@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- value-group scores/sec of the batched score_value + sample_from_scores hot path.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload all|c2_nich|...]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload all|c2_nich|...] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (prior + Mixture::score_value for every row x group +
 sample_from_scores) over one batch of synthetic rows with frozen group statistics.
@@ -18,6 +18,15 @@ ms_per_step / value / binding roofline / e2e --
           score kernel) and "rs" (NCCL reduce-scatter), each with the same table timed on one GPU in the same run.
 Single-feature table models (c1, c4) report the per-cell kernel as `value` (that is what the roofline measures)
 and the per-value CDF shortcut (SURVEY.md 8d, the library's default for those calls) beside it, flagged.
+
+--steps K is the step count of every timed loop: each configuration's event-timed steps and each e2e host-entry mode.
+Warm-up runs max(W, 3) steps.
+
+--dump-outputs DIR writes, after each configuration's timed steps, what its last step handed the caller (the sampled
+group index of every row; with --materialise the scores, with --sweep the refreshed prior and group sizes) as
+DIR/<workload>_<output>.npy in float32 (exact for the indices and sizes, which stay below 2^24).  Outputs longer than
+DUMP_ROWS rows keep every (rows // DUMP_ROWS)-th row from a seeded offset; with N > 1, row-sharded outputs are rank 0's
+shard.  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -49,6 +58,12 @@ WORKLOADS = {
 }
 HEADLINE = "c2_nich"
 SUB_N1 = ["c1_dd", "c1_dd_steady", "c3_crosscat", "c4_dpd", "c5_niw"]
+
+# --dump-outputs: at most 1M rows of a per-row output and 4096 rows of the [N][G] scores, 64 MB over all files
+DUMP_ROWS = 1 << 20
+DUMP_SCORE_ROWS = 4096
+DUMP_SEED = 7
+DUMP_MAX_BYTES = 64 << 20
 
 # committed ncu --set full summaries: dram__bytes of one launch of the config's dominant kernel
 NCU_SUMMARY = {
@@ -146,6 +161,15 @@ def make_workload(name, rank=0):
     w = getattr(synth, model)(seed, G, N, **cfg)
     feats = w["features"] if model == "crosscat" else [w]
     return dict(name=name, G=G, N=N, feats=feats, sizes=w["sizes"], u=w["u"])
+
+
+def write_outputs(outputs, out_dir):
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_MAX_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def model_id(capi, name):
@@ -354,6 +378,20 @@ class Bench:
         self.flush = torch.empty(256 * 1024 * 1024 // 4, device=self.dev, dtype=torch.float32)  # > 126 MB L2
         self.stream = torch.cuda.current_stream().cuda_stream
         self.peaks = Peaks(self.ctx)
+        self.outputs = {}
+
+    def keep_output(self, name, a):
+        """--dump-outputs: a host copy of one output (device tensor or numpy array), rows sampled past the limit"""
+        if not self.args.dump_outputs:
+            return
+        limit = DUMP_ROWS if a.ndim == 1 else DUMP_SCORE_ROWS
+        if a.shape[0] > limit:
+            stride = a.shape[0] // limit
+            rows = int(np.random.default_rng(DUMP_SEED).integers(stride)) + stride * np.arange(limit)
+            a = a[rows] if isinstance(a, np.ndarray) else a[self.torch.from_numpy(rows).to(a.device)]
+        if not isinstance(a, np.ndarray):
+            a = a.cpu().numpy()
+        self.outputs[name] = a.astype(np.float32)
 
     def barrier(self):
         self.torch.cuda.synchronize()
@@ -494,9 +532,11 @@ class Bench:
             ctx.set_option(capi.OPT_VALUE_CDF, 1)
             ms, t_wall, clocks = self.timed(step, steps, warmup, flush, sampler)
             a_cell = st["assign"].cpu().numpy()
+            self.keep_output(name + "_assign", a_cell)
             ctx.set_option(capi.OPT_VALUE_CDF, 0)
             ms_cdf, _, _ = self.timed(step, steps, warmup, flush)
             a_cdf = st["assign"].cpu().numpy()
+            self.keep_output(name + "_cdf_assign", a_cdf)
             rec["value_cdf_shortcut"] = {
                 "flag": "ALGORITHMIC SHORTCUT (SURVEY.md 8d): one table feature with frozen statistics -- the likelihood vector is "
                         "evaluated once per distinct VALUE, rows only search per-value CDF trees; N G / t is still reported. This is "
@@ -506,6 +546,12 @@ class Bench:
                 "index_agreement_with_per_cell_kernel": float(np.mean(a_cell == a_cdf)), "gpu_launches_per_step": 2}
         else:
             ms, t_wall, clocks = self.timed(step, steps, warmup, flush, sampler)
+            self.keep_output(name + "_assign", st["assign"])
+            if scores_buf is not None:
+                self.keep_output(name + "_scores", scores_buf)
+            if sweep:
+                self.keep_output(name + "_prior", st["prior"])
+                self.keep_output(name + "_group_sizes", sizes_dev)
         rec.update({"ms_per_step": ms, "value": cells / (ms * 1e-3), "wall_s_timed_region": t_wall,
                     "roofline": binding_roofline(name, wl, ms, self.peaks, materialise=scores_buf is not None),
                     "gpu_launches_per_step": launches_per_step(wl)})
@@ -516,7 +562,7 @@ class Bench:
             step()
             torch.cuda.synchronize()
             a_dev = st["assign"].cpu().numpy()
-            e2e, a_pin, a_page = self.e2e(wl, st, max(2, min(steps, 5)))
+            e2e, a_pin, a_page = self.e2e(wl, st, steps)
             rec["e2e"] = e2e
             rec["e2e_matches_device_assign"] = bool(np.array_equal(a_pin, a_dev) and np.array_equal(a_page, a_dev))
         if table_model:
@@ -613,22 +659,24 @@ def run_b200(args):
     torch = b.torch
     if args.feature_sharded and b.world > 1:
         r = b.run_feature_sharded("c3_crosscat", args.steps, args.warmup, "rs" if args.feature_sharded == "rs" else "push", args.row_shards)
+        b.keep_output("c3_crosscat_feature_sharded_%s_assign" % args.feature_sharded, b.last_full_assign)
         if b.rank == 0:
             print(json.dumps(r))
+            if args.dump_outputs:
+                write_outputs(b.outputs, args.dump_outputs)
         b.dist.destroy_process_group()
         return 0
     headline = HEADLINE if args.workload == "all" else args.workload
     sampler = ClockSampler(b.local_rank) if b.rank == 0 else None
     rec, clocks = b.run_rows(headline, args.steps, args.warmup, sampler=sampler, with_cpu=not args.no_cpu)
-    sub_steps = max(3, min(args.steps, 10))
     configs = {}
     if args.workload == "all":
         if b.world == 1:
             for name in SUB_N1:
-                r, _ = b.run_rows(name, sub_steps, args.warmup, with_cpu=not args.no_cpu)
+                r, _ = b.run_rows(name, args.steps, args.warmup, with_cpu=not args.no_cpu)
                 configs[name] = r
         else:
-            r, _ = b.run_rows("c4_dpd", sub_steps, args.warmup, with_e2e=False)
+            r, _ = b.run_rows("c4_dpd", args.steps, args.warmup, with_e2e=False)
             r["scaling"] = "weak"
             r["parallelism"] = "row shards: caches and prior replicated, every rank scores its own 10M-row shard, no collective"
             configs["c4_dpd_row_sharded"] = r
@@ -637,13 +685,14 @@ def run_b200(args):
                 variants.append(("hybrid_2x%d" % (b.world // 2), "push", b.world // 2))
             full_assign = {}
             for label, mode, row_shards in variants:
-                configs["c3_crosscat_feature_sharded_" + label] = b.run_feature_sharded("c3_crosscat", sub_steps, args.warmup, mode, row_shards)
+                configs["c3_crosscat_feature_sharded_" + label] = b.run_feature_sharded("c3_crosscat", args.steps, args.warmup, mode, row_shards)
                 full_assign[label] = b.last_full_assign
+                b.keep_output("c3_crosscat_feature_sharded_%s_assign" % label, b.last_full_assign)
             # the same table on ONE GPU in the same run (rank 0 only, the others wait): the strong-scaling reference
             t1 = torch.zeros(1, device=b.dev, dtype=torch.float64)
             if b.rank == 0:
                 world, b.world, dist, b.dist = b.world, 1, b.dist, None
-                r1, _ = b.run_rows("c3_crosscat", sub_steps, args.warmup, with_e2e=False)
+                r1, _ = b.run_rows("c3_crosscat", args.steps, args.warmup, with_e2e=False)
                 b.world, b.dist = world, dist
                 t1[0] = r1["ms_per_step"]
                 for label, _, _ in variants:
@@ -686,6 +735,8 @@ def run_b200(args):
     if configs:
         line["configs"] = configs
     print(json.dumps(line))
+    if args.dump_outputs:
+        write_outputs(b.outputs, args.dump_outputs)
     if b.dist is not None:
         b.dist.destroy_process_group()
     return 0
@@ -708,7 +759,13 @@ def main():
     ap.add_argument("--row-shards", type=int, default=1, help="with --feature-sharded push: feature x row hybrid")
     ap.add_argument("--tile-rows", type=int, default=65536, help="row tile of the feature-sharded reduce-scatter")
     ap.add_argument("--option", action="append", metavar="K=V", help="A/B runs: dist_b200_ctx_set_option(K, V) before anything runs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what each configuration's last step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if args.impl == "reference":
         return run_reference(args)
     return run_b200(args)

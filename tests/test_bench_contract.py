@@ -55,3 +55,52 @@ def test_reference_arm_runs_here():
     d = json.loads(out.stdout.strip().splitlines()[-1])
     assert d["impl"] == "reference" and BASE_KEYS <= set(d) and d["value"] > 0
     assert d["config"]["workload"] == "c1_dd"
+
+
+def test_steps_below_one_rejected():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=120)
+    assert out.returncode == 2 and "--steps" in out.stderr
+
+
+@pytest.mark.gpu
+def test_timed_loop_runs_the_requested_steps():
+    torch = pytest.importorskip("torch")
+    if not torch.cuda.is_available():
+        pytest.skip("no CUDA device")
+    import types
+    import bench
+    b = bench.Bench(types.SimpleNamespace(option=None, dump_outputs=None))
+    calls = []
+    for steps in (1, 7):
+        del calls[:]
+        ms, _, _ = b.timed(lambda: calls.append(1), steps, 0, flush=False)
+        assert len(calls) == 3 + steps and ms >= 0  # at least three warm-up steps, then exactly the timed ones
+    b.ctx.close()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_sampled_indices(tmp_path, oracle):
+    """--dump-outputs at c1: both timed paths' indices are what the oracle samples from the same scores and uniforms,
+    up to near-ties"""
+    import numpy as np
+    torch = pytest.importorskip("torch")
+    if not torch.cuda.is_available():
+        pytest.skip("no CUDA device")
+    import bench
+    import cases
+    from distributions_b200 import synth
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "c1_dd", "--steps", "2", "--warmup", "0",
+                          "--no-cpu", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2 and line["config"]["workload"] == "c1_dd"
+    assert sorted(os.listdir(str(tmp_path))) == ["c1_dd_assign.npy", "c1_dd_cdf_assign.npy"]
+    wl = bench.make_workload("c1_dd")
+    scores = cases.oracle_scores(oracle, wl["feats"], prior=oracle.py_prior(synth.PY_ALPHA, synth.PY_D, wl["sizes"]))
+    want = oracle.sample_rows(scores.copy(), wl["u"])
+    for f in ("c1_dd_assign.npy", "c1_dd_cdf_assign.npy"):
+        a = np.load(str(tmp_path / f))
+        assert a.dtype == np.float32 and a.shape == (wl["N"],) and np.array_equal(a, np.round(a))
+        got = a.astype(np.int32)
+        assert cases.explained_mismatch(scores.astype(np.float64), wl["u"], got, want, 2e-5).all(), f
+        assert np.mean(got == want) > 0.999, f
