@@ -17,7 +17,8 @@ OBJ_DIR = os.path.join(LIB_DIR, "obj")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 COMMON = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
           "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
-# per-file extra flags.  prep.cu keeps the reference's unfused multiply/add rounding.
+# per-file extra flags.  prep.cu keeps the reference's unfused multiply/add rounding; sample_values.cu shares its
+# posterior code (posterior.cuh).
 SOURCES = {
     "api.cu": [],
     "prep.cu": ["--fmad=false"],
@@ -39,6 +40,7 @@ SOURCES = {
     "microbench.cu": [],
     "stats.cu": [],
     "wire.cu": [],
+    "sample_values.cu": ["--fmad=false"],
 }
 
 

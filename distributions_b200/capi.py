@@ -49,6 +49,8 @@ SIGNATURES = {
     "dist_b200_rows_merge": (c_i, [c_p, c_p, c_i, c_p, c_i, c_p]),
     "dist_b200_rows_xchg_doubles": (c_i, [c_p, c_i, c_p]),
     "dist_b200_remove_rows_batch_host": (c_i, [c_p, c_p, c_i, c_p, c_p, c_sz]),
+    "dist_b200_sample_values_batch": (c_i, [c_p, c_p, c_i, c_p, c_sz, ctypes.c_uint64, ctypes.c_uint64, c_p, c_p]),
+    "dist_b200_sample_values_batch_host": (c_i, [c_p, c_p, c_i, c_p, c_sz, ctypes.c_uint64, ctypes.c_uint64, c_p]),
     "dist_b200_gp_set_log_prod": (c_i, [c_p, c_p, c_p]),
     "dist_b200_score_data_grid": (c_i, [c_p, c_p, c_sz, c_sz, c_p, c_p]),
     "dist_b200_score_data_grid_host": (c_i, [c_p, c_p, c_sz, c_sz, c_p]),
@@ -297,6 +299,30 @@ class Context:
         ca = (c_p * F)(*[_np_ptr(c) for c in cols])
         self.check(self.L.dist_b200_add_rows_batch_host(self.h, fa, F, ca, _np_ptr(assign), assign.size), "add_rows_batch_host")
 
+    def sample_values_batch(self, features, assign_dev, n_rows, columns_out, seed=0, row0=0, stream=None):
+        """batched Group::sample_value: columns_out[i][n] (device) <- a posterior-predictive draw of group assign_dev[n]
+        of features[i]; rows with an id outside [0, G) keep their values.  Draws depend on (seed, row0 + n, i) only."""
+        F, fa, ca = self._lists(features, columns_out)
+        self.check(self.L.dist_b200_sample_values_batch(self.h, fa, F, _dev_ptr(assign_dev), n_rows, int(seed), int(row0), ca, stream),
+                   "sample_values_batch")
+
+    def sample_values_batch_host(self, features, assign, seed=0, row0=0, out=None):
+        """host form: a list of one array per feature (COLUMN_DTYPE; niw [n][d]).  `out` (optional) supplies the arrays,
+        whose rows with an id outside [0, G) are left as they are; fresh arrays are zero-filled."""
+        F = len(features)
+        assign = np.ascontiguousarray(assign, dtype=np.int32)
+        n = assign.size
+        if out is None:
+            assert all(f.model != NIW or f.dim for f in features), "niw feature of unknown d: pass `out`"
+            out = [np.zeros((n, f.dim) if f.model == NIW else n, dtype=COLUMN_DTYPE[f.model]) for f in features]
+        for f, o in zip(features, out):
+            assert o.dtype == COLUMN_DTYPE[f.model] and o.flags.c_contiguous and o.shape[0] == n, "bad output array"
+        fa = (c_p * F)(*[f.h for f in features])
+        ca = (c_p * F)(*[_np_ptr(o) for o in out])
+        self.check(self.L.dist_b200_sample_values_batch_host(self.h, fa, F, _np_ptr(assign), n, int(seed), int(row0), ca),
+                   "sample_values_batch_host")
+        return out
+
     def count_assignments(self, assign_dev, n_rows, G, counts_dev, accumulate=False, stream=None):
         self.check(self.L.dist_b200_count_assignments(self.h, _dev_ptr(assign_dev), n_rows, G, _dev_ptr(counts_dev),
                                                       1 if accumulate else 0, stream), "count_assignments")
@@ -436,6 +462,7 @@ class Feature:
         h = c_p()
         ctx.check(ctx.L.dist_b200_feature_create(ctx.h, model, ctypes.byref(h)), "feature_create")
         self.h = h
+        self.dim = None  # niw: d of the last update_all (the row length of its columns)
 
     def close(self):
         if getattr(self, "h", None) and getattr(self.ctx, "h", None):
@@ -483,6 +510,7 @@ class Feature:
                                                cnt.shape[0], _np_ptr(cnt), stream), "dpd_update_all")
         elif m == NIW:
             mu, psi, cnt, sx, sxx = f32(w["mu"]), f32(w["psi"]), i32(w["count"]), f32(w["sum_x"]), f32(w["sum_xxT"])
+            self.dim = mu.size
             c.check(L.dist_b200_niw_update_all(self.h, mu.size, _np_ptr(mu), w["kappa"], _np_ptr(psi), w["nu"], cnt.size,
                                                _np_ptr(cnt), _np_ptr(sx), _np_ptr(sxx), stream), "niw_update_all")
         else:

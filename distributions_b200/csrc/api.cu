@@ -352,6 +352,7 @@ void dist_b200_feature_destroy(dist_b200_feature *f) {
     if (f->niw_tc) cudaFree(f->niw_tc);
     if (f->niw_stats) cudaFree(f->niw_stats);
     if (f->niw_shared_dev) cudaFree(f->niw_shared_dev);
+    if (f->sample_buf) cudaFree(f->sample_buf);
     if (f->stats) cudaFree(f->stats);
     if (f->alphas_dev) cudaFree(f->alphas_dev);
     if (f->log_prod_dev) cudaFree(f->log_prod_dev);
@@ -1058,6 +1059,107 @@ int dist_b200_add_rows_batch_host(dist_b200_ctx *ctx, dist_b200_feature *const *
 int dist_b200_remove_rows_batch_host(dist_b200_ctx *ctx, dist_b200_feature *const *features, int n_features,
                                      const void *const *columns_host, const int32_t *assign_host, size_t n_rows) {
     return rows_batch_host(ctx, features, n_features, columns_host, assign_host, n_rows, -1);
+}
+
+// ---- batched Group::sample_value (sample_values.cu) ----------------------------------------------------------------
+// arguments shared by the device and host forms; ERR_STATE for a feature without statistics or a G mismatch
+static int check_sample_args(dist_b200_ctx *ctx, dist_b200_feature *const *features, int n_features, const int32_t *assign,
+                             void *const *columns_out) {
+    if (n_features < 1 || !features || !assign || !columns_out) return fail(ctx, DIST_B200_ERR_INVALID, "sample_values: null argument");
+    for (int i = 0; i < n_features; ++i) {
+        const dist_b200_feature *f = features[i];
+        if (!f || f->ctx != ctx || !columns_out[i]) return fail(ctx, DIST_B200_ERR_INVALID, "sample_values: bad feature / output column");
+        const bool resident = f->model == DIST_B200_NIW ? f->niw_stats != nullptr
+                              : f->model == DIST_B200_DD ? f->stats && f->alphas_dev
+                              : f->model == DIST_B200_DPD ? f->stats && f->keys_dev : f->stats != nullptr;
+        if (f->G < 1 || !resident) return fail(ctx, DIST_B200_ERR_STATE, "sample_values: call update_all first");
+        if (f->G != features[0]->G) return fail(ctx, DIST_B200_ERR_STATE, "sample_values: features disagree on the number of groups");
+    }
+    return DIST_B200_OK;
+}
+
+static SampleSrc sample_src(const dist_b200_feature *f) {
+    SampleSrc src{};
+    src.model = f->model;
+    src.G = f->G;
+    src.dim = f->dim;
+    for (int k = 0; k < 4; ++k) src.shared[k] = f->shared[k];
+    switch (f->model) {
+        case DIST_B200_DD:
+            src.st0 = stat_ptr(f, 0);
+            src.alphas = f->alphas_dev;
+            break;
+        case DIST_B200_DPD:
+            src.shared[0] = f->alpha;
+            src.shared[1] = f->beta0;
+            src.st0 = f->stats;
+            src.alphas = reinterpret_cast<const float *>(dpd_betas(f));
+            src.keys_sorted = f->keys_dev;
+            src.key_rows = f->key_rows_dev;
+            break;
+        case DIST_B200_NIW:
+            src.shared[0] = f->kappa;
+            src.shared[1] = f->nu;
+            src.st0 = f->niw_stats;
+            src.st1 = reinterpret_cast<const uint32_t *>(niw_sum_x(f));
+            src.st2 = reinterpret_cast<const uint32_t *>(niw_sum_xxT(f));
+            src.alphas = f->niw_shared_dev;
+            break;
+        default:
+            src.st0 = stat_ptr(f, 0);
+            src.st1 = stat_ptr(f, 1);
+            src.st2 = f->model == DIST_B200_NICH ? stat_ptr(f, 2) : nullptr;
+    }
+    return src;
+}
+
+int dist_b200_sample_values_batch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                                  const int32_t *assign_dev, size_t n_rows, uint64_t seed, uint64_t row0,
+                                  void *const *columns_out_dev, void *stream) {
+    if (!ctx) return DIST_B200_ERR_INVALID;
+    dist_b200_feature *const *fs = const_cast<dist_b200_feature *const *>(features);
+    int rc = check_sample_args(ctx, fs, n_features, assign_dev, columns_out_dev);
+    if (rc || n_rows == 0) return rc;
+    cudaStream_t s = as_stream(stream);
+    if ((rc = wait_ready(ctx, features, n_features, s))) return rc;  // a preceding add / remove / update on another stream
+    for (int i = 0; i < n_features; ++i)
+        if ((rc = launch_sample_values(ctx, fs[i], sample_src(fs[i]), static_cast<uint32_t>(i), assign_dev, n_rows, seed, row0,
+                                       columns_out_dev[i], s)))
+            return rc;
+    return DIST_B200_OK;
+}
+
+// host buffers: the assignments and the output columns go up (rows the call skips keep their values), the columns come back
+int dist_b200_sample_values_batch_host(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                                       const int32_t *assign_host, size_t n_rows, uint64_t seed, uint64_t row0,
+                                       void *const *columns_out_host) {
+    if (!ctx) return DIST_B200_ERR_INVALID;
+    int rc = check_sample_args(ctx, const_cast<dist_b200_feature *const *>(features), n_features, assign_host, columns_out_host);
+    if (rc || n_rows == 0) return rc;
+    std::vector<size_t> off(n_features);
+    size_t total = 0;
+    for (int i = 0; i < n_features; ++i) {
+        off[i] = total;
+        total += round_up(column_bytes(features[i]) * n_rows, 256);
+    }
+    const size_t assign_off = total;
+    total += round_up(sizeof(int32_t) * n_rows, 256);
+    if ((rc = ensure_scratch(ctx, total + 256))) return rc;
+    cudaStream_t s = ctx->own_stream;
+    char *dev = static_cast<char *>(ctx->scratch_dev);
+    std::vector<void *> cols(n_features);
+    for (int i = 0; i < n_features; ++i) {
+        cols[i] = dev + off[i];
+        DISTB200_CUDA(ctx, cudaMemcpyAsync(cols[i], columns_out_host[i], column_bytes(features[i]) * n_rows, cudaMemcpyHostToDevice, s));
+    }
+    DISTB200_CUDA(ctx, cudaMemcpyAsync(dev + assign_off, assign_host, sizeof(int32_t) * n_rows, cudaMemcpyHostToDevice, s));
+    rc = dist_b200_sample_values_batch(ctx, features, n_features, reinterpret_cast<const int32_t *>(dev + assign_off), n_rows, seed,
+                                       row0, cols.data(), s);
+    if (rc == DIST_B200_OK)
+        for (int i = 0; i < n_features; ++i)
+            DISTB200_CUDA(ctx, cudaMemcpyAsync(columns_out_host[i], cols[i], column_bytes(features[i]) * n_rows, cudaMemcpyDeviceToHost, s));
+    DISTB200_CUDA(ctx, cudaStreamSynchronize(s));  // results on the host, the scratch free for the next upload
+    return rc;
 }
 
 int dist_b200_feature_add_rows(dist_b200_feature *f, const void *column_dev, const int32_t *assign_dev, size_t n_rows,

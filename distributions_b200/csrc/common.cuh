@@ -149,6 +149,8 @@ struct dist_b200_feature {
     uint32_t *niw_stats = nullptr;
     int niw_cap = 0;
     float *niw_shared_dev = nullptr;
+    void *sample_buf = nullptr;       // sample_values: per-group records of the prep pass (sample_values.cu)
+    size_t sample_bytes = 0;
 };
 
 namespace distb200 {
@@ -249,6 +251,19 @@ int launch_niw_tc_prep(dist_b200_ctx *ctx, int G, const float *recs, float *tc_b
 // scores != nullptr: [N][G] scores (optionally accumulated onto the buffer); scores == nullptr: the fused sampler writes assign[N]
 int launch_niw_tc(dist_b200_ctx *ctx, int G, const float *tc_buf, const void *values, size_t N, const float *prior,
                   float *scores, int accumulate, const float *u, int32_t *assign, cudaStream_t s);
+
+// sample_values.cu: batched Group::sample_value of one feature.  The device-resident statistics it reads:
+struct SampleSrc {
+    int model, G, dim;                // dim: dd dim / dpd V / niw d
+    float shared[4];                  // nich mu kappa sigmasq nu; gp alpha inv_beta; bnb alpha beta r; bb alpha beta;
+                                      // dpd alpha beta0; niw kappa nu
+    const uint32_t *st0, *st1, *st2;  // statistics arrays (see dist_b200_feature::stats); niw count | sum_x | sum_xxT
+    const float *alphas;              // dd alphas; dpd betas; niw mu[d] | psi[d][d]
+    const uint32_t *keys_sorted;      // dpd: dist_b200_feature::keys_dev / key_rows_dev
+    const int *key_rows;
+};
+int launch_sample_values(dist_b200_ctx *ctx, dist_b200_feature *f, const SampleSrc &src, uint32_t position, const int32_t *assign,
+                         size_t N, uint64_t seed, uint64_t row0, void *out, cudaStream_t s);
 
 // wire.cu: protobuf wire format of the reference (schema.proto) -> SoA.  Decoded feature: Shared floats
 // (+ dpd keys) and the statistics arrays in update_all's argument order.

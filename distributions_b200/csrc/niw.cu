@@ -20,6 +20,7 @@
 #include <cstring>
 
 #include "common.cuh"
+#include "posterior.cuh"
 
 namespace distb200 {
 
@@ -36,36 +37,8 @@ __global__ void niw_prep_kernel(int d, int dp, const float *__restrict__ mu, flo
     __shared__ double Winv[32][33];
     __shared__ double xbar[32], diff[32];
     const int g = blockIdx.x, tid = threadIdx.x;
-    const double n = static_cast<double>(count[g]);
-    const float *sx = sum_x + static_cast<size_t>(g) * d;
-    const float *sxx = sum_xxT + static_cast<size_t>(g) * d * d;
-    const double kap = kappa, post_kappa = kap + n, post_nu = static_cast<double>(nu) + n;
-    const double dof = post_nu - static_cast<double>(d) + 1.0;
-    if (tid < d) {
-        xbar[tid] = count[g] ? static_cast<double>(sx[tid]) / n : 0.0;
-        diff[tid] = xbar[tid] - static_cast<double>(mu[tid]);
-    }
-    __syncthreads();
-    for (int e = tid; e < d * d; e += blockDim.x) {
-        const int i = e / d, j = e % d;
-        const double c_n = static_cast<double>(sxx[e]) - static_cast<double>(sx[i]) * xbar[j] -
-                           xbar[i] * static_cast<double>(sx[j]) + n * xbar[i] * xbar[j];
-        const double post_psi = static_cast<double>(psi[e]) + c_n + kap * n / (kap + n) * diff[i] * diff[j];
-        S[i][j] = post_psi * (post_kappa + 1.0) / (post_kappa * dof);
-    }
-    __syncthreads();
-    // Cholesky (right-looking), lower triangle in place
-    for (int k = 0; k < d; ++k) {
-        if (tid == 0) S[k][k] = sqrt(S[k][k]);
-        __syncthreads();
-        if (tid > k && tid < d) S[tid][k] /= S[k][k];
-        __syncthreads();
-        for (int e = tid; e < d * d; e += blockDim.x) {
-            const int i = e / d, j = e % d;
-            if (j > k && i >= j) S[i][j] -= S[i][k] * S[j][k];
-        }
-        __syncthreads();
-    }
+    const double dof = niw_posterior_cholesky(d, mu, kappa, psi, nu, count[g], sum_x + static_cast<size_t>(g) * d,
+                                              sum_xxT + static_cast<size_t>(g) * d * d, S, xbar, diff);
     // W = L^-1 by forward substitution, one column per thread
     if (tid < d) {
         const int c = tid;
@@ -78,7 +51,7 @@ __global__ void niw_prep_kernel(int d, int dp, const float *__restrict__ mu, flo
     __syncthreads();
     float *rec = out + static_cast<size_t>(g) * niw_group_floats(dp);
     for (int i = tid; i < dp; i += blockDim.x)
-        rec[i] = i < d ? static_cast<float>(kap / (kap + n) * static_cast<double>(mu[i]) + n / (kap + n) * xbar[i]) : 0.f;
+        rec[i] = i < d ? static_cast<float>(niw_post_mu(kappa, count[g], mu[i], xbar[i])) : 0.f;
     for (int e = tid; e < dp * dp; e += blockDim.x) {
         const int i = e / dp, j = e % dp;
         rec[dp + e] = (i < d && j <= i) ? static_cast<float>(Winv[i][j]) : 0.f;

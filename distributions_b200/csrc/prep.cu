@@ -6,6 +6,7 @@
 #include <algorithm>
 
 #include "common.cuh"
+#include "posterior.cuh"
 
 namespace distb200 {
 
@@ -15,13 +16,8 @@ namespace distb200 {
 // with MUFU.LG2's base-2 logarithm directly.  The unscaled log_coeff_ is kept in `aux` for read-back.
 __device__ __forceinline__ void nich_prep_one(float mu, float kappa, float sigmasq, float nu, int32_t count, float mean,
                                               float ctv, float4 *params, float *aux, const NumericTables &t) {
-    const float cnt = static_cast<float>(count);
-    const float mu_1 = mu - mean;
-    const float post_kappa = kappa + cnt;
-    const float post_mu = (kappa * mu + mean * cnt) / post_kappa;
-    const float post_nu = nu + cnt;
-    const float post_sigmasq =
-        1.f / post_nu * (nu * sigmasq + ctv + (cnt * kappa * mu_1 * mu_1) / post_kappa);
+    const NichPost post = nich_plus_group(mu, kappa, sigmasq, nu, count, mean, ctv);
+    const float post_kappa = post.kappa, post_mu = post.mu, post_nu = post.nu, post_sigmasq = post.sigmasq;
     const float lambda = post_kappa / ((post_kappa + 1.f) * post_sigmasq);
     const float score = fast_lgamma_nu(post_nu, t.lgamma_nu3) +
                         0.5f * fast_log_table(lambda / (3.14159265358979f * post_nu), t.log2_table);
@@ -42,8 +38,8 @@ __global__ void nich_prep_kernel(float mu, float kappa, float sigmasq, float nu,
 
 // GammaPoisson: plus_group (gp.hpp:56-61) + Scorer::init (gp.hpp:198-207); {post_alpha, score_coeff, score, 0}
 __device__ __forceinline__ float4 gp_prep_one(float alpha, float inv_beta, uint32_t count, uint32_t sum, const NumericTables &t) {
-    const float post_alpha = alpha + static_cast<float>(sum);
-    const float post_inv_beta = inv_beta + static_cast<float>(count);
+    const float2 post = gp_plus_group(alpha, inv_beta, count, sum);
+    const float post_alpha = post.x, post_inv_beta = post.y;
     const float score_coeff = -fast_log_table(1.f + post_inv_beta, t.log2_table);
     const float score = -fast_lgamma_exact(post_alpha, t.lgamma5) +
                         post_alpha * (fast_log_table(post_inv_beta, t.log2_table) + score_coeff);
@@ -60,8 +56,8 @@ __global__ void gp_prep_kernel(float alpha, float inv_beta, int g0, int n, const
 // BetaNegativeBinomial: plus_group (bnb.hpp:57-63) + Scorer::init (bnb.hpp:200-211); {post_beta, alpha, score, 0}
 __device__ __forceinline__ float4 bnb_prep_one(float alpha, float beta, float r, uint32_t count, uint32_t sum,
                                                const NumericTables &t) {
-    const float post_alpha = alpha + r * static_cast<float>(count);
-    const float post_beta = beta + static_cast<float>(sum);
+    const float2 post = bnb_plus_group(alpha, beta, r, count, sum);
+    const float post_alpha = post.x, post_beta = post.y;
     const float a = post_alpha + r;
     const float score = fast_lgamma_exact(post_alpha + post_beta, t.lgamma5) - fast_lgamma_exact(post_alpha, t.lgamma5) -
                         fast_lgamma_exact(post_beta, t.lgamma5) + fast_lgamma_exact(a, t.lgamma5);
@@ -77,8 +73,8 @@ __global__ void bnb_prep_kernel(float alpha, float beta, float r, int g0, int n,
 
 // BetaBernoulli: update_all (bb.hpp:276-292); {heads_score, tails_score, 0, 0}
 __device__ __forceinline__ float4 bb_prep_one(float alpha, float beta, int32_t heads, int32_t tails, const NumericTables &t) {
-    const float h = alpha + static_cast<float>(heads);
-    const float tl = beta + static_cast<float>(tails);
+    const float2 post = bb_plus_group(alpha, beta, heads, tails);
+    const float h = post.x, tl = post.y;
     return make_float4(fast_log_table(h / (h + tl), t.log2_table), fast_log_table(tl / (h + tl), t.log2_table), 0.f, 0.f);
 }
 

@@ -136,6 +136,20 @@ class _Mixture:
         self.ctx.add_rows_batch_host([self.feature], [values], groupids)
         self._pull_groups(shared)
 
+    def sample_values(self, shared, groupids, seed=0, row0=0):
+        """batched Group::sample_value: one draw from the posterior predictive of group groupids[n] per row, with fresh
+        parameters per value (Sampler::init + eval), on the device.  A draw depends on (seed, row0 + n) and the group
+        only.  Returns an array of the model's Value type (bool for bb, [n][d] for niw)."""
+        gid = np.ascontiguousarray(groupids, np.int32).ravel()
+        assert gid.size == 0 or (gid.min() >= 0 and gid.max() < len(self.groups)), "bad group id"
+        out = self.ctx.sample_values_batch_host([self.feature], gid, seed, row0)[0]
+        return out.astype(bool) if self.model_id == capi.BB else out
+
+    def sample_value(self, shared, groupid, seed=0):
+        """Group::sample_value of one group"""
+        v = self.sample_values(shared, [groupid], seed)[0]
+        return v if self.model_id == capi.NIW else v.item()
+
 
 # ------------------------------------------------------------------------------------------------------
 class _NichShared(_Shared):

@@ -197,6 +197,26 @@ int dist_b200_rows_merge(dist_b200_ctx *ctx, dist_b200_feature *const *features,
  * features[i] (float / uint32 / int32, bool as uint8), assign_host the packed group ids.  Synchronous. */
 int dist_b200_add_rows_batch_host(dist_b200_ctx *ctx, dist_b200_feature *const *features, int n_features,
                                   const void *const *columns_host, const int32_t *assign_host, size_t n_rows);
+/* ---- batched Group::sample_value: posterior-predictive draws from the same device-resident statistics -------------
+ * For every row n with 0 <= assign_dev[n] < G, columns_out_dev[i][n] receives one draw from the posterior predictive of
+ * group assign_dev[n] of features[i]: fresh parameters per value, as Sampler::init + Sampler::eval do (nich.hpp, gp.hpp,
+ * bnb.hpp, bb.hpp, dd.hpp, dpd.hpp, niw.hpp), so rows are independent given the statistics.  Rows with a negative or
+ * out-of-range id are left untouched (as add_rows_batch skips them).  Output types are the column types of
+ * dist_b200_model (dpd: the key, 0xFFFFFFFF = OTHER; niw: rows of d floats), so the columns feed score_sample_batch and
+ * add_rows_batch unchanged.  All features share G (ERR_STATE otherwise, and for a feature before its first update_all).
+ * The launch waits on every feature's pending updates, so a preceding add_rows_batch is seen without a host synchronise.
+ * Random numbers: Philox4x32-10 keyed by `seed`, counter (global row row0 + n, position i of the feature in the list,
+ * draw index within the value).  A draw is a pure function of (seed, row0 + n, i, that group's statistics), independent
+ * of launch geometry, n_rows and chunking: row shards passing their own row0 reproduce a single call bit for bit.  Two
+ * features drawn in separate calls at the same list position get the same random stream: give such calls distinct seeds.
+ * The host form stages through the context (the output columns travel both ways, so skipped rows keep their values);
+ * its results are bit-identical to the device form.  Synchronous. */
+int dist_b200_sample_values_batch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                                  const int32_t *assign_dev, size_t n_rows, uint64_t seed, uint64_t row0,
+                                  void *const *columns_out_dev, void *stream);
+int dist_b200_sample_values_batch_host(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                                       const int32_t *assign_host, size_t n_rows, uint64_t seed, uint64_t row0,
+                                       void *const *columns_out_host);
 /* ---- score_data_grid: hyper-parameter inference over the same statistics ---------------------------
  * out[i] = log marginal likelihood of all groups of `f` under hyper-parameter setting i: the reference's
  * MixtureSlave::score_data_grid / score_data (mixture.hpp:427-438; nich.hpp:262-288, gp.hpp:220-241,

@@ -15,13 +15,16 @@
 //     counts(), empty_groupids(), sample_size(), init, add_value / remove_value (return whether a group
 //     was added / removed), score_value (OVERWRITES the caller's buffer)
 // What is new: Mixture::score_values / CrossCat::score_sample_values -- the batched entry that scores
-// N rows against frozen statistics and samples a group per row (SURVEY.md §3.3).
+// N rows against frozen statistics and samples a group per row (SURVEY.md §3.3); Mixture::sample_values /
+// CrossCat::sample_values -- batched Group::sample_value, one posterior-predictive draw per row on the device
+// (Sampler::init + Sampler::eval with fresh parameters per value), seeded explicitly instead of through rng_t.
 //
 // Group statistics live and mutate on the host exactly as in the reference (integer / float
 // bookkeeping, SURVEY §8 a20); every score -- per value or batched -- is computed by the sm_100a
 // kernels behind the C-ABI.  There is no CPU scoring path here: a failed C-ABI call throws
 // std::runtime_error (the reference's DIST_THROW_ON_ERROR behaviour, common.hpp:49-67).
-// Not mirrored (off the path): Sampler, sample_value, protobuf, Group::merge, gp log_prod.
+// Not mirrored (off the path): the per-group Sampler (one parameter draw shared by many values), protobuf,
+// Group::merge, gp log_prod.
 #pragma once
 
 #include <dist_b200.h>
@@ -55,7 +58,7 @@ template <class V> struct WireValue { typedef V type; };
 template <> struct WireValue<bool> { typedef uint8_t type; };
 }  // namespace detail
 
-struct rng_t {};  // scoring never draws (doc/overview.rst:213-220); kept so signatures match
+struct rng_t {};  // scoring never draws (doc/overview.rst:213-220) and sample_values takes a seed; kept so signatures match
 
 class Context {
   public:
@@ -586,6 +589,17 @@ class Mixture {
                     "score_values");
     }
 
+    // NEW: batched Group::sample_value.  out[n] receives one draw from the posterior predictive of group groupids[n]
+    // (fresh parameters per value, as Sampler::init + eval), computed on the device from its statistics.  A draw depends
+    // on (seed, row0 + n) and that group only; an id outside [0, G) leaves out[n] as it is.
+    void sample_values(const Shared &, const int32_t * groupids, size_t n, uint64_t seed, uint64_t row0, Value * out) const {
+        std::vector<typename detail::WireValue<Value>::type> wire(out, out + n);
+        const dist_b200_feature * feats[1] = {f_};
+        void * cols[1] = {wire.data()};
+        ctx_->check(dist_b200_sample_values_batch_host(ctx_->get(), feats, 1, groupids, n, seed, row0, cols), "sample_values");
+        for (size_t i = 0; i < n; ++i) out[i] = static_cast<Value>(wire[i]);
+    }
+
   private:
     std::shared_ptr<Context> ctx_;
     dist_b200_feature * f_ = nullptr;
@@ -719,6 +733,14 @@ class CrossCat {
         ctx_->check(dist_b200_score_sample_batch_host(ctx_->get(), feats_.data(), static_cast<int>(feats_.size()), cols_.data(), n,
                                                       prior, u, assign, scores),
                     "score_sample_values");
+    }
+
+    // batched Group::sample_value for every feature of the kind: columns_out[i] (host, the column type of feature i)
+    // receives, for every row n with 0 <= assign[n] < G, a posterior-predictive draw of group assign[n]
+    void sample_values(size_t n, const int32_t * assign, uint64_t seed, uint64_t row0, void * const * columns_out) {
+        ctx_->check(dist_b200_sample_values_batch_host(ctx_->get(), feats_.data(), static_cast<int>(feats_.size()), assign, n, seed,
+                                                       row0, columns_out),
+                    "sample_values");
     }
 
   private:
