@@ -5,6 +5,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <new>
 #include <numeric>
 
@@ -19,29 +20,7 @@ cudaStream_t as_stream(void *s) { return static_cast<cudaStream_t>(s); }
 
 int ensure_scratch(dist_b200_ctx *ctx, size_t bytes) {
     if (bytes <= ctx->scratch_bytes) return DIST_B200_OK;
-    if (ctx->scratch_dev) {
-        DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-        DISTB200_CUDA(ctx, cudaFree(ctx->scratch_dev));
-        ctx->scratch_dev = nullptr;
-        ctx->scratch_bytes = 0;
-    }
-    const size_t want = std::max<size_t>(bytes + bytes / 4, 1 << 20);
-    DISTB200_CUDA(ctx, cudaMalloc(&ctx->scratch_dev, want));
-    ctx->scratch_bytes = want;
-    return DIST_B200_OK;
-}
-
-int ensure_scores_scratch(dist_b200_ctx *ctx, size_t bytes) {
-    if (bytes <= ctx->scores_scratch_bytes) return DIST_B200_OK;
-    if (ctx->scores_scratch) {
-        DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-        DISTB200_CUDA(ctx, cudaFree(ctx->scores_scratch));
-        ctx->scores_scratch = nullptr;
-        ctx->scores_scratch_bytes = 0;
-    }
-    DISTB200_CUDA(ctx, cudaMalloc(&ctx->scores_scratch, bytes));
-    ctx->scores_scratch_bytes = bytes;
-    return DIST_B200_OK;
+    return grow(ctx, ctx->scratch_dev, ctx->scratch_bytes, std::max<size_t>(bytes + bytes / 4, 1 << 20));
 }
 
 int ensure_pinned(dist_b200_ctx *ctx, size_t bytes) {
@@ -67,94 +46,86 @@ size_t group_floats(const dist_b200_feature *f) {
     }
 }
 
-// device-side raw statistics: number of arrays and 4-byte elements per group of array a
+// floats of one niw record (niw.cu)
+size_t niw_rec_floats(int d) { return static_cast<size_t>(niw_padded_dim(d)) * (niw_padded_dim(d) + 1) + 4; }
+
+// device-side raw statistics: number of arrays, 4-byte elements per group of array a, and of all arrays
 int stat_arrays(const dist_b200_feature *f) {
     switch (f->model) {
-        case DIST_B200_NICH: return 3;
+        case DIST_B200_NICH: case DIST_B200_NIW: return 3;
         case DIST_B200_GP: case DIST_B200_BB: case DIST_B200_BNB: return 2;
-        case DIST_B200_DD: return 1;
-        default: return 0;
+        default: return 1;
     }
 }
-size_t stat_elems(const dist_b200_feature *f, int) { return f->model == DIST_B200_DD ? static_cast<size_t>(f->dim) : 1; }
-uint32_t *stat_ptr(const dist_b200_feature *f, int a) {
-    size_t off = 0;
-    for (int b = 0; b < a; ++b) off += stat_elems(f, b) * f->capacity;
-    return f->stats + off;
-}
-// (re)allocate the statistics arrays for the feature's current capacity, keeping the first old_G groups
-int ensure_stats(dist_b200_feature *f, int old_capacity, int old_G, bool keep) {
-    dist_b200_ctx *ctx = f->ctx;
-    const int na = stat_arrays(f);
-    if (na == 0) return DIST_B200_OK;
-    size_t words = 0;
-    for (int a = 0; a < na; ++a) words += stat_elems(f, a) * f->capacity;
-    if (f->stats && old_capacity == f->capacity && words <= f->stats_words) return DIST_B200_OK;
-    uint32_t *fresh = nullptr;
-    DISTB200_CUDA(ctx, cudaMalloc(&fresh, words * 4));
-    DISTB200_CUDA(ctx, cudaMemset(fresh, 0, words * 4));
-    if (f->stats) {
-        if (keep && old_capacity > 0) {
-            size_t off_old = 0, off_new = 0;
-            for (int a = 0; a < na; ++a) {
-                const size_t e = stat_elems(f, a);
-                DISTB200_CUDA(ctx, cudaMemcpy(fresh + off_new, f->stats + off_old, e * std::min(old_G, f->capacity) * 4, cudaMemcpyDeviceToDevice));
-                off_old += e * old_capacity;
-                off_new += e * f->capacity;
-            }
-        }
-        DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-        DISTB200_CUDA(ctx, cudaFree(f->stats));
+size_t stat_elems(const dist_b200_feature *f, int a) {
+    const size_t d = static_cast<size_t>(f->dim);
+    switch (f->model) {
+        case DIST_B200_DD: case DIST_B200_DPD: return d;
+        case DIST_B200_NIW: return a == 0 ? 1 : a == 1 ? d : d * d;
+        default: return 1;
     }
-    f->stats = fresh;
-    f->stats_words = words;
-    return DIST_B200_OK;
 }
-// copy `n` groups of statistics (device pointer, e.g. the freshly uploaded scratch) into array a from group g0
-int mirror_stats(dist_b200_feature *f, int a, const void *src_dev, int g0, int n, cudaStream_t s) {
-    if (!f->stats || n <= 0) return DIST_B200_OK;
-    const size_t e = stat_elems(f, a);
-    DISTB200_CUDA(f->ctx, cudaMemcpyAsync(stat_ptr(f, a) + e * g0, src_dev, e * n * 4, cudaMemcpyDeviceToDevice, s));
+size_t group_words(const dist_b200_feature *f) {
+    size_t n = 0;
+    for (int a = 0; a < stat_arrays(f); ++a) n += stat_elems(f, a);
+    return n;
+}
+bool stats_resident(const dist_b200_feature *f) { return f->stats[0] != nullptr; }
+
+// (re)allocate the statistics arrays for G groups, keeping the first G groups of the feature when `keep`.  Each model
+// keeps its growth slack: pooled and dd as their hot caches, dpd a quarter, niw a quarter + 8 groups.
+int reserve_stats(dist_b200_feature *f, int G, bool keep) {
+    const int na = stat_arrays(f), need = std::max(G, 1);
+    bool fits = need <= f->stats_cap;
+    for (int a = 0; a < na; ++a) fits = fits && 4 * stat_elems(f, a) * f->stats_cap <= f->stats_bytes[a];
+    if (fits) return DIST_B200_OK;
+    int cap;
+    if (f->model == DIST_B200_DPD) {
+        cap = static_cast<int>(round_up(static_cast<size_t>(need) + need / 4, 8));
+    } else if (f->model == DIST_B200_NIW) {
+        cap = need + need / 4 + 8;
+    } else {
+        const size_t c = round_up(static_cast<size_t>(need), 128);
+        cap = static_cast<int>(round_up(c + c / 2, 128));
+    }
+    for (int a = 0; a < na; ++a) {
+        const size_t e = 4 * stat_elems(f, a);
+        if (int rc = grow(f->ctx, f->stats[a], f->stats_bytes[a], e * cap, keep ? e * std::min(f->G, cap) : 0)) return rc;
+    }
+    f->stats_cap = cap;
     return DIST_B200_OK;
 }
 
-// (re)allocate the hot-layout buffer for `G` groups, zero-filled, padded to 128 groups so that the
-// score kernel may stage whole register tiles
+// (re)allocate the hot caches for G groups, keeping the first G groups of the feature when `keep`.  Pooled models and
+// dd: params (nich also aux), padded to 128 groups so that the score kernel may stage whole register tiles, and
+// zero-filled past the kept part.  dpd: the table, (V + 2) rows of G floats (every caller rebuilds it whole).  niw: the
+// records and, at d = 32, the tensor-core images.
 int ensure_params(dist_b200_feature *f, int G, bool keep) {
     dist_b200_ctx *ctx = f->ctx;
-    size_t bytes;
-    const int cap = static_cast<int>(round_up(static_cast<size_t>(std::max(G, 1)), 128));
-    if (f->model == DIST_B200_DPD) {
-        bytes = sizeof(float) * static_cast<size_t>(f->dim + 2) * G;  // table rows + OTHER row + shift row
-    } else {
-        bytes = sizeof(float) * group_floats(f) * cap;
+    const size_t need = static_cast<size_t>(std::max(G, 1));
+    int rc = DIST_B200_OK;
+    if (f->model == DIST_B200_NIW) {
+        const size_t rec = sizeof(float) * niw_rec_floats(f->dim), tc = sizeof(float) * niw_tc_floats(static_cast<int>(need));
+        if (rec * need > f->niw_bytes)
+            rc = grow(ctx, f->niw_buf, f->niw_bytes, rec * need + rec * need / 4, keep ? rec * f->G : 0);
+        if (!rc && f->dim == 32 && tc > f->niw_tc_bytes) rc = grow(ctx, f->niw_tc, f->niw_tc_bytes, tc + tc / 4);
+        return rc;
     }
-    const int old_capacity = f->capacity, old_G = f->G;
-    if (bytes <= f->params_bytes && (f->model == DIST_B200_DPD || cap <= f->capacity))
-        return ensure_stats(f, f->stats ? old_capacity : 0, old_G, keep);
-    void *fresh = nullptr;
-    const size_t want = f->model == DIST_B200_DPD ? bytes : sizeof(float) * group_floats(f) * round_up(cap + cap / 2, 128);
-    DISTB200_CUDA(ctx, cudaMalloc(&fresh, want));
-    DISTB200_CUDA(ctx, cudaMemset(fresh, 0, want));
-    if (f->params) {
-        if (keep) DISTB200_CUDA(ctx, cudaMemcpy(fresh, f->params, std::min(want, f->params_bytes), cudaMemcpyDeviceToDevice));
-        DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-        DISTB200_CUDA(ctx, cudaFree(f->params));
+    if (f->model == DIST_B200_DPD) {  // table rows + OTHER row + shift row
+        const size_t row = sizeof(float) * (f->dim + 2);
+        if (row * need > f->params_bytes) rc = grow(ctx, f->params, f->params_bytes, row * round_up(need + need / 4, 8));
+        f->capacity = static_cast<int>(f->params_bytes / row);
+        return rc;
     }
-    f->params = fresh;
-    f->params_bytes = want;
-    f->capacity = f->model == DIST_B200_DPD ? G : static_cast<int>(want / (sizeof(float) * group_floats(f)));
-    if (f->model == DIST_B200_NICH) {
-        float *aux = nullptr;
-        DISTB200_CUDA(ctx, cudaMalloc(&aux, sizeof(float) * f->capacity));
-        DISTB200_CUDA(ctx, cudaMemset(aux, 0, sizeof(float) * f->capacity));
-        if (f->aux) {
-            if (keep) DISTB200_CUDA(ctx, cudaMemcpy(aux, f->aux, sizeof(float) * std::min(f->capacity, f->G), cudaMemcpyDeviceToDevice));
-            DISTB200_CUDA(ctx, cudaFree(f->aux));
-        }
-        f->aux = aux;
+    const size_t gb = sizeof(float) * group_floats(f), cap = round_up(need, 128);
+    if (gb * cap > f->params_bytes) {
+        const size_t fresh = round_up(cap + cap / 2, 128);
+        if ((rc = grow(ctx, f->params, f->params_bytes, gb * fresh, keep ? f->params_bytes : 0, true))) return rc;
+        if (f->model == DIST_B200_NICH && (rc = grow(ctx, f->aux, f->aux_bytes, sizeof(float) * fresh, keep ? f->aux_bytes : 0, true)))
+            return rc;
     }
-    return ensure_stats(f, old_capacity, old_G, keep);
+    f->capacity = static_cast<int>(f->params_bytes / gb);
+    return DIST_B200_OK;
 }
 
 // copy host arrays into consecutive, 256-byte aligned regions of the context scratch
@@ -177,54 +148,42 @@ struct Upload {
     }
 };
 
-// dpd storage: table (V + 2) x capacity floats (dense stride G inside it), statistics counts[capacity][V] | betas[V]
-uint32_t *dpd_betas(const dist_b200_feature *f) { return f->stats + static_cast<size_t>(f->capacity) * f->dim; }
-int dpd_reserve(dist_b200_feature *f, int G, int V, bool keep) {
+// recompute the caches of groups [g0, g0 + n) from the resident statistics.  The prep launchers read group i of their
+// inputs from the pointers given and write cache g0 + i.
+int rebuild(dist_b200_feature *f, int g0, int n, cudaStream_t s) {
     dist_b200_ctx *ctx = f->ctx;
-    const int need = std::max(G, 1);
-    const bool fits = f->params && f->stats && need <= f->capacity &&
-                      f->params_bytes >= sizeof(float) * static_cast<size_t>(V + 2) * f->capacity &&
-                      f->stats_words >= static_cast<size_t>(f->capacity) * V + V;
-    if (fits) return DIST_B200_OK;
-    const int cap = static_cast<int>(round_up(static_cast<size_t>(need) + need / 4, 8));
-    void *params = nullptr;
-    uint32_t *stats = nullptr;
-    const size_t pbytes = sizeof(float) * static_cast<size_t>(V + 2) * cap, words = static_cast<size_t>(cap) * V + V;
-    DISTB200_CUDA(ctx, cudaMalloc(&params, pbytes));
-    DISTB200_CUDA(ctx, cudaMalloc(&stats, words * 4));
-    DISTB200_CUDA(ctx, cudaMemset(stats, 0, words * 4));
-    DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-    if (keep && f->stats && f->G > 0) {  // counts rows are contiguous; betas move with the capacity
-        DISTB200_CUDA(ctx, cudaMemcpy(stats, f->stats, sizeof(int32_t) * static_cast<size_t>(f->G) * V, cudaMemcpyDeviceToDevice));
-        DISTB200_CUDA(ctx, cudaMemcpy(stats + static_cast<size_t>(cap) * V, dpd_betas(f), sizeof(float) * V, cudaMemcpyDeviceToDevice));
-    }
-    if (f->params) DISTB200_CUDA(ctx, cudaFree(f->params));
-    if (f->stats) DISTB200_CUDA(ctx, cudaFree(f->stats));
-    f->params = params;
-    f->params_bytes = pbytes;
-    f->stats = stats;
-    f->stats_words = words;
-    f->capacity = cap;
-    return DIST_B200_OK;
-}
-
-// dpd caches: the canonical value-major table (dpd.hpp:471-497) + the scratch table_rows.cu re-lays it out into per call
-int dpd_rebuild(dist_b200_feature *f, const float *betas_dev, const int32_t *counts_dev, cudaStream_t s) {
-    dist_b200_ctx *ctx = f->ctx;
-    int rc = launch_dpd_prep(ctx, f->alpha, f->beta0, f->dim, betas_dev, f->G, counts_dev, static_cast<float *>(f->params), s);
-    if (rc || f->G < 1) return rc;
-    const size_t need = table_hot_floats(f->dim + 1, f->G);
-    if (need > f->dpd_hot_floats) {
-        if (f->dpd_hot) {
-            DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-            DISTB200_CUDA(ctx, cudaFree(f->dpd_hot));
-            f->dpd_hot = nullptr;
-            f->dpd_hot_floats = 0;
+    auto u32 = [&](int a) { return f->stats[a] + stat_elems(f, a) * g0; };
+    auto i32 = [&](int a) { return reinterpret_cast<const int32_t *>(u32(a)); };
+    auto f32 = [&](int a) { return reinterpret_cast<const float *>(u32(a)); };
+    float4 *params = static_cast<float4 *>(f->params);
+    switch (f->model) {
+        case DIST_B200_NICH: return launch_nich_prep(ctx, f->shared, f->G, g0, n, i32(0), f32(1), f32(2), params, f->aux, s);
+        case DIST_B200_GP:
+            f->gp_table_dirty = true;
+            f->log_prod_valid = false;
+            return launch_gp_prep(ctx, f->shared, g0, n, u32(0), u32(1), params, s);
+        case DIST_B200_BNB: return launch_bnb_prep(ctx, f->shared, g0, n, u32(0), u32(1), params, s);
+        case DIST_B200_BB: return launch_bb_prep(ctx, f->shared, g0, n, i32(0), i32(1), params, s);
+        case DIST_B200_DD:
+            return launch_dd_prep(ctx, f->dim, f->alphas_dev, f->alpha_sum, g0, n, i32(0), static_cast<float *>(f->params), s);
+        case DIST_B200_DPD: {  // the canonical value-major table (dpd.hpp:471-497), its stride is G
+            float *table = static_cast<float *>(f->params);
+            if (n == 1 && f->G > 1)
+                return launch_dpd_update_group(ctx, f->shared[0], f->shared[1], f->dim, f->alphas_dev, f->G, g0, i32(0), table, s);
+            int rc = launch_dpd_prep(ctx, f->shared[0], f->shared[1], f->dim, f->alphas_dev, f->G, i32(0), table, s);
+            if (rc || f->G < 1) return rc;
+            // + the scratch table_rows.cu re-lays the table out into per call
+            return grow(ctx, f->dpd_hot, f->dpd_hot_bytes, sizeof(float) * table_hot_floats(f->dim + 1, f->G));
         }
-        DISTB200_CUDA(ctx, cudaMalloc(&f->dpd_hot, need * sizeof(float)));
-        f->dpd_hot_floats = need;
+        case DIST_B200_NIW: {  // records, then the tensor-core images of all groups
+            const int d = f->dim;
+            int rc = launch_niw_prep(ctx, d, f->alphas_dev, f->shared[0], f->alphas_dev + d, f->shared[1], n, i32(0), f32(1), f32(2),
+                                     f->niw_buf + niw_rec_floats(d) * g0, s);
+            if (rc == DIST_B200_OK && d == 32 && f->niw_tc && f->G > 0) rc = launch_niw_tc_prep(ctx, f->G, f->niw_buf, f->niw_tc, s);
+            return rc;
+        }
+        default: return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "unknown model");
     }
-    return DIST_B200_OK;
 }
 
 bool check_feature(const dist_b200_feature *f, int model) { return f && f->ctx && f->model == model; }
@@ -233,8 +192,8 @@ bool check_feature(const dist_b200_feature *f, int model) { return f && f->ctx &
 int mark_ready(dist_b200_feature *f, int rc, cudaStream_t s) {
     if (rc != DIST_B200_OK) return rc;
     DISTB200_CUDA(f->ctx, cudaEventRecord(f->ready, s));
-    // the statistics were staged through the context's scratch buffer: drain the stream so the next
-    // host-side upload (possibly on another stream) cannot overwrite it under the prep kernel
+    // the update entries copy from the caller's host arrays asynchronously: drain the stream, so that every update
+    // returns with its work complete and the caller may reuse or free those arrays at once
     DISTB200_CUDA(f->ctx, cudaStreamSynchronize(s));
     return DIST_B200_OK;
 }
@@ -350,10 +309,9 @@ void dist_b200_feature_destroy(dist_b200_feature *f) {
     if (f->cdf_buf) cudaFree(f->cdf_buf);
     if (f->niw_buf) cudaFree(f->niw_buf);
     if (f->niw_tc) cudaFree(f->niw_tc);
-    if (f->niw_stats) cudaFree(f->niw_stats);
-    if (f->niw_shared_dev) cudaFree(f->niw_shared_dev);
     if (f->sample_buf) cudaFree(f->sample_buf);
-    if (f->stats) cudaFree(f->stats);
+    for (uint32_t *st : f->stats)
+        if (st) cudaFree(st);
     if (f->alphas_dev) cudaFree(f->alphas_dev);
     if (f->log_prod_dev) cudaFree(f->log_prod_dev);
     if (f->ready) cudaEventDestroy(f->ready);
@@ -363,122 +321,75 @@ void dist_b200_feature_destroy(dist_b200_feature *f) {
 int dist_b200_feature_model(const dist_b200_feature *f) { return f ? f->model : -1; }
 int dist_b200_feature_groups(const dist_b200_feature *f) { return f ? f->G : 0; }
 
+// update_all after the model's validation (f->dim, f->shared and f->alphas set): the Shared vector and the statistics
+// arrays (G groups each, in stats order) go straight into the resident buffers, then every cache is rebuilt
+static int write_all(dist_b200_feature *f, int G, std::initializer_list<const void *> arrays, void *stream) {
+    dist_b200_ctx *ctx = f->ctx;
+    cudaStream_t s = as_stream(stream);
+    int rc;
+    if ((rc = grow(ctx, f->alphas_dev, f->alphas_bytes, sizeof(float) * f->alphas.size())) || (rc = ensure_params(f, G, false)) ||
+        (rc = reserve_stats(f, G, false)))
+        return rc;
+    DISTB200_CUDA(ctx, cudaStreamWaitEvent(s, f->ready, 0));
+    if (!f->alphas.empty())
+        DISTB200_CUDA(ctx, cudaMemcpyAsync(f->alphas_dev, f->alphas.data(), sizeof(float) * f->alphas.size(), cudaMemcpyHostToDevice, s));
+    int a = 0;
+    for (const void *src : arrays) {
+        if (G) DISTB200_CUDA(ctx, cudaMemcpyAsync(f->stats[a], src, 4 * stat_elems(f, a) * G, cudaMemcpyHostToDevice, s));
+        ++a;
+    }
+    f->G = G;
+    return mark_ready(f, rebuild(f, 0, G, s), s);
+}
+
 int dist_b200_nich_update_all(dist_b200_feature *f, const float shared[4], int G, const int32_t *count,
                               const float *mean, const float *ctv, void *stream) {
     if (!check_feature(f, DIST_B200_NICH) || !shared || G < 0 || (G && (!count || !mean || !ctv))) return DIST_B200_ERR_INVALID;
-    dist_b200_ctx *ctx = f->ctx;
     std::memcpy(f->shared, shared, sizeof(float) * 4);
-    int rc = ensure_params(f, G, false);
-    if (rc) return rc;
-    if ((rc = ensure_scratch(ctx, 3 * round_up(sizeof(float) * G, 256) + 256))) return rc;
-    Upload up{ctx, as_stream(stream)};
-    const int32_t *c = up.put(count, G);
-    const float *m = up.put(mean, G);
-    const float *v = up.put(ctv, G);
-    if (up.err) return up.err;
-    f->G = G;
-    if ((rc = mirror_stats(f, 0, c, 0, G, as_stream(stream))) || (rc = mirror_stats(f, 1, m, 0, G, as_stream(stream))) ||
-        (rc = mirror_stats(f, 2, v, 0, G, as_stream(stream))))
-        return rc;
-    return mark_ready(f, launch_nich_prep(ctx, f->shared, G, 0, G, c, m, v, static_cast<float4 *>(f->params), f->aux, as_stream(stream)), as_stream(stream));
+    return write_all(f, G, {count, mean, ctv}, stream);
 }
 
 int dist_b200_gp_update_all(dist_b200_feature *f, const float shared[2], int G, const uint32_t *count,
                             const uint32_t *sum, void *stream) {
     if (!check_feature(f, DIST_B200_GP) || !shared || G < 0 || (G && (!count || !sum))) return DIST_B200_ERR_INVALID;
-    dist_b200_ctx *ctx = f->ctx;
     f->shared[0] = shared[0];
     f->shared[1] = shared[1];
-    int rc = ensure_params(f, G, false);
-    if (rc) return rc;
-    if ((rc = ensure_scratch(ctx, 2 * round_up(sizeof(float) * G, 256) + 256))) return rc;
-    Upload up{ctx, as_stream(stream)};
-    const uint32_t *c = up.put(count, G);
-    const uint32_t *sm = up.put(sum, G);
-    if (up.err) return up.err;
-    f->G = G;
-    f->gp_table_dirty = true;
-    f->log_prod_valid = false;
-    if ((rc = mirror_stats(f, 0, c, 0, G, as_stream(stream))) || (rc = mirror_stats(f, 1, sm, 0, G, as_stream(stream)))) return rc;
-    return mark_ready(f, launch_gp_prep(ctx, f->shared, 0, G, c, sm, static_cast<float4 *>(f->params), as_stream(stream)), as_stream(stream));
+    return write_all(f, G, {count, sum}, stream);
 }
 
 int dist_b200_bnb_update_all(dist_b200_feature *f, const float shared[2], uint32_t r, int G, const uint32_t *count,
                              const uint32_t *sum, void *stream) {
     if (!check_feature(f, DIST_B200_BNB) || !shared || G < 0 || (G && (!count || !sum))) return DIST_B200_ERR_INVALID;
-    dist_b200_ctx *ctx = f->ctx;
     f->shared[0] = shared[0];
     f->shared[1] = shared[1];
     f->shared[2] = static_cast<float>(r);  // the reference converts r to float wherever it enters (bnb.hpp:59,208)
-    int rc = ensure_params(f, G, false);
-    if (rc) return rc;
-    if ((rc = ensure_scratch(ctx, 2 * round_up(sizeof(float) * G, 256) + 256))) return rc;
-    Upload up{ctx, as_stream(stream)};
-    const uint32_t *c = up.put(count, G);
-    const uint32_t *sm = up.put(sum, G);
-    if (up.err) return up.err;
-    f->G = G;
-    if ((rc = mirror_stats(f, 0, c, 0, G, as_stream(stream))) || (rc = mirror_stats(f, 1, sm, 0, G, as_stream(stream)))) return rc;
-    return mark_ready(f, launch_bnb_prep(ctx, f->shared, 0, G, c, sm, static_cast<float4 *>(f->params), as_stream(stream)), as_stream(stream));
+    return write_all(f, G, {count, sum}, stream);
 }
 
 int dist_b200_bb_update_all(dist_b200_feature *f, const float shared[2], int G, const int32_t *heads,
                             const int32_t *tails, void *stream) {
     if (!check_feature(f, DIST_B200_BB) || !shared || G < 0 || (G && (!heads || !tails))) return DIST_B200_ERR_INVALID;
-    dist_b200_ctx *ctx = f->ctx;
     f->shared[0] = shared[0];
     f->shared[1] = shared[1];
-    int rc = ensure_params(f, G, false);
-    if (rc) return rc;
-    if ((rc = ensure_scratch(ctx, 2 * round_up(sizeof(float) * G, 256) + 256))) return rc;
-    Upload up{ctx, as_stream(stream)};
-    const int32_t *h = up.put(heads, G);
-    const int32_t *t = up.put(tails, G);
-    if (up.err) return up.err;
-    f->G = G;
-    if ((rc = mirror_stats(f, 0, h, 0, G, as_stream(stream))) || (rc = mirror_stats(f, 1, t, 0, G, as_stream(stream)))) return rc;
-    return mark_ready(f, launch_bb_prep(ctx, f->shared, 0, G, h, t, static_cast<float4 *>(f->params), as_stream(stream)), as_stream(stream));
+    return write_all(f, G, {heads, tails}, stream);
 }
 
 int dist_b200_dd_update_all(dist_b200_feature *f, int dim, const float *alphas, int G, const int32_t *counts,
                             void *stream) {
     if (!check_feature(f, DIST_B200_DD) || dim < 1 || !alphas || G < 0 || (G && !counts)) return DIST_B200_ERR_INVALID;
-    dist_b200_ctx *ctx = f->ctx;
-    if (dim > 256) return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "dd: dim > 256");
-    if (dim != f->dim) {  // layout changes: drop the old buffer
-        if (f->params) {
-            DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-            DISTB200_CUDA(ctx, cudaFree(f->params));
-        }
-        f->params = nullptr;
-        f->params_bytes = 0;
-        f->capacity = 0;
-    }
+    if (dim > 256) return fail(f->ctx, DIST_B200_ERR_UNSUPPORTED, "dd: dim > 256");
     f->dim = dim;
     f->alphas.assign(alphas, alphas + dim);
     float alpha_sum = 0;  // dd.hpp:404-407, sequential float sum
     for (int v = 0; v < dim; ++v) alpha_sum += alphas[v];
     f->alpha_sum = alpha_sum;
-    int rc = ensure_params(f, G, false);
-    if (rc) return rc;
-    if ((rc = ensure_scratch(ctx, round_up(sizeof(float) * dim, 256) + round_up(sizeof(int32_t) * static_cast<size_t>(G) * dim, 256) + 256))) return rc;
-    Upload up{ctx, as_stream(stream)};
-    const float *a = up.put(alphas, dim);
-    const int32_t *c = up.put(counts, static_cast<size_t>(G) * dim);
-    if (up.err) return up.err;
-    f->G = G;
-    if (!f->alphas_dev) DISTB200_CUDA(ctx, cudaMalloc(&f->alphas_dev, sizeof(float) * 256));
-    DISTB200_CUDA(ctx, cudaMemcpyAsync(f->alphas_dev, a, sizeof(float) * dim, cudaMemcpyDeviceToDevice, as_stream(stream)));
-    if ((rc = mirror_stats(f, 0, c, 0, G, as_stream(stream)))) return rc;
-    return mark_ready(f, launch_dd_prep(ctx, dim, a, alpha_sum, 0, G, c, static_cast<float *>(f->params), as_stream(stream)), as_stream(stream));
+    return write_all(f, G, {counts}, stream);
 }
 
 int dist_b200_dpd_update_all(dist_b200_feature *f, float alpha, float beta0, int V, const uint32_t *keys,
                              const float *betas, int G, const int32_t *counts, void *stream) {
     if (!check_feature(f, DIST_B200_DPD) || V < 1 || !keys || !betas || G < 0 || (G && !counts)) return DIST_B200_ERR_INVALID;
     dist_b200_ctx *ctx = f->ctx;
-    f->alpha = alpha;
-    f->beta0 = beta0;
     // value -> table row: identity when keys are 0..V-1, else sorted keys + binary search on device
     bool dense = true;
     for (int v = 0; v < V; ++v) dense = dense && keys[v] == static_cast<uint32_t>(v);
@@ -490,51 +401,22 @@ int dist_b200_dpd_update_all(dist_b200_feature *f, float alpha, float beta0, int
         for (int i = 0; i < V; ++i) sorted[i] = keys[order[i]];
         for (int i = 1; i < V; ++i)
             if (sorted[i] == sorted[i - 1]) return fail(ctx, DIST_B200_ERR_INVALID, "dpd: duplicate key");
-        if (f->keys_dev) {
-            DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-            DISTB200_CUDA(ctx, cudaFree(f->keys_dev));
-            DISTB200_CUDA(ctx, cudaFree(f->key_rows_dev));
-            f->keys_dev = nullptr;
-            f->key_rows_dev = nullptr;
-        }
-        DISTB200_CUDA(ctx, cudaMalloc(&f->keys_dev, sizeof(uint32_t) * V));
-        DISTB200_CUDA(ctx, cudaMalloc(&f->key_rows_dev, sizeof(int) * V));
-        DISTB200_CUDA(ctx, cudaMemcpy(f->keys_dev, sorted.data(), sizeof(uint32_t) * V, cudaMemcpyHostToDevice));
-        DISTB200_CUDA(ctx, cudaMemcpy(f->key_rows_dev, order.data(), sizeof(int) * V, cudaMemcpyHostToDevice));
+        int rc;
+        if ((rc = grow(ctx, f->keys_dev, f->keys_bytes, sizeof(uint32_t) * V)) || (rc = grow(ctx, f->key_rows_dev, f->key_rows_bytes, sizeof(int) * V)))
+            return rc;
+        cudaStream_t s = as_stream(stream);
+        DISTB200_CUDA(ctx, cudaStreamWaitEvent(s, f->ready, 0));
+        DISTB200_CUDA(ctx, cudaMemcpyAsync(f->keys_dev, sorted.data(), sizeof(uint32_t) * V, cudaMemcpyHostToDevice, s));
+        DISTB200_CUDA(ctx, cudaMemcpyAsync(f->key_rows_dev, order.data(), sizeof(int) * V, cudaMemcpyHostToDevice, s));
+        DISTB200_CUDA(ctx, cudaStreamSynchronize(s));  // the host vectors go out of scope
         f->keys.assign(keys, keys + V);
     }
     f->keys_dense = dense;
     f->dim = V;
+    f->shared[0] = alpha;
+    f->shared[1] = beta0;
     f->alphas.assign(betas, betas + V);
-    int rc = dpd_reserve(f, G, V, false);
-    if (rc) return rc;
-    if ((rc = ensure_scratch(ctx, round_up(sizeof(float) * V, 256) + round_up(sizeof(int32_t) * static_cast<size_t>(G) * V, 256) + 256))) return rc;
-    Upload up{ctx, as_stream(stream)};
-    const float *b = up.put(betas, V);
-    const int32_t *c = up.put(counts, static_cast<size_t>(G) * V);
-    if (up.err) return up.err;
-    f->G = G;
-    DISTB200_CUDA(ctx, cudaMemcpyAsync(f->stats, c, sizeof(int32_t) * static_cast<size_t>(G) * V, cudaMemcpyDeviceToDevice, as_stream(stream)));
-    DISTB200_CUDA(ctx, cudaMemcpyAsync(dpd_betas(f), b, sizeof(float) * V, cudaMemcpyDeviceToDevice, as_stream(stream)));
-    return mark_ready(f, dpd_rebuild(f, b, c, as_stream(stream)), as_stream(stream));
-}
-
-static int niw_reserve(dist_b200_feature *f, int G, int keep);
-static int32_t *niw_count(const dist_b200_feature *f) { return reinterpret_cast<int32_t *>(f->niw_stats); }
-static float *niw_sum_x(const dist_b200_feature *f) { return reinterpret_cast<float *>(f->niw_stats) + f->niw_cap; }
-static float *niw_sum_xxT(const dist_b200_feature *f) {
-    return reinterpret_cast<float *>(f->niw_stats) + f->niw_cap + static_cast<size_t>(f->niw_cap) * f->dim;
-}
-// records of groups [g0, g0 + n) (and the tensor-core images) from the resident statistics
-static int niw_rebuild(dist_b200_feature *f, int g0, int n, cudaStream_t s) {
-    dist_b200_ctx *ctx = f->ctx;
-    const int d = f->dim;
-    const size_t dd = static_cast<size_t>(d) * d;
-    const size_t rec = static_cast<size_t>(niw_padded_dim(d)) * (niw_padded_dim(d) + 1) + 4;
-    int rc = launch_niw_prep(ctx, d, f->niw_shared_dev, f->kappa, f->niw_shared_dev + d, f->nu, n, niw_count(f) + g0,
-                             niw_sum_x(f) + static_cast<size_t>(g0) * d, niw_sum_xxT(f) + g0 * dd, f->niw_buf + rec * g0, s);
-    if (rc == DIST_B200_OK && d == 32 && f->niw_tc && f->G > 0) rc = launch_niw_tc_prep(ctx, f->G, f->niw_buf, f->niw_tc, s);
-    return rc;
+    return write_all(f, G, {counts}, stream);
 }
 
 int dist_b200_niw_update_all(dist_b200_feature *f, int d, const float *mu, float kappa, const float *psi,
@@ -546,274 +428,78 @@ int dist_b200_niw_update_all(dist_b200_feature *f, int d, const float *mu, float
     if (d > 32) return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "niw: d > 32");
     if (!(kappa > 0.f) || !(nu > static_cast<float>(d) - 1.f))
         return fail(ctx, DIST_B200_ERR_INVALID, "niw: need kappa > 0 and nu > d - 1 (niw.hpp:121,132)");
-    if (f->niw_stats && f->dim != d) {  // the statistics layout depends on d
-        DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-        DISTB200_CUDA(ctx, cudaFree(f->niw_stats));
-        f->niw_stats = nullptr;
-        f->niw_cap = 0;
-    }
     f->dim = d;
-    {
-        int rcr = niw_reserve(f, G, 0);
-        if (rcr) return rcr;
-    }
-    const size_t dd = static_cast<size_t>(d) * d;
-    int rc = ensure_scratch(ctx, round_up(4 * d, 256) + round_up(4 * dd, 256) + round_up(4 * static_cast<size_t>(G), 256) +
-                                     round_up(4 * static_cast<size_t>(G) * d, 256) + round_up(4 * G * dd, 256) + 256);
-    if (rc) return rc;
-    Upload up{ctx, as_stream(stream)};
-    const float *mu_d = up.put(mu, d);
-    const float *psi_d = up.put(psi, dd);
-    const int32_t *cnt_d = up.put(count, G);
-    const float *sx_d = up.put(sum_x, static_cast<size_t>(G) * d);
-    const float *sxx_d = up.put(sum_xxT, static_cast<size_t>(G) * dd);
-    if (up.err) return up.err;
-    f->dim = d;
-    f->G = G;
-    f->kappa = kappa;
-    f->nu = nu;
-    f->mu.assign(mu, mu + d);
-    f->psi.assign(psi, psi + dd);
-    cudaStream_t s = as_stream(stream);
-    DISTB200_CUDA(ctx, cudaMemcpyAsync(f->niw_shared_dev, mu_d, sizeof(float) * d, cudaMemcpyDeviceToDevice, s));
-    DISTB200_CUDA(ctx, cudaMemcpyAsync(f->niw_shared_dev + d, psi_d, sizeof(float) * dd, cudaMemcpyDeviceToDevice, s));
-    if (G > 0) {
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(niw_count(f), cnt_d, sizeof(int32_t) * G, cudaMemcpyDeviceToDevice, s));
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(niw_sum_x(f), sx_d, sizeof(float) * G * d, cudaMemcpyDeviceToDevice, s));
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(niw_sum_xxT(f), sxx_d, sizeof(float) * G * dd, cudaMemcpyDeviceToDevice, s));
-    }
-    return mark_ready(f, niw_rebuild(f, 0, G, s), s);
+    f->shared[0] = kappa;
+    f->shared[1] = nu;
+    f->alphas.assign(mu, mu + d);
+    f->alphas.insert(f->alphas.end(), psi, psi + static_cast<size_t>(d) * d);
+    return write_all(f, G, {count, sum_x, sum_xxT}, stream);
 }
 
-// NormalInverseWishart: one group's record (posterior, whitening matrix, constants) from its raw statistics
-// {int32 count; float sum_x[d]; float sum_xxT[d][d]} (niw.hpp:187-190, :247-276), then the tensor-core block records
-static int niw_update_group(dist_b200_feature *f, int groupid, const void *stats, cudaStream_t s) {
-    dist_b200_ctx *ctx = f->ctx;
-    const int d = f->dim;
-    const size_t dd = static_cast<size_t>(d) * d;
-    if (f->mu.size() != static_cast<size_t>(d) || f->psi.size() != dd) return fail(ctx, DIST_B200_ERR_STATE, "niw update_group: call update_all first");
-    if (!f->niw_stats || groupid >= f->niw_cap) return fail(ctx, DIST_B200_ERR_STATE, "niw update_group: call update_all first");
-    int rc = ensure_scratch(ctx, round_up(4 * d, 256) + round_up(4 * dd, 256) + 512);
-    if (rc) return rc;
-    const char *p = static_cast<const char *>(stats);
-    Upload up{ctx, s};
-    const int32_t *cnt_d = up.put(reinterpret_cast<const int32_t *>(p), 1);
-    const float *sx_d = up.put(reinterpret_cast<const float *>(p + 4), d);
-    const float *sxx_d = up.put(reinterpret_cast<const float *>(p + 4 + 4 * d), dd);
-    if (up.err) return up.err;
-    DISTB200_CUDA(ctx, cudaStreamWaitEvent(s, f->ready, 0));
-    DISTB200_CUDA(ctx, cudaMemcpyAsync(niw_count(f) + groupid, cnt_d, sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
-    DISTB200_CUDA(ctx, cudaMemcpyAsync(niw_sum_x(f) + static_cast<size_t>(groupid) * d, sx_d, sizeof(float) * d, cudaMemcpyDeviceToDevice, s));
-    DISTB200_CUDA(ctx, cudaMemcpyAsync(niw_sum_xxT(f) + groupid * dd, sxx_d, sizeof(float) * dd, cudaMemcpyDeviceToDevice, s));
-    return mark_ready(f, niw_rebuild(f, groupid, 1, s), s);
-}
-
-// (re)allocate the niw record buffers for G groups, keeping the first `keep` records
-static int niw_reserve(dist_b200_feature *f, int G, int keep) {
-    dist_b200_ctx *ctx = f->ctx;
-    const int d = f->dim;
-    const size_t rec = static_cast<size_t>(niw_padded_dim(d)) * (niw_padded_dim(d) + 1) + 4;
-    const size_t bytes = sizeof(float) * rec * std::max(G, 1);
-    if (bytes > f->niw_bytes) {
-        const size_t want = bytes + bytes / 4;
-        float *fresh = nullptr;
-        DISTB200_CUDA(ctx, cudaMalloc(&fresh, want));
-        DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-        if (f->niw_buf) {
-            if (keep > 0) DISTB200_CUDA(ctx, cudaMemcpy(fresh, f->niw_buf, sizeof(float) * rec * keep, cudaMemcpyDeviceToDevice));
-            DISTB200_CUDA(ctx, cudaFree(f->niw_buf));
-        }
-        f->niw_buf = fresh;
-        f->niw_bytes = want;
-    }
-    if (!f->niw_shared_dev) DISTB200_CUDA(ctx, cudaMalloc(&f->niw_shared_dev, sizeof(float) * (32 + 32 * 32)));
-    if (G > f->niw_cap || !f->niw_stats) {
-        const int cap = std::max(G, 1) + std::max(G, 1) / 4 + 8;
-        const size_t dd = static_cast<size_t>(d) * d;
-        uint32_t *fresh = nullptr;
-        DISTB200_CUDA(ctx, cudaMalloc(&fresh, sizeof(uint32_t) * static_cast<size_t>(cap) * (1 + d + dd)));
-        DISTB200_CUDA(ctx, cudaMemset(fresh, 0, sizeof(uint32_t) * static_cast<size_t>(cap) * (1 + d + dd)));
-        DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-        if (f->niw_stats) {
-            if (keep > 0) {
-                DISTB200_CUDA(ctx, cudaMemcpy(fresh, niw_count(f), sizeof(int32_t) * keep, cudaMemcpyDeviceToDevice));
-                DISTB200_CUDA(ctx, cudaMemcpy(fresh + cap, niw_sum_x(f), sizeof(float) * keep * d, cudaMemcpyDeviceToDevice));
-                DISTB200_CUDA(ctx, cudaMemcpy(fresh + cap + static_cast<size_t>(cap) * d, niw_sum_xxT(f), sizeof(float) * keep * dd, cudaMemcpyDeviceToDevice));
-            }
-            DISTB200_CUDA(ctx, cudaFree(f->niw_stats));
-        }
-        f->niw_stats = fresh;
-        f->niw_cap = cap;
-    }
-    if (d == 32) {
-        const size_t tc_bytes = sizeof(float) * niw_tc_floats(std::max(G, 1));
-        if (tc_bytes > f->niw_tc_bytes) {
-            if (f->niw_tc) {
-                DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-                DISTB200_CUDA(ctx, cudaFree(f->niw_tc));
-                f->niw_tc = nullptr;
-            }
-            DISTB200_CUDA(ctx, cudaMalloc(&f->niw_tc, tc_bytes + tc_bytes / 4));
-            f->niw_tc_bytes = tc_bytes + tc_bytes / 4;
-        }
-    }
-    return DIST_B200_OK;
-}
-
+// the record of one group is its slice of each statistics array, in update_all's order (dist_b200.h)
 int dist_b200_feature_update_group(dist_b200_feature *f, int groupid, const void *stats, void *stream) {
     if (!f || !f->ctx || !stats) return DIST_B200_ERR_INVALID;
     dist_b200_ctx *ctx = f->ctx;
     if (groupid < 0 || groupid >= f->G) return fail(ctx, DIST_B200_ERR_INVALID, "update_group: bad groupid");
-    int rc = ensure_scratch(ctx, 4096 + sizeof(int32_t) * 256);
-    if (rc) return rc;
     cudaStream_t s = as_stream(stream);
     DISTB200_CUDA(ctx, cudaStreamWaitEvent(s, f->ready, 0));
-    Upload up{ctx, s};
-    switch (f->model) {
-        case DIST_B200_NICH: {
-            const char *p = static_cast<const char *>(stats);
-            const int32_t *c = up.put(reinterpret_cast<const int32_t *>(p), 1);
-            const float *m = up.put(reinterpret_cast<const float *>(p + 4), 1);
-            const float *v = up.put(reinterpret_cast<const float *>(p + 8), 1);
-            if (up.err) return up.err;
-            if ((rc = mirror_stats(f, 0, c, groupid, 1, s)) || (rc = mirror_stats(f, 1, m, groupid, 1, s)) ||
-                (rc = mirror_stats(f, 2, v, groupid, 1, s)))
-                return rc;
-            return mark_ready(f, launch_nich_prep(ctx, f->shared, f->G, groupid, 1, c, m, v, static_cast<float4 *>(f->params), f->aux, s), s);
-        }
-        case DIST_B200_GP: {
-            const uint32_t *p = static_cast<const uint32_t *>(stats);
-            const uint32_t *c = up.put(p, 1);
-            const uint32_t *sm = up.put(p + 1, 1);
-            if (up.err) return up.err;
-            f->gp_table_dirty = true;
-            f->log_prod_valid = false;
-            if ((rc = mirror_stats(f, 0, c, groupid, 1, s)) || (rc = mirror_stats(f, 1, sm, groupid, 1, s))) return rc;
-            return mark_ready(f, launch_gp_prep(ctx, f->shared, groupid, 1, c, sm, static_cast<float4 *>(f->params), s), s);
-        }
-        case DIST_B200_BNB: {
-            const uint32_t *p = static_cast<const uint32_t *>(stats);
-            const uint32_t *c = up.put(p, 1);
-            const uint32_t *sm = up.put(p + 1, 1);
-            if (up.err) return up.err;
-            if ((rc = mirror_stats(f, 0, c, groupid, 1, s)) || (rc = mirror_stats(f, 1, sm, groupid, 1, s))) return rc;
-            return mark_ready(f, launch_bnb_prep(ctx, f->shared, groupid, 1, c, sm, static_cast<float4 *>(f->params), s), s);
-        }
-        case DIST_B200_BB: {
-            const int32_t *p = static_cast<const int32_t *>(stats);
-            const int32_t *h = up.put(p, 1);
-            const int32_t *t = up.put(p + 1, 1);
-            if (up.err) return up.err;
-            if ((rc = mirror_stats(f, 0, h, groupid, 1, s)) || (rc = mirror_stats(f, 1, t, groupid, 1, s))) return rc;
-            return mark_ready(f, launch_bb_prep(ctx, f->shared, groupid, 1, h, t, static_cast<float4 *>(f->params), s), s);
-        }
-        case DIST_B200_DD: {
-            const float *a = up.put(f->alphas.data(), f->dim);
-            const int32_t *c = up.put(static_cast<const int32_t *>(stats), f->dim);
-            if (up.err) return up.err;
-            if ((rc = mirror_stats(f, 0, c, groupid, 1, s))) return rc;
-            return mark_ready(f, launch_dd_prep(ctx, f->dim, a, f->alpha_sum, groupid, 1, c, static_cast<float *>(f->params), s), s);
-        }
-        case DIST_B200_DPD: {  // stats: the group's dense counts[V], in update_all's key order
-            const int V = f->dim;
-            if ((rc = ensure_scratch(ctx, round_up(sizeof(int32_t) * V, 256) + 256))) return rc;
-            Upload up2{ctx, s};
-            const int32_t *c = up2.put(static_cast<const int32_t *>(stats), V);
-            if (up2.err) return up2.err;
-            int32_t *row = reinterpret_cast<int32_t *>(f->stats) + static_cast<size_t>(groupid) * V;
-            DISTB200_CUDA(ctx, cudaMemcpyAsync(row, c, sizeof(int32_t) * V, cudaMemcpyDeviceToDevice, s));
-            return mark_ready(f, launch_dpd_update_group(ctx, f->alpha, f->beta0, V, reinterpret_cast<const float *>(dpd_betas(f)), f->G, groupid,
-                                                         row, static_cast<float *>(f->params), s), s);
-        }
-        case DIST_B200_NIW: return niw_update_group(f, groupid, stats, s);
-        default:
-            return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "update_group: unknown model");
+    const char *rec = static_cast<const char *>(stats);
+    for (int a = 0; a < stat_arrays(f); ++a) {
+        const size_t e = stat_elems(f, a);
+        DISTB200_CUDA(ctx, cudaMemcpyAsync(f->stats[a] + e * groupid, rec, 4 * e, cudaMemcpyHostToDevice, s));
+        rec += 4 * e;
     }
+    return mark_ready(f, rebuild(f, groupid, 1, s), s);
 }
 
+// a fresh group is Group::init (all-zero statistics) followed by update_group (mixture.hpp:361-369)
 int dist_b200_feature_add_group(dist_b200_feature *f, void *stream) {
     if (!f || !f->ctx) return DIST_B200_ERR_INVALID;
     dist_b200_ctx *ctx = f->ctx;
-    if (f->model == DIST_B200_DPD) {
-        // a fresh empty group: one more zero counts row; the dense table's stride is G, so it is rebuilt (O(V G))
-        if (f->G < 1 && !f->stats) return fail(ctx, DIST_B200_ERR_STATE, "add_group: call update_all first");
-        int rc = dpd_reserve(f, f->G + 1, f->dim, true);
-        if (rc) return rc;
-        cudaStream_t s = as_stream(stream);
-        DISTB200_CUDA(ctx, cudaStreamWaitEvent(s, f->ready, 0));
-        DISTB200_CUDA(ctx, cudaMemsetAsync(f->stats + static_cast<size_t>(f->G) * f->dim, 0, sizeof(int32_t) * f->dim, s));
-        f->G += 1;
-        return mark_ready(f, dpd_rebuild(f, reinterpret_cast<const float *>(dpd_betas(f)), reinterpret_cast<const int32_t *>(f->stats), s), s);
-    }
-    if (f->model == DIST_B200_NIW) {
-        if (f->mu.empty()) return fail(ctx, DIST_B200_ERR_STATE, "add_group: call update_all first");
-        int rc = niw_reserve(f, f->G + 1, f->G);
-        if (rc) return rc;
-        f->G += 1;
-        std::vector<float> zeros(1 + f->dim + static_cast<size_t>(f->dim) * f->dim, 0.f);  // Group::init: count = 0, sums = 0
-        return niw_update_group(f, f->G - 1, zeros.data(), as_stream(stream));
-    }
-    int rc = ensure_params(f, f->G + 1, true);
-    if (rc) return rc;
-    f->G += 1;
-    // a fresh group is Group::init (all-zero statistics) followed by update_group (mixture.hpp:361-369)
-    int32_t zeros[256];
-    std::memset(zeros, 0, sizeof(zeros));
-    return dist_b200_feature_update_group(f, f->G - 1, zeros, stream);
+    if (!stats_resident(f)) return fail(ctx, DIST_B200_ERR_STATE, "add_group: call update_all first");
+    const int g = f->G;
+    int rc;
+    if ((rc = ensure_params(f, g + 1, true)) || (rc = reserve_stats(f, g + 1, true))) return rc;
+    cudaStream_t s = as_stream(stream);
+    DISTB200_CUDA(ctx, cudaStreamWaitEvent(s, f->ready, 0));
+    for (int a = 0; a < stat_arrays(f); ++a)
+        DISTB200_CUDA(ctx, cudaMemsetAsync(f->stats[a] + stat_elems(f, a) * g, 0, 4 * stat_elems(f, a), s));
+    f->G = g + 1;
+    // the dpd table's stride is G: it is rebuilt whole (O(V G))
+    return mark_ready(f, f->model == DIST_B200_DPD ? rebuild(f, 0, f->G, s) : rebuild(f, g, 1, s), s);
 }
 
+// packed_remove: the last group moves into the hole (vector.hpp:47-51)
 int dist_b200_feature_remove_group(dist_b200_feature *f, int groupid, void *stream) {
     if (!f || !f->ctx) return DIST_B200_ERR_INVALID;
     dist_b200_ctx *ctx = f->ctx;
     if (groupid < 0 || groupid >= f->G) return fail(ctx, DIST_B200_ERR_INVALID, "remove_group: bad groupid");
-    if (f->model == DIST_B200_DPD) {  // packed_remove on the counts rows, then the dense table again
-        cudaStream_t s = as_stream(stream);
-        DISTB200_CUDA(ctx, cudaStreamWaitEvent(s, f->ready, 0));
-        const int last = f->G - 1, V = f->dim;
-        if (groupid != last)
-            DISTB200_CUDA(ctx, cudaMemcpyAsync(f->stats + static_cast<size_t>(groupid) * V, f->stats + static_cast<size_t>(last) * V,
-                                               sizeof(int32_t) * V, cudaMemcpyDeviceToDevice, s));
-        f->G = last;
-        return mark_ready(f, dpd_rebuild(f, reinterpret_cast<const float *>(dpd_betas(f)), reinterpret_cast<const int32_t *>(f->stats), s), s);
+    cudaStream_t s = as_stream(stream);
+    DISTB200_CUDA(ctx, cudaStreamWaitEvent(s, f->ready, 0));
+    const int last = f->G - 1;
+    for (int a = 0; a < stat_arrays(f) && groupid != last; ++a) {
+        const size_t e = stat_elems(f, a);
+        DISTB200_CUDA(ctx, cudaMemcpyAsync(f->stats[a] + e * groupid, f->stats[a] + e * last, 4 * e, cudaMemcpyDeviceToDevice, s));
     }
+    f->G = last;
+    if (f->model == DIST_B200_DPD) return mark_ready(f, rebuild(f, 0, last, s), s);  // stride G again
+    int rc = DIST_B200_OK;
     if (f->model == DIST_B200_NIW) {
-        cudaStream_t s = as_stream(stream);
-        DISTB200_CUDA(ctx, cudaStreamWaitEvent(s, f->ready, 0));
-        const size_t rec = static_cast<size_t>(niw_padded_dim(f->dim)) * (niw_padded_dim(f->dim) + 1) + 4;
-        const int last = f->G - 1;
-        if (groupid != last) {
-            const int d = f->dim;
-            const size_t dd = static_cast<size_t>(d) * d;
+        const size_t rec = niw_rec_floats(f->dim);
+        if (groupid != last)
             DISTB200_CUDA(ctx, cudaMemcpyAsync(f->niw_buf + rec * groupid, f->niw_buf + rec * last, sizeof(float) * rec, cudaMemcpyDeviceToDevice, s));
-            DISTB200_CUDA(ctx, cudaMemcpyAsync(niw_count(f) + groupid, niw_count(f) + last, sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
-            DISTB200_CUDA(ctx, cudaMemcpyAsync(niw_sum_x(f) + static_cast<size_t>(groupid) * d, niw_sum_x(f) + static_cast<size_t>(last) * d,
-                                               sizeof(float) * d, cudaMemcpyDeviceToDevice, s));
-            DISTB200_CUDA(ctx, cudaMemcpyAsync(niw_sum_xxT(f) + groupid * dd, niw_sum_xxT(f) + last * dd, sizeof(float) * dd, cudaMemcpyDeviceToDevice, s));
-        }
-        f->G = last;
-        int rc = DIST_B200_OK;
-        if (f->dim == 32 && f->niw_tc && f->G > 0) rc = launch_niw_tc_prep(ctx, f->G, f->niw_buf, f->niw_tc, s);
+        if (f->dim == 32 && f->niw_tc && last > 0) rc = launch_niw_tc_prep(ctx, last, f->niw_buf, f->niw_tc, s);
         return mark_ready(f, rc, s);
     }
     const size_t gb = sizeof(float) * group_floats(f);
     char *base = static_cast<char *>(f->params);
-    const int last = f->G - 1;
-    if (groupid != last)  // packed_remove: move the last group into the hole (vector.hpp:47-51)
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(base + gb * groupid, base + gb * last, gb, cudaMemcpyDeviceToDevice, as_stream(stream)));
-    DISTB200_CUDA(ctx, cudaMemsetAsync(base + gb * last, 0, gb, as_stream(stream)));
+    if (groupid != last) DISTB200_CUDA(ctx, cudaMemcpyAsync(base + gb * groupid, base + gb * last, gb, cudaMemcpyDeviceToDevice, s));
+    DISTB200_CUDA(ctx, cudaMemsetAsync(base + gb * last, 0, gb, s));
+    if (f->aux && groupid != last)
+        DISTB200_CUDA(ctx, cudaMemcpyAsync(f->aux + groupid, f->aux + last, sizeof(float), cudaMemcpyDeviceToDevice, s));
     f->gp_table_dirty = true;
     f->log_prod_valid = false;
-    if (f->stats && groupid != last) {
-        for (int a = 0; a < stat_arrays(f); ++a) {
-            const size_t e = stat_elems(f, a);
-            DISTB200_CUDA(ctx, cudaMemcpyAsync(stat_ptr(f, a) + e * groupid, stat_ptr(f, a) + e * last, e * 4, cudaMemcpyDeviceToDevice,
-                                               as_stream(stream)));
-        }
-    }
-    if (f->aux && groupid != last)
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(f->aux + groupid, f->aux + last, sizeof(float), cudaMemcpyDeviceToDevice, as_stream(stream)));
-    f->G = last;
-    return mark_ready(f, DIST_B200_OK, as_stream(stream));
+    return mark_ready(f, rc, s);
 }
 
 // batched Group::add_value over many features of one kind.  Everything is enqueued on `stream`: the
@@ -848,7 +534,7 @@ static int rows_batch(dist_b200_ctx *ctx, dist_b200_feature *const *features, in
     for (int i = 0; i < n_features; ++i) {
         dist_b200_feature *f = features[i];
         if (!f || f->ctx != ctx || (phase != kRowsMerge && !columns_dev[i])) return fail(ctx, DIST_B200_ERR_INVALID, "add_rows: bad feature / column");
-        if (f->G < 1 || !(f->model == DIST_B200_NIW ? f->niw_stats : f->stats)) return fail(ctx, DIST_B200_ERR_STATE, "add_rows: call update_all first");
+        if (f->G < 1 || !stats_resident(f)) return fail(ctx, DIST_B200_ERR_STATE, "add_rows: call update_all first");
         if (pooled_model(f->model)) {
             acc_need = std::max(acc_need, add_rows_acc_bytes(f->G) * std::min(n_features, kAddBatch));
             ++n_pooled;
@@ -863,20 +549,11 @@ static int rows_batch(dist_b200_ctx *ctx, dist_b200_feature *const *features, in
     acc_need += table_tmp + niw_tmp;
     // exchange layout: the pooled features' [4][G] blocks first (list order), then the count tables (list order)
     size_t table_off = phase == kRowsBoth ? 0 : static_cast<size_t>(n_pooled) * 4 * features[0]->G;
-    if (acc_need > ctx->add_acc_bytes) {
-        if (ctx->add_acc) {
-            DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-            DISTB200_CUDA(ctx, cudaFree(ctx->add_acc));
-            ctx->add_acc = nullptr;
-            ctx->add_acc_bytes = 0;
-        }
-        DISTB200_CUDA(ctx, cudaMalloc(&ctx->add_acc, acc_need));
-        ctx->add_acc_bytes = acc_need;
-    }
+    int rc = grow(ctx, ctx->add_acc, ctx->add_acc_bytes, acc_need);
+    if (rc) return rc;
     if (!ctx->add_done) DISTB200_CUDA(ctx, cudaEventCreateWithFlags(&ctx->add_done, cudaEventDisableTiming));
     DISTB200_CUDA(ctx, cudaStreamWaitEvent(s, ctx->add_done, 0));  // the previous batch may have run on another stream
-    int rc = wait_ready(ctx, features, n_features, s);
-    if (rc) return rc;
+    if ((rc = wait_ready(ctx, features, n_features, s))) return rc;
 
     AddBatch b{};
     b.sign = sign;
@@ -910,7 +587,7 @@ static int rows_batch(dist_b200_ctx *ctx, dist_b200_feature *const *features, in
             r = launch_add_rows_counts(ctx, f, columns_dev[i], assign_dev, n_rows, +1, s, tmp);
             if (!r) r = launch_counts_to_doubles(ctx, tmp, xchg + table_off, cells, s);
         } else {
-            r = launch_merge_counts(ctx, reinterpret_cast<int32_t *>(f->stats), xchg + table_off, cells, sign, s);
+            r = launch_merge_counts(ctx, reinterpret_cast<int32_t *>(f->stats[0]), xchg + table_off, cells, sign, s);
         }
         table_off += cells;
         return r;
@@ -928,9 +605,9 @@ static int rows_batch(dist_b200_ctx *ctx, dist_b200_feature *const *features, in
                 b.G = G;
                 AddDesc &d = b.d[b.n++];
                 d.column = columns_dev ? columns_dev[i] : nullptr;
-                d.st0 = stat_ptr(f, 0);
-                d.st1 = stat_ptr(f, 1);
-                d.st2 = f->model == DIST_B200_NICH ? stat_ptr(f, 2) : nullptr;
+                d.st0 = f->stats[0];
+                d.st1 = f->stats[1];
+                d.st2 = f->stats[2];
                 d.params = static_cast<float4 *>(f->params);
                 d.aux = f->aux;
                 for (int k = 0; k < 4; ++k) d.shared[k] = f->shared[k];
@@ -941,30 +618,24 @@ static int rows_batch(dist_b200_ctx *ctx, dist_b200_feature *const *features, in
                 }
             } break;
             case DIST_B200_DD:
-                if (!f->alphas_dev) return fail(ctx, DIST_B200_ERR_STATE, "add_rows: dd alphas not resident (update_all first)");
-                if ((rc = table_counts(f, i))) return rc;
-                if (phase == kRowsAccumulate) break;
-                if ((rc = launch_dd_prep(ctx, f->dim, f->alphas_dev, f->alpha_sum, 0, G, reinterpret_cast<const int32_t *>(stat_ptr(f, 0)),
-                                         static_cast<float *>(f->params), s)))
-                    return rc;
-                break;
             case DIST_B200_DPD:
                 if ((rc = table_counts(f, i))) return rc;
                 if (phase == kRowsAccumulate) break;
-                if ((rc = dpd_rebuild(f, reinterpret_cast<const float *>(dpd_betas(f)), reinterpret_cast<const int32_t *>(f->stats), s)))
-                    return rc;
+                if ((rc = rebuild(f, 0, G, s))) return rc;
                 break;
             case DIST_B200_NIW: {  // per-group SYRK into a [G][1 + d + d^2] double block (niw_stats.cu), then the records again
                 const int d = f->dim;
-                const size_t per = 1 + static_cast<size_t>(d) + static_cast<size_t>(d) * d;
+                const size_t per = group_words(f);
                 char *area = static_cast<char *>(ctx->add_acc) + pooled_bytes + table_tmp;
                 double *acc = phase == kRowsBoth ? reinterpret_cast<double *>(area) : xchg + table_off;
                 void *work = area + round_up(sizeof(double) * G * per, 256);
                 if (phase != kRowsMerge && (rc = launch_niw_accumulate(ctx, G, d, columns_dev[i], assign_dev, n_rows, acc, work, s))) return rc;
                 table_off += G * per;
                 if (phase == kRowsAccumulate) break;
-                if ((rc = launch_niw_apply(ctx, G, d, sign, acc, niw_count(f), niw_sum_x(f), niw_sum_xxT(f), s))) return rc;
-                if ((rc = niw_rebuild(f, 0, G, s))) return rc;
+                if ((rc = launch_niw_apply(ctx, G, d, sign, acc, reinterpret_cast<int32_t *>(f->stats[0]), reinterpret_cast<float *>(f->stats[1]),
+                                           reinterpret_cast<float *>(f->stats[2]), s)))
+                    return rc;
+                if ((rc = rebuild(f, 0, G, s))) return rc;
             } break;
             default: return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "add_rows: unsupported model");
         }
@@ -991,9 +662,7 @@ int dist_b200_rows_xchg_doubles(dist_b200_feature *const *features, int n_featur
     for (int i = 0; i < n_features; ++i) {
         const dist_b200_feature *f = features[i];
         if (!f) return DIST_B200_ERR_INVALID;
-        n += pooled_model(f->model) ? static_cast<size_t>(4) * f->G
-             : f->model == DIST_B200_NIW ? static_cast<size_t>(f->G) * (1 + f->dim + static_cast<size_t>(f->dim) * f->dim)
-                                         : static_cast<size_t>(f->G) * f->dim;
+        n += static_cast<size_t>(f->G) * (pooled_model(f->model) ? 4 : group_words(f));
     }
     *n_doubles = n;
     return DIST_B200_OK;
@@ -1069,10 +738,7 @@ static int check_sample_args(dist_b200_ctx *ctx, dist_b200_feature *const *featu
     for (int i = 0; i < n_features; ++i) {
         const dist_b200_feature *f = features[i];
         if (!f || f->ctx != ctx || !columns_out[i]) return fail(ctx, DIST_B200_ERR_INVALID, "sample_values: bad feature / output column");
-        const bool resident = f->model == DIST_B200_NIW ? f->niw_stats != nullptr
-                              : f->model == DIST_B200_DD ? f->stats && f->alphas_dev
-                              : f->model == DIST_B200_DPD ? f->stats && f->keys_dev : f->stats != nullptr;
-        if (f->G < 1 || !resident) return fail(ctx, DIST_B200_ERR_STATE, "sample_values: call update_all first");
+        if (f->G < 1 || !stats_resident(f)) return fail(ctx, DIST_B200_ERR_STATE, "sample_values: call update_all first");
         if (f->G != features[0]->G) return fail(ctx, DIST_B200_ERR_STATE, "sample_values: features disagree on the number of groups");
     }
     return DIST_B200_OK;
@@ -1084,32 +750,12 @@ static SampleSrc sample_src(const dist_b200_feature *f) {
     src.G = f->G;
     src.dim = f->dim;
     for (int k = 0; k < 4; ++k) src.shared[k] = f->shared[k];
-    switch (f->model) {
-        case DIST_B200_DD:
-            src.st0 = stat_ptr(f, 0);
-            src.alphas = f->alphas_dev;
-            break;
-        case DIST_B200_DPD:
-            src.shared[0] = f->alpha;
-            src.shared[1] = f->beta0;
-            src.st0 = f->stats;
-            src.alphas = reinterpret_cast<const float *>(dpd_betas(f));
-            src.keys_sorted = f->keys_dev;
-            src.key_rows = f->key_rows_dev;
-            break;
-        case DIST_B200_NIW:
-            src.shared[0] = f->kappa;
-            src.shared[1] = f->nu;
-            src.st0 = f->niw_stats;
-            src.st1 = reinterpret_cast<const uint32_t *>(niw_sum_x(f));
-            src.st2 = reinterpret_cast<const uint32_t *>(niw_sum_xxT(f));
-            src.alphas = f->niw_shared_dev;
-            break;
-        default:
-            src.st0 = stat_ptr(f, 0);
-            src.st1 = stat_ptr(f, 1);
-            src.st2 = f->model == DIST_B200_NICH ? stat_ptr(f, 2) : nullptr;
-    }
+    src.st0 = f->stats[0];
+    src.st1 = f->stats[1];
+    src.st2 = f->stats[2];
+    src.alphas = f->alphas_dev;
+    src.keys_sorted = f->keys_dev;
+    src.key_rows = f->key_rows_dev;
     return src;
 }
 
@@ -1184,15 +830,7 @@ int dist_b200_gp_set_log_prod(dist_b200_feature *f, const float *log_prod_host, 
     if (!check_feature(f, DIST_B200_GP) || !log_prod_host) return DIST_B200_ERR_INVALID;
     dist_b200_ctx *ctx = f->ctx;
     if (f->G < 1) return fail(ctx, DIST_B200_ERR_STATE, "gp_set_log_prod: call update_all first");
-    if (f->log_prod_dev && f->log_prod_cap < f->capacity) {
-        DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-        DISTB200_CUDA(ctx, cudaFree(f->log_prod_dev));
-        f->log_prod_dev = nullptr;
-    }
-    if (!f->log_prod_dev) {
-        DISTB200_CUDA(ctx, cudaMalloc(&f->log_prod_dev, sizeof(float) * f->capacity));
-        f->log_prod_cap = f->capacity;
-    }
+    if (int rc = grow(ctx, f->log_prod_dev, f->log_prod_bytes, sizeof(float) * f->capacity)) return rc;
     cudaStream_t s = as_stream(stream);
     DISTB200_CUDA(ctx, cudaMemcpyAsync(f->log_prod_dev, log_prod_host, sizeof(float) * f->G, cudaMemcpyHostToDevice, s));
     DISTB200_CUDA(ctx, cudaStreamSynchronize(s));  // pageable source
@@ -1205,7 +843,7 @@ int dist_b200_score_data_grid(dist_b200_feature *f, const float *shareds_dev, si
     if (!f || !f->ctx) return DIST_B200_ERR_INVALID;
     dist_b200_ctx *ctx = f->ctx;
     if (!shareds_dev || !out_dev) return fail(ctx, DIST_B200_ERR_INVALID, "score_data_grid: null argument");
-    if (f->G < 1 || !(f->model == DIST_B200_NIW ? f->niw_stats : f->stats)) return fail(ctx, DIST_B200_ERR_STATE, "score_data_grid: call update_all first");
+    if (f->G < 1 || !stats_resident(f)) return fail(ctx, DIST_B200_ERR_STATE, "score_data_grid: call update_all first");
     if (stride < shared_stride(f)) return fail(ctx, DIST_B200_ERR_INVALID, "score_data_grid: stride shorter than the model's packed Shared");
     if (f->model == DIST_B200_GP && !f->log_prod_valid)
         return fail(ctx, DIST_B200_ERR_STATE, "score_data_grid: gp needs Group::log_prod (dist_b200_gp_set_log_prod) after the last statistics change");
@@ -1213,40 +851,20 @@ int dist_b200_score_data_grid(dist_b200_feature *f, const float *shareds_dev, si
     cudaStream_t s = as_stream(stream);
     DISTB200_CUDA(ctx, cudaStreamWaitEvent(s, f->ready, 0));
     // the double accumulators live next to the add_value accumulators (same event guards both)
-    const size_t need = sizeof(double) * n_grid;
-    if (need > ctx->add_acc_bytes) {
-        if (ctx->add_acc) {
-            DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-            DISTB200_CUDA(ctx, cudaFree(ctx->add_acc));
-            ctx->add_acc = nullptr;
-            ctx->add_acc_bytes = 0;
-        }
-        DISTB200_CUDA(ctx, cudaMalloc(&ctx->add_acc, need));
-        ctx->add_acc_bytes = need;
-    }
+    int rc = grow(ctx, ctx->add_acc, ctx->add_acc_bytes, sizeof(double) * n_grid);
+    if (rc) return rc;
     if (!ctx->add_done) DISTB200_CUDA(ctx, cudaEventCreateWithFlags(&ctx->add_done, cudaEventDisableTiming));
     DISTB200_CUDA(ctx, cudaStreamWaitEvent(s, ctx->add_done, 0));
+    double *acc = static_cast<double *>(ctx->add_acc);
     if (f->model == DIST_B200_NIW) {
-        DISTB200_CUDA(ctx, cudaMemsetAsync(ctx->add_acc, 0, sizeof(double) * n_grid, s));
-        int rcn = launch_niw_score_data(ctx, f->G, f->dim, niw_count(f), niw_sum_x(f), niw_sum_xxT(f), shareds_dev, n_grid, stride,
-                                        static_cast<double *>(ctx->add_acc), s);
-        if (!rcn) rcn = launch_score_data_finish(ctx, n_grid, static_cast<const double *>(ctx->add_acc), out_dev, s);
-        if (rcn) return rcn;
-        DISTB200_CUDA(ctx, cudaEventRecord(ctx->add_done, s));
-        return DIST_B200_OK;
-    }
-    const uint32_t *st0, *st1 = nullptr, *st2 = nullptr;
-    const float *betas = nullptr;
-    if (f->model == DIST_B200_DPD) {
-        st0 = f->stats;
-        betas = reinterpret_cast<const float *>(dpd_betas(f));
+        DISTB200_CUDA(ctx, cudaMemsetAsync(acc, 0, sizeof(double) * n_grid, s));
+        rc = launch_niw_score_data(ctx, f->G, f->dim, reinterpret_cast<const int32_t *>(f->stats[0]), reinterpret_cast<const float *>(f->stats[1]),
+                                   reinterpret_cast<const float *>(f->stats[2]), shareds_dev, n_grid, stride, acc, s);
+        if (!rc) rc = launch_score_data_finish(ctx, n_grid, acc, out_dev, s);
     } else {
-        st0 = stat_ptr(f, 0);
-        if (stat_arrays(f) > 1) st1 = stat_ptr(f, 1);
-        if (stat_arrays(f) > 2) st2 = stat_ptr(f, 2);
+        rc = launch_score_data(ctx, f, f->stats[0], f->stats[1], f->stats[2], f->alphas_dev, f->log_prod_dev, shareds_dev, n_grid, stride,
+                               acc, out_dev, s);
     }
-    int rc = launch_score_data(ctx, f, st0, st1, st2, betas, f->log_prod_dev, shareds_dev, n_grid, stride,
-                               static_cast<double *>(ctx->add_acc), out_dev, s);
     if (rc) return rc;
     DISTB200_CUDA(ctx, cudaEventRecord(ctx->add_done, s));
     return DIST_B200_OK;
@@ -1415,17 +1033,9 @@ int dist_b200_feature_dump_groups_wire(dist_b200_feature *f, void *out, size_t c
                                        void *stream) {
     if (!f || !f->ctx) return DIST_B200_ERR_INVALID;
     dist_b200_ctx *ctx = f->ctx;
-    if (!(f->model == DIST_B200_NIW ? f->niw_stats : f->stats) || f->G < 1)
-        return fail(ctx, DIST_B200_ERR_STATE, "dump_groups_wire: no device statistics (update_all first)");
+    if (!stats_resident(f) || f->G < 1) return fail(ctx, DIST_B200_ERR_STATE, "dump_groups_wire: no device statistics (update_all first)");
     const size_t g = static_cast<size_t>(f->G);
-    size_t words;
-    switch (f->model) {
-        case DIST_B200_NICH: case DIST_B200_GP: words = 3 * g; break;
-        case DIST_B200_BNB: case DIST_B200_BB: words = 2 * g; break;
-        case DIST_B200_DD: case DIST_B200_DPD: words = g * f->dim; break;
-        case DIST_B200_NIW: words = g * (1 + f->dim + static_cast<size_t>(f->dim) * f->dim); break;
-        default: return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "dump_groups_wire: unsupported model");
-    }
+    const size_t words = g * (group_words(f) + (f->model == DIST_B200_GP ? 1 : 0));  // gp: + Group::log_prod
     std::vector<uint32_t> st(words, 0);
     size_t got = 0;
     int rc = dist_b200_feature_download_stats(f, st.data(), 4 * words, &got, stream);  // synchronises
@@ -1450,35 +1060,17 @@ int dist_b200_feature_download_stats(const dist_b200_feature *f, void *out_host,
                                      void *stream) {
     if (!f || !f->ctx || !out_host) return DIST_B200_ERR_INVALID;
     dist_b200_ctx *ctx = f->ctx;
-    if (!(f->model == DIST_B200_NIW ? f->niw_stats : f->stats))
-        return fail(ctx, DIST_B200_ERR_STATE, "download_stats: no device statistics (update_all first)");
+    if (!stats_resident(f)) return fail(ctx, DIST_B200_ERR_STATE, "download_stats: no device statistics (update_all first)");
+    const size_t total = 4 * group_words(f) * f->G;
+    if (n_bytes) *n_bytes = total;
+    if (total > capacity_bytes) return fail(ctx, DIST_B200_ERR_INVALID, "download_stats: buffer too small");
     cudaStream_t s = as_stream(stream);
     DISTB200_CUDA(ctx, cudaStreamWaitEvent(s, f->ready, 0));
     char *out = static_cast<char *>(out_host);
-    size_t total = 0;
-    if (f->model == DIST_B200_NIW) {  // count[G] | sum_x[G][d] | sum_xxT[G][d][d]
-        const size_t g = static_cast<size_t>(f->G), d = static_cast<size_t>(f->dim);
-        total = 4 * g * (1 + d + d * d);
-        if (n_bytes) *n_bytes = total;
-        if (total > capacity_bytes) return fail(ctx, DIST_B200_ERR_INVALID, "download_stats: buffer too small");
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(out, niw_count(f), 4 * g, cudaMemcpyDeviceToHost, s));
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(out + 4 * g, niw_sum_x(f), 4 * g * d, cudaMemcpyDeviceToHost, s));
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(out + 4 * g * (1 + d), niw_sum_xxT(f), 4 * g * d * d, cudaMemcpyDeviceToHost, s));
-    } else if (f->model == DIST_B200_DPD) {
-        total = sizeof(int32_t) * static_cast<size_t>(f->G) * f->dim;
-        if (n_bytes) *n_bytes = total;
-        if (total > capacity_bytes) return fail(ctx, DIST_B200_ERR_INVALID, "download_stats: buffer too small");
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(out, f->stats, total, cudaMemcpyDeviceToHost, s));
-    } else {
-        for (int a = 0; a < stat_arrays(f); ++a) total += stat_elems(f, a) * f->G * 4;
-        if (n_bytes) *n_bytes = total;
-        if (total > capacity_bytes) return fail(ctx, DIST_B200_ERR_INVALID, "download_stats: buffer too small");
-        size_t off = 0;
-        for (int a = 0; a < stat_arrays(f); ++a) {
-            const size_t b = stat_elems(f, a) * f->G * 4;
-            DISTB200_CUDA(ctx, cudaMemcpyAsync(out + off, stat_ptr(f, a), b, cudaMemcpyDeviceToHost, s));
-            off += b;
-        }
+    for (int a = 0; a < stat_arrays(f); ++a) {
+        const size_t b = 4 * stat_elems(f, a) * f->G;
+        DISTB200_CUDA(ctx, cudaMemcpyAsync(out, f->stats[a], b, cudaMemcpyDeviceToHost, s));
+        out += b;
     }
     DISTB200_CUDA(ctx, cudaStreamSynchronize(s));
     return DIST_B200_OK;
@@ -1594,6 +1186,9 @@ static int queue_gp_table(dist_b200_ctx *ctx, dist_b200_feature *f, GpTableBatch
     return DIST_B200_OK;
 }
 
+// the GammaPoisson value table: [capacity][x] | [x][capacity]
+static size_t gp_table_bytes(const dist_b200_feature *f) { return sizeof(float) * 2 * kGpTableX * f->capacity; }
+
 // stale tables are queued in `tb`; the caller launches the remainder before the score kernel
 static int fill_desc(dist_b200_ctx *ctx, const dist_b200_feature *cf, const void *column, bool multi, FeatDesc &d,
                      GpTableBatch &tb, cudaStream_t s) {
@@ -1606,14 +1201,8 @@ static int fill_desc(dist_b200_ctx *ctx, const dist_b200_feature *cf, const void
     d.cap = f->capacity;
     d.pad_ = 0;
     if (multi && f->model == DIST_B200_GP) {
-        if (f->gp_table_cap < f->capacity) {
-            if (f->gp_table) {
-                DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-                DISTB200_CUDA(ctx, cudaFree(f->gp_table));
-                f->gp_table = nullptr;
-            }
-            DISTB200_CUDA(ctx, cudaMalloc(&f->gp_table, sizeof(float) * 2 * kGpTableX * f->capacity));  // [capacity][x] | [x][capacity]
-            f->gp_table_cap = f->capacity;
+        if (gp_table_bytes(f) > f->gp_table_bytes) {
+            if (int rc = grow(ctx, f->gp_table, f->gp_table_bytes, gp_table_bytes(f))) return rc;
             f->gp_table_dirty = true;
         }
         if (f->gp_table_dirty) {
@@ -1638,7 +1227,7 @@ static int refresh_gp_tables(dist_b200_ctx *ctx, const dist_b200_feature *const 
     bool any = false;
     for (int f = 0; f < F; ++f) {
         if (!features[f] || features[f]->model != DIST_B200_GP) continue;
-        const bool stale = features[f]->gp_table_dirty || features[f]->gp_table_cap < features[f]->capacity;
+        const bool stale = features[f]->gp_table_dirty || features[f]->gp_table_bytes < gp_table_bytes(features[f]);
         int rc = fill_desc(ctx, features[f], nullptr, true, scratch_desc, tb, s);
         if (rc) return rc;
         any = any || stale;
@@ -1684,18 +1273,8 @@ static int score_dispatch(dist_b200_ctx *ctx, const dist_b200_feature *const *fe
         (features[0]->model == DIST_B200_DPD || features[0]->model == DIST_B200_DD || features[0]->model == DIST_B200_BB)) {
         dist_b200_feature *f = const_cast<dist_b200_feature *>(features[0]);
         const int R = f->model == DIST_B200_DPD ? f->dim + 1 : (f->model == DIST_B200_DD ? f->dim : 2);
-        const size_t need = value_cdf_floats(R, G);
-        if (need > f->cdf_floats) {
-            if (f->cdf_buf) {
-                DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-                DISTB200_CUDA(ctx, cudaFree(f->cdf_buf));
-                f->cdf_buf = nullptr;
-                f->cdf_floats = 0;
-            }
-            DISTB200_CUDA(ctx, cudaMalloc(&f->cdf_buf, need * sizeof(float)));
-            f->cdf_floats = need;
-        }
-        const int rc = launch_value_cdf(ctx, f, f->cdf_buf, columns[0], N, prior, u, assign, s);
+        int rc = grow(ctx, f->cdf_buf, f->cdf_bytes, sizeof(float) * value_cdf_floats(R, G));
+        if (!rc) rc = launch_value_cdf(ctx, f, f->cdf_buf, columns[0], N, prior, u, assign, s);
         if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;
     }
     if (n_solo == 0) {
@@ -1730,8 +1309,7 @@ static int score_dispatch(dist_b200_ctx *ctx, const dist_b200_feature *const *fe
     }
     float *buf = scores;
     if (!buf) {
-        int rc = ensure_scores_scratch(ctx, sizeof(float) * N * G);
-        if (rc) return rc;
+        if (int rc = grow(ctx, ctx->scores_scratch, ctx->scores_scratch_bytes, sizeof(float) * N * G)) return rc;
         buf = static_cast<float *>(ctx->scores_scratch);
     }
     FeatList fl;

@@ -89,7 +89,7 @@ struct dist_b200_ctx {
     void *xpack = nullptr;            // niw tensor path: rows packed into A-operand images
     size_t xpack_bytes = 0;
     float *bbt = nullptr;             // kSub cross-cat kernel: compact [heads | tails] rows of the list's BetaBernoulli features
-    size_t bbt_floats = 0;
+    size_t bbt_bytes = 0;
     void *scores_scratch = nullptr;   // [N][G] buffer of the materialising dispatch paths
     size_t scores_scratch_bytes = 0;
     cudaStream_t own_stream = nullptr, own_stream2 = nullptr;
@@ -104,51 +104,50 @@ struct dist_b200_feature {
     dist_b200_ctx *ctx = nullptr;
     int model = 0;
     int G = 0;          // packed group count
-    int capacity = 0;   // allocated groups
+    int capacity = 0;   // groups allocated in the hot caches (params, aux, gp_table, log_prod_dev)
     int dim = 0;        // dd: dim, dpd: V, niw: d
-    // hyper-parameters of the last update_all (needed by update_group / add_group)
+    // scalar hyper-parameters of the last update_all (needed by update_group / add_group): nich mu kappa sigmasq nu;
+    // gp alpha inv_beta; bnb alpha beta r; bb alpha beta; dpd alpha beta0; niw kappa nu
     float shared[4] = {0, 0, 0, 0};
-    std::vector<float> alphas;        // dd alphas / dpd betas
+    std::vector<float> alphas;        // host copy of alphas_dev
     std::vector<uint32_t> keys;       // dpd keys as given to update_all (the order of the counts columns)
     bool keys_dense = false;          // dpd: keys == 0..V-1
-    float alpha = 0, beta0 = 0;       // dpd
     float alpha_sum = 0;              // dd
     // device buffers
     void *params = nullptr;           // hot layout (see FeatDesc::params)
     size_t params_bytes = 0;
     float *aux = nullptr;             // nich: unscaled log_coeff_ per group (capacity floats)
+    size_t aux_bytes = 0;
     float *gp_table = nullptr;        // gp: [capacity][kGpTableX] tabulated terms for values < kGpTableX
-    int gp_table_cap = 0;
+    size_t gp_table_bytes = 0;
     bool gp_table_dirty = true;
     cudaEvent_t ready = nullptr;      // recorded after every cache mutation; scoring streams wait on it
-    // device-resident raw group statistics (mirror of the host Groups; the state that batched
-    // add_value updates in place): arrays of `capacity` groups, 4-byte elements
-    //   nich: count | mean | count_times_variance     gp: count | sum     bb: heads | tails
-    //   dd: counts[capacity][dim]                      dpd: counts[G][V] | betas[V]
-    uint32_t *stats = nullptr;
-    size_t stats_words = 0;
-    float *alphas_dev = nullptr;      // dd: alphas, resident for device-side cache rebuilds
+    // device-resident raw group statistics (mirror of the host Groups; the state that batched add_value updates in
+    // place): stat_arrays arrays in update_all's argument order, each holding stats_cap groups of stat_elems 4-byte
+    // elements
+    //   nich: count | mean | count_times_variance     gp, bnb: count | sum     bb: heads | tails
+    //   dd: counts[dim]     dpd: counts[V]     niw: count | sum_x[d] | sum_xxT[d][d]
+    uint32_t *stats[3] = {nullptr, nullptr, nullptr};
+    size_t stats_bytes[3] = {0, 0, 0};
+    int stats_cap = 0;
+    float *alphas_dev = nullptr;      // the Shared vector: dd alphas, dpd betas, niw mu[d] | psi[d][d]
+    size_t alphas_bytes = 0;
     float *log_prod_dev = nullptr;    // gp: Group::log_prod per group (read by score_data only)
-    int log_prod_cap = 0;
+    size_t log_prod_bytes = 0;
     bool log_prod_valid = false;      // cleared by every statistics mutation that does not maintain it
     float *dpd_hot = nullptr;         // dpd: per-call scratch of table_rows.cu (the table with prior / row max folded in)
-    size_t dpd_hot_floats = 0;
+    size_t dpd_hot_bytes = 0;
     float *cdf_buf = nullptr;         // dpd / dd / bb: per-value CDF trees (rebuilt per scoring call: they carry the prior)
-    size_t cdf_floats = 0;
+    size_t cdf_bytes = 0;
     uint32_t *keys_dev = nullptr;     // dpd sorted keys
+    size_t keys_bytes = 0;
     int *key_rows_dev = nullptr;      // dpd: table row of sorted key i
+    size_t key_rows_bytes = 0;
     // niw
-    float *niw_buf = nullptr;
+    float *niw_buf = nullptr;         // per-group records (posterior, whitening matrix, constants)
     size_t niw_bytes = 0;
     float *niw_tc = nullptr;          // d = 32: tensor-core operand images, b vectors, constants
     size_t niw_tc_bytes = 0;
-    float kappa = 0, nu = 0;
-    std::vector<float> mu, psi;
-    // niw: device-resident raw statistics over niw_cap groups (the state batched add_value updates in place):
-    // count[niw_cap] | sum_x[niw_cap][d] | sum_xxT[niw_cap][d][d]; and the Shared's mu[d] | psi[d][d]
-    uint32_t *niw_stats = nullptr;
-    int niw_cap = 0;
-    float *niw_shared_dev = nullptr;
     void *sample_buf = nullptr;       // sample_values: per-group records of the prep pass (sample_values.cu)
     size_t sample_bytes = 0;
 };
@@ -167,6 +166,30 @@ inline int fail(dist_b200_ctx *ctx, int code, const std::string &msg) {
             return ::distb200::fail((ctx), DIST_B200_ERR_CUDA,                                     \
                                     std::string(#call) + ": " + cudaGetErrorString(e__));          \
     } while (0)
+
+// Grow-only device buffer: when `bytes` exceeds the allocation `have`, `buf` is replaced by an allocation of `bytes`.
+// The first `keep` bytes of the old contents move over, and with `zero` the rest is zero-filled.  The device is
+// synchronised before the old buffer is freed: kernels on any stream may still read it.
+template <class T>
+int grow(dist_b200_ctx *ctx, T *&buf, size_t &have, size_t bytes, size_t keep = 0, bool zero = false) {
+    if (bytes <= have) return DIST_B200_OK;
+    if (buf) DISTB200_CUDA(ctx, cudaDeviceSynchronize());
+    if (buf && !keep) {  // freed first: the peak use stays one buffer
+        DISTB200_CUDA(ctx, cudaFree(buf));
+        buf = nullptr;
+        have = 0;
+    }
+    void *fresh = nullptr;
+    DISTB200_CUDA(ctx, cudaMalloc(&fresh, bytes));
+    if (zero) DISTB200_CUDA(ctx, cudaMemset(static_cast<char *>(fresh) + keep, 0, bytes - keep));
+    if (buf) DISTB200_CUDA(ctx, cudaMemcpy(fresh, buf, keep, cudaMemcpyDeviceToDevice));
+    // the fill and the copy run on the legacy stream: they complete before any stream uses the buffer
+    if (buf || zero) DISTB200_CUDA(ctx, cudaDeviceSynchronize());
+    if (buf) DISTB200_CUDA(ctx, cudaFree(buf));
+    buf = static_cast<T *>(fresh);
+    have = bytes;
+    return DIST_B200_OK;
+}
 
 // ---- kernel launchers implemented in the .cu files --------------------------------------------
 // prep.cu
@@ -257,8 +280,8 @@ struct SampleSrc {
     int model, G, dim;                // dim: dd dim / dpd V / niw d
     float shared[4];                  // nich mu kappa sigmasq nu; gp alpha inv_beta; bnb alpha beta r; bb alpha beta;
                                       // dpd alpha beta0; niw kappa nu
-    const uint32_t *st0, *st1, *st2;  // statistics arrays (see dist_b200_feature::stats); niw count | sum_x | sum_xxT
-    const float *alphas;              // dd alphas; dpd betas; niw mu[d] | psi[d][d]
+    const uint32_t *st0, *st1, *st2;  // statistics arrays (see dist_b200_feature::stats)
+    const float *alphas;              // dist_b200_feature::alphas_dev
     const uint32_t *keys_sorted;      // dpd: dist_b200_feature::keys_dev / key_rows_dev
     const int *key_rows;
 };

@@ -638,17 +638,7 @@ int launch_niw_tc(dist_b200_ctx *ctx, int G, const float *tc_buf, const void *va
     const size_t sxbytes = (ntiles * sizeof(float) + 255) / 256 * 256;
     const size_t Gpad = static_cast<size_t>(nb) * kTcGroupsPerBlock;
     const size_t scratch_bytes = fused ? static_cast<size_t>(grid) * kChunkTiles * kTcRows * Gpad * sizeof(float) : 0;
-    const size_t need = xbytes + sxbytes + scratch_bytes;
-    if (need > ctx->xpack_bytes) {
-        if (ctx->xpack) {
-            DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-            DISTB200_CUDA(ctx, cudaFree(ctx->xpack));
-            ctx->xpack = nullptr;
-            ctx->xpack_bytes = 0;
-        }
-        DISTB200_CUDA(ctx, cudaMalloc(&ctx->xpack, need));
-        ctx->xpack_bytes = need;
-    }
+    if (int rc = grow(ctx, ctx->xpack, ctx->xpack_bytes, xbytes + sxbytes + scratch_bytes)) return rc;
     unsigned char *base = static_cast<unsigned char *>(ctx->xpack);
     NiwTcArgs a{};
     a.G = G;

@@ -341,17 +341,7 @@ static size_t sample_buf_bytes(const SampleSrc &src) {
 int launch_sample_values(dist_b200_ctx *ctx, dist_b200_feature *f, const SampleSrc &src, uint32_t position, const int32_t *assign,
                          size_t N, uint64_t seed, uint64_t row0, void *out, cudaStream_t s) {
     if (N == 0 || src.G <= 0) return DIST_B200_OK;
-    const size_t need = sample_buf_bytes(src);
-    if (need > f->sample_bytes) {
-        if (f->sample_buf) {
-            DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-            DISTB200_CUDA(ctx, cudaFree(f->sample_buf));
-            f->sample_buf = nullptr;
-            f->sample_bytes = 0;
-        }
-        DISTB200_CUDA(ctx, cudaMalloc(&f->sample_buf, need));
-        f->sample_bytes = need;
-    }
+    if (int rc = grow(ctx, f->sample_buf, f->sample_bytes, sample_buf_bytes(src))) return rc;
     char *buf = static_cast<char *>(f->sample_buf);
     SampleArgs a{};
     a.G = src.G;

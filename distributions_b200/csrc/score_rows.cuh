@@ -983,17 +983,7 @@ static int launch_tiers(dist_b200_ctx *ctx, const FeatList &feats, const RowsArg
             const int Gpad = (a.G + 127) / 128 * 128;  // <= every feature's capacity (ensure_params pads to 128 groups)
             int n_bb = 0;
             for (int f = 0; f < feats.n; ++f) n_bb += feats.f[f].kind == DIST_B200_BB ? 1 : 0;
-            const size_t need = static_cast<size_t>(n_bb) * 2 * Gpad;
-            if (need > ctx->bbt_floats) {
-                if (ctx->bbt) {
-                    DISTB200_CUDA(ctx, cudaDeviceSynchronize());
-                    DISTB200_CUDA(ctx, cudaFree(ctx->bbt));
-                    ctx->bbt = nullptr;
-                    ctx->bbt_floats = 0;
-                }
-                DISTB200_CUDA(ctx, cudaMalloc(&ctx->bbt, need * sizeof(float)));
-                ctx->bbt_floats = need;
-            }
+            if (int rc = grow(ctx, ctx->bbt, ctx->bbt_bytes, sizeof(float) * n_bb * 2 * Gpad)) return rc;
             FeatList local = feats;
             for (int f = 0, k = 0; f < local.n; ++f)
                 if (local.f[f].kind == DIST_B200_BB) {

@@ -301,7 +301,7 @@ int launch_add_rows_counts(dist_b200_ctx *ctx, dist_b200_feature *f, const void 
     a.N = N;
     a.column = column;
     a.assign = assign;
-    a.counts = dst ? dst : reinterpret_cast<int32_t *>(f->stats);  // dd: counts[G][dim]; dpd: counts[G][V]
+    a.counts = dst ? dst : reinterpret_cast<int32_t *>(f->stats[0]);  // dd: counts[G][dim]; dpd: counts[G][V]
     a.keys = f->keys_dev;
     a.key_rows = f->key_rows_dev;
     const size_t cells = static_cast<size_t>(f->G) * f->dim;
