@@ -73,6 +73,9 @@ SIGNATURES = {
     "dist_b200_score_batch": (c_i, [c_p, c_p, c_i, c_p, c_sz, c_p, c_p, c_i, c_p]),
     "dist_b200_score_sample_batch": (c_i, [c_p, c_p, c_i, c_p, c_sz, c_p, c_p, c_p, c_p, c_p]),
     "dist_b200_sample_from_scores": (c_i, [c_p, c_p, c_sz, c_i, c_p, c_p, c_p]),
+    "dist_b200_score_logp_batch": (c_i, [c_p, c_p, c_i, c_p, c_sz, c_p, c_p, c_p]),
+    "dist_b200_score_logp_batch_host": (c_i, [c_p, c_p, c_i, c_p, c_sz, c_p, c_p]),
+    "dist_b200_logp_from_scores": (c_i, [c_p, c_p, c_sz, c_i, c_p, c_p]),
     "dist_b200_peer_alloc": (c_i, [c_p, c_sz, ctypes.POINTER(c_p), c_p]),
     "dist_b200_peer_open": (c_i, [c_p, c_p, ctypes.POINTER(c_p)]),
     "dist_b200_peer_close": (c_i, [c_p, c_p]),
@@ -370,6 +373,16 @@ class Context:
         self.check(self.L.dist_b200_sample_from_scores(self.h, _dev_ptr(scores), n_rows, G, _dev_ptr(u), _dev_ptr(assign),
                                                        stream), "sample_from_scores")
 
+    def score_logp_batch(self, features, columns, n_rows, prior, logp, stream=None):
+        """logp[n] (device, float32) <- log sum_g exp(prior[g] + sum_f score_f(columns[f][n]; g)); prior may be None"""
+        F, fa, ca = self._lists(features, columns)
+        self.check(self.L.dist_b200_score_logp_batch(self.h, fa, F, ca, n_rows, _dev_ptr(prior), _dev_ptr(logp), stream),
+                   "score_logp_batch")
+
+    def logp_from_scores(self, scores, n_rows, G, logp, stream=None):
+        """logp[n] <- log sum_g exp(scores[n][g]) over materialised [n_rows][G] scores (device)"""
+        self.check(self.L.dist_b200_logp_from_scores(self.h, _dev_ptr(scores), n_rows, G, _dev_ptr(logp), stream), "logp_from_scores")
+
     # -- feature shards over peer memory ---------------------------------------------------------
     def peer_alloc(self, nbytes):
         """cudaMalloc a buffer and return (device pointer, 64-byte IPC handle)"""
@@ -427,6 +440,24 @@ class Context:
         self.check(self.L.dist_b200_score_sample_batch_host(self.h, fa, F, ca, n, _np_ptr(prior), _np_ptr(u), _np_ptr(assign),
                                                             _np_ptr(scores)), "score_sample_batch_host")
         return assign, scores
+
+    def score_logp_batch_host(self, features, columns, prior=None, logp_out=None):
+        """Host-buffer form of score_logp_batch: returns the float32 logp of every row.  Page-locked arrays (and a
+        page-locked `logp_out`) take the zero-copy route, as in score_sample_batch_host."""
+        F = len(features)
+        cols = [np.ascontiguousarray(c, dtype=COLUMN_DTYPE[f.model]) for f, c in zip(features, columns)]
+        f0 = features[0]
+        n = cols[0].shape[0] if f0.model == NIW and cols[0].ndim == 2 else cols[0].size // (f0.dim if f0.model == NIW else 1)
+        for f, c in zip(features, cols):
+            assert c.size == n * (f.dim if f.model == NIW else 1), "columns of different lengths"
+        fa = (c_p * F)(*[f.h for f in features])
+        ca = (c_p * F)(*[c.ctypes.data for c in cols])
+        prior = None if prior is None else np.ascontiguousarray(prior, dtype=np.float32)
+        logp = logp_out if logp_out is not None else np.empty(n, dtype=np.float32)
+        assert logp.dtype == np.float32 and logp.size == n and logp.flags.c_contiguous
+        self.check(self.L.dist_b200_score_logp_batch_host(self.h, fa, F, ca, n, _np_ptr(prior), _np_ptr(logp)),
+                   "score_logp_batch_host")
+        return logp
 
     def host_register(self, array):
         """page-lock a numpy array in place (once): later host-entry calls on it are zero-copy"""

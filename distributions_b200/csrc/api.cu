@@ -1240,11 +1240,12 @@ static int refresh_gp_tables(dist_b200_ctx *ctx, const dist_b200_feature *const 
     return DIST_B200_OK;
 }
 
+// logp != nullptr (assign = scores = nullptr): logp[n] = log sum_g exp(prior[g] + sum_f score_f) per row
 static int score_dispatch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int F,
                           const void *const *columns, size_t N, const float *prior, const float *u,
-                          int32_t *assign, float *scores, int accumulate, cudaStream_t s) {
+                          int32_t *assign, float *scores, int accumulate, cudaStream_t s, float *logp = nullptr) {
     if (!ctx || !features || !columns || F < 1) return DIST_B200_ERR_INVALID;
-    if (!assign && !scores) return fail(ctx, DIST_B200_ERR_INVALID, "score: no output requested");
+    if (!assign && !scores && !logp) return fail(ctx, DIST_B200_ERR_INVALID, "score: no output requested");
     if (assign && !u) return fail(ctx, DIST_B200_ERR_INVALID, "score_sample: u is required");
     if (accumulate && prior) return fail(ctx, DIST_B200_ERR_INVALID, "score: prior is an overwrite, not valid with accumulate");
     const int G = features[0] ? features[0]->G : 0;
@@ -1277,6 +1278,16 @@ static int score_dispatch(dist_b200_ctx *ctx, const dist_b200_feature *const *fe
         if (!rc) rc = launch_value_cdf(ctx, f, f->cdf_buf, columns[0], N, prior, u, assign, s);
         if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;
     }
+    // the logp form of the same shortcut: a table feature's log-normaliser is a function of the value alone, so it is one
+    // log-sum-exp per table row and a gather per data row (DIST_B200_OPT_VALUE_CDF = 1 keeps the per-cell kernels here too)
+    if (F == 1 && logp && ctx->opt[DIST_B200_OPT_VALUE_CDF] != 1 &&
+        (features[0]->model == DIST_B200_DPD || features[0]->model == DIST_B200_DD || features[0]->model == DIST_B200_BB)) {
+        dist_b200_feature *f = const_cast<dist_b200_feature *>(features[0]);
+        const int R = f->model == DIST_B200_DPD ? f->dim + 1 : (f->model == DIST_B200_DD ? f->dim : 2);
+        int rc = grow(ctx, f->cdf_buf, f->cdf_bytes, sizeof(float) * R);
+        if (!rc) rc = launch_value_logp(ctx, f, f->cdf_buf, columns[0], N, prior, logp, s);
+        if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;
+    }
     if (n_solo == 0) {
         if (F > kMaxFeatures) return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "score: more than 512 features in one call");
         FeatList fl;
@@ -1288,7 +1299,7 @@ static int score_dispatch(dist_b200_ctx *ctx, const dist_b200_feature *const *fe
             if (rc) return rc;
         }
         if (int rc = launch_gp_table_batch(ctx, tb, s)) return rc;
-        return launch_score_rows(ctx, fl, G, N, prior, u, assign, scores, accumulate, s);
+        return launch_score_rows(ctx, fl, G, N, prior, u, assign, scores, accumulate, s, nullptr, logp);
     }
     // one NIW<32> feature, sampling only: quadratic forms, scores and sample_from_scores in one tcgen05 kernel
     if (F == 1 && features[0]->model == DIST_B200_NIW && features[0]->dim == 32 && features[0]->niw_tc && assign && !scores &&
@@ -1300,7 +1311,8 @@ static int score_dispatch(dist_b200_ctx *ctx, const dist_b200_feature *const *fe
         const int rc = launch_niw_rows_small(ctx, features[0], columns[0], N, prior, u, assign, s);
         if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;
     }
-    if (F == 1 && features[0]->model == DIST_B200_DPD) {
+    // logp over dpd / niw (alone or in a mixed list): the scores are materialised and reduced by logp_scores_kernel
+    if (F == 1 && features[0]->model == DIST_B200_DPD && !logp) {
         if (assign && !scores && !accumulate && ctx->opt[DIST_B200_OPT_TABLE_KERNEL] != 1) {
             const int rc = launch_table_rows(ctx, features[0], columns[0], N, prior, u, assign, s);
             if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;
@@ -1340,6 +1352,7 @@ static int score_dispatch(dist_b200_ctx *ctx, const dist_b200_feature *const *fe
         started = true;
     }
     if (assign) return launch_sample_scores(ctx, buf, N, G, u, assign, s);
+    if (logp) return launch_logp_scores(ctx, buf, N, G, logp, s);
     return DIST_B200_OK;
 }
 
@@ -1357,6 +1370,21 @@ int dist_b200_score_sample_batch(dist_b200_ctx *ctx, const dist_b200_feature *co
     if (!assign_dev) return ctx ? fail(ctx, DIST_B200_ERR_INVALID, "score_sample_batch: assign_dev is null") : DIST_B200_ERR_INVALID;
     return score_dispatch(ctx, features, n_features, columns_dev, n_rows, prior_dev, u_dev, assign_dev, scores_dev, 0,
                           as_stream(stream));
+}
+
+int dist_b200_score_logp_batch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                               const void *const *columns_dev, size_t n_rows, const float *prior_dev, float *logp_dev,
+                               void *stream) {
+    if (!logp_dev) return ctx ? fail(ctx, DIST_B200_ERR_INVALID, "score_logp_batch: logp_dev is null") : DIST_B200_ERR_INVALID;
+    return score_dispatch(ctx, features, n_features, columns_dev, n_rows, prior_dev, nullptr, nullptr, nullptr, 0,
+                          as_stream(stream), logp_dev);
+}
+
+int dist_b200_logp_from_scores(dist_b200_ctx *ctx, const float *scores_dev, size_t n_rows, int G, float *logp_dev,
+                               void *stream) {
+    if (!ctx) return DIST_B200_ERR_INVALID;
+    if (!scores_dev || !logp_dev || G < 1) return fail(ctx, DIST_B200_ERR_INVALID, "logp_from_scores: null buffer or G < 1");
+    return launch_logp_scores(ctx, scores_dev, n_rows, G, logp_dev, as_stream(stream));
 }
 
 int dist_b200_sample_from_scores(dist_b200_ctx *ctx, const float *scores_dev, size_t n_rows, int G,
@@ -1449,17 +1477,18 @@ static size_t value_bytes(const dist_b200_feature *f) {
     }
 }
 
-int dist_b200_score_sample_batch_host(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int F,
-                                      const void *const *columns_host, size_t N, const float *prior_host,
-                                      const float *u_host, int32_t *assign_host, float *scores_host) {
-    if (!ctx || !features || !columns_host || F < 1 || F > kMaxFeatures || !u_host || !assign_host) return DIST_B200_ERR_INVALID;
+// The host-buffer form of score_dispatch.  Its per-row output is 4 bytes: the sampled group (u_host and assign_host given)
+// or the row's log-normaliser (logp_host given, no u).
+static int score_host(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int F, const void *const *columns_host, size_t N,
+                      const float *prior_host, const float *u_host, int32_t *assign_host, float *logp_host, float *scores_host) {
+    void *out_host = logp_host ? static_cast<void *>(logp_host) : static_cast<void *>(assign_host);
     for (int f = 0; f < F; ++f)
         if (!features[f] || !columns_host[f]) return fail(ctx, DIST_B200_ERR_INVALID, "score_sample_host: null feature / column");
     const int G = features[0]->G;
     if (G < 1) return fail(ctx, DIST_B200_ERR_STATE, "score_sample_host: no groups");
     if (N == 0) return DIST_B200_OK;
     // layout of the staging area (identical in pinned host memory and on the device):
-    //   columns | prior | u | assign | scores(optional, device only + host out)
+    //   columns | prior | u (sampling only) | per-row output | scores(optional, device only + host out)
     std::vector<size_t> col_off(F);
     size_t off = 0;
     for (int f = 0; f < F; ++f) {
@@ -1469,9 +1498,9 @@ int dist_b200_score_sample_batch_host(dist_b200_ctx *ctx, const dist_b200_featur
     const size_t prior_off = off;
     off += round_up(sizeof(float) * G, 256);
     const size_t u_off = off;
-    off += round_up(sizeof(float) * N, 256);
+    if (u_host) off += round_up(sizeof(float) * N, 256);
     const size_t in_bytes = off;
-    const size_t assign_off = off;
+    const size_t out_off = off;
     off += round_up(sizeof(int32_t) * N, 256);
     const size_t scores_off = off;
     if (scores_host) off += round_up(sizeof(float) * N * G, 256);
@@ -1493,8 +1522,15 @@ int dist_b200_score_sample_batch_host(dist_b200_ctx *ctx, const dist_b200_featur
     };
     std::vector<char> col_pinned(F);
     for (int f = 0; f < F; ++f) col_pinned[f] = is_pinned(columns_host[f]) ? 1 : 0;
-    const bool u_pinned = is_pinned(u_host), assign_pinned = is_pinned(assign_host);
+    const bool u_pinned = !u_host || is_pinned(u_host), out_pinned = is_pinned(out_host);
     const bool scores_pinned = scores_host && is_pinned(scores_host);
+
+    // per-row output of rows [lo, lo + n) at `out` (device / mapped), u of those rows at `uu`
+    auto dispatch = [&](const void *const *cols, size_t n, const float *pr, const float *uu, char *out, float *sc, cudaStream_t str) {
+        return score_dispatch(ctx, features, F, cols, n, pr, uu, logp_host ? nullptr : reinterpret_cast<int32_t *>(out), sc, 0, str,
+                              logp_host ? reinterpret_cast<float *>(out) : nullptr);
+    };
+    auto dev_u = [&](size_t lo) { return u_host ? reinterpret_cast<const float *>(dev + u_off) + lo : nullptr; };
 
     // Row chunks are pipelined over two streams: the H2D copy of chunk k+1 and the D2H copy of chunk
     // k-1 overlap the kernels of chunk k (rows are independent given frozen statistics).
@@ -1507,7 +1543,7 @@ int dist_b200_score_sample_batch_host(dist_b200_ctx *ctx, const dist_b200_featur
     // the math row tile by row tile with no chunking, no staging copies and no second stream.
     // DIST_B200_OPT_HOST_ZEROCOPY: 0 = when all buffers are page-locked, 1 = never, 2 = same as 0 (A/B runs).
     {
-        bool all_pinned = u_pinned && assign_pinned && !scores_host;
+        bool all_pinned = u_pinned && out_pinned && !scores_host;
         for (int f = 0; f < F; ++f) all_pinned = all_pinned && col_pinned[f];
         // niw keeps the staged path: its row images are built by a separate pack kernel, which would read the rows over
         // PCIe without any math to hide behind (measured: c5 e2e 6.1e10 staged vs 4.1e10 zero-copy)
@@ -1522,11 +1558,12 @@ int dist_b200_score_sample_batch_host(dist_b200_ctx *ctx, const dist_b200_featur
                 zc_cols[f] = dp;
             }
             const float *u_zc = nullptr;
-            int32_t *assign_zc = nullptr;
-            if (ok) ok = cudaHostGetDevicePointer(&dp, const_cast<float *>(u_host), 0) == cudaSuccess;
-            u_zc = static_cast<const float *>(dp);
-            if (ok) ok = cudaHostGetDevicePointer(&dp, assign_host, 0) == cudaSuccess;
-            assign_zc = static_cast<int32_t *>(dp);
+            if (ok && u_host) {
+                ok = cudaHostGetDevicePointer(&dp, const_cast<float *>(u_host), 0) == cudaSuccess;
+                u_zc = static_cast<const float *>(dp);
+            }
+            if (ok) ok = cudaHostGetDevicePointer(&dp, out_host, 0) == cudaSuccess;
+            char *out_zc = static_cast<char *>(dp);
             if (ok) {
                 const float *prior_zc = nullptr;
                 if (prior_host) {  // the prior vector is re-read per table row by the dpd / dd kernels: it goes to the device
@@ -1535,7 +1572,7 @@ int dist_b200_score_sample_batch_host(dist_b200_ctx *ctx, const dist_b200_featur
                         return fail(ctx, DIST_B200_ERR_CUDA, "score_sample_host: prior upload");
                     prior_zc = reinterpret_cast<const float *>(dev + prior_off);
                 }
-                rc = score_dispatch(ctx, features, F, zc_cols.data(), N, prior_zc, u_zc, assign_zc, nullptr, 0, st[0]);
+                rc = dispatch(zc_cols.data(), N, prior_zc, u_zc, out_zc, nullptr, st[0]);
                 cudaError_t e = cudaStreamSynchronize(st[0]);
                 if (rc) return rc;
                 if (e != cudaSuccess) return fail(ctx, DIST_B200_ERR_CUDA, std::string("score_sample_host: ") + cudaGetErrorString(e));
@@ -1556,11 +1593,12 @@ int dist_b200_score_sample_batch_host(dist_b200_ctx *ctx, const dist_b200_featur
     // five chunks measured best at 1M rows (DIST_B200_OPT_HOST_CHUNKS overrides it for A/B runs)
     const size_t max_chunks = ctx->opt[DIST_B200_OPT_HOST_CHUNKS] > 0 ? static_cast<size_t>(ctx->opt[DIST_B200_OPT_HOST_CHUNKS]) : 5;
     size_t nchunks = std::min<size_t>(max_chunks, std::max<size_t>(1, N / min_chunk));
-    // niw launches share the context's packed-row buffer and mixed dpd lists its single scores buffer: their kernels stay
-    // on ONE stream in chunk order; only the H2D copies of the later chunks run ahead on the second stream
+    // niw launches share the context's packed-row buffer and mixed dpd lists (and a dpd logp, which may materialise) its
+    // single scores buffer: their kernels stay on ONE stream in chunk order; only the H2D copies of the later chunks run
+    // ahead on the second stream
     bool one_compute_stream = false;
     for (int f = 0; f < F; ++f)
-        if (features[f]->model == DIST_B200_NIW || (features[f]->model == DIST_B200_DPD && F > 1)) one_compute_stream = true;
+        if (features[f]->model == DIST_B200_NIW || (features[f]->model == DIST_B200_DPD && (F > 1 || logp_host))) one_compute_stream = true;
     if (one_compute_stream && scores_host) nchunks = 1;
     // chunk boundaries: equal interior chunks, half-size first and last ones -- the first H2D copy and the
     // last D2H copy are the only transfers no kernel hides
@@ -1602,12 +1640,14 @@ int dist_b200_score_sample_batch_host(dist_b200_ctx *ctx, const dist_b200_featur
                 }
                 ce = cudaMemcpyAsync(dev + col_off[f] + vb * lo, src, vb * n, cudaMemcpyHostToDevice, st[1]);
             }
-            const char *src = reinterpret_cast<const char *>(u_host + lo);
-            if (!u_pinned) {
-                std::memcpy(pin + u_off + 4 * lo, src, 4 * n);
-                src = pin + u_off + 4 * lo;
+            if (u_host) {
+                const char *src = reinterpret_cast<const char *>(u_host + lo);
+                if (!u_pinned) {
+                    std::memcpy(pin + u_off + 4 * lo, src, 4 * n);
+                    src = pin + u_off + 4 * lo;
+                }
+                if (ce == cudaSuccess) ce = cudaMemcpyAsync(dev + u_off + 4 * lo, src, 4 * n, cudaMemcpyHostToDevice, st[1]);
             }
-            if (ce == cudaSuccess) ce = cudaMemcpyAsync(dev + u_off + 4 * lo, src, 4 * n, cudaMemcpyHostToDevice, st[1]);
             if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&ready[k], cudaEventDisableTiming);
             if (ce == cudaSuccess) ce = cudaEventRecord(ready[k], st[1]);
         }
@@ -1616,16 +1656,14 @@ int dist_b200_score_sample_batch_host(dist_b200_ctx *ctx, const dist_b200_featur
             if (n == 0) continue;
             ce = cudaStreamWaitEvent(st[0], ready[k], 0);
             for (int f = 0; f < F; ++f) cols[f] = dev + col_off[f] + value_bytes(features[f]) * lo;
-            if (ce == cudaSuccess)
-                rc = score_dispatch(ctx, features, F, cols.data(), n, prior_dev, reinterpret_cast<const float *>(dev + u_off) + lo,
-                                    reinterpret_cast<int32_t *>(dev + assign_off) + lo, nullptr, 0, st[0]);
+            if (ce == cudaSuccess) rc = dispatch(cols.data(), n, prior_dev, dev_u(lo), dev + out_off + 4 * lo, nullptr, st[0]);
         }
-        int32_t *adst = assign_pinned ? assign_host : reinterpret_cast<int32_t *>(pin + assign_off);
-        if (ce == cudaSuccess && rc == DIST_B200_OK) ce = cudaMemcpyAsync(adst, dev + assign_off, 4 * N, cudaMemcpyDeviceToHost, st[0]);
+        void *odst = out_pinned ? out_host : pin + out_off;
+        if (ce == cudaSuccess && rc == DIST_B200_OK) ce = cudaMemcpyAsync(odst, dev + out_off, 4 * N, cudaMemcpyDeviceToHost, st[0]);
         cleanup();
         if (rc) return rc;
         if (ce != cudaSuccess) return fail(ctx, DIST_B200_ERR_CUDA, std::string("score_sample_host: ") + cudaGetErrorString(ce));
-        if (!assign_pinned) std::memcpy(assign_host, pin + assign_off, sizeof(int32_t) * N);
+        if (!out_pinned) std::memcpy(out_host, pin + out_off, 4 * N);
         return DIST_B200_OK;
     }
     for (size_t k = 0; k + 1 < bounds.size(); ++k) {
@@ -1642,7 +1680,7 @@ int dist_b200_score_sample_batch_host(dist_b200_ctx *ctx, const dist_b200_featur
             DISTB200_CUDA(ctx, cudaMemcpyAsync(dev + col_off[f] + vb * lo, src, vb * n, cudaMemcpyHostToDevice, s));
             cols[f] = dev + col_off[f] + vb * lo;
         }
-        {
+        if (u_host) {
             const char *src = reinterpret_cast<const char *>(u_host + lo);
             if (!u_pinned) {
                 std::memcpy(pin + u_off + 4 * lo, src, 4 * n);
@@ -1650,15 +1688,14 @@ int dist_b200_score_sample_batch_host(dist_b200_ctx *ctx, const dist_b200_featur
             }
             DISTB200_CUDA(ctx, cudaMemcpyAsync(dev + u_off + 4 * lo, src, 4 * n, cudaMemcpyHostToDevice, s));
         }
-        rc = score_dispatch(ctx, features, F, cols.data(), n, prior_dev, reinterpret_cast<const float *>(dev + u_off) + lo,
-                            reinterpret_cast<int32_t *>(dev + assign_off) + lo, scores_dev ? scores_dev + lo * G : nullptr, 0, s);
+        rc = dispatch(cols.data(), n, prior_dev, dev_u(lo), dev + out_off + 4 * lo, scores_dev ? scores_dev + lo * G : nullptr, s);
         if (rc) {  // copies of earlier chunks into the caller's buffers may still be in flight
             cudaStreamSynchronize(st[0]);
             cudaStreamSynchronize(st[1]);
             return rc;
         }
-        int32_t *adst = assign_pinned ? assign_host + lo : reinterpret_cast<int32_t *>(pin + assign_off) + lo;
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(adst, dev + assign_off + 4 * lo, 4 * n, cudaMemcpyDeviceToHost, s));
+        char *odst = (out_pinned ? static_cast<char *>(out_host) : pin + out_off) + 4 * lo;
+        DISTB200_CUDA(ctx, cudaMemcpyAsync(odst, dev + out_off + 4 * lo, 4 * n, cudaMemcpyDeviceToHost, s));
         if (scores_host)
             DISTB200_CUDA(ctx, cudaMemcpyAsync(scores_host + lo * G, scores_dev + lo * G, sizeof(float) * n * G,
                                                cudaMemcpyDeviceToHost, s));
@@ -1666,8 +1703,23 @@ int dist_b200_score_sample_batch_host(dist_b200_ctx *ctx, const dist_b200_featur
     (void)scores_pinned;
     DISTB200_CUDA(ctx, cudaStreamSynchronize(st[0]));
     DISTB200_CUDA(ctx, cudaStreamSynchronize(st[1]));
-    if (!assign_pinned) std::memcpy(assign_host, pin + assign_off, sizeof(int32_t) * N);
+    if (!out_pinned) std::memcpy(out_host, pin + out_off, 4 * N);
     return DIST_B200_OK;
+}
+
+int dist_b200_score_sample_batch_host(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int F,
+                                      const void *const *columns_host, size_t N, const float *prior_host,
+                                      const float *u_host, int32_t *assign_host, float *scores_host) {
+    if (!ctx || !features || !columns_host || F < 1 || F > kMaxFeatures || !u_host || !assign_host) return DIST_B200_ERR_INVALID;
+    return score_host(ctx, features, F, columns_host, N, prior_host, u_host, assign_host, nullptr, scores_host);
+}
+
+int dist_b200_score_logp_batch_host(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int F,
+                                    const void *const *columns_host, size_t N, const float *prior_host, float *logp_host) {
+    if (!ctx) return DIST_B200_ERR_INVALID;
+    if (!features || !columns_host || F < 1 || F > kMaxFeatures || !logp_host)
+        return fail(ctx, DIST_B200_ERR_INVALID, "score_logp_batch_host: null argument");
+    return score_host(ctx, features, F, columns_host, N, prior_host, nullptr, nullptr, logp_host, nullptr);
 }
 
 int dist_b200_host_register(dist_b200_ctx *ctx, void *ptr, size_t bytes) {

@@ -218,10 +218,11 @@ int launch_score_data(dist_b200_ctx *ctx, const dist_b200_feature *f, const uint
                       size_t n_grid, size_t stride, double *acc, float *out_dev, cudaStream_t s);
 int launch_unpack_caches(dist_b200_ctx *ctx, const dist_b200_feature *f, float *out_dev, cudaStream_t s);
 
-// score_rows.cu: rows mapped to lanes, groups looped (nich / gp / bb / small-dim dd, any F)
+// score_rows.cu: rows mapped to lanes, groups looped (nich / gp / bb / small-dim dd, any F).  logp != nullptr (with
+// assign = scores = nullptr): logp[n] = log sum_g exp(prior[g] + scores of row n)
 int launch_score_rows(dist_b200_ctx *ctx, const FeatList &feats, int G, size_t N, const float *prior,
                       const float *u, int32_t *assign, float *scores, int accumulate, cudaStream_t s,
-                      const PushTargets *push = nullptr);
+                      const PushTargets *push = nullptr, float *logp = nullptr);
 int launch_gp_table_batch(dist_b200_ctx *ctx, const GpTableBatch &b, cudaStream_t s);
 // stats.cu: batched Group::add_value (segmented reduction of assigned rows into the device-side statistics)
 // pooled models: accumulate `b.n` features in one launch (b.acc zeroed by the launcher), then merge + rebuild caches
@@ -243,6 +244,8 @@ int launch_gather_rows(dist_b200_ctx *ctx, const dist_b200_feature *f, const voi
                        cudaStream_t s);
 int launch_sample_scores(dist_b200_ctx *ctx, const float *scores, size_t N, int G, const float *u,
                          int32_t *assign, cudaStream_t s, int n_slots = 1, size_t slot_stride = 0);
+// logp[n] = log sum_g exp(scores[n][g]) over materialised [N][G] scores
+int launch_logp_scores(dist_b200_ctx *ctx, const float *scores, size_t N, int G, float *logp, cudaStream_t s);
 // table_rows.cu: single table feature (dpd / dd / bb)
 size_t table_hot_floats(int R, int G);
 int launch_table_rows(dist_b200_ctx *ctx, const dist_b200_feature *f, const void *column, size_t N, const float *prior,
@@ -250,6 +253,9 @@ int launch_table_rows(dist_b200_ctx *ctx, const dist_b200_feature *f, const void
 size_t value_cdf_floats(int R, int G);
 int launch_value_cdf(dist_b200_ctx *ctx, const dist_b200_feature *f, float *buf, const void *column, size_t N,
                      const float *prior, const float *u, int32_t *assign, cudaStream_t s);
+// the logp form of the per-value shortcut: one log-normaliser per table row (`buf`: table rows floats), then a gather
+int launch_value_logp(dist_b200_ctx *ctx, const dist_b200_feature *f, float *buf, const void *column, size_t N,
+                      const float *prior, float *logp, cudaStream_t s);
 // niw.cu
 int niw_padded_dim(int d);
 int launch_niw_prep(dist_b200_ctx *ctx, int d, const float *mu, float kappa, const float *psi, float nu, int G,

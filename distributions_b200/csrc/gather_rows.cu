@@ -283,4 +283,35 @@ int launch_sample_scores(dist_b200_ctx *ctx, const float *scores, size_t N, int 
     return launch_gather(ctx, a, s);
 }
 
+// logp[n] = log sum_g exp(scores[n][g]): one warp per row, coalesced reads, the row maximum then the sum of exp
+constexpr int kLogpWarps = 8;
+__global__ void __launch_bounds__(kLogpWarps * 32) logp_scores_kernel(const float *__restrict__ scores, size_t N, int G,
+                                                                       float *__restrict__ logp) {
+    const unsigned full = 0xffffffffu;
+    const int lane = threadIdx.x & 31;
+    const size_t step = static_cast<size_t>(gridDim.x) * kLogpWarps;
+    for (size_t n = static_cast<size_t>(blockIdx.x) * kLogpWarps + (threadIdx.x >> 5); n < N; n += step) {
+        const float *row = scores + n * static_cast<size_t>(G);
+        float m = -INFINITY;
+        for (int g = lane; g < G; g += 32) m = fmaxf(m, __ldg(row + g));
+#pragma unroll
+        for (int o = 16; o; o >>= 1) m = fmaxf(m, __shfl_xor_sync(full, m, o));
+        const float nm = fminf(-m * kLog2e, 3.0e38f);  // finite when the whole row is -inf: the sum is then 0
+        float sum = 0.f;
+        for (int g = lane; g < G; g += 32) sum += mufu_ex2(fmaf(__ldg(row + g), kLog2e, nm));
+#pragma unroll
+        for (int o = 16; o; o >>= 1) sum += __shfl_xor_sync(full, sum, o);
+        if (lane == 0) logp[n] = logp_finish(nm, sum);
+    }
+}
+
+int launch_logp_scores(dist_b200_ctx *ctx, const float *scores, size_t N, int G, float *logp, cudaStream_t s) {
+    if (N == 0) return DIST_B200_OK;
+    const size_t want = (N + kLogpWarps - 1) / kLogpWarps, cap = static_cast<size_t>(ctx->sm_count) * 16;
+    logp_scores_kernel<<<static_cast<unsigned>(want < cap ? want : cap), kLogpWarps * 32, 0, s>>>(scores, N, G, logp);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail(ctx, DIST_B200_ERR_CUDA, std::string("logp_scores launch: ") + cudaGetErrorString(e));
+    return DIST_B200_OK;
+}
+
 }  // namespace distb200

@@ -35,6 +35,7 @@ struct NichRowsArgs {
     const float *values;
     const float *u;
     int32_t *assign;
+    float *logp;           // nich_logp_kernel: log sum_g exp(prior + score) per row
 };
 
 // geometry of the block-private parameter copy and the per-row slot pairs
@@ -471,6 +472,142 @@ __global__ void __launch_bounds__(kNrThreads, kBlocks) nich_rows2_kernel(const N
             nich2_tile<kPoly, 1>(g, x1, u1, row1, a.N, a.assign);
         }
     }
+}
+
+// ------------------------------------------------------------------------------------------------
+// nich_logp_kernel: the row log-normaliser with nich_rows2_kernel's static reference.  The weights it sums are
+// e_g = 2^((s_g - M*) log2 e), so logp = M* + ln(sum_g e_g) needs no slots and no walk, and a thread carries its four rows
+// across all the tiles.  Rows whose sum falls below 2^-40 are re-evaluated with their own maximum (nich2_row_logp).
+__device__ __noinline__ float nich2_row_logp(const Nich2Geom &g, float x) {  // ln sum_g 2^(arg_g), arg on the lg2 scale
+    float m = -INFINITY;
+    for (int gi = 0; gi < g.G; ++gi) m = fmaxf(m, nich2_arg(g, gi, x));
+    if (m == -INFINITY) return -INFINITY;
+    float total = 0.f;
+    for (int gi = 0; gi < g.G; ++gi) total += mufu_ex2(nich2_arg(g, gi, x) - m);
+    return (m + log2f(total)) * kLn2;
+}
+
+template <int kPoly>
+__global__ void __launch_bounds__(kNrThreads, 2) nich_logp_kernel(const NichRowsArgs a) {
+    extern __shared__ __align__(16) float smem[];
+    __shared__ float red[kNrThreads / 32];
+    constexpr int R = kN2Rows;
+    Nich2Geom g;
+    g.G = a.G;
+    g.nchunks = (a.G + kNrChunk - 1) / kNrChunk;
+    const int Gpad = g.nchunks * kNrChunk;
+    g.cps = (g.nchunks + kSlots - 1) / kSlots;
+    g.nslots = (g.nchunks + g.cps - 1) / g.cps;
+    g.slot_groups = g.cps * kNrChunk;
+    float4 *caches = reinterpret_cast<float4 *>(smem);
+    g.caches = caches;
+    g.slots = nullptr;
+    const int tid = threadIdx.x;
+    // M* as in nich_rows2_kernel; 0 when every group sits at -inf, so that the weights are 0 and not NaN
+    float m = -INFINITY;
+    for (int gi = tid; gi < a.G; gi += kNrThreads) m = fmaxf(m, a.params[gi].w + (a.prior ? a.prior[gi] : 0.f));
+#pragma unroll
+    for (int o = 16; o; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+    if ((tid & 31) == 0) red[tid >> 5] = m;
+    __syncthreads();
+    m = red[0];
+#pragma unroll
+    for (int w = 1; w < kNrThreads / 32; ++w) m = fmaxf(m, red[w]);
+    if (m == -INFINITY) m = 0.f;
+    for (int p = tid; p < Gpad / 2; p += kNrThreads) {  // the block-private copy of nich_rows2_kernel
+        float4 q[2];
+        float sc[2], co[2];
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+            const int gi = 2 * p + k;
+            q[k] = a.params[gi < a.G ? gi : 0];
+            const float s = q[k].w + (a.prior ? a.prior[gi < a.G ? gi : 0] : 0.f);
+            sc[k] = gi < a.G ? (s - m) * kLog2e : -INFINITY;
+            co[k] = static_cast<float>(static_cast<double>(q[k].z) * 1.4426950408889634);
+        }
+        const int at = 2 * p + (2 * p) / g.slot_groups;
+        caches[at] = make_float4(-q[0].x, -q[1].x, q[0].y, q[1].y);
+        caches[at + 1] = make_float4(co[0], co[1], sc[0], sc[1]);
+    }
+    __syncthreads();
+
+    const uint64_t one2 = f2_pack(1.f, 1.f);
+    const size_t tile_rows = static_cast<size_t>(kNrThreads) * R;
+    const size_t ntiles = (a.N + tile_rows - 1) / tile_rows;
+    for (size_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
+        size_t row[R];
+        float x[R];
+        uint64_t x2[R], sa[R], sb[R];  // two partial sums per row: even / odd pairs
+#pragma unroll
+        for (int r = 0; r < R; ++r) {
+            row[r] = t * tile_rows + static_cast<size_t>(r) * kNrThreads + tid;
+            x[r] = __ldg(a.values + (row[r] < a.N ? row[r] : a.N - 1));  // clamp: compute on a real row, discard the result
+            x2[r] = f2_pack(x[r], x[r]);
+            sa[r] = sb[r] = f2_pack(0.f, 0.f);
+        }
+        for (int c = 0; c < g.nchunks; ++c) {
+            const float4 *p4 = g.caches + c * kNrChunk + c / g.cps;
+#pragma unroll
+            for (int j = 0; j < kNrChunk; j += 2) {  // parameters once, all rows; the weights of nich2_tile
+                const float4 qa = p4[j], qb = p4[j + 1];
+#pragma unroll
+                for (int r = 0; r < R; ++r) {
+                    const uint64_t d2 = f2_add(x2[r], f2_pack(qa.x, qa.y));
+                    const uint64_t z2 = f2_fma(f2_mul(f2_pack(qa.z, qa.w), f2_mul(d2, d2)), one2, one2);
+                    float za, zb;
+                    f2_unpack(z2, za, zb);
+                    const uint64_t a2 = f2_fma(f2_pack(qb.x, qb.y), f2_pack(fast_log2_cell(za), fast_log2_cell(zb)), f2_pack(qb.z, qb.w));
+                    uint64_t e2;
+                    if (((j / 2) * kPoly) % 16 < kPoly) {
+                        e2 = poly_ex2_pair(a2);
+                    } else {
+                        float ea, eb;
+                        f2_unpack(a2, ea, eb);
+                        e2 = f2_pack(mufu_ex2(ea), mufu_ex2(eb));
+                    }
+                    if (j & 2) sb[r] = f2_add(sb[r], e2);
+                    else sa[r] = f2_add(sa[r], e2);
+                }
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < R; ++r) {
+            float a0, a1;
+            f2_unpack(f2_add(sa[r], sb[r]), a0, a1);
+            const float total = a0 + a1;
+            const float lp = total >= kN2Redo ? m + logf(total) : m + nich2_row_logp(g, x[r]);  // an outlier to every group
+            if (row[r] < a.N) a.logp[row[r]] = lp;
+        }
+    }
+}
+
+int launch_nich_logp(dist_b200_ctx *ctx, const float4 *params, const void *column, int G, size_t N, const float *prior,
+                     float *logp, cudaStream_t s) {
+    if (G <= 128 || !logp) return DIST_B200_ERR_UNSUPPORTED;
+    const int nchunks = (G + kNrChunk - 1) / kNrChunk;
+    const int cps = (nchunks + kSlots - 1) / kSlots;
+    const int nslots = (nchunks + cps - 1) / cps;
+    const size_t smem = sizeof(float4) * (nchunks * kNrChunk + nslots);
+    if (smem > 220 * 1024) return DIST_B200_ERR_UNSUPPORTED;
+    NichRowsArgs a{};
+    a.G = G;
+    a.N = N;
+    a.params = params;
+    a.prior = prior;
+    a.values = static_cast<const float *>(column);
+    a.logp = logp;
+    auto kern = nich_logp_kernel<kN2PolyDefault>;
+    DISTB200_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    int per_sm = 0;
+    DISTB200_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kNrThreads, smem));
+    if (per_sm < 1) per_sm = 1;
+    const size_t tile_rows = static_cast<size_t>(kNrThreads) * kN2Rows;
+    const size_t ntiles = (N + tile_rows - 1) / tile_rows;
+    const size_t cap = static_cast<size_t>(ctx->sm_count) * per_sm;
+    kern<<<static_cast<unsigned>(ntiles < cap ? ntiles : cap), kNrThreads, smem, s>>>(a);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail(ctx, DIST_B200_ERR_CUDA, std::string("nich_logp launch: ") + cudaGetErrorString(e));
+    return DIST_B200_OK;
 }
 
 template <int kPoly, int RT = kN2Rows, int kBlocks = 2>

@@ -61,6 +61,10 @@ __device__ __forceinline__ float fast_log_cell(float x) { return fast_log2_cell(
 // returns garbage denormals there, fmath.hpp:455-458; both are < 1.2e-38 of the row maximum).
 __device__ __forceinline__ float fast_exp_neg(float x) { return mufu_ex2(x * kLog2e); }
 
+// log sum_g exp(s_g) from a reference nm = -(m log2 e) and sum = sum_g 2^(s_g log2 e + nm): ln(sum) - nm ln 2.  A row
+// whose every term is -inf has sum = 0 (nm finite: the callers clamp it) and gets -inf, never NaN.
+__device__ __forceinline__ float logp_finish(float nm, float sum) { return fmaf(-nm, kLn2, logf(sum)); }
+
 // floor(log2 y) for positive y from the exponent field (special.hpp:127-146; subnormals via clz)
 __device__ __forceinline__ int float_exponent(float y) {
     const int x = __float_as_int(y);

@@ -36,7 +36,7 @@ int launch_gp_table_batch(dist_b200_ctx *ctx, const GpTableBatch &b, cudaStream_
 
 int launch_score_rows(dist_b200_ctx *ctx, const FeatList &feats, int G, size_t N, const float *prior,
                       const float *u, int32_t *assign, float *scores, int accumulate, cudaStream_t s,
-                      const PushTargets *push) {
+                      const PushTargets *push, float *logp) {
     if (N == 0 || G == 0) return DIST_B200_OK;
     RowsArgs a{};
     if (push) {
@@ -54,7 +54,8 @@ int launch_score_rows(dist_b200_ctx *ctx, const FeatList &feats, int G, size_t N
     a.scores = scores;
     a.accumulate = accumulate;
     a.t = ctx->tables;
-    if (!assign && !scores) return fail(ctx, DIST_B200_ERR_INVALID, "score_rows: nothing to produce");
+    a.logp = logp;
+    if (!assign && !scores && !logp) return fail(ctx, DIST_B200_ERR_INVALID, "score_rows: nothing to produce");
     if (feats.n == 1) {
         int rc = DIST_B200_ERR_UNSUPPORTED;
         switch (feats.f[0].kind) {

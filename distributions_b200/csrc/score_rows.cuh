@@ -16,6 +16,8 @@
 //
 //   G <= CHUNK  : the whole score row lives in registers; max, exp, running total and the
 //                 `t -= l[i]; t <= 0` walk are the reference's loops verbatim.
+//   logp mode   : neither sample nor scores: per row an online (negated scaled max, sum of exp) pair is merged across
+//                 the tiles (no slots, no walk) and log sum_g exp(score) is written.
 //   G  > CHUNK  : per tile (negated scaled max, sum of exp) pairs are merged into at most kSlots
 //                 slots kept in shared memory; a walk over the slots finds the one holding
 //                 u * total, then each thread re-scores just that slot's tiles for its own row
@@ -233,14 +235,16 @@ struct RowsArgs {
     int n_push;
     size_t row0, block_rows;
     float *push[kMaxPushOwners];
+    float *logp;  // logp mode (kSample = kScores = false): logp[n] = log sum_g exp(score of row n, group g)
 };
 
 // kSub (feature lists whose caches stream, more groups than one register tile, sampling only): per tile the row keeps
 // the tile's maximum and the sums of exp over SUB-SLOTS of 16 groups, so that the draw is located down to 16 groups
 // from the main pass and only those are re-scored (from global memory, through the transposed GammaPoisson tables).
 constexpr int kSubGroups = 16;
+// (logp mode: no minimum of resident blocks -- the register cap the others take would make its online pair spill)
 template <int CHUNK, int KIND, bool kSample, bool kScores, int THREADS, bool kSub = false>
-__global__ void __launch_bounds__(THREADS, THREADS == 128 ? (is_dd_scaled(KIND) ? 5 : 3) : (CHUNK <= 32 ? (KIND >= 0 ? 4 : 3) : (CHUNK <= 64 ? 2 : 1)))
+__global__ void __launch_bounds__(THREADS, (!kSample && !kScores) ? 1 : THREADS == 128 ? (is_dd_scaled(KIND) ? 5 : 3) : (CHUNK <= 32 ? (KIND >= 0 ? 4 : 3) : (CHUNK <= 64 ? 2 : 1)))
 score_rows_kernel(const __grid_constant__ FeatList feats, const RowsArgs a) {
     constexpr int kThreads = THREADS;  // block size of this instantiation
     static_assert(!kSub || (KIND < 0 && kSample && !kScores && CHUNK % kSubGroups == 0), "kSub: streaming feature lists, sampling only");
@@ -253,6 +257,7 @@ score_rows_kernel(const __grid_constant__ FeatList feats, const RowsArgs a) {
     // against lgamma(post_alpha + v) -- adding the prior before that cancellation would cost ~1e-5
     constexpr bool kFold = kSingle && KIND != DIST_B200_GP && KIND != DIST_B200_BNB;
     constexpr bool kNich = KIND == DIST_B200_NICH || KIND == kKindNichPacked;
+    constexpr bool kLogp = !kSample && !kScores;
     const int G = a.G;
     const int nchunks = (G + CHUNK - 1) / CHUNK;
     const int Gpad = nchunks * CHUNK;
@@ -389,6 +394,7 @@ score_rows_kernel(const __grid_constant__ FeatList feats, const RowsArgs a) {
         if (!valid) row = row_end - 1;  // clamp: compute on a real row, discard the result
         float slot_m = INFINITY, slot_s = 0.f;  // slot being merged: negated scaled max, sum of exp
         float nmax = 0.f, tres = 0.f;           // finalisation state: row's negated scaled max, remaining draw
+        float lp_m = INFINITY, lp_s = 0.f;      // logp mode: the row's negated scaled max and sum of exp so far
         int sel = 0, count = 0, result = 0;
         const float urow = kPrefetch ? pre_u : (kSample ? a.u[row] : 0.f);
         const uint32_t vrow = pre_v;
@@ -554,6 +560,30 @@ score_rows_kernel(const __grid_constant__ FeatList feats, const RowsArgs a) {
                         }
                     }
                 }
+            }
+
+            if (kLogp) {
+                // the tile's (negated scaled max, sum of exp) pair merged into the row's, as the multi-tile sampler merges
+                // a slot; nm is finite also when every group of the tile sits at -inf (its sum is then 0, not NaN)
+                float m = acc[0];
+#pragma unroll
+                for (int j = 1; j < CHUNK; ++j) m = fmaxf(m, acc[j]);
+                const float nm = fminf(-m * kLog2e, 3.0e38f);
+                const uint64_t l2e2 = f2_pack(kLog2e, kLog2e), nm2 = f2_pack(nm, nm);
+                uint64_t s2 = f2_pack(0.f, 0.f);
+#pragma unroll
+                for (int j = 0; j < CHUNK; j += 2) {
+                    float ea, eb;
+                    f2_unpack(f2_fma(f2_pack(acc[j], acc[j + 1]), l2e2, nm2), ea, eb);
+                    s2 = f2_add(s2, f2_pack(mufu_ex2(ea), mufu_ex2(eb)));
+                }
+                float se, so;
+                f2_unpack(s2, se, so);
+                const float s = se + so;
+                const float dlt = lp_m - nm;
+                const float e = mufu_ex2(-fabsf(dlt));
+                lp_s = dlt > 0.f ? fmaf(lp_s, e, s) : fmaf(s, e, lp_s);
+                lp_m = fminf(lp_m, nm);
             }
 
             if (kSample && is_dd_scaled(KIND)) {
@@ -868,6 +898,7 @@ score_rows_kernel(const __grid_constant__ FeatList feats, const RowsArgs a) {
             }
         }
         if (kSample && valid) a.assign[row] = result;
+        if (kLogp && valid) a.logp[row] = logp_finish(lp_m, lp_s);
     }  // row tiles
 }
 
@@ -910,9 +941,18 @@ static int launch_variant(dist_b200_ctx *ctx, const FeatList &feats, RowsArgs a,
     return DIST_B200_OK;
 }
 
+int launch_crosscat_tile32(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s);
+int launch_crosscat_tile64(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s);
+int launch_crosscat_ksub(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s);
+
 template <int CHUNK, int KIND, int THREADS>
 static int launch_modes(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s) {
     const bool sample = a.assign != nullptr, scores = a.scores != nullptr;
+    if (a.logp) {
+        // a feature list does not fit a 128-group logp tile in registers: two 64-group tiles instead
+        if constexpr (KIND < 0 && CHUNK == 128) return launch_crosscat_tile64(ctx, feats, a, s);
+        else return launch_variant<CHUNK, KIND, false, false, THREADS>(ctx, feats, a, s);
+    }
     if (sample && scores) return launch_variant<CHUNK, KIND, true, true, THREADS>(ctx, feats, a, s);
     if (sample) return launch_variant<CHUNK, KIND, true, false, THREADS>(ctx, feats, a, s);
     return launch_variant<CHUNK, KIND, false, true, THREADS>(ctx, feats, a, s);
@@ -937,9 +977,6 @@ static __global__ void __launch_bounds__(256) bb_compact_kernel(const __grid_con
 // latency) -- DIST_B200_OPT_SMALL_TILE selects the alternatives for A/B runs.  G > 128: 32-group tiles.
 // the feature-list (KIND = -1) instantiations are the heaviest to compile: they live in three translation units
 // (score_rows.cu: 128-group tiles; score_rows_cc32.cu: 32-group tiles + kSub; score_rows_cc64.cu: 64-group tiles)
-int launch_crosscat_tile32(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s);
-int launch_crosscat_tile64(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s);
-int launch_crosscat_ksub(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s);
 template <int KIND>
 static int launch_tile32(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s) {
     if constexpr (KIND < 0) return launch_crosscat_tile32(ctx, feats, a, s);

@@ -531,6 +531,122 @@ static size_t value_cdf_tree_floats(int R, int G) {
     return per;
 }
 
+// ------------------------------------------------------------------------------------------------
+// (3) the logp form of (2): per table row r, lse[r] = log sum_g exp(prior_g + T[r][g]) (one warp per row: the reduction
+// of value_guide_build_kernel without the prefix sums and guide), then logp[n] = lse[key_row(value n)].
+__global__ void __launch_bounds__(kGuideWarps * 32) value_logp_build_kernel(const GuideArgs a) {
+    const int lane = threadIdx.x & 31;
+    const int r = blockIdx.x * kGuideWarps + (threadIdx.x >> 5);
+    if (r >= a.R) return;
+    const unsigned full = 0xffffffffu;
+    float m = -INFINITY;
+    for (int g = lane; g < a.G; g += 32) m = fmaxf(m, (a.prior ? a.prior[g] : 0.f) + guide_table_score(a, r, g));
+#pragma unroll
+    for (int o = 16; o; o >>= 1) m = fmaxf(m, __shfl_xor_sync(full, m, o));
+    const float nm = fminf(-m * kLog2e, 3.0e38f);  // finite when the whole row is -inf: the sum is then 0
+    float sum = 0.f;
+    for (int g = lane; g < a.G; g += 32) sum += mufu_ex2(fmaf((a.prior ? a.prior[g] : 0.f) + guide_table_score(a, r, g), kLog2e, nm));
+#pragma unroll
+    for (int o = 16; o; o >>= 1) sum += __shfl_xor_sync(full, sum, o);
+    if (lane == 0) a.total[r] = logp_finish(nm, sum);
+}
+
+struct ValueLogpArgs {
+    KeyMap km;
+    size_t N;
+    const float *lse;
+    const uint32_t *values;
+    int value_bytes;
+    float *logp;
+};
+
+__device__ __forceinline__ uint32_t table_value(const ValueLogpArgs &a, size_t n) {
+    return a.value_bytes == 1 ? (reinterpret_cast<const uint8_t *>(a.values)[n] ? 1u : 0u) : a.values[n];
+}
+
+// kVec = 4: four consecutive rows per thread with 16-byte loads and stores, as value_guide_sample_kernel
+template <int kVec>
+__global__ void __launch_bounds__(256) value_logp_gather_kernel(const ValueLogpArgs a) {
+    const size_t step = static_cast<size_t>(gridDim.x) * blockDim.x;
+    const size_t first = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (kVec == 4) {
+        const size_t nq = a.N / 4;
+        for (size_t q = first; q < nq; q += step) {
+            uint32_t v[4];
+            if (a.value_bytes == 1) {
+                const uchar4 b = reinterpret_cast<const uchar4 *>(a.values)[q];
+                v[0] = b.x ? 1u : 0u, v[1] = b.y ? 1u : 0u, v[2] = b.z ? 1u : 0u, v[3] = b.w ? 1u : 0u;
+            } else {
+                const uint4 w = reinterpret_cast<const uint4 *>(a.values)[q];
+                v[0] = w.x, v[1] = w.y, v[2] = w.z, v[3] = w.w;
+            }
+            float lp[4];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) lp[i] = __ldg(a.lse + key_row(a.km, v[i]));
+            reinterpret_cast<float4 *>(a.logp)[q] = make_float4(lp[0], lp[1], lp[2], lp[3]);
+        }
+        const size_t n = nq * 4 + first;  // the ragged tail
+        if (n < a.N) a.logp[n] = __ldg(a.lse + key_row(a.km, table_value(a, n)));
+    } else {
+        for (size_t n = first; n < a.N; n += step) a.logp[n] = __ldg(a.lse + key_row(a.km, table_value(a, n)));
+    }
+}
+
+// value -> table row of a single table feature (dd values are clamped to dim - 1 like the row-mapped kernel does)
+static int table_key_map(const dist_b200_feature *f, int &R, KeyMap &km) {
+    switch (f->model) {
+        case DIST_B200_DPD:
+            R = f->dim + 1;
+            km = KeyMap{f->dim, f->keys_dense ? 1 : 0, f->keys_dev, f->key_rows_dev};
+            return DIST_B200_OK;
+        case DIST_B200_DD:
+            R = f->dim;
+            km = KeyMap{f->dim - 1, 1, nullptr, nullptr};
+            return DIST_B200_OK;
+        case DIST_B200_BB:
+            R = 2;
+            km = KeyMap{1, 1, nullptr, nullptr};
+            return DIST_B200_OK;
+        default: return DIST_B200_ERR_UNSUPPORTED;
+    }
+}
+
+// single table feature, logp only.  `buf` holds R floats (feature-owned scratch).  DIST_B200_ERR_UNSUPPORTED below 4 R rows
+// (the same threshold as the sampler): the caller takes the per-cell kernels
+int launch_value_logp(dist_b200_ctx *ctx, const dist_b200_feature *f, float *buf, const void *column, size_t N,
+                      const float *prior, float *logp, cudaStream_t s) {
+    if (N == 0 || f->G == 0) return DIST_B200_OK;
+    int R;
+    KeyMap km{};
+    if (table_key_map(f, R, km)) return DIST_B200_ERR_UNSUPPORTED;
+    if (N < 4 * static_cast<size_t>(R)) return DIST_B200_ERR_UNSUPPORTED;
+    GuideArgs b{};
+    b.model = f->model;
+    b.G = f->G;
+    b.R = R;
+    b.vdim = f->dim;
+    b.params = f->params;
+    b.prior = prior;
+    b.total = buf;
+    value_logp_build_kernel<<<(R + kGuideWarps - 1) / kGuideWarps, kGuideWarps * 32, 0, s>>>(b);
+    ValueLogpArgs a{};
+    a.km = km;
+    a.N = N;
+    a.lse = buf;
+    a.values = static_cast<const uint32_t *>(column);
+    a.value_bytes = f->model == DIST_B200_BB ? 1 : 4;
+    a.logp = logp;
+    const bool vec = N >= 1024 && ((reinterpret_cast<uintptr_t>(column) | reinterpret_cast<uintptr_t>(logp)) & 15) == 0;
+    const size_t want = ((vec ? N / 4 : N) + 255) / 256;
+    const size_t cap = static_cast<size_t>(ctx->sm_count) * 8;
+    const unsigned grid = static_cast<unsigned>(want < cap ? want : cap);
+    if (vec) value_logp_gather_kernel<4><<<grid, 256, 0, s>>>(a);
+    else value_logp_gather_kernel<1><<<grid, 256, 0, s>>>(a);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail(ctx, DIST_B200_ERR_CUDA, std::string("value_logp launch: ") + cudaGetErrorString(e));
+    return DIST_B200_OK;
+}
+
 // single table feature, sampling only.  `buf` holds value_cdf_floats(R, G) floats (feature-owned scratch).
 int launch_value_cdf(dist_b200_ctx *ctx, const dist_b200_feature *f, float *buf, const void *column, size_t N,
                      const float *prior, const float *u, int32_t *assign, cudaStream_t s) {

@@ -131,6 +131,15 @@ class _Mixture:
         vals = np.ascontiguousarray(values, dtype=capi.COLUMN_DTYPE[self.model_id])
         return self.ctx.score_sample_batch_host([self.feature], [vals], prior, np.ascontiguousarray(u, np.float32), want_scores)
 
+    def score_logp(self, shared, values, prior=None):
+        """float32 logp[n] = log sum_g exp(prior[g] + score_value_group(g, values[n])) on the device, without the [n][G]
+        scores.  With the clustering's Pitman-Yor vector as `prior` this is the log posterior-predictive density of each
+        value under the mixture (niw: values is [n][d])."""
+        vals = np.ascontiguousarray(values, dtype=capi.COLUMN_DTYPE[self.model_id])
+        if self.model_id == capi.NIW:
+            vals = vals.reshape(-1, shared.dim)
+        return self.ctx.score_logp_batch_host([self.feature], [vals], prior)
+
     def add_values(self, shared, values, groupids):
         """batched add_value: one segmented reduction on the device, then the Groups are read back"""
         self.ctx.add_rows_batch_host([self.feature], [values], groupids)

@@ -350,6 +350,35 @@ int dist_b200_score_sample_batch(dist_b200_ctx *ctx, const dist_b200_feature *co
 int dist_b200_sample_from_scores(dist_b200_ctx *ctx, const float *scores_dev, size_t n_rows, int G,
                                  const float *u_dev, int32_t *assign_dev, void *stream);
 
+/* ---- row log-likelihood: how probable is each row under the mixture ---------------------------------------------
+ * dist_b200_score_logp_batch: for every row n,
+ *   logp_dev[n] = log sum_{g < G} exp(prior_dev[g] + sum_f score_f(columns_dev[f][n]; g))      (natural log, float32)
+ * prior_dev may be NULL (= 0).  With the Pitman-Yor vector of dist_b200_prior_pitman_yor (group sizes including the empty
+ * group; the prior weights then sum to 1) this is the log posterior-predictive density of the row under the mixture: the
+ * quantity the reference's frozen-mixture example forms per pixel as exp(scores).sum() (examples/mixture/main.py:143-160)
+ * with log_sum_exp as its primitive (src/random.cc:77-92).
+ *   - logp_dev is OVERWRITTEN; there is no accumulate form.  The [N][G] scores are not materialised for row-mapped
+ *     features (nich / gp / bnb / bb / dd, any list of them) and single table features; dpd in per-cell mode, niw and mixed
+ *     lists containing them go through the context's scores buffer.
+ *   - A row whose every term is -inf (e.g. a prior of -inf everywhere) gets -inf, never NaN.
+ *   - Same feature-list rules, column types and error codes as dist_b200_score_sample_batch (ERR_STATE for a feature
+ *     before its first update_all or features that disagree on G).  Waits on every feature's pending updates (ready
+ *     events), like the other score entries, so a preceding add_rows_batch on another stream is seen.
+ *   - Conditional densities: logp(A | B) = logp(features A and B) - logp(features B), two calls over nested feature lists
+ *     with the same prior.
+ * dist_b200_score_logp_batch_host: the same with host buffers (staged / zero-copy as dist_b200_score_sample_batch_host;
+ * results bit-identical to the device form).  Synchronous.
+ * dist_b200_logp_from_scores: the reduction alone over materialised [N][G] scores, e.g. a score_batch result or the sum
+ * of feature-shard slots the caller formed (the counterpart of dist_b200_sample_from_scores). */
+int dist_b200_score_logp_batch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                               const void *const *columns_dev, size_t n_rows, const float *prior_dev,
+                               float *logp_dev, void *stream);
+int dist_b200_score_logp_batch_host(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                                    const void *const *columns_host, size_t n_rows, const float *prior_host,
+                                    float *logp_host);
+int dist_b200_logp_from_scores(dist_b200_ctx *ctx, const float *scores_dev, size_t n_rows, int G,
+                               float *logp_dev, void *stream);
+
 /* ---- feature shards over NVLink peer memory (one process per GPU) ----------------------------------
  * scores[n][g] = prior[g] + sum_f s_f[n][g] is a sum over features (SURVEY.md §8e).  With the features of
  * a kind sharded over K ranks, each rank scores its features for every row and stores the partial row

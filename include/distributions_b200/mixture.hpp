@@ -15,7 +15,8 @@
 //     counts(), empty_groupids(), sample_size(), init, add_value / remove_value (return whether a group
 //     was added / removed), score_value (OVERWRITES the caller's buffer)
 // What is new: Mixture::score_values / CrossCat::score_sample_values -- the batched entry that scores
-// N rows against frozen statistics and samples a group per row (SURVEY.md §3.3); Mixture::sample_values /
+// N rows against frozen statistics and samples a group per row (SURVEY.md §3.3); Mixture::score_logp_values /
+// CrossCat::score_logp_values -- the log-likelihood of each row under the mixture; Mixture::sample_values /
 // CrossCat::sample_values -- batched Group::sample_value, one posterior-predictive draw per row on the device
 // (Sampler::init + Sampler::eval with fresh parameters per value), seeded explicitly instead of through rng_t.
 //
@@ -589,6 +590,16 @@ class Mixture {
                     "score_values");
     }
 
+    // NEW: row log-likelihood.  logp[n] = log sum_g exp(prior[g] + score_value_group(g, values[n])), computed on the device
+    // without the [n][G] scores; with the Pitman-Yor prior vector the log posterior-predictive density of values[n].
+    template <class T>
+    void score_logp_values(const Shared &, const T * values, size_t n, const float * prior, float * logp) const {
+        std::vector<typename detail::WireValue<Value>::type> wire(values, values + n);
+        const dist_b200_feature * feats[1] = {f_};
+        const void * cols[1] = {wire.data()};
+        ctx_->check(dist_b200_score_logp_batch_host(ctx_->get(), feats, 1, cols, n, prior, logp), "score_logp_values");
+    }
+
     // NEW: batched Group::sample_value.  out[n] receives one draw from the posterior predictive of group groupids[n]
     // (fresh parameters per value, as Sampler::init + eval), computed on the device from its statistics.  A draw depends
     // on (seed, row0 + n) and that group only; an id outside [0, G) leaves out[n] as it is.
@@ -733,6 +744,14 @@ class CrossCat {
         ctx_->check(dist_b200_score_sample_batch_host(ctx_->get(), feats_.data(), static_cast<int>(feats_.size()), cols_.data(), n,
                                                       prior, u, assign, scores),
                     "score_sample_values");
+    }
+
+    // logp[n] = log sum_g exp(prior[g] + sum_f score_f(row n; g)) for n rows of the kind's features (conditional densities:
+    // the difference of two calls over nested feature lists)
+    void score_logp_values(size_t n, const float * prior, float * logp) {
+        ctx_->check(dist_b200_score_logp_batch_host(ctx_->get(), feats_.data(), static_cast<int>(feats_.size()), cols_.data(), n, prior,
+                                                    logp),
+                    "score_logp_values");
     }
 
     // batched Group::sample_value for every feature of the kind: columns_out[i] (host, the column type of feature i)
