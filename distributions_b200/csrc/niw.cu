@@ -57,14 +57,17 @@ __global__ void niw_prep_kernel(int d, int dp, const float *__restrict__ mu, flo
         rec[dp + e] = (i < d && j <= i) ? static_cast<float>(Winv[i][j]) : 0.f;
     }
     if (tid == 0) {
-        double det = 1.0;
-        for (int i = 0; i < d; ++i) det *= S[i][i] * S[i][i];
+        double det = 1.0, logdet = 0.0;
+        for (int i = 0; i < d; ++i) {
+            det *= S[i][i] * S[i][i];
+            logdet += 2.0 * log(S[i][i]);
+        }
         // score_mv_student_t's constant terms, with its float/double mix (random.hpp:166-178)
         const float dof_f = static_cast<float>(dof);
         const float log_pi = 1.1447298858494002f;
         const float term1 = fast_lgamma_exact(static_cast<float>(dof_f / 2. + static_cast<float>(d) / 2.), t.lgamma5) -
                             fast_lgamma_exact(static_cast<float>(dof_f / 2.), t.lgamma5);
-        const float term2 = static_cast<float>(-0.5 * fast_log_table(static_cast<float>(det), t.log2_table) -
+        const float term2 = static_cast<float>(-0.5 * niw_log_det(det, logdet, t.log2_table) -
                                                static_cast<float>(d) / 2. * (fast_log_table(dof_f, t.log2_table) + log_pi));
         float *k4 = rec + dp + dp * dp;
         k4[0] = term1 + term2;

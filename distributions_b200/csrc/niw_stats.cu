@@ -218,15 +218,6 @@ __device__ double chol_logdet_free(double (*S)[33], int d, int tid, int nthreads
     return det_out[1];
 }
 
-// fast_log(det) as the reference writes it while det is a normal float; beyond that (the reference's float determinant()
-// has overflowed / flushed to zero -- at d = 32 it always does -- and its score_data is meaningless) the log of the
-// determinant itself, as the reference's exact-math Python flavour computes it (dbg/models/niw.py:213,216)
-__device__ float niw_log_det(const double *det, const NumericTables &t) {
-    const float f = static_cast<float>(det[0]);
-    if (isfinite(f) && f >= 1.17549435e-38f) return fast_log_table(f, t.log2_table);
-    return static_cast<float>(det[1]);
-}
-
 __device__ float lmultigamma_dev(int d, float a, const NumericTables &t) {  // special.hpp:278-286
     const float log_pi = 1.1447298858494002f;
     const float term1 = static_cast<float>(0.25 * static_cast<float>(d * (d - 1))) * log_pi;
@@ -273,9 +264,9 @@ __global__ void __launch_bounds__(64) niw_score_data_kernel(const NiwScoreDataAr
         const float log_pi = 1.1447298858494002f;
         const float post_nu = nu + static_cast<float>(cnt), post_kappa = kappa + static_cast<float>(cnt);
         const float score = lmultigamma_dev(d, static_cast<float>(post_nu * 0.5), t) +
-                            static_cast<float>(nu * 0.5) * niw_log_det(det_prior, t) -
+                            static_cast<float>(nu * 0.5) * niw_log_det(det_prior[0], det_prior[1], t.log2_table) -
                             static_cast<float>(static_cast<float>(cnt * d) * 0.5) * log_pi - lmultigamma_dev(d, static_cast<float>(nu * 0.5), t) -
-                            static_cast<float>(post_nu * 0.5) * niw_log_det(det_post, t) +
+                            static_cast<float>(post_nu * 0.5) * niw_log_det(det_post[0], det_post[1], t.log2_table) +
                             static_cast<float>(static_cast<float>(d) * 0.5) * fast_log_table(kappa / post_kappa, t.log2_table);
         atomicAdd(a.acc + blockIdx.y, static_cast<double>(score));
     }

@@ -55,6 +55,17 @@ __device__ __forceinline__ float fast_log2_cell(float x) {
 }
 __device__ __forceinline__ float fast_log_cell(float x) { return fast_log2_cell(x) * kLn2; }
 
+// The log-determinant of an NIW scale matrix (score_mv_student_t's constant, Group::score_data): fast_log(det) as the
+// reference writes it while det is a normal float; beyond that (the reference's float determinant() has overflowed to
+// inf or flushed to 0, and its result is meaningless) the log of the determinant itself, logdet = sum_i 2 ln L_ii, as the
+// reference's exact-math Python flavour computes it (dbg/models/niw.py:213,216).  At d = 32 the window is a geometric-mean
+// per-dimension variance in about [0.065, 16].
+__device__ __forceinline__ float niw_log_det(double det, double logdet, const float *__restrict__ log2_table) {
+    const float f = static_cast<float>(det);
+    if (isfinite(f) && f >= 1.17549435e-38f) return fast_log_table(f, log2_table);
+    return static_cast<float>(logdet);
+}
+
 // fast_exp as used by scores_to_likelihoods (random.cc:94-106): argument = score - max <= 0.
 // fmath::exp is exp() to 4e-7 (source) / 5e-6 (the -ffast-math build); MUFU.EX2 of x*log2(e) is
 // within 2^-22 + the rounding of the product.  Results below 2^-126 flush to 0 (the reference
@@ -153,8 +164,9 @@ __device__ __forceinline__ uint64_t f2_fma(uint64_t a, uint64_t b, uint64_t c) {
     return r;
 }
 
-// exp2 of a pair on the FMA pipe (Cody-Waite split + degree-5 minimax polynomial, 2.1e-7 relative: the accuracy class of
-// MUFU.EX2's 2^-22), for arguments <= ~0.  The sampling kernels are bound by the MUFU pipe (16 lanes / clock / SM) while the
+// exp2 of a pair on the FMA pipe (Cody-Waite split + degree-5 polynomial, <= 2.21e-7 relative over every fp32
+// argument in [-1, 0], hence over every reachable fractional part: the accuracy class of MUFU.EX2's 2^-22; the constant
+// term is exactly 1, so integer arguments give exact powers of two), for arguments <= ~0.  The sampling kernels are bound by the MUFU pipe (16 lanes / clock / SM) while the
 // FMA pipe idles: a share of their exp2 takes this route instead of MUFU.EX2 (the softmax trick of recent attention
 // kernels; nich_rows.cu: kPoly of every 16 pairs).  x + 1.5 * 2^23 rounds x to the nearest integer n in the low mantissa bits, f = x - n lies
 // in [-0.5, 0.5], and 2^n is applied by adding n to the exponent field; below -125 the argument is clamped (2^-125 of
@@ -170,7 +182,7 @@ __device__ __forceinline__ uint64_t poly_ex2_pair(uint64_t x2) {
     p2 = f2_fma(p2, f2, f2_pack(0.05550713092088699f, 0.05550713092088699f));
     p2 = f2_fma(p2, f2, f2_pack(0.24022120237350464f, 0.24022120237350464f));
     p2 = f2_fma(p2, f2, f2_pack(0.6931469440460205f, 0.6931469440460205f));
-    p2 = f2_fma(p2, f2, f2_pack(1.0000001192092896f, 1.0000001192092896f));
+    p2 = f2_fma(p2, f2, f2_pack(1.f, 1.f));
     float pa, pb, ra, rb;
     f2_unpack(p2, pa, pb);
     f2_unpack(r2, ra, rb);

@@ -461,6 +461,12 @@ __global__ void numerics_probe_kernel(int fn, size_t n, const float *__restrict_
         case 4: y = fast_log_factorial(__float_as_uint(x), t.log_factorial, t.lgamma5); break;
         case 5: y = fast_log_cell(x); break;
         case 6: y = fast_lgamma_exact(x, t.lgamma5); break;
+        case 7: {  // poly_ex2_pair, both halves fed x
+            float lo, hi;
+            f2_unpack(poly_ex2_pair(f2_pack(x, x)), lo, hi);
+            y = lo;
+            break;
+        }
     }
     out[i] = y;
 }

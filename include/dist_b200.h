@@ -330,7 +330,15 @@ int dist_b200_prior_pitman_yor_host(dist_b200_ctx *ctx, float alpha, float d, in
  *   accumulate != 0 : scores_dev[n][g] += sum_f ...        (the slave's ACCUMULATE semantic)
  *   accumulate == 0 : scores_dev[n][g]  = prior_dev[g] + sum_f ... (prior_dev may be NULL = 0;
  *                     this is clustering's OVERWRITE, clustering.hpp:195-208, followed by the slaves)
- * scores_dev is [N][G] row-major float32. */
+ * scores_dev is [N][G] row-major float32.
+ * Precondition of the continuous models: the log argument of a cell, nich's 1 + precision (x - mean)^2 and niw's
+ * 1 + q / dof, must be finite in float32.  A cell whose argument overflows scores -inf (the reference's table gives
+ * 128 ln 2); a row that overflows in every group gets -inf from score_logp_batch and an unspecified draw.  On the niw
+ * d = 32 tensor-core route such a row also makes the other rows of its 128-row tile score NaN (tile-wide scale).
+ * niw d = 32 (tensor cores): the quadratic form's error follows |W x| + |W mu'|, not |W (x - mu')|.  It matches the FP32
+ * kernel's accuracy on data and prior mean within a few standard deviations of the origin (measured); at 1e2 - 1e3
+ * standard deviations, or beside a row ~1e4 x larger in its 128-row tile, it loses precision (DESIGN §6).
+ * DIST_B200_OPT_NIW_PATH = 1 is translation-invariant. */
 int dist_b200_score_batch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
                           const void *const *columns_dev, size_t n_rows, const float *prior_dev,
                           float *scores_dev, int accumulate, void *stream);
@@ -433,7 +441,10 @@ int dist_b200_score_value_host(dist_b200_ctx *ctx, const dist_b200_feature *feat
 /* ---- numerics probes (parity tests of the device functions against special.hpp / fmath.hpp).
  * fn: 0 fast_log (table form, as used by the cache rebuilds)   1 fast_exp (sampler form)
  *     2 fast_lgamma   3 fast_lgamma_nu   4 fast_log_factorial (input bits as uint32)
- *     5 fast_log (per-cell form: truncated mantissa + MUFU.LG2) */
+ *     5 fast_log (per-cell form: truncated mantissa + MUFU.LG2; the argument must be finite: inf gives inf, where the
+ *       table gives 128 ln 2 -- see the nich / niw score entries)
+ *     6 fast_lgamma (exact restatement of the cache rebuilds)
+ *     7 exp2 on the FMA pipe (poly_ex2_pair of the sampling kernels; arguments below -125 give 2^-125) */
 int dist_b200_numerics_probe(dist_b200_ctx *ctx, int fn, size_t n, const float *in_dev, float *out_dev,
                              void *stream);
 

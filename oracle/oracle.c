@@ -567,6 +567,15 @@ static double invert(int d, double *a, double *inv) {
     return det;
 }
 
+/* fast_log(det) as the reference writes it, while det is a normal float; beyond that (the reference's float determinant()
+ * has overflowed to inf or flushed to 0, and its score is meaningless) the log of the
+ * determinant itself, as the reference's exact-math Python flavour computes it (dbg/models/niw.py:213,216) */
+static float log_det(double det, double logabsdet) {
+    const float f = (float)det;
+    if (isfinite(f) && f >= 1.17549435e-38f) return orc_fast_log(f);
+    return (float)logabsdet;
+}
+
 void orc_niw_score_rows(int d, const float *mu, float kappa, const float *psi, float nu, size_t G,
                         const int32_t *count, const float *sum_x, const float *sum_xxT, size_t n,
                         const float *values, float *scores) {
@@ -599,7 +608,7 @@ void orc_niw_score_rows(int d, const float *mu, float kappa, const float *psi, f
         for (size_t k = 0; k < dd; ++k) sig_inv[g * dd + k] = (float)inv[k];
         /* score_mv_student_t, random.hpp:160-185 (mixed float/double arithmetic as written) */
         float term1 = orc_fast_lgamma((float)(dof / 2. + (float)d / 2.)) - orc_fast_lgamma((float)(dof / 2.));
-        float term2 = (float)(-0.5 * orc_fast_log((float)det) - (float)d / 2. * (orc_fast_log(dof) + log_pi));
+        float term2 = (float)(-0.5 * log_det(det, g_logabsdet) - (float)d / 2. * (orc_fast_log(dof) + log_pi));
         konst[g * 3 + 0] = term1 + term2;
         konst[g * 3 + 1] = (float)(-0.5 * (dof + (float)d));
         konst[g * 3 + 2] = dof;
@@ -625,15 +634,6 @@ void orc_niw_score_rows(int d, const float *mu, float kappa, const float *psi, f
 /* Group::score_data (niw.hpp:296-308) summed over the groups, as SmallMixtureSlave's data scorer does for a model
  * without a FastMixture (mixture.hpp:300-319); lmultigamma is special.hpp:278-286.  The determinants are taken by
  * the Gauss-Jordan above in double (the reference: Eigen's float determinant(); Eigen is absent here). */
-/* fast_log(det) as the reference writes it, while det is a normal float; beyond that (the reference's float determinant()
- * has overflowed to inf or flushed to 0 -- at d = 32 it always does -- and its score_data is meaningless) the log of the
- * determinant itself, as the reference's exact-math Python flavour computes it (dbg/models/niw.py:213,216) */
-static float log_det(double det, double logabsdet) {
-    const float f = (float)det;
-    if (isfinite(f) && f >= 1.17549435e-38f) return orc_fast_log(f);
-    return (float)logabsdet;
-}
-
 static float orc_lmultigamma(int d, float a) {
     const float log_pi = 1.1447298858494002f;
     const float term1 = (float)(0.25 * (float)(d * (d - 1))) * log_pi;

@@ -117,7 +117,7 @@ def test_numerics_device_functions(ctx, oracle):
         0: np.concatenate([np.logspace(-37, 38, 200001), -np.logspace(-5, 5, 1001), [0.0, np.inf]]),
         2: np.logspace(-3, 9.6, 200001),
         3: np.logspace(-3, 9.6, 200001),
-        5: np.concatenate([np.logspace(0, 30, 200001), 1 + np.logspace(-7, 0, 50001)]),
+        5: np.concatenate([np.logspace(0, 30, 200001), 1 + np.logspace(-7, 0, 50001), [np.finfo(np.float32).max]]),
         6: np.logspace(-3, 9.6, 200001),
     }
     tol = {0: 0.0, 2: 1e-6, 3: 2e-6, 5: 5e-7, 6: 1e-6}
@@ -133,6 +133,11 @@ def test_numerics_device_functions(ctx, oracle):
         err = np.abs(got - want) / (1 + np.abs(want))
         err = np.where(got == want, 0.0, err)
         assert err.max() <= tol[fn], (fn, err.max(), x[np.argmax(err)])
+    # the per-cell log needs a finite argument (DESIGN §4): at inf it gives inf, where the table gives 128 ln 2
+    xd = dev(np.array([np.inf], np.float32))
+    out = torch.empty_like(xd)
+    ctx.numerics_probe(5, xd, out, 1)
+    assert out.cpu().numpy()[0] == np.inf
     # fast_exp on the sampler's domain: relative to the restated fmath::exp
     x = np.linspace(-87.0, 0.0, 200001).astype(np.float32)
     xd = dev(x)
@@ -149,6 +154,35 @@ def test_numerics_device_functions(ctx, oracle):
     out = torch.empty_like(xd)
     ctx.numerics_probe(4, xd, out, n.size)
     np.testing.assert_allclose(out.cpu().numpy(), oracle.fast_log_factorial(n), rtol=1e-6)
+
+
+def test_numerics_poly_ex2(ctx):
+    """fn 7, poly_ex2_pair (the sampling kernels' exp2 on the FMA pipe) against float64 exp2: relative 2.21e-7 over every
+    fp32 in [-1, -2^-30] (every fractional part x - round(x) the range reduction can produce, at full resolution; below
+    2^-30 the polynomial is 1 to within an ulp) and on a grid of [-125, 0], exact powers of two at integers, exactly 2^-125
+    below the clamp"""
+    bits = torch.arange(0xB0800000 - 2 ** 32, 0xBF800000 - 2 ** 32 + 1, device="cuda", dtype=torch.int64).to(torch.int32)
+    xe = bits.view(torch.float32)
+    ye = torch.empty_like(xe)
+    ctx.numerics_probe(7, xe, ye, xe.numel())
+    torch.cuda.synchronize()
+    err = (ye.double() / torch.exp2(xe.double()) - 1).abs()
+    assert float(err.max()) <= 2.21e-7, (float(err.max()), float(xe[int(torch.argmax(err))]))
+    del bits, xe, ye, err
+    x = np.concatenate([np.linspace(-125.0, 0.0, 2000001), -np.logspace(-30, 0, 10001), [0.0, -0.5, 0.5 - 1.0]]).astype(np.float32)
+    ints = np.arange(-125, 1).astype(np.float32)
+    below = np.array([-125.5, -126.0, -150.0, -1e30, -np.inf], np.float32)
+    xa = np.concatenate([x, ints, below])
+    xd = dev(xa)
+    out = torch.empty_like(xd)
+    ctx.numerics_probe(7, xd, out, xa.size)
+    torch.cuda.synchronize()
+    got = out.cpu().numpy().astype(np.float64)
+    g_x, g_i, g_b = got[:x.size], got[x.size:x.size + ints.size], got[x.size + ints.size:]
+    err = np.abs(g_x / np.exp2(x.astype(np.float64)) - 1)
+    assert err.max() <= 2.21e-7, (err.max(), x[np.argmax(err)])
+    assert np.array_equal(g_i, np.exp2(ints.astype(np.float64)))
+    assert np.all(g_b == 2.0 ** -125)
 
 
 def test_prior(ctx, oracle, golden):
