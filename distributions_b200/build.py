@@ -36,6 +36,7 @@ SOURCES = {
     "peer.cu": [],
     "niw.cu": [],
     "niw_tc.cu": [],
+    "niw_tc_wide.cu": [],
     "niw_stats.cu": [],
     "microbench.cu": [],
     "stats.cu": [],

@@ -99,7 +99,7 @@ int reserve_stats(dist_b200_feature *f, int G, bool keep) {
 // (re)allocate the hot caches for G groups, keeping the first G groups of the feature when `keep`.  Pooled models and
 // dd: params (nich also aux), padded to 128 groups so that the score kernel may stage whole register tiles, and
 // zero-filled past the kept part.  dpd: the table, (V + 2) rows of G floats (every caller rebuilds it whole).  niw: the
-// records and, at d = 32, the tensor-core images.
+// records and, at d = 32 and d > 32, the tensor-core images (sized by d).
 int ensure_params(dist_b200_feature *f, int G, bool keep) {
     dist_b200_ctx *ctx = f->ctx;
     const size_t need = static_cast<size_t>(std::max(G, 1));
@@ -109,6 +109,10 @@ int ensure_params(dist_b200_feature *f, int G, bool keep) {
         if (rec * need > f->niw_bytes)
             rc = grow(ctx, f->niw_buf, f->niw_bytes, rec * need + rec * need / 4, keep ? rec * f->G : 0);
         if (!rc && f->dim == 32 && tc > f->niw_tc_bytes) rc = grow(ctx, f->niw_tc, f->niw_tc_bytes, tc + tc / 4);
+        if (!rc && f->dim > 32) {
+            const size_t wide = sizeof(float) * niw_tc_wide_floats(static_cast<int>(need), f->dim);
+            if (wide > f->niw_tc_bytes) rc = grow(ctx, f->niw_tc, f->niw_tc_bytes, wide + wide / 4);
+        }
         return rc;
     }
     if (f->model == DIST_B200_DPD) {  // table rows + OTHER row + shift row
@@ -180,6 +184,7 @@ int rebuild(dist_b200_feature *f, int g0, int n, cudaStream_t s) {
             int rc = launch_niw_prep(ctx, d, f->alphas_dev, f->shared[0], f->alphas_dev + d, f->shared[1], n, i32(0), f32(1), f32(2),
                                      f->niw_buf + niw_rec_floats(d) * g0, s);
             if (rc == DIST_B200_OK && d == 32 && f->niw_tc && f->G > 0) rc = launch_niw_tc_prep(ctx, f->G, f->niw_buf, f->niw_tc, s);
+            if (rc == DIST_B200_OK && d > 32 && f->G > 0) rc = launch_niw_tc_wide_prep(ctx, f->G, d, f->niw_buf, f->niw_tc, s);
             return rc;
         }
         default: return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "unknown model");
@@ -425,7 +430,7 @@ int dist_b200_niw_update_all(dist_b200_feature *f, int d, const float *mu, float
     if (!check_feature(f, DIST_B200_NIW) || d < 1 || !mu || !psi || G < 0 || (G && (!count || !sum_x || !sum_xxT)))
         return DIST_B200_ERR_INVALID;
     dist_b200_ctx *ctx = f->ctx;
-    if (d > 32) return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "niw: d > 32");
+    if (d > 128) return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "niw: d > 128 (the group prep holds a d x d double Cholesky factor in shared memory)");
     if (!(kappa > 0.f) || !(nu > static_cast<float>(d) - 1.f))
         return fail(ctx, DIST_B200_ERR_INVALID, "niw: need kappa > 0 and nu > d - 1 (niw.hpp:121,132)");
     f->dim = d;
@@ -489,6 +494,7 @@ int dist_b200_feature_remove_group(dist_b200_feature *f, int groupid, void *stre
         if (groupid != last)
             DISTB200_CUDA(ctx, cudaMemcpyAsync(f->niw_buf + rec * groupid, f->niw_buf + rec * last, sizeof(float) * rec, cudaMemcpyDeviceToDevice, s));
         if (f->dim == 32 && f->niw_tc && last > 0) rc = launch_niw_tc_prep(ctx, last, f->niw_buf, f->niw_tc, s);
+        if (f->dim > 32 && last > 0) rc = launch_niw_tc_wide_prep(ctx, last, f->dim, f->niw_buf, f->niw_tc, s);
         return mark_ready(f, rc, s);
     }
     const size_t gb = sizeof(float) * group_floats(f);

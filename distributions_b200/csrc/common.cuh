@@ -146,7 +146,7 @@ struct dist_b200_feature {
     // niw
     float *niw_buf = nullptr;         // per-group records (posterior, whitening matrix, constants)
     size_t niw_bytes = 0;
-    float *niw_tc = nullptr;          // d = 32: tensor-core operand images, b vectors, constants
+    float *niw_tc = nullptr;          // d = 32 and 32 < d <= 128: tensor-core operand images, b vectors, constants
     size_t niw_tc_bytes = 0;
     void *sample_buf = nullptr;       // sample_values: per-group records of the prep pass (sample_values.cu)
     size_t sample_bytes = 0;
@@ -280,6 +280,12 @@ int launch_niw_tc_prep(dist_b200_ctx *ctx, int G, const float *recs, float *tc_b
 // scores != nullptr: [N][G] scores (optionally accumulated onto the buffer); scores == nullptr: the fused sampler writes assign[N]
 int launch_niw_tc(dist_b200_ctx *ctx, int G, const float *tc_buf, const void *values, size_t N, const float *prior,
                   float *scores, int accumulate, const float *u, int32_t *assign, cudaStream_t s);
+// niw_tc_wide.cu (tcgen05 / TMEM path, 32 < d <= 128, materialising): per-stage operand images built from the records
+size_t niw_tc_wide_floats(int G, int d);
+int launch_niw_tc_wide_prep(dist_b200_ctx *ctx, int G, int d, const float *recs, float *tc_buf, cudaStream_t s);
+// [N][G] scores of x - mu0 (mu0 = Shared.mu, the centre the records' b vectors were built around), optionally accumulated
+int launch_niw_tc_wide(dist_b200_ctx *ctx, int G, int d, const float *tc_buf, const float *mu0, const void *values, size_t N,
+                       const float *prior, float *scores, int accumulate, cudaStream_t s);
 
 // sample_values.cu: batched Group::sample_value of one feature.  The device-resident statistics it reads:
 struct SampleSrc {

@@ -77,6 +77,77 @@ __global__ void niw_prep_kernel(int d, int dp, const float *__restrict__ mu, flo
     }
 }
 
+// 32 < d <= 128: the same record at DP = 64 / 128, except that its first DP floats hold b = W (mu' - mu0) (mu0 = Shared.mu)
+// instead of mu' -- the tensor-core route scores x - mu0 against it (niw_tc_wide.cu).  One block of kNiwWideThreads per
+// group; a double [128][129] matrix is 132 KB, so W = L^-1 overwrites L in place (dynamic shared memory).
+constexpr int kNiwWideThreads = 256;
+constexpr int kNiwWideLd = 129;
+constexpr size_t kNiwWidePrepSmem = sizeof(double) * (128 * kNiwWideLd + 4 * 128);
+
+__global__ void __launch_bounds__(kNiwWideThreads) niw_prep_wide_kernel(int d, int dp, const float *__restrict__ mu, float kappa,
+                                                                        const float *__restrict__ psi, float nu,
+                                                                        const int32_t *__restrict__ count, const float *__restrict__ sum_x,
+                                                                        const float *__restrict__ sum_xxT, float *__restrict__ out,
+                                                                        NumericTables t) {
+    extern __shared__ double wsm[];
+    double(*S)[kNiwWideLd] = reinterpret_cast<double(*)[kNiwWideLd]>(wsm);  // sigma, then L (lower), then W = L^-1 (lower)
+    double *xbar = wsm + 128 * kNiwWideLd, *diff = xbar + 128, *col = diff + 128, *dm = col + 128;
+    __shared__ double det_s[2];
+    const int g = blockIdx.x, tid = threadIdx.x;
+    const double dof = niw_posterior_cholesky<kNiwWideLd>(d, mu, kappa, psi, nu, count[g], sum_x + static_cast<size_t>(g) * d,
+                                                          sum_xxT + static_cast<size_t>(g) * d * d, S, xbar, diff);
+    if (tid == 0) {
+        double det = 1.0, logdet = 0.0;
+        for (int i = 0; i < d; ++i) {
+            det *= S[i][i] * S[i][i];
+            logdet += 2.0 * log(S[i][i]);
+        }
+        det_s[0] = det;
+        det_s[1] = logdet;
+    }
+    if (tid < d) dm[tid] = niw_post_mu(kappa, count[g], mu[tid], xbar[tid]) - static_cast<double>(mu[tid]);
+    // in-place inverse, right to left: with L = [l 0; c L2], W = [1/l 0; -L2^-1 c / l  L2^-1], so column j of W needs
+    // column j of L (saved first) and the columns right of j, which already hold W
+    for (int j = d - 1; j >= 0; --j) {
+        __syncthreads();
+        if (tid > j && tid < d) col[tid] = S[tid][j];
+        __syncthreads();
+        const double ljj = S[j][j];
+        __syncthreads();
+        if (tid > j && tid < d) {
+            double s = 0.0;
+            for (int k = j + 1; k <= tid; ++k) s += S[tid][k] * col[k];
+            S[tid][j] = -s / ljj;
+        }
+        if (tid == j) S[j][j] = 1.0 / ljj;
+    }
+    __syncthreads();
+    float *rec = out + static_cast<size_t>(g) * niw_group_floats(dp);
+    for (int i = tid; i < dp; i += blockDim.x) {
+        double b = 0.0;
+        if (i < d)
+            for (int k = 0; k <= i; ++k) b += S[i][k] * dm[k];
+        rec[i] = static_cast<float>(b);
+    }
+    for (int e = tid; e < dp * dp; e += blockDim.x) {
+        const int i = e / dp, j = e % dp;
+        rec[dp + e] = (i < d && j <= i) ? static_cast<float>(S[i][j]) : 0.f;
+    }
+    if (tid == 0) {  // as niw_prep_kernel
+        const float dof_f = static_cast<float>(dof);
+        const float log_pi = 1.1447298858494002f;
+        const float term1 = fast_lgamma_exact(static_cast<float>(dof_f / 2. + static_cast<float>(d) / 2.), t.lgamma5) -
+                            fast_lgamma_exact(static_cast<float>(dof_f / 2.), t.lgamma5);
+        const float term2 = static_cast<float>(-0.5 * niw_log_det(det_s[0], det_s[1], t.log2_table) -
+                                               static_cast<float>(d) / 2. * (fast_log_table(dof_f, t.log2_table) + log_pi));
+        float *k4 = rec + dp + dp * dp;
+        k4[0] = term1 + term2;
+        k4[1] = static_cast<float>(-0.5 * (dof_f + static_cast<float>(d))) * kLn2;
+        k4[2] = 1.f / dof_f;
+        k4[3] = 0.f;
+    }
+}
+
 int niw_padded_dim(int d);
 
 constexpr int kNiwThreads = 128;
@@ -473,12 +544,19 @@ int launch_niw_rows_small(dist_b200_ctx *ctx, const dist_b200_feature *f, const 
     return launch_niw_rows_t<8, 2>(ctx, a, s);
 }
 
-int niw_padded_dim(int d) { return d <= 4 ? 4 : (d <= 8 ? 8 : (d <= 16 ? 16 : 32)); }
+int niw_padded_dim(int d) { return d <= 4 ? 4 : (d <= 8 ? 8 : (d <= 16 ? 16 : (d <= 32 ? 32 : (d <= 64 ? 64 : 128)))); }
 
 int launch_niw_prep(dist_b200_ctx *ctx, int d, const float *mu, float kappa, const float *psi, float nu, int G,
                     const int32_t *count, const float *sum_x, const float *sum_xxT, float *recs, cudaStream_t s) {
     if (G <= 0) return DIST_B200_OK;
-    niw_prep_kernel<<<G, 64, 0, s>>>(d, niw_padded_dim(d), mu, kappa, psi, nu, count, sum_x, sum_xxT, recs, ctx->tables);
+    if (d <= 32) {
+        niw_prep_kernel<<<G, 64, 0, s>>>(d, niw_padded_dim(d), mu, kappa, psi, nu, count, sum_x, sum_xxT, recs, ctx->tables);
+    } else {
+        DISTB200_CUDA(ctx, cudaFuncSetAttribute(niw_prep_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                static_cast<int>(kNiwWidePrepSmem)));
+        niw_prep_wide_kernel<<<G, kNiwWideThreads, kNiwWidePrepSmem, s>>>(d, niw_padded_dim(d), mu, kappa, psi, nu, count, sum_x,
+                                                                           sum_xxT, recs, ctx->tables);
+    }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail(ctx, DIST_B200_ERR_CUDA, std::string("niw prep launch: ") + cudaGetErrorString(e));
     return DIST_B200_OK;
@@ -487,6 +565,8 @@ int launch_niw_prep(dist_b200_ctx *ctx, int d, const float *mu, float kappa, con
 int launch_niw_scores(dist_b200_ctx *ctx, const dist_b200_feature *f, const void *values, size_t N,
                       const float *prior, float *scores, int accumulate, cudaStream_t s) {
     if (N == 0 || f->G == 0) return DIST_B200_OK;
+    // 32 < d <= 128: tcgen05 on x - mu0, the only route there
+    if (f->dim > 32) return launch_niw_tc_wide(ctx, f->G, f->dim, f->niw_tc, f->alphas_dev, values, N, prior, scores, accumulate, s);
     // d = 32: tcgen05 with split fp16 operands; DIST_B200_OPT_NIW_PATH = 1 keeps the FP32 CUDA-core kernel for A/B runs
     if (f->dim == 32 && f->niw_tc && ctx->opt[DIST_B200_OPT_NIW_PATH] == 0) {
         const int rc = launch_niw_tc(ctx, f->G, f->niw_tc, values, N, prior, scores, accumulate, nullptr, nullptr, s);

@@ -122,6 +122,57 @@ __global__ void __launch_bounds__(kNsThreads) niw_accumulate_kernel(const NiwAcc
     }
 }
 
+// 32 < d <= 128: the d x d SYRK tiled over the output -- a work item is (unit, chunk of 4 x 256 matrix entries), so every
+// thread still holds 4 accumulators; a unit's rows are staged once per chunk (they come from L2 after the first).
+__global__ void __launch_bounds__(kNsThreads) niw_accumulate_wide_kernel(const NiwAccArgs a) {
+    __shared__ float xs[32][129];
+    const int tid = threadIdx.x, d = a.d, dd = d * d;
+    constexpr int kChunk = 4 * kNsThreads;
+    const int nchunks = (dd + kChunk - 1) / kChunk;
+    const long long total = static_cast<long long>(a.unit_off[a.G]) * nchunks;
+    for (long long w = blockIdx.x; w < total; w += gridDim.x) {
+        const int u = static_cast<int>(w / nchunks), ch = static_cast<int>(w - static_cast<long long>(u) * nchunks);
+        int lo = 0, hi = a.G;
+        while (hi - lo > 1) {
+            const int mid = (lo + hi) >> 1;
+            if (a.unit_off[mid] <= u) lo = mid;
+            else hi = mid;
+        }
+        const int g = lo;
+        const int first = a.offsets[g] + (u - a.unit_off[g]) * kNsSlice;
+        const int last = min(first + kNsSlice, a.offsets[g + 1]);
+        int ei[4], ej[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const int e = ch * kChunk + tid + kNsThreads * k;
+            ei[k] = e < dd ? e / d : -1;
+            ej[k] = e < dd ? e % d : 0;
+        }
+        double m[4] = {0.0, 0.0, 0.0, 0.0}, sx = 0.0;
+        for (int r0 = first; r0 < last; r0 += 32) {
+            const int nr = min(32, last - r0);
+            __syncthreads();
+            for (int e = tid; e < 32 * d; e += kNsThreads) {
+                const int r = e / d, k = e - r * d;
+                xs[r][k] = r < nr ? a.values[static_cast<size_t>(a.perm[r0 + r]) * d + k] : 0.f;
+            }
+            __syncthreads();
+            for (int r = 0; r < nr; ++r) {
+#pragma unroll
+                for (int k = 0; k < 4; ++k)
+                    if (ei[k] >= 0) m[k] = fma(static_cast<double>(xs[r][ei[k]]), static_cast<double>(xs[r][ej[k]]), m[k]);
+                if (ch == 0 && tid < d) sx += static_cast<double>(xs[r][tid]);
+            }
+        }
+        double *out = a.acc + static_cast<size_t>(g) * (1 + d + dd);
+        if (ch == 0 && tid == 0) atomicAdd(out, static_cast<double>(last - first));
+        if (ch == 0 && tid < d) atomicAdd(out + 1 + tid, sx);
+#pragma unroll
+        for (int k = 0; k < 4; ++k)
+            if (ei[k] >= 0) atomicAdd(out + 1 + d + ch * kChunk + tid + kNsThreads * k, m[k]);
+    }
+}
+
 // resident float statistics += sign * accumulated block; a group the batch empties is reset to exact zeros (what
 // Group::init gives the next value that joins it; the reference's float subtraction leaves rounding residue there)
 __global__ void niw_apply_kernel(int G, int d, int sign, const double *__restrict__ acc, int32_t *__restrict__ count,
@@ -168,7 +219,12 @@ int launch_niw_accumulate(dist_b200_ctx *ctx, int G, int d, const void *values, 
     niw_scatter_kernel<<<static_cast<unsigned>(want < cap ? want : cap), 256, 0, s>>>(assign, N, G, cursor, perm);
     NiwAccArgs a{G, d, static_cast<const float *>(values), offsets, unit_off, perm, acc};
     const size_t units_bound = N / kNsSlice + G + 1;
-    niw_accumulate_kernel<<<static_cast<unsigned>(units_bound < cap ? units_bound : cap), kNsThreads, 0, s>>>(a);
+    if (d <= 32) {
+        niw_accumulate_kernel<<<static_cast<unsigned>(units_bound < cap ? units_bound : cap), kNsThreads, 0, s>>>(a);
+    } else {
+        const size_t items = units_bound * ((static_cast<size_t>(d) * d + 4 * kNsThreads - 1) / (4 * kNsThreads));
+        niw_accumulate_wide_kernel<<<static_cast<unsigned>(items < cap ? items : cap), kNsThreads, 0, s>>>(a);
+    }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail(ctx, DIST_B200_ERR_CUDA, std::string("niw add_rows launch: ") + cudaGetErrorString(e));
     return DIST_B200_OK;
@@ -272,6 +328,72 @@ __global__ void __launch_bounds__(64) niw_score_data_kernel(const NiwScoreDataAr
     }
 }
 
+// 32 < d <= 128: one [d][129] double matrix (dynamic shared memory) serves both factorisations in turn -- the prior's
+// psi first, then the posterior's -- with the Cholesky of chol_logdet_free.
+constexpr int kSdWideLd = 129;
+constexpr size_t kSdWideSmem = sizeof(double) * (128 * kSdWideLd + 2 * 128);
+
+__global__ void __launch_bounds__(128) niw_score_data_wide_kernel(const NiwScoreDataArgs a, NumericTables t) {
+    extern __shared__ double sdm[];
+    double(*S)[kSdWideLd] = reinterpret_cast<double(*)[kSdWideLd]>(sdm);
+    double *xbar = sdm + 128 * kSdWideLd, *diff = xbar + 128;
+    __shared__ double det_prior[2], det_post[2];
+    const int g = blockIdx.x, tid = threadIdx.x, d = a.d;
+    const float *sh = a.shareds + blockIdx.y * a.stride;
+    const float kappa = sh[0], nu = sh[1];
+    const float *mu = sh + 2, *psi = sh + 2 + d;
+    const float *sx = a.sum_x + static_cast<size_t>(g) * d, *sxx = a.sum_xxT + static_cast<size_t>(g) * d * d;
+    const int cnt = a.count[g];
+    const double n = cnt, kap = kappa;
+    auto chol = [&](double *det_out) {
+        for (int k = 0; k < d; ++k) {
+            if (tid == 0) S[k][k] = sqrt(S[k][k]);
+            __syncthreads();
+            if (tid > k && tid < d) S[tid][k] /= S[k][k];
+            __syncthreads();
+            for (int e = tid; e < d * d; e += blockDim.x) {
+                const int i = e / d, j = e % d;
+                if (j > k && i >= j) S[i][j] -= S[i][k] * S[j][k];
+            }
+            __syncthreads();
+        }
+        if (tid == 0) {
+            double det = 1.0, logdet = 0.0;
+            for (int i = 0; i < d; ++i) {
+                det *= S[i][i] * S[i][i];
+                logdet += 2.0 * log(S[i][i]);
+            }
+            det_out[0] = det;
+            det_out[1] = logdet;
+        }
+        __syncthreads();
+    };
+    for (int e = tid; e < d * d; e += blockDim.x) S[e / d][e % d] = static_cast<double>(psi[e]);
+    if (tid < d) {
+        xbar[tid] = cnt ? static_cast<double>(sx[tid]) / n : 0.0;
+        diff[tid] = xbar[tid] - static_cast<double>(mu[tid]);
+    }
+    __syncthreads();
+    chol(det_prior);
+    for (int e = tid; e < d * d; e += blockDim.x) {
+        const int i = e / d, j = e % d;
+        const double c_n = static_cast<double>(sxx[e]) - static_cast<double>(sx[i]) * xbar[j] - xbar[i] * static_cast<double>(sx[j]) + n * xbar[i] * xbar[j];
+        S[i][j] = static_cast<double>(psi[e]) + c_n + kap * n / (kap + n) * diff[i] * diff[j];
+    }
+    __syncthreads();
+    chol(det_post);
+    if (tid == 0) {  // as niw_score_data_kernel
+        const float log_pi = 1.1447298858494002f;
+        const float post_nu = nu + static_cast<float>(cnt), post_kappa = kappa + static_cast<float>(cnt);
+        const float score = lmultigamma_dev(d, static_cast<float>(post_nu * 0.5), t) +
+                            static_cast<float>(nu * 0.5) * niw_log_det(det_prior[0], det_prior[1], t.log2_table) -
+                            static_cast<float>(static_cast<float>(cnt * d) * 0.5) * log_pi - lmultigamma_dev(d, static_cast<float>(nu * 0.5), t) -
+                            static_cast<float>(post_nu * 0.5) * niw_log_det(det_post[0], det_post[1], t.log2_table) +
+                            static_cast<float>(static_cast<float>(d) * 0.5) * fast_log_table(kappa / post_kappa, t.log2_table);
+        atomicAdd(a.acc + blockIdx.y, static_cast<double>(score));
+    }
+}
+
 int launch_niw_score_data(dist_b200_ctx *ctx, int G, int d, const int32_t *count, const float *sum_x, const float *sum_xxT,
                           const float *shareds_dev, size_t n_grid, size_t stride, double *acc, cudaStream_t s) {
     if (n_grid == 0 || G <= 0) return DIST_B200_OK;
@@ -281,7 +403,13 @@ int launch_niw_score_data(dist_b200_ctx *ctx, int G, int d, const int32_t *count
         const size_t n = n_grid - i0 < 65535 ? n_grid - i0 : 65535;
         b.shareds = shareds_dev + i0 * stride;
         b.acc = acc + i0;
-        niw_score_data_kernel<<<dim3(static_cast<unsigned>(G), static_cast<unsigned>(n)), 64, 0, s>>>(b, ctx->tables);
+        if (d <= 32) {
+            niw_score_data_kernel<<<dim3(static_cast<unsigned>(G), static_cast<unsigned>(n)), 64, 0, s>>>(b, ctx->tables);
+        } else {
+            DISTB200_CUDA(ctx, cudaFuncSetAttribute(niw_score_data_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                    static_cast<int>(kSdWideSmem)));
+            niw_score_data_wide_kernel<<<dim3(static_cast<unsigned>(G), static_cast<unsigned>(n)), 128, kSdWideSmem, s>>>(b, ctx->tables);
+        }
     }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail(ctx, DIST_B200_ERR_CUDA, std::string("niw score_data launch: ") + cudaGetErrorString(e));

@@ -41,10 +41,11 @@ __device__ __forceinline__ float2 bb_plus_group(float alpha, float beta, int32_t
 // NormalInverseWishart: Shared::plus_group (niw.hpp:82-103) for one group's statistics (count, sum_x[d], sum_xxT[d][d])
 // and the Cholesky factor of the Student-t scale of Scorer::eval (niw.hpp:343-361),
 //   sigma = psi' (kappa' + 1) / (kappa' dof),  dof = nu' - d + 1,
-// in double.  Block-cooperative: every thread of the block calls it (d <= 32).  On return S[i][j], j <= i, holds L with
-// sigma = L L^T (the upper triangle is scratch), xbar the group mean; the return value is dof.
+// in double.  Block-cooperative: every thread of the block calls it (d <= LD - 1 and d <= blockDim.x).  On return S[i][j],
+// j <= i, holds L with sigma = L L^T (the upper triangle is scratch), xbar the group mean; the return value is dof.
+template <int LD>
 __device__ __forceinline__ double niw_posterior_cholesky(int d, const float *mu, float kappa, const float *psi, float nu,
-                                                         int32_t count, const float *sx, const float *sxx, double (*S)[33],
+                                                         int32_t count, const float *sx, const float *sxx, double (*S)[LD],
                                                          double *xbar, double *diff) {
     const int tid = threadIdx.x;
     const double n = static_cast<double>(count);

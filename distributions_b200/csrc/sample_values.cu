@@ -251,6 +251,31 @@ __global__ void niw_sample_prep_kernel(const SampleSrc src, float *__restrict__ 
     if (tid == 0) rec[W + d * W] = static_cast<float>(0.5 * dof);
 }
 
+// 32 < d <= 128: the same record with niw_wide_cols(d) columns per Lt row; a double [128][129] matrix (dynamic shared memory)
+__host__ __device__ constexpr int niw_wide_cols(int d) { return (d + 31) / 32 * 32; }
+__host__ __device__ constexpr int niw_wide_sample_floats(int d) { return niw_wide_cols(d) * (d + 1) + 1; }
+constexpr int kNiwWideLd = 129;
+constexpr size_t kNiwWideSampleSmem = sizeof(double) * (128 * kNiwWideLd + 2 * 128);
+
+__global__ void __launch_bounds__(256) niw_sample_prep_wide_kernel(const SampleSrc src, float *__restrict__ out) {
+    extern __shared__ double ssm[];
+    double(*S)[kNiwWideLd] = reinterpret_cast<double(*)[kNiwWideLd]>(ssm);
+    double *xbar = ssm + 128 * kNiwWideLd, *diff = xbar + 128;
+    const int g = blockIdx.x, tid = threadIdx.x, d = src.dim, W = niw_wide_cols(d);
+    const float *mu = src.alphas, *psi = src.alphas + d;
+    const int32_t count = reinterpret_cast<const int32_t *>(src.st0)[g];
+    const float *sx = reinterpret_cast<const float *>(src.st1) + static_cast<size_t>(g) * d;
+    const float *sxx = reinterpret_cast<const float *>(src.st2) + static_cast<size_t>(g) * d * d;
+    const double dof = niw_posterior_cholesky<kNiwWideLd>(d, mu, src.shared[0], psi, src.shared[1], count, sx, sxx, S, xbar, diff);
+    float *rec = out + static_cast<size_t>(g) * niw_wide_sample_floats(d);
+    for (int i = tid; i < W; i += blockDim.x) rec[i] = i < d ? static_cast<float>(niw_post_mu(src.shared[0], count, mu[i], xbar[i])) : 0.f;
+    for (int e = tid; e < d * W; e += blockDim.x) {
+        const int k = e / W, i = e % W;
+        rec[W + e] = (i < d && i >= k) ? static_cast<float>(S[i][k]) : 0.f;
+    }
+    if (tid == 0) rec[W + d * W] = static_cast<float>(0.5 * dof);
+}
+
 // ---- rows ----------------------------------------------------------------------------------------------------------
 template <int MODEL>
 __global__ void __launch_bounds__(256) sample_rows_kernel(const SampleArgs a) {
@@ -319,6 +344,52 @@ __global__ void __launch_bounds__(256) niw_sample_rows_kernel(const SampleArgs a
     }
 }
 
+// 32 < d <= 128: one warp per row, lane c owns coordinates c, c + 32, ...: z_c from block c of the row's stream, the
+// chi-square from block max(32, d) on (lane 0), so no block serves two quantities
+__global__ void __launch_bounds__(256) niw_sample_rows_wide_kernel(const SampleArgs a) {
+    const int lane = threadIdx.x & 31, d = a.d, W = a.W;
+    const size_t warp = (static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+    const size_t warps = (static_cast<size_t>(gridDim.x) * blockDim.x) >> 5;
+    for (size_t n = warp; n < a.N; n += warps) {
+        const int g = a.assign[n];
+        if (g < 0 || g >= a.G) continue;
+        const float *rec = a.niw + static_cast<size_t>(g) * a.niw_stride;
+        float z[4] = {0.f, 0.f, 0.f, 0.f}, s = 0.f;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const int c = lane + 32 * j;
+            if (c < d) {
+                ValueRng r(a.seed, a.row0 + n, a.feature, c);
+                z[j] = static_cast<float>(r.normal());
+            }
+        }
+        if (lane == 0) {
+            const double h = rec[W + d * W];
+            ValueRng r(a.seed, a.row0 + n, a.feature, d > 32 ? d : 32);
+            s = static_cast<float>(exp(0.5 * (log(h) - log_gamma_draw(r, h))));
+        }
+        s = __shfl_sync(0xffffffffu, s, 0);
+        float acc[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+        for (int jk = 0; jk < 4; ++jk) {
+            if (32 * jk >= d) break;
+            for (int kk = 0; kk < 32; ++kk) {
+                const int k = 32 * jk + kk;
+                const float zk = __shfl_sync(0xffffffffu, z[jk], kk);
+                if (k >= d) continue;
+#pragma unroll
+                for (int j = 0; j < 4; ++j)
+                    if (32 * j < W) acc[j] = fmaf(rec[W + k * W + lane + 32 * j], zk, acc[j]);  // zero above L's diagonal
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const int c = lane + 32 * j;
+            if (c < d) static_cast<float *>(a.out)[n * d + c] = fmaf(s, acc[j], rec[c]);
+        }
+    }
+}
+
 }  // namespace
 
 #define SAMPLE_LAUNCH_CHECK(ctx)                                                                               \
@@ -333,7 +404,7 @@ static size_t sample_buf_bytes(const SampleSrc &src) {
     switch (src.model) {
         case DIST_B200_DD: return round_up(G * src.dim * 8, 256) + round_up(G * src.dim * 4, 256);
         case DIST_B200_DPD: return round_up(G * (src.dim + 1) * 8, 256) + round_up(G * (src.dim + 1) * 4, 256) + round_up(4 * static_cast<size_t>(src.dim), 256);
-        case DIST_B200_NIW: return G * niw_sample_floats(src.dim) * 4;
+        case DIST_B200_NIW: return G * (src.dim > 32 ? niw_wide_sample_floats(src.dim) : niw_sample_floats(src.dim)) * 4;
         default: return G * sizeof(Rec);
     }
 }
@@ -377,6 +448,20 @@ int launch_sample_values(dist_b200_ctx *ctx, dist_b200_feature *f, const SampleS
         } break;
         case DIST_B200_NIW: {
             float *recs = reinterpret_cast<float *>(buf);
+            if (src.dim > 32) {
+                DISTB200_CUDA(ctx, cudaFuncSetAttribute(niw_sample_prep_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                        static_cast<int>(kNiwWideSampleSmem)));
+                niw_sample_prep_wide_kernel<<<src.G, 256, kNiwWideSampleSmem, s>>>(src, recs);
+                SAMPLE_LAUNCH_CHECK(ctx);
+                a.d = src.dim;
+                a.W = niw_wide_cols(src.dim);
+                a.niw = recs;
+                a.niw_stride = niw_wide_sample_floats(src.dim);
+                const unsigned nb = static_cast<unsigned>(std::max<size_t>(1, std::min<size_t>((N * 32 + threads - 1) / threads,
+                                                                                               static_cast<size_t>(ctx->sm_count) * 32)));
+                niw_sample_rows_wide_kernel<<<nb, threads, 0, s>>>(a);
+                break;
+            }
             niw_sample_prep_kernel<<<src.G, 64, 0, s>>>(src, recs);
             SAMPLE_LAUNCH_CHECK(ctx);
             a.d = src.dim;

@@ -269,7 +269,8 @@ int wire_decode(dist_b200_ctx *ctx, int model, const void *shared_msg, size_t sh
         case DIST_B200_NIW: {  // schema.proto:147-161; Shared::protobuf_load niw.hpp:105-134, Group::protobuf_load :192-216
             if (!parse(shared_msg, shared_len, "\0ffff", sh)) return bad("malformed NormalInverseWishart.Shared");
             const size_t d = sh.f[1].size();
-            if (d < 1 || d > 32) return bad("NormalInverseWishart.Shared: dim must be 1..32");
+            if (d < 1) return bad("NormalInverseWishart.Shared: dim must be at least 1");
+            if (d > 128) return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "wire: NormalInverseWishart.Shared: dim above 128 is not supported");
             if (sh.f[2].empty() || sh.f[4].empty()) return bad("NormalInverseWishart.Shared: missing required field");
             if (sh.f[3].size() != d * d) return bad("NormalInverseWishart.Shared: psi is not dim x dim (niw.hpp:92-94)");
             const float kappa = sh.f[2].back(), nu = sh.f[4].back();
@@ -454,8 +455,8 @@ int wire_encode_shared(dist_b200_ctx *ctx, int model, const float *shared, size_
         }
         case DIST_B200_NIW: {  // mu, kappa, psi, nu (niw.hpp:136-156)
             size_t d = 1;
-            while (d <= 32 && 2 + d + d * d != n_shared) ++d;
-            if (!shared || d > 32) break;
+            while (d <= 128 && 2 + d + d * d != n_shared) ++d;
+            if (!shared || d > 128) break;
             for (size_t k = 0; k < d; ++k) put_float(1, shared[2 + k]);
             put_float(2, shared[0]);
             for (size_t k = 0; k < d * d; ++k) put_float(3, shared[2 + d + k]);

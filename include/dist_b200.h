@@ -73,7 +73,8 @@ typedef enum {
                                       2 = the shortcut with 8-ary tree search instead of the guide-table walk (G <= 1024) */
     DIST_B200_OPT_ROW_TILE = 1,    /* score_rows register tile for G > 128: 0 = default (32; 64 when the [N][G] scores are written), else 32 / 64 */
     DIST_B200_OPT_HOST_CHUNKS = 2, /* row chunks of the host-buffer entry: 0 = default (5) */
-    DIST_B200_OPT_NIW_PATH = 3,    /* d = 32: 0 = tcgen05 kernel, split fp16 operands (default), 1 = FP32 CUDA-core kernel */
+    DIST_B200_OPT_NIW_PATH = 3,    /* d = 32: 0 = tcgen05 kernel, split fp16 operands (default), 1 = FP32 CUDA-core kernel;
+                                      no effect at other d (32 < d <= 128 has one route, the centred tcgen05 kernel) */
     DIST_B200_OPT_TABLE_KERNEL = 4,/* dpd no-shortcut kernel: 0 = register kernel on the lane-segment layout (owner lane's walk staged through
                                       shared memory), 1 = round-1 gather kernel, 2 = register kernel with the walk inside the row loop (G in (384, 512]) */
     DIST_B200_OPT_SMALL_TILE = 5,  /* score_rows, single feature, 64 < G <= 128: 0 = default, 1 = one 128-group tile x 256 threads
@@ -128,7 +129,10 @@ int dist_b200_dpd_update_all(dist_b200_feature *f, float alpha, float beta0, int
 /* NormalInverseWishart<d> has no Mixture in the reference; this is the batched form of looping
  * Group::score_value over groups (mixture.hpp:321-337 semantics; niw.hpp:82-103, :343-361,
  * random.hpp:160-185).  psi and sum_xxT[g] are [d][d] row-major; Group = {count, sum_x, sum_xxT}
- * (niw.hpp:187-190). */
+ * (niw.hpp:187-190).  1 <= d <= 128; d > 128 returns DIST_B200_ERR_UNSUPPORTED (the group prep holds a d x d double
+ * Cholesky factor in shared memory).  Scoring routes by d: d <= 8 sampling only, the fused FP32 kernel; d <= 32 the FP32
+ * CUDA-core kernel, except d = 32: tcgen05 with split fp16 operands (DIST_B200_OPT_NIW_PATH); 32 < d <= 128: tcgen05 on
+ * x - mu (Shared.mu) padded to 64 / 128, scores materialised and sampled / reduced by the stand-alone kernels. */
 int dist_b200_niw_update_all(dist_b200_feature *f, int d, const float *mu, float kappa, const float *psi,
                              float nu, int G, const int32_t *count, const float *sum_x,
                              const float *sum_xxT, void *stream);
@@ -209,6 +213,8 @@ int dist_b200_add_rows_batch_host(dist_b200_ctx *ctx, dist_b200_feature *const *
  * draw index within the value).  A draw is a pure function of (seed, row0 + n, i, that group's statistics), independent
  * of launch geometry, n_rows and chunking: row shards passing their own row0 reproduce a single call bit for bit.  Two
  * features drawn in separate calls at the same list position get the same random stream: give such calls distinct seeds.
+ * niw: coordinate c of a row draws its normal from block c of the row's stream and the chi-square from block max(32, d)
+ * on, so no block serves two quantities at any d <= 128 (the draws at d <= 32 use block 32, as before).
  * The host form stages through the context (the output columns travel both ways, so skipped rows keep their values);
  * its results are bit-identical to the device form.  Synchronous. */
 int dist_b200_sample_values_batch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
@@ -338,7 +344,12 @@ int dist_b200_prior_pitman_yor_host(dist_b200_ctx *ctx, float alpha, float d, in
  * niw d = 32 (tensor cores): the quadratic form's error follows |W x| + |W mu'|, not |W (x - mu')|.  It matches the FP32
  * kernel's accuracy on data and prior mean within a few standard deviations of the origin (measured); at 1e2 - 1e3
  * standard deviations, or beside a row ~1e4 x larger in its 128-row tile, it loses precision (DESIGN §6).
- * DIST_B200_OPT_NIW_PATH = 1 is translation-invariant. */
+ * DIST_B200_OPT_NIW_PATH = 1 is translation-invariant.
+ * niw 32 < d <= 128 (tensor cores, centred): the rows are split after subtracting Shared.mu and the groups' offsets
+ * W (mu' - mu) are formed in double, so the error follows |W (x - mu)| + |W (mu' - mu)| -- the data's spread around the
+ * prior mean, not its offset from the origin -- within the derived bound of DESIGN §6 ("d > 32").  As at d = 32 the scale
+ * is per 128-row tile: a row far larger than its tile-mates (|x - mu| ~ 1e4 x) costs them precision, and a row whose
+ * scaled square overflows makes them NaN. */
 int dist_b200_score_batch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
                           const void *const *columns_dev, size_t n_rows, const float *prior_dev,
                           float *scores_dev, int accumulate, void *stream);
