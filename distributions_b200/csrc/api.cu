@@ -37,6 +37,65 @@ int ensure_pinned(dist_b200_ctx *ctx, size_t bytes) {
     return DIST_B200_OK;
 }
 
+// Host arrays staged through the context scratch: region() lays out 256-byte aligned regions, reserve() grows the
+// device scratch (and the page-locked mirror ctx->pinned over the first `mirror` bytes, same offsets), put / get copy
+// between host arrays and regions, through the mirror when asked.  Every stream it was handed is drained when it leaves
+// scope, on every return path: no copy into the caller's buffers or out of the mirror is still queued when an entry
+// returns, and the next host entry may overwrite the scratch.
+struct Staging {
+    dist_b200_ctx *ctx;
+    cudaStream_t streams[2];
+    int n_streams;
+    size_t bytes = 0;
+    Staging(dist_b200_ctx *c, cudaStream_t s) : ctx(c), streams{s, s}, n_streams(1) {}
+    Staging(dist_b200_ctx *c, cudaStream_t s0, cudaStream_t s1) : ctx(c), streams{s0, s1}, n_streams(2) {}
+    ~Staging() {
+        for (int i = 0; i < n_streams; ++i) cudaStreamSynchronize(streams[i]);
+    }
+    size_t region(size_t n) {
+        const size_t off = bytes;
+        bytes += round_up(n, 256);
+        return off;
+    }
+    int reserve(size_t mirror = 0) {
+        if (int rc = ensure_pinned(ctx, mirror)) return rc;
+        return ensure_scratch(ctx, bytes + 256);
+    }
+    template <class T = char>
+    T *dev(size_t off) const { return reinterpret_cast<T *>(static_cast<char *>(ctx->scratch_dev) + off); }
+    char *pin(size_t off) const { return static_cast<char *>(ctx->pinned) + off; }
+    int put(size_t off, const void *host, size_t n, cudaStream_t s, bool via_mirror = false) {
+        if (via_mirror) host = std::memcpy(pin(off), host, n);
+        DISTB200_CUDA(ctx, cudaMemcpyAsync(dev(off), host, n, cudaMemcpyHostToDevice, s));
+        return DIST_B200_OK;
+    }
+    // via the mirror the bytes land at pin(off): the caller copies them out after drain()
+    int get(void *host, size_t off, size_t n, cudaStream_t s, bool via_mirror = false) {
+        DISTB200_CUDA(ctx, cudaMemcpyAsync(via_mirror ? pin(off) : host, dev(off), n, cudaMemcpyDeviceToHost, s));
+        return DIST_B200_OK;
+    }
+    int drain() {
+        for (int i = 0; i < n_streams; ++i) DISTB200_CUDA(ctx, cudaStreamSynchronize(streams[i]));
+        n_streams = 0;  // drained: nothing left for the destructor
+        return DIST_B200_OK;
+    }
+};
+
+// a clustering prior over G host group sizes on `s`: launch(sizes_dev, prior, s) writes prior_dev or, with prior_host,
+// the scratch that is copied out to the host array
+template <class Launch>
+int prior_from_host_sizes(dist_b200_ctx *ctx, int G, const int32_t *group_sizes, float *prior_dev, float *prior_host,
+                          cudaStream_t s, Launch launch) {
+    Staging stage(ctx, s);
+    const size_t sizes_off = stage.region(sizeof(int32_t) * G), out_off = stage.region(sizeof(float) * G);
+    int rc;
+    if ((rc = stage.reserve()) || (rc = stage.put(sizes_off, group_sizes, sizeof(int32_t) * G, s)) ||
+        (rc = launch(stage.dev<const int32_t>(sizes_off), prior_host ? stage.dev<float>(out_off) : prior_dev, s)) ||
+        (prior_host && (rc = stage.get(prior_host, out_off, sizeof(float) * G, s))))
+        return rc;
+    return stage.drain();
+}
+
 
 // per-group floats of the hot layout
 size_t group_floats(const dist_b200_feature *f) {
@@ -131,26 +190,6 @@ int ensure_params(dist_b200_feature *f, int G, bool keep) {
     f->capacity = static_cast<int>(f->params_bytes / gb);
     return DIST_B200_OK;
 }
-
-// copy host arrays into consecutive, 256-byte aligned regions of the context scratch
-struct Upload {
-    dist_b200_ctx *ctx;
-    cudaStream_t s;
-    size_t off = 0;
-    int err = DIST_B200_OK;
-    template <class T>
-    const T *put(const T *host, size_t n) {
-        if (err) return nullptr;
-        char *dst = static_cast<char *>(ctx->scratch_dev) + off;
-        cudaError_t e = cudaMemcpyAsync(dst, host, n * sizeof(T), cudaMemcpyHostToDevice, s);
-        if (e != cudaSuccess) {
-            err = fail(ctx, DIST_B200_ERR_CUDA, std::string("upload: ") + cudaGetErrorString(e));
-            return nullptr;
-        }
-        off += round_up(n * sizeof(T), 256);
-        return reinterpret_cast<const T *>(dst);
-    }
-};
 
 // recompute the caches of groups [g0, g0 + n) from the resident statistics.  The prep launchers read group i of their
 // inputs from the pointers given and write cache g0 + i.
@@ -691,7 +730,7 @@ int dist_b200_remove_rows_batch(dist_b200_ctx *ctx, dist_b200_feature *const *fe
 }
 
 // bytes of one value of the feature's column: bool as uint8, niw a row of d floats, everything else 4 bytes
-static size_t column_bytes(const dist_b200_feature *f) {
+static size_t value_bytes(const dist_b200_feature *f) {
     return f->model == DIST_B200_BB ? 1 : f->model == DIST_B200_NIW ? 4 * static_cast<size_t>(f->dim) : 4;
 }
 
@@ -701,29 +740,24 @@ static int rows_batch_host(dist_b200_ctx *ctx, dist_b200_feature *const *feature
     if (!ctx) return DIST_B200_ERR_INVALID;
     if (n_features < 1 || !features || !columns_host || !assign_host) return fail(ctx, DIST_B200_ERR_INVALID, "add_rows_host: null argument");
     if (n_rows == 0) return DIST_B200_OK;
-    std::vector<size_t> off(n_features);
-    size_t total = 0;
-    for (int i = 0; i < n_features; ++i) {
+    for (int i = 0; i < n_features; ++i)
         if (!features[i] || !columns_host[i]) return fail(ctx, DIST_B200_ERR_INVALID, "add_rows_host: null feature / column");
-        off[i] = total;
-        total += round_up(column_bytes(features[i]) * n_rows, 256);
-    }
-    const size_t assign_off = total;
-    total += round_up(sizeof(int32_t) * n_rows, 256);
-    int rc = ensure_scratch(ctx, total + 256);
-    if (rc) return rc;
     cudaStream_t s = ctx->own_stream;
-    char *dev = static_cast<char *>(ctx->scratch_dev);
+    Staging stage(ctx, s);
+    std::vector<size_t> off(n_features);
+    for (int i = 0; i < n_features; ++i) off[i] = stage.region(value_bytes(features[i]) * n_rows);
+    const size_t assign_off = stage.region(sizeof(int32_t) * n_rows);
+    int rc = stage.reserve();
+    if (rc) return rc;
     std::vector<const void *> cols(n_features);
     for (int i = 0; i < n_features; ++i) {
-        const size_t vb = column_bytes(features[i]);
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(dev + off[i], columns_host[i], vb * n_rows, cudaMemcpyHostToDevice, s));
-        cols[i] = dev + off[i];
+        if ((rc = stage.put(off[i], columns_host[i], value_bytes(features[i]) * n_rows, s))) return rc;
+        cols[i] = stage.dev(off[i]);
     }
-    DISTB200_CUDA(ctx, cudaMemcpyAsync(dev + assign_off, assign_host, sizeof(int32_t) * n_rows, cudaMemcpyHostToDevice, s));
-    rc = rows_batch(ctx, features, n_features, cols.data(), reinterpret_cast<const int32_t *>(dev + assign_off), n_rows, sign, s);
-    DISTB200_CUDA(ctx, cudaStreamSynchronize(s));  // the scratch is free for the next upload
-    return rc;
+    if ((rc = stage.put(assign_off, assign_host, sizeof(int32_t) * n_rows, s)) ||
+        (rc = rows_batch(ctx, features, n_features, cols.data(), stage.dev<const int32_t>(assign_off), n_rows, sign, s)))
+        return rc;
+    return stage.drain();
 }
 
 int dist_b200_add_rows_batch_host(dist_b200_ctx *ctx, dist_b200_feature *const *features, int n_features,
@@ -788,30 +822,24 @@ int dist_b200_sample_values_batch_host(dist_b200_ctx *ctx, const dist_b200_featu
     if (!ctx) return DIST_B200_ERR_INVALID;
     int rc = check_sample_args(ctx, const_cast<dist_b200_feature *const *>(features), n_features, assign_host, columns_out_host);
     if (rc || n_rows == 0) return rc;
-    std::vector<size_t> off(n_features);
-    size_t total = 0;
-    for (int i = 0; i < n_features; ++i) {
-        off[i] = total;
-        total += round_up(column_bytes(features[i]) * n_rows, 256);
-    }
-    const size_t assign_off = total;
-    total += round_up(sizeof(int32_t) * n_rows, 256);
-    if ((rc = ensure_scratch(ctx, total + 256))) return rc;
     cudaStream_t s = ctx->own_stream;
-    char *dev = static_cast<char *>(ctx->scratch_dev);
+    Staging stage(ctx, s);
+    std::vector<size_t> off(n_features);
+    for (int i = 0; i < n_features; ++i) off[i] = stage.region(value_bytes(features[i]) * n_rows);
+    const size_t assign_off = stage.region(sizeof(int32_t) * n_rows);
+    if ((rc = stage.reserve())) return rc;
     std::vector<void *> cols(n_features);
     for (int i = 0; i < n_features; ++i) {
-        cols[i] = dev + off[i];
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(cols[i], columns_out_host[i], column_bytes(features[i]) * n_rows, cudaMemcpyHostToDevice, s));
+        cols[i] = stage.dev(off[i]);
+        if ((rc = stage.put(off[i], columns_out_host[i], value_bytes(features[i]) * n_rows, s))) return rc;
     }
-    DISTB200_CUDA(ctx, cudaMemcpyAsync(dev + assign_off, assign_host, sizeof(int32_t) * n_rows, cudaMemcpyHostToDevice, s));
-    rc = dist_b200_sample_values_batch(ctx, features, n_features, reinterpret_cast<const int32_t *>(dev + assign_off), n_rows, seed,
-                                       row0, cols.data(), s);
-    if (rc == DIST_B200_OK)
-        for (int i = 0; i < n_features; ++i)
-            DISTB200_CUDA(ctx, cudaMemcpyAsync(columns_out_host[i], cols[i], column_bytes(features[i]) * n_rows, cudaMemcpyDeviceToHost, s));
-    DISTB200_CUDA(ctx, cudaStreamSynchronize(s));  // results on the host, the scratch free for the next upload
-    return rc;
+    if ((rc = stage.put(assign_off, assign_host, sizeof(int32_t) * n_rows, s)) ||
+        (rc = dist_b200_sample_values_batch(ctx, features, n_features, stage.dev<const int32_t>(assign_off), n_rows, seed, row0,
+                                            cols.data(), s)))
+        return rc;
+    for (int i = 0; i < n_features; ++i)
+        if ((rc = stage.get(columns_out_host[i], off[i], value_bytes(features[i]) * n_rows, s))) return rc;
+    return stage.drain();
 }
 
 int dist_b200_feature_add_rows(dist_b200_feature *f, const void *column_dev, const int32_t *assign_dev, size_t n_rows,
@@ -882,17 +910,15 @@ int dist_b200_score_data_grid_host(dist_b200_feature *f, const float *shareds_ho
     dist_b200_ctx *ctx = f->ctx;
     if (!shareds_host || !out_host) return fail(ctx, DIST_B200_ERR_INVALID, "score_data_grid: null argument");
     if (n_grid == 0) return DIST_B200_OK;
-    const size_t in_bytes = round_up(sizeof(float) * n_grid * stride, 256);
-    int rc = ensure_scratch(ctx, in_bytes + sizeof(float) * n_grid + 256);
-    if (rc) return rc;
     cudaStream_t s = ctx->own_stream;
-    char *dev = static_cast<char *>(ctx->scratch_dev);
-    DISTB200_CUDA(ctx, cudaMemcpyAsync(dev, shareds_host, sizeof(float) * n_grid * stride, cudaMemcpyHostToDevice, s));
-    rc = dist_b200_score_data_grid(f, reinterpret_cast<const float *>(dev), n_grid, stride, reinterpret_cast<float *>(dev + in_bytes), s);
-    if (rc == DIST_B200_OK)
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(out_host, dev + in_bytes, sizeof(float) * n_grid, cudaMemcpyDeviceToHost, s));
-    DISTB200_CUDA(ctx, cudaStreamSynchronize(s));
-    return rc;
+    Staging stage(ctx, s);
+    const size_t in_off = stage.region(sizeof(float) * n_grid * stride), out_off = stage.region(sizeof(float) * n_grid);
+    int rc;
+    if ((rc = stage.reserve()) || (rc = stage.put(in_off, shareds_host, sizeof(float) * n_grid * stride, s)) ||
+        (rc = dist_b200_score_data_grid(f, stage.dev<const float>(in_off), n_grid, stride, stage.dev<float>(out_off), s)) ||
+        (rc = stage.get(out_host, out_off, sizeof(float) * n_grid, s)))
+        return rc;
+    return stage.drain();
 }
 
 // ---- protobuf wire format (schema.proto) -> update_all (SURVEY 8f rank 4) --------------------------
@@ -1125,15 +1151,8 @@ int dist_b200_feature_download_caches(const dist_b200_feature *f, float *out_hos
 int dist_b200_prior_pitman_yor(dist_b200_ctx *ctx, float alpha, float d, int G, const int32_t *group_sizes,
                                float *prior_dev, void *stream) {
     if (!ctx || G < 1 || !group_sizes || !prior_dev) return DIST_B200_ERR_INVALID;
-    int rc = ensure_scratch(ctx, sizeof(int32_t) * G + 256);
-    if (rc) return rc;
-    Upload up{ctx, as_stream(stream)};
-    const int32_t *sz = up.put(group_sizes, G);
-    if (up.err) return up.err;
-    int rc2 = launch_prior_prep(ctx, alpha, d, G, sz, prior_dev, as_stream(stream));
-    if (rc2) return rc2;
-    DISTB200_CUDA(ctx, cudaStreamSynchronize(as_stream(stream)));  // scratch (group sizes) is free again
-    return DIST_B200_OK;
+    return prior_from_host_sizes(ctx, G, group_sizes, prior_dev, nullptr, as_stream(stream),
+                                 [&](const int32_t *sz, float *out, cudaStream_t s) { return launch_prior_prep(ctx, alpha, d, G, sz, out, s); });
 }
 
 // LowEntropy clustering prior (clustering.hpp:245-331 through MixtureDriver::score_value): overwrite semantics
@@ -1146,33 +1165,16 @@ int dist_b200_prior_low_entropy_dev(dist_b200_ctx *ctx, int dataset_size, int G,
 int dist_b200_prior_low_entropy_host(dist_b200_ctx *ctx, int dataset_size, int G, const int32_t *group_sizes,
                                      float *prior_host) {
     if (!ctx || G < 1 || !group_sizes || !prior_host || dataset_size < 1) return DIST_B200_ERR_INVALID;
-    int rc = ensure_scratch(ctx, round_up(sizeof(int32_t) * G, 256) + sizeof(float) * G + 256);
-    if (rc) return rc;
-    cudaStream_t s = ctx->own_stream;
-    Upload up{ctx, s};
-    const int32_t *sz = up.put(group_sizes, G);
-    if (up.err) return up.err;
-    float *out = reinterpret_cast<float *>(static_cast<char *>(ctx->scratch_dev) + up.off);
-    if ((rc = launch_low_entropy_prep(ctx, dataset_size, G, sz, out, s))) return rc;
-    DISTB200_CUDA(ctx, cudaMemcpyAsync(prior_host, out, sizeof(float) * G, cudaMemcpyDeviceToHost, s));
-    DISTB200_CUDA(ctx, cudaStreamSynchronize(s));
-    return DIST_B200_OK;
+    return prior_from_host_sizes(ctx, G, group_sizes, nullptr, prior_host, ctx->own_stream, [&](const int32_t *sz, float *out, cudaStream_t s) {
+        return launch_low_entropy_prep(ctx, dataset_size, G, sz, out, s);
+    });
 }
 
 int dist_b200_prior_pitman_yor_host(dist_b200_ctx *ctx, float alpha, float d, int G, const int32_t *group_sizes,
                                     float *prior_host) {
     if (!ctx || G < 1 || !group_sizes || !prior_host) return DIST_B200_ERR_INVALID;
-    int rc = ensure_scratch(ctx, round_up(sizeof(int32_t) * G, 256) + sizeof(float) * G + 256);
-    if (rc) return rc;
-    cudaStream_t s = ctx->own_stream;
-    Upload up{ctx, s};
-    const int32_t *sz = up.put(group_sizes, G);
-    if (up.err) return up.err;
-    float *out = reinterpret_cast<float *>(static_cast<char *>(ctx->scratch_dev) + up.off);
-    if ((rc = launch_prior_prep(ctx, alpha, d, G, sz, out, s))) return rc;
-    DISTB200_CUDA(ctx, cudaMemcpyAsync(prior_host, out, sizeof(float) * G, cudaMemcpyDeviceToHost, s));
-    DISTB200_CUDA(ctx, cudaStreamSynchronize(s));
-    return DIST_B200_OK;
+    return prior_from_host_sizes(ctx, G, group_sizes, nullptr, prior_host, ctx->own_stream,
+                                 [&](const int32_t *sz, float *out, cudaStream_t s) { return launch_prior_prep(ctx, alpha, d, G, sz, out, s); });
 }
 
 // ---- the hot path ---------------------------------------------------------------------------
@@ -1475,14 +1477,6 @@ int dist_b200_sample_from_slots(dist_b200_ctx *ctx, const float *slots_dev, int 
     return launch_sample_scores(ctx, slots_dev, n_rows, G, u_dev, assign_dev, as_stream(stream), n_slots, slot_stride);
 }
 
-static size_t value_bytes(const dist_b200_feature *f) {
-    switch (f->model) {
-        case DIST_B200_BB: return 1;
-        case DIST_B200_NIW: return sizeof(float) * f->dim;
-        default: return 4;
-    }
-}
-
 // The host-buffer form of score_dispatch.  Its per-row output is 4 bytes: the sampled group (u_host and assign_host given)
 // or the row's log-normaliser (logp_host given, no u).
 static int score_host(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int F, const void *const *columns_host, size_t N,
@@ -1493,29 +1487,20 @@ static int score_host(dist_b200_ctx *ctx, const dist_b200_feature *const *featur
     const int G = features[0]->G;
     if (G < 1) return fail(ctx, DIST_B200_ERR_STATE, "score_sample_host: no groups");
     if (N == 0) return DIST_B200_OK;
-    // layout of the staging area (identical in pinned host memory and on the device):
-    //   columns | prior | u (sampling only) | per-row output | scores(optional, device only + host out)
+    // Row chunks are pipelined over two streams: the H2D copy of chunk k+1 and the D2H copy of chunk
+    // k-1 overlap the kernels of chunk k (rows are independent given frozen statistics).
+    cudaStream_t st[2] = {ctx->own_stream, ctx->own_stream2};
+    Staging stage(ctx, st[0], st[1]);
+    // layout of the staging area (identical in the page-locked mirror and on the device):
+    //   columns | prior | u (sampling only) | per-row output | scores (optional, device only + host out)
     std::vector<size_t> col_off(F);
-    size_t off = 0;
-    for (int f = 0; f < F; ++f) {
-        col_off[f] = off;
-        off += round_up(value_bytes(features[f]) * N, 256);
-    }
-    const size_t prior_off = off;
-    off += round_up(sizeof(float) * G, 256);
-    const size_t u_off = off;
-    if (u_host) off += round_up(sizeof(float) * N, 256);
-    const size_t in_bytes = off;
-    const size_t out_off = off;
-    off += round_up(sizeof(int32_t) * N, 256);
-    const size_t scores_off = off;
-    if (scores_host) off += round_up(sizeof(float) * N * G, 256);
-    (void)in_bytes;
+    for (int f = 0; f < F; ++f) col_off[f] = stage.region(value_bytes(features[f]) * N);
+    const size_t prior_off = stage.region(sizeof(float) * G);
+    const size_t u_off = stage.region(u_host ? sizeof(float) * N : 0);
+    const size_t out_off = stage.region(sizeof(int32_t) * N);
+    const size_t scores_off = stage.region(scores_host ? sizeof(float) * N * G : 0);
     int rc;
-    if ((rc = ensure_pinned(ctx, scores_off))) return rc;
-    if ((rc = ensure_scratch(ctx, off + 256))) return rc;
-    char *pin = static_cast<char *>(ctx->pinned);
-    char *dev = static_cast<char *>(ctx->scratch_dev);
+    if ((rc = stage.reserve(scores_off))) return rc;
     // A caller buffer that is already page-locked (cudaHostAlloc / cudaHostRegister / torch pin_memory)
     // is copied from / to directly; pageable buffers go through the context's pinned staging area.
     auto is_pinned = [](const void *p) {
@@ -1529,21 +1514,18 @@ static int score_host(dist_b200_ctx *ctx, const dist_b200_feature *const *featur
     std::vector<char> col_pinned(F);
     for (int f = 0; f < F; ++f) col_pinned[f] = is_pinned(columns_host[f]) ? 1 : 0;
     const bool u_pinned = !u_host || is_pinned(u_host), out_pinned = is_pinned(out_host);
-    const bool scores_pinned = scores_host && is_pinned(scores_host);
 
     // per-row output of rows [lo, lo + n) at `out` (device / mapped), u of those rows at `uu`
     auto dispatch = [&](const void *const *cols, size_t n, const float *pr, const float *uu, char *out, float *sc, cudaStream_t str) {
         return score_dispatch(ctx, features, F, cols, n, pr, uu, logp_host ? nullptr : reinterpret_cast<int32_t *>(out), sc, 0, str,
                               logp_host ? reinterpret_cast<float *>(out) : nullptr);
     };
-    auto dev_u = [&](size_t lo) { return u_host ? reinterpret_cast<const float *>(dev + u_off) + lo : nullptr; };
 
-    // Row chunks are pipelined over two streams: the H2D copy of chunk k+1 and the D2H copy of chunk
-    // k-1 overlap the kernels of chunk k (rows are independent given frozen statistics).
-    cudaStream_t st[2] = {ctx->own_stream, ctx->own_stream2};
     if ((rc = wait_ready(ctx, features, F, st[0]))) return rc;
     if ((rc = refresh_gp_tables(ctx, features, F, st[0]))) return rc;  // before the second stream starts reading them
-    const float *prior_dev = nullptr;
+    // the prior vector is re-read per table row by the dpd / dd kernels: it goes to the device on every route
+    const float *prior_dev = prior_host ? stage.dev<const float>(prior_off) : nullptr;
+    if (prior_host && (rc = stage.put(prior_off, prior_host, sizeof(float) * G, st[0], true))) return rc;
     // Zero-copy: when every caller buffer is page-locked, the kernels read the rows straight from host memory and write
     // the assignments straight back (device-accessible under unified addressing): ONE launch, the PCIe transfers overlap
     // the math row tile by row tile with no chunking, no staging copies and no second stream.
@@ -1571,29 +1553,16 @@ static int score_host(dist_b200_ctx *ctx, const dist_b200_feature *const *featur
             if (ok) ok = cudaHostGetDevicePointer(&dp, out_host, 0) == cudaSuccess;
             char *out_zc = static_cast<char *>(dp);
             if (ok) {
-                const float *prior_zc = nullptr;
-                if (prior_host) {  // the prior vector is re-read per table row by the dpd / dd kernels: it goes to the device
-                    std::memcpy(pin + prior_off, prior_host, sizeof(float) * G);
-                    if (cudaMemcpyAsync(dev + prior_off, pin + prior_off, sizeof(float) * G, cudaMemcpyHostToDevice, st[0]) != cudaSuccess)
-                        return fail(ctx, DIST_B200_ERR_CUDA, "score_sample_host: prior upload");
-                    prior_zc = reinterpret_cast<const float *>(dev + prior_off);
-                }
-                rc = dispatch(zc_cols.data(), N, prior_zc, u_zc, out_zc, nullptr, st[0]);
-                cudaError_t e = cudaStreamSynchronize(st[0]);
-                if (rc) return rc;
-                if (e != cudaSuccess) return fail(ctx, DIST_B200_ERR_CUDA, std::string("score_sample_host: ") + cudaGetErrorString(e));
-                return DIST_B200_OK;
+                if ((rc = dispatch(zc_cols.data(), N, prior_dev, u_zc, out_zc, nullptr, st[0]))) return rc;
+                return stage.drain();
             }
             cudaGetLastError();  // not mappable: fall through to the staged path
         }
     }
     if ((rc = wait_ready(ctx, features, F, st[1]))) return rc;
     if (prior_host) {
-        std::memcpy(pin + prior_off, prior_host, sizeof(float) * G);
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(dev + prior_off, pin + prior_off, sizeof(float) * G, cudaMemcpyHostToDevice, st[0]));
         DISTB200_CUDA(ctx, cudaEventRecord(ctx->ev, st[0]));
         DISTB200_CUDA(ctx, cudaStreamWaitEvent(st[1], ctx->ev, 0));
-        prior_dev = reinterpret_cast<const float *>(dev + prior_off);
     }
     const size_t min_chunk = 32768;
     // five chunks measured best at 1M rows (DIST_B200_OPT_HOST_CHUNKS overrides it for A/B runs)
@@ -1623,93 +1592,30 @@ static int score_host(dist_b200_ctx *ctx, const dist_b200_feature *const *featur
         for (size_t at = chunk; at < N; at += chunk) bounds.push_back(at);
     }
     bounds.push_back(N);
+    // with more than one chunk, one compute stream takes the copies on the second stream and the kernels on the first
+    one_compute_stream = one_compute_stream && bounds.size() > 2;
     std::vector<const void *> cols(F);
-    float *scores_dev = scores_host ? reinterpret_cast<float *>(dev + scores_off) : nullptr;
-    if (one_compute_stream && bounds.size() > 2) {
-        // copies of all chunks on the second stream, one event each; the kernels follow on the first stream
-        std::vector<cudaEvent_t> ready(bounds.size() - 1, nullptr);
-        auto cleanup = [&]() {
-            cudaStreamSynchronize(st[0]);
-            cudaStreamSynchronize(st[1]);
-            for (cudaEvent_t e : ready)
-                if (e) cudaEventDestroy(e);
-        };
-        cudaError_t ce = cudaSuccess;
-        for (size_t k = 0; k + 1 < bounds.size() && ce == cudaSuccess; ++k) {
-            const size_t lo = bounds[k], n = bounds[k + 1] - lo;
-            for (int f = 0; f < F && ce == cudaSuccess; ++f) {
-                const size_t vb = value_bytes(features[f]);
-                const char *src = static_cast<const char *>(columns_host[f]) + vb * lo;
-                if (!col_pinned[f]) {
-                    std::memcpy(pin + col_off[f] + vb * lo, src, vb * n);
-                    src = pin + col_off[f] + vb * lo;
-                }
-                ce = cudaMemcpyAsync(dev + col_off[f] + vb * lo, src, vb * n, cudaMemcpyHostToDevice, st[1]);
-            }
-            if (u_host) {
-                const char *src = reinterpret_cast<const char *>(u_host + lo);
-                if (!u_pinned) {
-                    std::memcpy(pin + u_off + 4 * lo, src, 4 * n);
-                    src = pin + u_off + 4 * lo;
-                }
-                if (ce == cudaSuccess) ce = cudaMemcpyAsync(dev + u_off + 4 * lo, src, 4 * n, cudaMemcpyHostToDevice, st[1]);
-            }
-            if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&ready[k], cudaEventDisableTiming);
-            if (ce == cudaSuccess) ce = cudaEventRecord(ready[k], st[1]);
-        }
-        for (size_t k = 0; k + 1 < bounds.size() && ce == cudaSuccess && rc == DIST_B200_OK; ++k) {
-            const size_t lo = bounds[k], n = bounds[k + 1] - lo;
-            if (n == 0) continue;
-            ce = cudaStreamWaitEvent(st[0], ready[k], 0);
-            for (int f = 0; f < F; ++f) cols[f] = dev + col_off[f] + value_bytes(features[f]) * lo;
-            if (ce == cudaSuccess) rc = dispatch(cols.data(), n, prior_dev, dev_u(lo), dev + out_off + 4 * lo, nullptr, st[0]);
-        }
-        void *odst = out_pinned ? out_host : pin + out_off;
-        if (ce == cudaSuccess && rc == DIST_B200_OK) ce = cudaMemcpyAsync(odst, dev + out_off, 4 * N, cudaMemcpyDeviceToHost, st[0]);
-        cleanup();
-        if (rc) return rc;
-        if (ce != cudaSuccess) return fail(ctx, DIST_B200_ERR_CUDA, std::string("score_sample_host: ") + cudaGetErrorString(ce));
-        if (!out_pinned) std::memcpy(out_host, pin + out_off, 4 * N);
-        return DIST_B200_OK;
-    }
     for (size_t k = 0; k + 1 < bounds.size(); ++k) {
         const size_t lo = bounds[k], n = bounds[k + 1] - lo;
-        if (n == 0) continue;
-        cudaStream_t s = st[k & 1];
+        const cudaStream_t cs = one_compute_stream ? st[1] : st[k & 1], ks = one_compute_stream ? st[0] : st[k & 1];
         for (int f = 0; f < F; ++f) {
-            const size_t vb = value_bytes(features[f]);
-            const char *src = static_cast<const char *>(columns_host[f]) + vb * lo;
-            if (!col_pinned[f]) {
-                std::memcpy(pin + col_off[f] + vb * lo, src, vb * n);
-                src = pin + col_off[f] + vb * lo;
-            }
-            DISTB200_CUDA(ctx, cudaMemcpyAsync(dev + col_off[f] + vb * lo, src, vb * n, cudaMemcpyHostToDevice, s));
-            cols[f] = dev + col_off[f] + vb * lo;
+            const size_t vb = value_bytes(features[f]), at = col_off[f] + vb * lo;
+            if ((rc = stage.put(at, static_cast<const char *>(columns_host[f]) + vb * lo, vb * n, cs, !col_pinned[f]))) return rc;
+            cols[f] = stage.dev(at);
         }
-        if (u_host) {
-            const char *src = reinterpret_cast<const char *>(u_host + lo);
-            if (!u_pinned) {
-                std::memcpy(pin + u_off + 4 * lo, src, 4 * n);
-                src = pin + u_off + 4 * lo;
-            }
-            DISTB200_CUDA(ctx, cudaMemcpyAsync(dev + u_off + 4 * lo, src, 4 * n, cudaMemcpyHostToDevice, s));
+        if (u_host && (rc = stage.put(u_off + 4 * lo, u_host + lo, 4 * n, cs, !u_pinned))) return rc;
+        if (cs != ks) {
+            DISTB200_CUDA(ctx, cudaEventRecord(ctx->ev, cs));
+            DISTB200_CUDA(ctx, cudaStreamWaitEvent(ks, ctx->ev, 0));
         }
-        rc = dispatch(cols.data(), n, prior_dev, dev_u(lo), dev + out_off + 4 * lo, scores_dev ? scores_dev + lo * G : nullptr, s);
-        if (rc) {  // copies of earlier chunks into the caller's buffers may still be in flight
-            cudaStreamSynchronize(st[0]);
-            cudaStreamSynchronize(st[1]);
+        if ((rc = dispatch(cols.data(), n, prior_dev, u_host ? stage.dev<const float>(u_off) + lo : nullptr, stage.dev(out_off + 4 * lo),
+                           scores_host ? stage.dev<float>(scores_off) + lo * G : nullptr, ks)) ||
+            (rc = stage.get(static_cast<char *>(out_host) + 4 * lo, out_off + 4 * lo, 4 * n, ks, !out_pinned)) ||
+            (scores_host && (rc = stage.get(scores_host + lo * G, scores_off + sizeof(float) * lo * G, sizeof(float) * n * G, ks))))
             return rc;
-        }
-        char *odst = (out_pinned ? static_cast<char *>(out_host) : pin + out_off) + 4 * lo;
-        DISTB200_CUDA(ctx, cudaMemcpyAsync(odst, dev + out_off + 4 * lo, 4 * n, cudaMemcpyDeviceToHost, s));
-        if (scores_host)
-            DISTB200_CUDA(ctx, cudaMemcpyAsync(scores_host + lo * G, scores_dev + lo * G, sizeof(float) * n * G,
-                                               cudaMemcpyDeviceToHost, s));
     }
-    (void)scores_pinned;
-    DISTB200_CUDA(ctx, cudaStreamSynchronize(st[0]));
-    DISTB200_CUDA(ctx, cudaStreamSynchronize(st[1]));
-    if (!out_pinned) std::memcpy(out_host, pin + out_off, 4 * N);
+    if ((rc = stage.drain())) return rc;
+    if (!out_pinned) std::memcpy(out_host, stage.pin(out_off), 4 * N);
     return DIST_B200_OK;
 }
 
