@@ -25,6 +25,9 @@ SOURCES = {
     "score_rows.cu": [],
     "score_rows_cc32.cu": [],
     "score_rows_cc64.cu": [],
+    "score_rows_masked.cu": [],
+    "score_rows_masked_cc.cu": [],
+    "missing.cu": [],
     "score_rows_nich.cu": [],
     "nich_rows.cu": [],
     "score_rows_gp.cu": [],

@@ -90,6 +90,13 @@ SIGNATURES = {
     "dist_b200_host_unregister": (c_i, [c_p, c_p]),
     "dist_b200_numerics_probe": (c_i, [c_p, c_i, c_sz, c_p, c_p, c_p]),
     "dist_b200_pipe_peak": (c_i, [c_p, c_i, ctypes.POINTER(ctypes.c_double)]),
+    "dist_b200_score_batch_masked": (c_i, [c_p, c_p, c_i, c_p, c_sz, c_p, c_p, c_i, c_p, c_p]),
+    "dist_b200_score_sample_batch_masked": (c_i, [c_p, c_p, c_i, c_p, c_sz, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "dist_b200_score_logp_batch_masked": (c_i, [c_p, c_p, c_i, c_p, c_sz, c_p, c_p, c_p, c_p]),
+    "dist_b200_add_rows_batch_masked": (c_i, [c_p, c_p, c_i, c_p, c_p, c_sz, c_p, c_p]),
+    "dist_b200_remove_rows_batch_masked": (c_i, [c_p, c_p, c_i, c_p, c_p, c_sz, c_p, c_p]),
+    "dist_b200_rows_accumulate_masked": (c_i, [c_p, c_p, c_i, c_p, c_p, c_sz, c_p, c_p, c_p]),
+    "dist_b200_sample_values_batch_masked": (c_i, [c_p, c_p, c_i, c_p, c_sz, ctypes.c_uint64, ctypes.c_uint64, c_p, c_p, c_p]),
 }
 
 
@@ -131,6 +138,31 @@ def _dev_ptr(t):
     if isinstance(t, int):
         return t
     return t.data_ptr()
+
+
+def pack_observed(mask):
+    """a bool column (numpy or torch, True = observed) -> the observed-mask words of the *_masked entries:
+    ceil(N / 32) uint32, bit n % 32 of word n / 32 = mask[n] (np.packbits little-endian bit order, read as little-endian
+    uint32; bits past N are 0).  Returns the type it was given: a numpy array, or a torch tensor on the input's device."""
+    torch_in = not isinstance(mask, np.ndarray) and hasattr(mask, "detach")
+    m = mask.detach().cpu().numpy() if torch_in else np.asarray(mask)
+    m = np.ascontiguousarray(m, dtype=bool).reshape(-1)
+    n_words = (m.size + 31) // 32
+    b = np.zeros(4 * n_words, dtype=np.uint8)
+    b[:(m.size + 7) // 8] = np.packbits(m, bitorder="little")
+    words = b.view("<u4").astype(np.uint32)
+    if torch_in:
+        import torch
+        return torch.from_numpy(words.view(np.int32).copy()).to(mask.device)
+    return words
+
+
+def _masks(observed, F):
+    """observed: None or one entry per feature (None = fully observed, else a device tensor / pointer of mask words)"""
+    if observed is None:
+        return None
+    assert len(observed) == F, "observed: one entry per feature"
+    return (c_p * F)(*[_dev_ptr(o) for o in observed])
 
 
 def wire_decode(model, shared_msg, group_msgs):
@@ -256,9 +288,14 @@ class Context:
         self.check(self.L.dist_b200_prior_pitman_yor_host(self.h, alpha, d, sizes.size, _np_ptr(sizes), _np_ptr(out)), "prior_pitman_yor_host")
         return out
 
-    def add_rows_batch(self, features, columns, assign_dev, n_rows, stream=None):
-        """batched Group::add_value for all features of one kind; nothing is drained, later calls order behind it"""
+    def add_rows_batch(self, features, columns, assign_dev, n_rows, stream=None, observed=None):
+        """batched Group::add_value for all features of one kind; nothing is drained, later calls order behind it.
+        observed: None, or per feature None / pack_observed words on the device (a missing cell is not added)"""
         F, fa, ca = self._lists(features, columns)
+        if observed is not None:
+            self.check(self.L.dist_b200_add_rows_batch_masked(self.h, fa, F, ca, _dev_ptr(assign_dev), n_rows, _masks(observed, F),
+                                                              stream), "add_rows_batch_masked")
+            return
         self.check(self.L.dist_b200_add_rows_batch(self.h, fa, F, ca, _dev_ptr(assign_dev), n_rows, stream), "add_rows_batch")
 
     def rows_xchg_doubles(self, features):
@@ -269,9 +306,13 @@ class Context:
         self.check(self.L.dist_b200_rows_xchg_doubles(fa, F, ctypes.byref(n)), "rows_xchg_doubles")
         return int(n.value)
 
-    def rows_accumulate(self, features, columns, assign_dev, n_rows, xchg_dev, stream=None):
+    def rows_accumulate(self, features, columns, assign_dev, n_rows, xchg_dev, stream=None, observed=None):
         """row shards: this rank's accumulators into xchg_dev (rows_xchg_doubles float64; then all-reduce, then rows_merge)"""
         F, fa, ca = self._lists(features, columns)
+        if observed is not None:
+            self.check(self.L.dist_b200_rows_accumulate_masked(self.h, fa, F, ca, _dev_ptr(assign_dev), n_rows, _dev_ptr(xchg_dev),
+                                                               _masks(observed, F), stream), "rows_accumulate_masked")
+            return
         self.check(self.L.dist_b200_rows_accumulate(self.h, fa, F, ca, _dev_ptr(assign_dev), n_rows, _dev_ptr(xchg_dev), stream),
                    "rows_accumulate")
 
@@ -280,9 +321,13 @@ class Context:
         fa = (c_p * F)(*[f.h for f in features])
         self.check(self.L.dist_b200_rows_merge(self.h, fa, F, _dev_ptr(xchg_dev), sign, stream), "rows_merge")
 
-    def remove_rows_batch(self, features, columns, assign_dev, n_rows, stream=None):
-        """batched Group::remove_value: the rows leave the groups assign_dev names"""
+    def remove_rows_batch(self, features, columns, assign_dev, n_rows, stream=None, observed=None):
+        """batched Group::remove_value: the rows leave the groups assign_dev names (observed: as in add_rows_batch)"""
         F, fa, ca = self._lists(features, columns)
+        if observed is not None:
+            self.check(self.L.dist_b200_remove_rows_batch_masked(self.h, fa, F, ca, _dev_ptr(assign_dev), n_rows,
+                                                                 _masks(observed, F), stream), "remove_rows_batch_masked")
+            return
         self.check(self.L.dist_b200_remove_rows_batch(self.h, fa, F, ca, _dev_ptr(assign_dev), n_rows, stream), "remove_rows_batch")
 
     def remove_rows_batch_host(self, features, columns, assign):
@@ -302,10 +347,15 @@ class Context:
         ca = (c_p * F)(*[_np_ptr(c) for c in cols])
         self.check(self.L.dist_b200_add_rows_batch_host(self.h, fa, F, ca, _np_ptr(assign), assign.size), "add_rows_batch_host")
 
-    def sample_values_batch(self, features, assign_dev, n_rows, columns_out, seed=0, row0=0, stream=None):
+    def sample_values_batch(self, features, assign_dev, n_rows, columns_out, seed=0, row0=0, stream=None, observed=None):
         """batched Group::sample_value: columns_out[i][n] (device) <- a posterior-predictive draw of group assign_dev[n]
-        of features[i]; rows with an id outside [0, G) keep their values.  Draws depend on (seed, row0 + n, i) only."""
+        of features[i]; rows with an id outside [0, G) keep their values.  Draws depend on (seed, row0 + n, i) only.
+        observed (imputation): per feature None / mask words; only MISSING cells are drawn (None: nothing is drawn)."""
         F, fa, ca = self._lists(features, columns_out)
+        if observed is not None:
+            self.check(self.L.dist_b200_sample_values_batch_masked(self.h, fa, F, _dev_ptr(assign_dev), n_rows, int(seed), int(row0),
+                                                                   ca, _masks(observed, F), stream), "sample_values_batch_masked")
+            return
         self.check(self.L.dist_b200_sample_values_batch(self.h, fa, F, _dev_ptr(assign_dev), n_rows, int(seed), int(row0), ca, stream),
                    "sample_values_batch")
 
@@ -359,13 +409,24 @@ class Context:
         ca = (c_p * F)(*[_dev_ptr(c) for c in columns])
         return F, fa, ca
 
-    def score_batch(self, features, columns, n_rows, prior, scores, accumulate=False, stream=None):
+    def score_batch(self, features, columns, n_rows, prior, scores, accumulate=False, stream=None, observed=None):
         F, fa, ca = self._lists(features, columns)
+        if observed is not None:
+            self.check(self.L.dist_b200_score_batch_masked(self.h, fa, F, ca, n_rows, _dev_ptr(prior), _dev_ptr(scores),
+                                                           1 if accumulate else 0, _masks(observed, F), stream), "score_batch_masked")
+            return
         self.check(self.L.dist_b200_score_batch(self.h, fa, F, ca, n_rows, _dev_ptr(prior), _dev_ptr(scores),
                                                 1 if accumulate else 0, stream), "score_batch")
 
-    def score_sample_batch(self, features, columns, n_rows, prior, u, assign, scores=None, stream=None):
+    def score_sample_batch(self, features, columns, n_rows, prior, u, assign, scores=None, stream=None, observed=None):
+        """observed: None, or per feature None (fully observed) / pack_observed words on the device; a missing cell
+        contributes 0 to every group's score"""
         F, fa, ca = self._lists(features, columns)
+        if observed is not None:
+            self.check(self.L.dist_b200_score_sample_batch_masked(self.h, fa, F, ca, n_rows, _dev_ptr(prior), _dev_ptr(u),
+                                                                  _dev_ptr(assign), _dev_ptr(scores), _masks(observed, F), stream),
+                       "score_sample_batch_masked")
+            return
         self.check(self.L.dist_b200_score_sample_batch(self.h, fa, F, ca, n_rows, _dev_ptr(prior), _dev_ptr(u),
                                                        _dev_ptr(assign), _dev_ptr(scores), stream), "score_sample_batch")
 
@@ -373,9 +434,14 @@ class Context:
         self.check(self.L.dist_b200_sample_from_scores(self.h, _dev_ptr(scores), n_rows, G, _dev_ptr(u), _dev_ptr(assign),
                                                        stream), "sample_from_scores")
 
-    def score_logp_batch(self, features, columns, n_rows, prior, logp, stream=None):
-        """logp[n] (device, float32) <- log sum_g exp(prior[g] + sum_f score_f(columns[f][n]; g)); prior may be None"""
+    def score_logp_batch(self, features, columns, n_rows, prior, logp, stream=None, observed=None):
+        """logp[n] (device, float32) <- log sum_g exp(prior[g] + sum_f score_f(columns[f][n]; g)); prior may be None.
+        observed: as in score_sample_batch (a missing cell's term is left out of the sum)"""
         F, fa, ca = self._lists(features, columns)
+        if observed is not None:
+            self.check(self.L.dist_b200_score_logp_batch_masked(self.h, fa, F, ca, n_rows, _dev_ptr(prior), _dev_ptr(logp),
+                                                                _masks(observed, F), stream), "score_logp_batch_masked")
+            return
         self.check(self.L.dist_b200_score_logp_batch(self.h, fa, F, ca, n_rows, _dev_ptr(prior), _dev_ptr(logp), stream),
                    "score_logp_batch")
 

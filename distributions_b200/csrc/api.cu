@@ -307,6 +307,7 @@ void dist_b200_ctx_destroy(dist_b200_ctx *ctx) {
     if (ctx->add_acc) cudaFree(ctx->add_acc);
     if (ctx->add_done) cudaEventDestroy(ctx->add_done);
     if (ctx->scores_scratch) cudaFree(ctx->scores_scratch);
+    if (ctx->missing_scratch) cudaFree(ctx->missing_scratch);
     if (ctx->xpack) cudaFree(ctx->xpack);
     if (ctx->bbt) cudaFree(ctx->bbt);
     if (ctx->pinned) cudaFreeHost(ctx->pinned);
@@ -559,9 +560,11 @@ static bool pooled_model(int model) {
     return model == DIST_B200_NICH || model == DIST_B200_GP || model == DIST_B200_BB || model == DIST_B200_BNB;
 }
 
+// observed (accumulating phases): per feature NULL or a mask (dist_b200.h).  The pooled, count-table and niw kernels skip
+// a missing cell themselves (their masked instantiations); pooled batches keep up to kAddBatch features whatever the masks
 static int rows_batch(dist_b200_ctx *ctx, dist_b200_feature *const *features, int n_features,
                       const void *const *columns_dev, const int32_t *assign_dev, size_t n_rows, int sign, void *stream,
-                      int phase = kRowsBoth, double *xchg = nullptr) {
+                      int phase = kRowsBoth, double *xchg = nullptr, const uint32_t *const *observed = nullptr) {
     if (!ctx) return DIST_B200_ERR_INVALID;
     if (n_features < 0 || (n_features && !features) || (phase != kRowsMerge && ((n_features && !columns_dev) || !assign_dev)))
         return fail(ctx, DIST_B200_ERR_INVALID, "add_rows: null argument");
@@ -605,6 +608,8 @@ static int rows_batch(dist_b200_ctx *ctx, dist_b200_feature *const *features, in
     b.N = n_rows;
     b.assign = assign_dev;
     b.acc = static_cast<char *>(ctx->add_acc);
+    AddMasks bm{};  // the pending pooled batch's observed masks (bm.m[k] for b.d[k])
+    auto mask_of = [&](int i) -> const uint32_t * { return observed && phase != kRowsMerge ? observed[i] : nullptr; };
     int flushed = 0;  // pooled features already processed = index of b.d[0] in the exchange buffer
     auto flush = [&]() -> int {
         if (b.n == 0) return DIST_B200_OK;
@@ -612,11 +617,12 @@ static int rows_batch(dist_b200_ctx *ctx, dist_b200_feature *const *features, in
         b.xchg = phase == kRowsMerge ? xchg : nullptr;
         b.xchg_first = flushed;
         int r = DIST_B200_OK;
-        if (phase != kRowsMerge) r = launch_add_rows_pooled(ctx, b, s);
+        if (phase != kRowsMerge) r = launch_add_rows_pooled(ctx, b, s, &bm);
         if (!r && phase == kRowsAccumulate) r = launch_pack_accumulators(ctx, b, xchg, s);
         if (!r && phase != kRowsAccumulate) r = launch_merge_prep_batch(ctx, b, s);
         flushed += b.n;
         b.n = 0;
+        bm = AddMasks{};
         return r;
     };
     // count tables (dd / dpd).  Single GPU: the rows go straight into the feature's table.  Exchange: accumulate = this
@@ -625,11 +631,11 @@ static int rows_batch(dist_b200_ctx *ctx, dist_b200_feature *const *features, in
         const size_t cells = static_cast<size_t>(f->G) * f->dim;
         int r = DIST_B200_OK;
         if (phase == kRowsBoth) {
-            r = launch_add_rows_counts(ctx, f, columns_dev[i], assign_dev, n_rows, sign, s);
+            r = launch_add_rows_counts(ctx, f, columns_dev[i], assign_dev, n_rows, sign, s, nullptr, mask_of(i));
         } else if (phase == kRowsAccumulate) {
             int32_t *tmp = reinterpret_cast<int32_t *>(static_cast<char *>(ctx->add_acc) + pooled_bytes);
             DISTB200_CUDA(ctx, cudaMemsetAsync(tmp, 0, sizeof(int32_t) * cells, s));
-            r = launch_add_rows_counts(ctx, f, columns_dev[i], assign_dev, n_rows, +1, s, tmp);
+            r = launch_add_rows_counts(ctx, f, columns_dev[i], assign_dev, n_rows, +1, s, tmp, mask_of(i));
             if (!r) r = launch_counts_to_doubles(ctx, tmp, xchg + table_off, cells, s);
         } else {
             r = launch_merge_counts(ctx, reinterpret_cast<int32_t *>(f->stats[0]), xchg + table_off, cells, sign, s);
@@ -648,6 +654,7 @@ static int rows_batch(dist_b200_ctx *ctx, dist_b200_feature *const *features, in
                 if (b.n == kAddBatch || (b.n && b.G != G))
                     if ((rc = flush())) return rc;
                 b.G = G;
+                bm.m[b.n] = mask_of(i);
                 AddDesc &d = b.d[b.n++];
                 d.column = columns_dev ? columns_dev[i] : nullptr;
                 d.st0 = f->stats[0];
@@ -674,7 +681,9 @@ static int rows_batch(dist_b200_ctx *ctx, dist_b200_feature *const *features, in
                 char *area = static_cast<char *>(ctx->add_acc) + pooled_bytes + table_tmp;
                 double *acc = phase == kRowsBoth ? reinterpret_cast<double *>(area) : xchg + table_off;
                 void *work = area + round_up(sizeof(double) * G * per, 256);
-                if (phase != kRowsMerge && (rc = launch_niw_accumulate(ctx, G, d, columns_dev[i], assign_dev, n_rows, acc, work, s))) return rc;
+                if (phase != kRowsMerge &&
+                    (rc = launch_niw_accumulate(ctx, G, d, columns_dev[i], assign_dev, n_rows, acc, work, s, mask_of(i))))
+                    return rc;
                 table_off += G * per;
                 if (phase == kRowsAccumulate) break;
                 if ((rc = launch_niw_apply(ctx, G, d, sign, acc, reinterpret_cast<int32_t *>(f->stats[0]), reinterpret_cast<float *>(f->stats[1]),
@@ -727,6 +736,25 @@ int dist_b200_add_rows_batch(dist_b200_ctx *ctx, dist_b200_feature *const *featu
 int dist_b200_remove_rows_batch(dist_b200_ctx *ctx, dist_b200_feature *const *features, int n_features,
                                 const void *const *columns_dev, const int32_t *assign_dev, size_t n_rows, void *stream) {
     return rows_batch(ctx, features, n_features, columns_dev, assign_dev, n_rows, -1, stream);
+}
+
+int dist_b200_rows_accumulate_masked(dist_b200_ctx *ctx, dist_b200_feature *const *features, int n_features,
+                                     const void *const *columns_dev, const int32_t *assign_dev, size_t n_rows, double *xchg_dev,
+                                     const uint32_t *const *observed_dev, void *stream) {
+    return rows_batch(ctx, features, n_features, columns_dev, assign_dev, n_rows, +1, stream, kRowsAccumulate, xchg_dev,
+                      observed_dev);
+}
+
+int dist_b200_add_rows_batch_masked(dist_b200_ctx *ctx, dist_b200_feature *const *features, int n_features,
+                                    const void *const *columns_dev, const int32_t *assign_dev, size_t n_rows,
+                                    const uint32_t *const *observed_dev, void *stream) {
+    return rows_batch(ctx, features, n_features, columns_dev, assign_dev, n_rows, +1, stream, kRowsBoth, nullptr, observed_dev);
+}
+
+int dist_b200_remove_rows_batch_masked(dist_b200_ctx *ctx, dist_b200_feature *const *features, int n_features,
+                                       const void *const *columns_dev, const int32_t *assign_dev, size_t n_rows,
+                                       const uint32_t *const *observed_dev, void *stream) {
+    return rows_batch(ctx, features, n_features, columns_dev, assign_dev, n_rows, -1, stream, kRowsBoth, nullptr, observed_dev);
 }
 
 // bytes of one value of the feature's column: bool as uint8, niw a row of d floats, everything else 4 bytes
@@ -812,6 +840,29 @@ int dist_b200_sample_values_batch(dist_b200_ctx *ctx, const dist_b200_feature *c
         if ((rc = launch_sample_values(ctx, fs[i], sample_src(fs[i]), static_cast<uint32_t>(i), assign_dev, n_rows, seed, row0,
                                        columns_out_dev[i], s)))
             return rc;
+    return DIST_B200_OK;
+}
+
+// imputation: the unmasked kernels over an assignment vector that keeps only the missing cells' rows (mask_assign, keep = 0),
+// so every drawn cell is the unmasked call's draw for the same (seed, row, position) and every other cell is untouched
+int dist_b200_sample_values_batch_masked(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                                         const int32_t *assign_dev, size_t n_rows, uint64_t seed, uint64_t row0,
+                                         void *const *columns_out_dev, const uint32_t *const *observed_dev, void *stream) {
+    if (!ctx) return DIST_B200_ERR_INVALID;
+    dist_b200_feature *const *fs = const_cast<dist_b200_feature *const *>(features);
+    int rc = check_sample_args(ctx, fs, n_features, assign_dev, columns_out_dev);
+    if (rc || n_rows == 0 || !observed_dev) return rc;
+    cudaStream_t s = as_stream(stream);
+    if ((rc = wait_ready(ctx, features, n_features, s))) return rc;
+    if ((rc = grow(ctx, ctx->missing_scratch, ctx->missing_scratch_bytes, sizeof(int32_t) * n_rows))) return rc;
+    int32_t *missing_assign = static_cast<int32_t *>(ctx->missing_scratch);
+    for (int i = 0; i < n_features; ++i) {
+        if (!observed_dev[i]) continue;  // fully observed: nothing to impute
+        if ((rc = launch_mask_assign(ctx, assign_dev, observed_dev[i], n_rows, 0, missing_assign, s)) ||
+            (rc = launch_sample_values(ctx, fs[i], sample_src(fs[i]), static_cast<uint32_t>(i), missing_assign, n_rows, seed, row0,
+                                       columns_out_dev[i], s)))
+            return rc;
+    }
     return DIST_B200_OK;
 }
 
@@ -1248,30 +1299,40 @@ static int refresh_gp_tables(dist_b200_ctx *ctx, const dist_b200_feature *const 
     return DIST_B200_OK;
 }
 
-// logp != nullptr (assign = scores = nullptr): logp[n] = log sum_g exp(prior[g] + sum_f score_f) per row
-static int score_dispatch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int F,
-                          const void *const *columns, size_t N, const float *prior, const float *u,
-                          int32_t *assign, float *scores, int accumulate, cudaStream_t s, float *logp = nullptr) {
+// argument checks of every score entry; G = the list's number of groups
+static int check_score_args(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int F, const void *const *columns,
+                            const float *prior, const float *u, const int32_t *assign, const float *scores, int accumulate,
+                            const float *logp, int &G) {
     if (!ctx || !features || !columns || F < 1) return DIST_B200_ERR_INVALID;
     if (!assign && !scores && !logp) return fail(ctx, DIST_B200_ERR_INVALID, "score: no output requested");
     if (assign && !u) return fail(ctx, DIST_B200_ERR_INVALID, "score_sample: u is required");
     if (accumulate && prior) return fail(ctx, DIST_B200_ERR_INVALID, "score: prior is an overwrite, not valid with accumulate");
-    const int G = features[0] ? features[0]->G : 0;
+    G = features[0] ? features[0]->G : 0;
     if (G < 1) return fail(ctx, DIST_B200_ERR_STATE, "score: feature 0 has no groups (call update_all)");
     for (int f = 0; f < F; ++f) {
         if (!features[f] || !columns[f]) return fail(ctx, DIST_B200_ERR_INVALID, "score: null feature / column");
         if (features[f]->ctx != ctx) return fail(ctx, DIST_B200_ERR_INVALID, "score: feature belongs to another context");
         if (features[f]->G != G) return fail(ctx, DIST_B200_ERR_STATE, "score: features disagree on the number of groups");
     }
+    return DIST_B200_OK;
+}
+
+// Row-mapped models (nich/gp/bb/dd) fuse into one launch.  dpd (value-major table, warp per row) and
+// niw (dense contraction) have their own kernels: alone they run directly, in mixed lists the scores
+// are materialised, every feature accumulates, and the stand-alone sampler finishes.
+static bool solo(const dist_b200_feature *f) { return f->model == DIST_B200_DPD || f->model == DIST_B200_NIW; }
+
+// logp != nullptr (assign = scores = nullptr): logp[n] = log sum_g exp(prior[g] + sum_f score_f) per row
+static int score_dispatch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int F,
+                          const void *const *columns, size_t N, const float *prior, const float *u,
+                          int32_t *assign, float *scores, int accumulate, cudaStream_t s, float *logp = nullptr) {
+    int G = 0;
+    if (int rc = check_score_args(ctx, features, F, columns, prior, u, assign, scores, accumulate, logp, G)) return rc;
     if (N == 0) return DIST_B200_OK;
     {
         int rcw = wait_ready(ctx, features, F, s);
         if (rcw) return rcw;
     }
-    // Row-mapped models (nich/gp/bb/dd) fuse into one launch.  dpd (value-major table, warp per row) and
-    // niw (dense contraction) have their own kernels: alone they run directly, in mixed lists the scores
-    // are materialised, every feature accumulates, and the stand-alone sampler finishes.
-    auto solo = [](const dist_b200_feature *f) { return f->model == DIST_B200_DPD || f->model == DIST_B200_NIW; };
     int n_solo = 0;
     for (int f = 0; f < F; ++f) n_solo += solo(features[f]) ? 1 : 0;
     // ONE table feature (dpd / dd / bb), sampling only: every row with the same value has the same likelihood
@@ -1362,6 +1423,103 @@ static int score_dispatch(dist_b200_ctx *ctx, const dist_b200_feature *const *fe
     if (assign) return launch_sample_scores(ctx, buf, N, G, u, assign, s);
     if (logp) return launch_logp_scores(ctx, buf, N, G, logp, s);
     return DIST_B200_OK;
+}
+
+// ---- missing cells (dist_b200.h: "Missing cells") ----
+static bool any_mask(const uint32_t *const *observed, int F) {
+    for (int f = 0; observed && f < F; ++f)
+        if (observed[f]) return true;
+    return false;
+}
+
+// All-NULL masks take the unmasked dispatch.  Otherwise: every feature row-mapped -> one launch of the masked feature-list
+// kernel; dpd / niw in the list -> the row-mapped features' scores from the masked kernel into [N][G], each masked dpd /
+// niw feature scored alone into a second [N][G] buffer and added where observed (masked_accumulate), fully observed ones
+// accumulated directly as in the unmasked dispatch, then the stand-alone sampler or log-sum-exp.
+static int score_masked(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int F, const void *const *columns,
+                        const uint32_t *const *observed, size_t N, const float *prior, const float *u, int32_t *assign,
+                        float *scores, int accumulate, cudaStream_t s, float *logp = nullptr) {
+    if (!any_mask(observed, F)) return score_dispatch(ctx, features, F, columns, N, prior, u, assign, scores, accumulate, s, logp);
+    int G = 0;
+    if (int rc = check_score_args(ctx, features, F, columns, prior, u, assign, scores, accumulate, logp, G)) return rc;
+    if (N == 0) return DIST_B200_OK;
+    int rc = wait_ready(ctx, features, F, s);
+    if (rc) return rc;
+    int n_solo = 0, n_masked_solo = 0;
+    for (int f = 0; f < F; ++f) {
+        n_solo += solo(features[f]) ? 1 : 0;
+        n_masked_solo += solo(features[f]) && observed[f] ? 1 : 0;
+    }
+    if (F - n_solo > kMaxFeatures) return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "score: more than 512 features in one call");
+    FeatList fl;
+    MaskList ml;
+    fl.n = 0;
+    GpTableBatch tb;
+    tb.n = 0;
+    for (int f = 0; f < F; ++f) {
+        if (solo(features[f])) continue;
+        ml.m[fl.n] = observed[f];
+        if ((rc = fill_desc(ctx, features[f], columns[f], F > 1, fl.f[fl.n++], tb, s))) return rc;
+    }
+    if ((rc = launch_gp_table_batch(ctx, tb, s))) return rc;
+    if (n_solo == 0) return launch_score_rows_masked(ctx, fl, ml, G, N, prior, u, assign, scores, accumulate, logp, s);
+    const size_t cells = N * static_cast<size_t>(G);
+    float *buf = scores;
+    if (!buf) {
+        if ((rc = grow(ctx, ctx->scores_scratch, ctx->scores_scratch_bytes, sizeof(float) * cells))) return rc;
+        buf = static_cast<float *>(ctx->scores_scratch);
+    }
+    float *tmp = nullptr;
+    if (n_masked_solo) {
+        if ((rc = grow(ctx, ctx->missing_scratch, ctx->missing_scratch_bytes, sizeof(float) * cells))) return rc;
+        tmp = static_cast<float *>(ctx->missing_scratch);
+    }
+    bool started = accumulate != 0;
+    if (fl.n) {
+        if ((rc = launch_score_rows_masked(ctx, fl, ml, G, N, prior, nullptr, nullptr, buf, accumulate, nullptr, s))) return rc;
+        started = true;
+    }
+    for (int f = 0; f < F; ++f) {
+        const dist_b200_feature *feat = features[f];
+        if (!solo(feat)) continue;
+        const bool m = observed[f] != nullptr;
+        float *dst = m ? tmp : buf;
+        const float *p = m || started ? nullptr : prior;
+        const int acc = !m && started ? 1 : 0;
+        if (feat->model == DIST_B200_DPD) rc = launch_gather_rows(ctx, feat, columns[f], N, p, nullptr, nullptr, dst, acc, s);
+        else rc = launch_niw_scores(ctx, feat, columns[f], N, p, dst, acc, s);
+        if (!rc && m) rc = launch_masked_accumulate(ctx, buf, tmp, observed[f], N, G, started ? nullptr : prior, started ? 1 : 0, s);
+        if (rc) return rc;
+        started = true;
+    }
+    if (assign) return launch_sample_scores(ctx, buf, N, G, u, assign, s);
+    if (logp) return launch_logp_scores(ctx, buf, N, G, logp, s);
+    return DIST_B200_OK;
+}
+
+int dist_b200_score_batch_masked(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                                 const void *const *columns_dev, size_t n_rows, const float *prior_dev, float *scores_dev,
+                                 int accumulate, const uint32_t *const *observed_dev, void *stream) {
+    if (!scores_dev) return ctx ? fail(ctx, DIST_B200_ERR_INVALID, "score_batch: scores_dev is null") : DIST_B200_ERR_INVALID;
+    return score_masked(ctx, features, n_features, columns_dev, observed_dev, n_rows, prior_dev, nullptr, nullptr, scores_dev,
+                        accumulate, as_stream(stream));
+}
+
+int dist_b200_score_sample_batch_masked(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                                        const void *const *columns_dev, size_t n_rows, const float *prior_dev,
+                                        const float *u_dev, int32_t *assign_dev, float *scores_dev,
+                                        const uint32_t *const *observed_dev, void *stream) {
+    if (!assign_dev) return ctx ? fail(ctx, DIST_B200_ERR_INVALID, "score_sample_batch: assign_dev is null") : DIST_B200_ERR_INVALID;
+    return score_masked(ctx, features, n_features, columns_dev, observed_dev, n_rows, prior_dev, u_dev, assign_dev, scores_dev, 0,
+                        as_stream(stream));
+}
+
+int dist_b200_score_logp_batch_masked(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                                      const void *const *columns_dev, size_t n_rows, const float *prior_dev, float *logp_dev,
+                                      const uint32_t *const *observed_dev, void *stream) {
+    if (!logp_dev) return ctx ? fail(ctx, DIST_B200_ERR_INVALID, "score_logp_batch: logp_dev is null") : DIST_B200_ERR_INVALID;
+    return score_masked(ctx, features, n_features, columns_dev, observed_dev, n_rows, prior_dev, nullptr, nullptr, nullptr, 0,
+                        as_stream(stream), logp_dev);
 }
 
 int dist_b200_score_batch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,

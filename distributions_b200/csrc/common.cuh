@@ -41,6 +41,12 @@ struct FeatList {
     FeatDesc f[kMaxFeatures];
 };
 
+// observed masks of a feature list: m[f] is NULL (feature f fully observed) or ceil(N / 32) words, bit n % 32 of word
+// n / 32 set when row n's cell of feature f is observed (a separate kernel parameter: FeatList's layout is unchanged)
+struct MaskList {
+    const uint32_t *m[kMaxFeatures];
+};
+
 // GammaPoisson value tables of many features rebuilt in one launch (grid.y = feature)
 constexpr int kGpTableBatch = 128;
 struct GpTableBatch {
@@ -72,6 +78,11 @@ struct AddBatch {
     int xchg_first;              // index of d[0] in that buffer
     AddDesc d[kAddBatch];
 };
+// observed masks of an AddBatch's features (dist_b200.h, missing cells): m[f] for d[f], NULL = fully observed.  A
+// separate kernel parameter of the masked kernels, so AddBatch keeps its layout.
+struct AddMasks {
+    const uint32_t *m[kAddBatch];
+};
 
 }  // namespace distb200
 
@@ -92,6 +103,8 @@ struct dist_b200_ctx {
     size_t bbt_bytes = 0;
     void *scores_scratch = nullptr;   // [N][G] buffer of the materialising dispatch paths
     size_t scores_scratch_bytes = 0;
+    void *missing_scratch = nullptr;  // masked entries: per-feature [N] assignments, or one feature's [N][G] scores
+    size_t missing_scratch_bytes = 0;
     cudaStream_t own_stream = nullptr, own_stream2 = nullptr;
     cudaEvent_t ev = nullptr;
     void *add_acc = nullptr;          // batched add_value: per-feature accumulators (stats.cu)
@@ -224,19 +237,29 @@ int launch_score_rows(dist_b200_ctx *ctx, const FeatList &feats, int G, size_t N
                       const float *u, int32_t *assign, float *scores, int accumulate, cudaStream_t s,
                       const PushTargets *push = nullptr, float *logp = nullptr);
 int launch_gp_table_batch(dist_b200_ctx *ctx, const GpTableBatch &b, cudaStream_t s);
+// score_rows_masked*.cu: the feature-list kernel with missing cells (every feature row-mapped; assign, scores or logp)
+int launch_score_rows_masked(dist_b200_ctx *ctx, const FeatList &feats, const MaskList &masks, int G, size_t N,
+                             const float *prior, const float *u, int32_t *assign, float *scores, int accumulate,
+                             float *logp, cudaStream_t s);
+// missing.cu: out[n] = assign[n] where row n's bit equals `keep` (1: observed cells, 0: missing cells), else -1
+int launch_mask_assign(dist_b200_ctx *ctx, const int32_t *assign, const uint32_t *observed, size_t N, int keep, int32_t *out,
+                       cudaStream_t s);
+// scores[n][g] = base + (bit of row n ? tmp[n][g] : 0), base = scores[n][g] (accumulate) or prior[g] (or 0 without a prior)
+int launch_masked_accumulate(dist_b200_ctx *ctx, float *scores, const float *tmp, const uint32_t *observed, size_t N, int G,
+                             const float *prior, int accumulate, cudaStream_t s);
 // stats.cu: batched Group::add_value (segmented reduction of assigned rows into the device-side statistics)
 // pooled models: accumulate `b.n` features in one launch (b.acc zeroed by the launcher), then merge + rebuild caches
-int launch_add_rows_pooled(dist_b200_ctx *ctx, const AddBatch &b, cudaStream_t s);
+int launch_add_rows_pooled(dist_b200_ctx *ctx, const AddBatch &b, cudaStream_t s, const AddMasks *masks = nullptr);
 int launch_merge_prep_batch(dist_b200_ctx *ctx, const AddBatch &b, cudaStream_t s);  // prep.cu
 int launch_pack_accumulators(dist_b200_ctx *ctx, const AddBatch &b, double *xchg, cudaStream_t s);  // prep.cu
 // dd / dpd: counts updated in place
 int launch_add_rows_counts(dist_b200_ctx *ctx, dist_b200_feature *f, const void *column, const int32_t *assign, size_t N,
-                           int sign, cudaStream_t s, int32_t *dst = nullptr);
+                           int sign, cudaStream_t s, int32_t *dst = nullptr, const uint32_t *observed = nullptr);
 int launch_counts_to_doubles(dist_b200_ctx *ctx, const int32_t *src, double *dst, size_t n, cudaStream_t s);
 int launch_merge_counts(dist_b200_ctx *ctx, int32_t *counts, const double *delta, size_t n, int sign, cudaStream_t s);
 size_t add_rows_acc_bytes(int G);
 int launch_count_assignments(dist_b200_ctx *ctx, const int32_t *assign, size_t N, int G, int32_t *counts, int accumulate,
-                             cudaStream_t s);
+                             cudaStream_t s, const uint32_t *observed = nullptr);
 // gather_rows.cu: one warp per row, groups mapped to lanes (value-major tables: dpd, wide dd) and the
 // stand-alone sampler over materialised scores
 int launch_gather_rows(dist_b200_ctx *ctx, const dist_b200_feature *f, const void *column, size_t N,
@@ -269,7 +292,7 @@ int launch_score_data_finish(dist_b200_ctx *ctx, size_t n_grid, const double *ac
 inline size_t round_up(size_t x, size_t m) { return (x + m - 1) / m * m; }
 size_t niw_add_rows_bytes(int G, int d, size_t N);
 int launch_niw_accumulate(dist_b200_ctx *ctx, int G, int d, const void *values, const int32_t *assign, size_t N, double *acc,
-                          void *work, cudaStream_t s);
+                          void *work, cudaStream_t s, const uint32_t *observed = nullptr);
 int launch_niw_apply(dist_b200_ctx *ctx, int G, int d, int sign, const double *acc, int32_t *count, float *sum_x, float *sum_xxT,
                      cudaStream_t s);
 int launch_niw_score_data(dist_b200_ctx *ctx, int G, int d, const int32_t *count, const float *sum_x, const float *sum_xxT,

@@ -68,6 +68,18 @@ __global__ void __launch_bounds__(256) niw_scatter_kernel(const int32_t *__restr
     }
 }
 
+// the same, leaving out rows whose cell is missing (bit n % 32 of observed[n / 32] is 0): the accumulate kernels read
+// rows through perm only, so the histogram (count_observed_kernel) and this scatter are all that a mask changes
+__global__ void __launch_bounds__(256) niw_scatter_masked_kernel(const int32_t *__restrict__ assign, size_t N, int G,
+                                                                 int32_t *__restrict__ cursor, int32_t *__restrict__ perm,
+                                                                 const uint32_t *__restrict__ observed) {
+    for (size_t n = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; n < N; n += static_cast<size_t>(gridDim.x) * blockDim.x) {
+        const int g = assign[n];
+        const bool obs = (__ldg(observed + (n >> 5)) >> (n & 31)) & 1u;
+        if (obs && g >= 0 && g < G) perm[atomicAdd(&cursor[g], 1)] = static_cast<int32_t>(n);
+    }
+}
+
 struct NiwAccArgs {
     int G, d;
     const float *values;  // [N][d]
@@ -203,7 +215,7 @@ size_t niw_add_rows_bytes(int G, int d, size_t N) {
 
 // accumulate the rows' {count, sum_x, sum_xxT} per group into acc (zeroed here); work = niw_add_rows_bytes() scratch
 int launch_niw_accumulate(dist_b200_ctx *ctx, int G, int d, const void *values, const int32_t *assign, size_t N, double *acc,
-                          void *work, cudaStream_t s) {
+                          void *work, cudaStream_t s, const uint32_t *observed) {
     if (G <= 0) return DIST_B200_OK;
     if (N > 0x7FFFFFFFull) return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "niw add_rows: more than 2^31 rows in one batch");
     DISTB200_CUDA(ctx, cudaMemsetAsync(acc, 0, sizeof(double) * static_cast<size_t>(G) * (1 + d + d * d), s));
@@ -212,11 +224,12 @@ int launch_niw_accumulate(dist_b200_ctx *ctx, int G, int d, const void *values, 
     const size_t gi = round_up(sizeof(int32_t) * (static_cast<size_t>(G) + 1), 256);
     int32_t *hist = reinterpret_cast<int32_t *>(p), *offsets = reinterpret_cast<int32_t *>(p + gi), *cursor = reinterpret_cast<int32_t *>(p + 2 * gi),
             *unit_off = reinterpret_cast<int32_t *>(p + 3 * gi), *perm = reinterpret_cast<int32_t *>(p + 4 * gi);
-    int rc = launch_count_assignments(ctx, assign, N, G, hist, 0, s);
+    int rc = launch_count_assignments(ctx, assign, N, G, hist, 0, s, observed);
     if (rc) return rc;
     niw_scan_kernel<<<1, 1024, 0, s>>>(NiwScanArgs{G, hist, offsets, cursor, unit_off});
     const size_t want = (N + 255) / 256, cap = static_cast<size_t>(ctx->sm_count) * 8;
-    niw_scatter_kernel<<<static_cast<unsigned>(want < cap ? want : cap), 256, 0, s>>>(assign, N, G, cursor, perm);
+    if (observed) niw_scatter_masked_kernel<<<static_cast<unsigned>(want < cap ? want : cap), 256, 0, s>>>(assign, N, G, cursor, perm, observed);
+    else niw_scatter_kernel<<<static_cast<unsigned>(want < cap ? want : cap), 256, 0, s>>>(assign, N, G, cursor, perm);
     NiwAccArgs a{G, d, static_cast<const float *>(values), offsets, unit_off, perm, acc};
     const size_t units_bound = N / kNsSlice + G + 1;
     if (d <= 32) {

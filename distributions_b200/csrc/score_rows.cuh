@@ -242,12 +242,25 @@ struct RowsArgs {
 // the tile's maximum and the sums of exp over SUB-SLOTS of 16 groups, so that the draw is located down to 16 groups
 // from the main pass and only those are re-scored (from global memory, through the transposed GammaPoisson tables).
 constexpr int kSubGroups = 16;
+// Missing cells (feature lists only, MaskList in common.cuh).  A warp's 32 rows share one mask word: row tiles are
+// multiples of 32 rows.
+__device__ __forceinline__ bool cell_observed(const uint32_t *m, size_t row) {
+    return !m || ((__ldg(m + (row >> 5)) >> (row & 31)) & 1u);
+}
+// mask of feature f: none without masks (the unmasked kernel), else read from the kernel's MaskList parameter
+__device__ __forceinline__ const uint32_t *mask_of(int) { return nullptr; }
+__device__ __forceinline__ const uint32_t *mask_of(int f, const MaskList &ml) { return ml.m[f]; }
+
 // (logp mode: no minimum of resident blocks -- the register cap the others take would make its online pair spill)
-template <int CHUNK, int KIND, bool kSample, bool kScores, int THREADS, bool kSub = false>
+// Masks: empty, or one MaskList (score_rows_masked*.cu, feature lists with missing cells: a lane whose cell is missing
+// sits that feature out).  Without masks the kernel is the unmasked one instruction for instruction.
+template <int CHUNK, int KIND, bool kSample, bool kScores, int THREADS, bool kSub = false, typename... Masks>
 __global__ void __launch_bounds__(THREADS, (!kSample && !kScores) ? 1 : THREADS == 128 ? (is_dd_scaled(KIND) ? 5 : 3) : (CHUNK <= 32 ? (KIND >= 0 ? 4 : 3) : (CHUNK <= 64 ? 2 : 1)))
-score_rows_kernel(const __grid_constant__ FeatList feats, const RowsArgs a) {
+score_rows_kernel(const __grid_constant__ FeatList feats, const RowsArgs a, Masks... masks) {
+    constexpr bool kMask = sizeof...(Masks) > 0;
     constexpr int kThreads = THREADS;  // block size of this instantiation
     static_assert(!kSub || (KIND < 0 && kSample && !kScores && CHUNK % kSubGroups == 0), "kSub: streaming feature lists, sampling only");
+    static_assert(!kMask || KIND < 0, "masks: feature-list kernels only");
     constexpr int kSubPer = CHUNK / kSubGroups;  // sub-slots per tile
     extern __shared__ __align__(16) float smem[];
     // layout: coeff[33*8] | logfact[64] | prior[Gpad] | tile[8 warps][32][33] (kScores) |
@@ -457,6 +470,7 @@ score_rows_kernel(const __grid_constant__ FeatList feats, const RowsArgs a) {
                     const int st = kind_stride(fd.kind, fd.vdim);
                     uint32_t xn = 0;
                     const float *pb;
+                    const bool obs = kMask ? cell_observed(mask_of(f, masks...), row) : true;
                     if (resident) {
                         if (f + 1 < F) xn = load_value(feats.f[f + 1].kind, feats.f[f + 1].column, row);
                         pb = caches + res_off + static_cast<size_t>(g0) * st;
@@ -475,8 +489,11 @@ score_rows_kernel(const __grid_constant__ FeatList feats, const RowsArgs a) {
                             xb = word;
                         }
                     }
-                    accumulate_feature<CHUNK, false>(fd.kind, xb, pb, fd.vdim, acc, coeff, logfact,
-                                                     static_cast<const float4 *>(fd.aux) + g0);
+                    // a missing cell adds nothing: its lane sits out this feature (no arithmetic on the value it holds, so
+                    // an inf / NaN term of that value cannot reach the sum)
+                    if (!kMask || obs)
+                        accumulate_feature<CHUNK, false>(fd.kind, xb, pb, fd.vdim, acc, coeff, logfact,
+                                                         static_cast<const float4 *>(fd.aux) + g0);
                     if (resident) xb = xn;
                 }
                 if (!resident) __syncthreads();  // the ring is refilled by the next tile's prologue
@@ -814,6 +831,7 @@ score_rows_kernel(const __grid_constant__ FeatList feats, const RowsArgs a) {
             for (int j = 0; j < kSubGroups; ++j) sc16[j] = prior_s[gb + j];
             for (int f = 0; f < F; ++f) {
                 const FeatDesc &fd = feats.f[f];
+                if (kMask && !cell_observed(mask_of(f, masks...), row)) continue;  // the main pass added 0 for this cell
                 const uint32_t xv = load_value(fd.kind, fd.column, row);
                 if (fd.kind == kKindGpTable && xv < static_cast<uint32_t>(kGpTableX)) {
                     // transposed table [value][capacity] behind the [capacity][value] one: 64 contiguous bytes
@@ -879,6 +897,7 @@ score_rows_kernel(const __grid_constant__ FeatList feats, const RowsArgs a) {
                     } else
                     for (int f = 0; f < F; ++f) {
                         const FeatDesc &fd = feats.f[f];
+                        if (kMask && !cell_observed(mask_of(f, masks...), row)) continue;
                         const uint32_t xv = load_value(fd.kind, fd.column, row);
                         if (fd.kind == kKindGpTable && xv >= static_cast<uint32_t>(kGpTableX))
                             s += gp_term(static_cast<const float4 *>(fd.aux)[g], xv, coeff, logfact);
@@ -905,8 +924,8 @@ score_rows_kernel(const __grid_constant__ FeatList feats, const RowsArgs a) {
 
 // ---------------------------------------------------------------------------------------------
 // launchers (header templates: every score_rows_*.cu instantiates the variants of its own model)
-template <int CHUNK, int KIND, bool kSample, bool kScores, int THREADS, bool kSub = false>
-static int launch_variant(dist_b200_ctx *ctx, const FeatList &feats, RowsArgs a, cudaStream_t s) {
+template <int CHUNK, int KIND, bool kSample, bool kScores, int THREADS, bool kSub = false, bool kMask = false>
+static int launch_variant(dist_b200_ctx *ctx, const FeatList &feats, RowsArgs a, cudaStream_t s, const MaskList *masks = nullptr) {
     constexpr int kThreads = THREADS;
     const int G = a.G;
     const int nchunks = (G + CHUNK - 1) / CHUNK;
@@ -927,15 +946,26 @@ static int launch_variant(dist_b200_ctx *ctx, const FeatList &feats, RowsArgs a,
     a.stage_floats = CHUNK * max_stride;
     const size_t smem = fixed + (a.resident ? cache_floats : kStages * (static_cast<size_t>(a.stage_floats) + kThreads)) * sizeof(float);
     if (smem > 227 * 1024) return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "score_rows: group caches exceed shared memory");
-    auto kern = score_rows_kernel<CHUNK, KIND, kSample, kScores, kThreads, kSub>;
-    DISTB200_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    int per_sm = 0;
-    DISTB200_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, smem));
-    if (per_sm < 1) per_sm = 1;
-    const size_t ntiles = (a.N + kThreads - 1) / kThreads;
-    const size_t max_blocks = static_cast<size_t>(ctx->sm_count) * per_sm;
-    const unsigned grid = static_cast<unsigned>(ntiles < max_blocks ? ntiles : max_blocks);
-    kern<<<grid, kThreads, smem, s>>>(feats, a);
+    auto run = [&](auto kern, auto... extra) -> int {
+        DISTB200_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+        int per_sm = 0;
+        DISTB200_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, smem));
+        if (per_sm < 1) per_sm = 1;
+        const size_t ntiles = (a.N + kThreads - 1) / kThreads;
+        const size_t max_blocks = static_cast<size_t>(ctx->sm_count) * per_sm;
+        const unsigned grid = static_cast<unsigned>(ntiles < max_blocks ? ntiles : max_blocks);
+        kern<<<grid, kThreads, smem, s>>>(feats, a, extra...);
+        return DIST_B200_OK;
+    };
+    int rc;
+    if constexpr (kMask) {
+        void (*kern)(FeatList, RowsArgs, MaskList) = score_rows_kernel<CHUNK, KIND, kSample, kScores, kThreads, kSub, MaskList>;
+        rc = run(kern, *masks);
+    } else {
+        void (*kern)(FeatList, RowsArgs) = score_rows_kernel<CHUNK, KIND, kSample, kScores, kThreads, kSub>;
+        rc = run(kern);
+    }
+    if (rc) return rc;
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return fail(ctx, DIST_B200_ERR_CUDA, std::string("score_rows launch: ") + cudaGetErrorString(e));
     return DIST_B200_OK;
@@ -969,6 +999,34 @@ static __global__ void __launch_bounds__(256) bb_compact_kernel(const __grid_con
         out[g] = q.x;
         out[Gpad + g] = q.y;
     }
+}
+
+// the kSub kernel serves feature lists whose 32-group-tile caches do not fit the resident budget
+static bool ksub_wanted(const FeatList &feats, int G) {
+    size_t cache_bytes = 0;
+    for (int f = 0; f < feats.n; ++f)
+        cache_bytes += sizeof(float) * static_cast<size_t>((G + 31) / 32 * 32) * kind_stride(feats.f[f].kind, feats.f[f].vdim);
+    return cache_bytes > kResidentBudget;
+}
+
+// `local` = `feats` with every BetaBernoulli feature pointed at a compact copy of its caches for the kSub re-score
+static int ksub_list(dist_b200_ctx *ctx, const FeatList &feats, int G, FeatList &local, cudaStream_t s) {
+    const int Gpad = (G + 127) / 128 * 128;  // <= every feature's capacity (ensure_params pads to 128 groups)
+    int n_bb = 0;
+    for (int f = 0; f < feats.n; ++f) n_bb += feats.f[f].kind == DIST_B200_BB ? 1 : 0;
+    if (int rc = grow(ctx, ctx->bbt, ctx->bbt_bytes, sizeof(float) * n_bb * 2 * Gpad)) return rc;
+    local = feats;
+    for (int f = 0, k = 0; f < local.n; ++f)
+        if (local.f[f].kind == DIST_B200_BB) {
+            local.f[f].aux = ctx->bbt + static_cast<size_t>(k++) * 2 * Gpad;
+            local.f[f].cap = Gpad;
+        }
+    if (n_bb) {
+        bb_compact_kernel<<<dim3((Gpad + 255) / 256, local.n), 256, 0, s>>>(local, Gpad);
+        cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return fail(ctx, DIST_B200_ERR_CUDA, std::string("bb_compact launch: ") + cudaGetErrorString(e));
+    }
+    return DIST_B200_OK;
 }
 
 // Register tile.  G <= 128: the whole row in one tile (the sampler is then the reference's loops on registers);
@@ -1013,25 +1071,9 @@ static int launch_tiers(dist_b200_ctx *ctx, const FeatList &feats, const RowsArg
         // feature lists too large to keep resident (a cross-cat kind): the 128-group streaming tiles of the G <= 128 case
         // with sub-slot bookkeeping (kSub); measured at 256 features against the 32-group tiles + per-cell re-score of a whole
         // slot from global memory: G = 256, 1M rows 53.4 -> 14.9 ms; G = 1024, 100k rows 15.3 -> 7.19 ms
-        size_t cache_bytes = 0;
-        for (int f = 0; f < feats.n; ++f)
-            cache_bytes += sizeof(float) * static_cast<size_t>((a.G + 31) / 32 * 32) * kind_stride(feats.f[f].kind, feats.f[f].vdim);
-        if (cache_bytes > kResidentBudget) {
-            const int Gpad = (a.G + 127) / 128 * 128;  // <= every feature's capacity (ensure_params pads to 128 groups)
-            int n_bb = 0;
-            for (int f = 0; f < feats.n; ++f) n_bb += feats.f[f].kind == DIST_B200_BB ? 1 : 0;
-            if (int rc = grow(ctx, ctx->bbt, ctx->bbt_bytes, sizeof(float) * n_bb * 2 * Gpad)) return rc;
-            FeatList local = feats;
-            for (int f = 0, k = 0; f < local.n; ++f)
-                if (local.f[f].kind == DIST_B200_BB) {
-                    local.f[f].aux = ctx->bbt + static_cast<size_t>(k++) * 2 * Gpad;
-                    local.f[f].cap = Gpad;
-                }
-            if (n_bb) {
-                bb_compact_kernel<<<dim3((Gpad + 255) / 256, local.n), 256, 0, s>>>(local, Gpad);
-                cudaError_t e = cudaGetLastError();
-                if (e != cudaSuccess) return fail(ctx, DIST_B200_ERR_CUDA, std::string("bb_compact launch: ") + cudaGetErrorString(e));
-            }
+        if (ksub_wanted(feats, a.G)) {
+            FeatList local;
+            if (int rc = ksub_list(ctx, feats, a.G, local, s)) return rc;
             const int rc = launch_crosscat_ksub(ctx, local, a, s);
             if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;  // (too many groups for the sub-slot sums in shared memory)
         }

@@ -52,9 +52,22 @@ __device__ __forceinline__ void load4(const T *p, size_t q, T (&v)[4]) {
     }
 }
 
-template <bool kVec, typename T, typename Fn>
+// kMask: `observed` (NULL = every row) holds one bit per row (dist_b200.h, missing cells); a row whose bit is 0 reaches `fn`
+// with group -1, which every caller skips -- so the row's cell is left out of this feature only.  Four consecutive rows
+// from a multiple of 4 share one mask word.
+__device__ __forceinline__ int32_t observed_or_skip(const uint32_t *observed, size_t n, int32_t g) {
+    return !observed || ((__ldg(observed + (n >> 5)) >> (n & 31)) & 1u) ? g : -1;
+}
+__device__ __forceinline__ void mask4(const uint32_t *observed, size_t q, int32_t (&g)[4]) {
+    if (!observed) return;
+    const uint32_t bits = __ldg(observed + ((4 * q) >> 5)) >> ((4 * q) & 31);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) g[k] = (bits >> k) & 1u ? g[k] : -1;
+}
+
+template <bool kVec, bool kMask = false, typename T, typename Fn>
 __device__ __forceinline__ void for_each_row(const int32_t *__restrict__ assign, const T *__restrict__ col, size_t N, int threads,
-                                             Fn &&fn) {
+                                             Fn &&fn, const uint32_t *__restrict__ observed = nullptr) {
     const size_t stride = static_cast<size_t>(gridDim.x) * threads;
     const size_t first = static_cast<size_t>(blockIdx.x) * threads + threadIdx.x;
     if constexpr (kVec) {
@@ -67,6 +80,10 @@ __device__ __forceinline__ void for_each_row(const int32_t *__restrict__ assign,
             load4(assign, q + stride, g1);
             load4(col, q, x0);
             load4(col, q + stride, x1);
+            if constexpr (kMask) {
+                mask4(observed, q, g0);
+                mask4(observed, q + stride, g1);
+            }
 #pragma unroll
             for (int k = 0; k < 4; ++k) fn(g0[k], x0[k]);
 #pragma unroll
@@ -77,20 +94,30 @@ __device__ __forceinline__ void for_each_row(const int32_t *__restrict__ assign,
             T x0[4];
             load4(assign, q, g0);
             load4(col, q, x0);
+            if constexpr (kMask) mask4(observed, q, g0);
 #pragma unroll
             for (int k = 0; k < 4; ++k) fn(g0[k], x0[k]);
         }
         const size_t n = 4 * n4 + first;  // the last N % 4 rows
-        if (n < N) fn(assign[n], col[n]);
+        if constexpr (kMask) {
+            if (n < N) fn(observed_or_skip(observed, n, assign[n]), col[n]);
+        } else {
+            if (n < N) fn(assign[n], col[n]);
+        }
     } else {
-        for (size_t n = first; n < N; n += stride) fn(assign[n], col[n]);
+        if constexpr (kMask) {
+            for (size_t n = first; n < N; n += stride) fn(observed_or_skip(observed, n, assign[n]), col[n]);
+        } else {
+            for (size_t n = first; n < N; n += stride) fn(assign[n], col[n]);
+        }
     }
 }
 
 // ---------------------------------------------------------------------------------------------
 // pooled models: grid (row tiles, features)
-template <bool kSmem, bool kVec>
-__global__ void __launch_bounds__(kAddThreads) add_rows_pooled_kernel(const AddBatch b) {
+// kMask: `observed` (NULL = fully observed) is the mask of feature d[blockIdx.y]
+template <bool kSmem, bool kVec, bool kMask>
+__device__ __forceinline__ void add_rows_pooled(const AddBatch &b, const uint32_t *observed) {
     extern __shared__ __align__(8) unsigned char add_smem[];
     const int G = b.G;
     const AddDesc &d = b.d[blockIdx.y];
@@ -123,7 +150,7 @@ __global__ void __launch_bounds__(kAddThreads) add_rows_pooled_kernel(const AddB
     // warp's popular groups are therefore combined in registers first (masked butterfly, one atomic per
     // peeled group); lanes of unpopular groups go direct.
     if (model == DIST_B200_NICH) {
-        for_each_row<kVec>(b.assign, static_cast<const float *>(d.column), b.N, kAddThreads, [&](int g, float xf) {
+        for_each_row<kVec, kMask>(b.assign, static_cast<const float *>(d.column), b.N, kAddThreads, [&](int g, float xf) {
             const unsigned active = __activemask();
             const int lane = threadIdx.x & 31;
             bool pending = g >= 0 && g < G;
@@ -157,18 +184,18 @@ __global__ void __launch_bounds__(kAddThreads) add_rows_pooled_kernel(const AddB
                 atomicAdd(&ax[g], x);
                 atomicAdd(&axx[g], xx);
             }
-        });
+        }, observed);
     } else if (model == DIST_B200_GP || model == DIST_B200_BNB) {
-        for_each_row<kVec>(b.assign, static_cast<const uint32_t *>(d.column), b.N, kAddThreads, [&](int g, uint32_t x) {
+        for_each_row<kVec, kMask>(b.assign, static_cast<const uint32_t *>(d.column), b.N, kAddThreads, [&](int g, uint32_t x) {
             if (g < 0 || g >= G) return;
             atomicAdd(&ca[g], 1);
             atomicAdd(reinterpret_cast<unsigned int *>(&cb[g]), x);
-        });
+        }, observed);
     } else {  // bb
-        for_each_row<kVec>(b.assign, static_cast<const uint8_t *>(d.column), b.N, kAddThreads, [&](int g, uint8_t x) {
+        for_each_row<kVec, kMask>(b.assign, static_cast<const uint8_t *>(d.column), b.N, kAddThreads, [&](int g, uint8_t x) {
             if (g < 0 || g >= G) return;
             atomicAdd(x != 0 ? &ca[g] : &cb[g], 1);
-        });
+        }, observed);
     }
     if (kSmem) {
         __syncthreads();
@@ -181,6 +208,19 @@ __global__ void __launch_bounds__(kAddThreads) add_rows_pooled_kernel(const AddB
             }
         }
     }
+}
+
+// ---------------------------------------------------------------------------------------------
+
+template <bool kSmem, bool kVec>
+__global__ void __launch_bounds__(kAddThreads) add_rows_pooled_kernel(const AddBatch b) {
+    add_rows_pooled<kSmem, kVec, false>(b, nullptr);
+}
+
+// the same with per-feature observed masks (masks.m[f] for feature d[f])
+template <bool kSmem, bool kVec>
+__global__ void __launch_bounds__(kAddThreads) add_rows_pooled_masked_kernel(const AddBatch b, const AddMasks masks) {
+    add_rows_pooled<kSmem, kVec, true>(b, masks.m[blockIdx.y]);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -206,8 +246,8 @@ __device__ __forceinline__ int dpd_row(const CountArgs &a, uint32_t value) {
     return (lo < a.dim && a.keys[lo] == value) ? a.key_rows[lo] : -1;
 }
 
-template <bool kSmem, bool kVec>
-__global__ void __launch_bounds__(kAddThreads) add_rows_counts_kernel(const CountArgs a) {
+template <bool kSmem, bool kVec, bool kMask>
+__device__ __forceinline__ void add_rows_counts(const CountArgs &a, const uint32_t *observed) {
     extern __shared__ int32_t bins[];
     const int cells = a.G * a.dim;
     if (kSmem) {
@@ -216,7 +256,7 @@ __global__ void __launch_bounds__(kAddThreads) add_rows_counts_kernel(const Coun
     }
     int32_t *dst = kSmem ? bins : a.counts;
     // dd values are int32 ids, dpd values uint32 keys: both stream as uint32
-    for_each_row<kVec>(a.assign, static_cast<const uint32_t *>(a.column), a.N, kAddThreads, [&](int g, uint32_t x) {
+    for_each_row<kVec, kMask>(a.assign, static_cast<const uint32_t *>(a.column), a.N, kAddThreads, [&](int g, uint32_t x) {
         int cell = -1;
         if (g >= 0 && g < a.G) {
             if (a.model == DIST_B200_DD) {
@@ -229,7 +269,7 @@ __global__ void __launch_bounds__(kAddThreads) add_rows_counts_kernel(const Coun
         if (cell < 0) return;
         if (a.sign > 0) atomicAdd(&dst[cell], 1);
         else atomicAdd(&dst[cell], -1);
-    });
+    }, observed);
     if (kSmem) {
         __syncthreads();
         for (int i = threadIdx.x; i < cells; i += kAddThreads)
@@ -238,22 +278,45 @@ __global__ void __launch_bounds__(kAddThreads) add_rows_counts_kernel(const Coun
 }
 
 template <bool kSmem, bool kVec>
-__global__ void __launch_bounds__(kAddThreads) count_assignments_kernel(const int32_t *__restrict__ assign, size_t N, int G,
-                                                                        int32_t *__restrict__ counts) {
+__global__ void __launch_bounds__(kAddThreads) add_rows_counts_kernel(const CountArgs a) {
+    add_rows_counts<kSmem, kVec, false>(a, nullptr);
+}
+
+template <bool kSmem, bool kVec>
+__global__ void __launch_bounds__(kAddThreads) add_rows_counts_masked_kernel(const CountArgs a, const uint32_t *observed) {
+    add_rows_counts<kSmem, kVec, true>(a, observed);
+}
+
+// kMask: rows whose bit in `observed` is 0 are not counted (the niw histogram of a feature with missing cells)
+template <bool kSmem, bool kVec, bool kMask>
+__device__ __forceinline__ void count_assignments(const int32_t *__restrict__ assign, size_t N, int G, int32_t *__restrict__ counts,
+                                                  const uint32_t *observed) {
     extern __shared__ int32_t bins[];
     if (kSmem) {
         for (int i = threadIdx.x; i < G; i += kAddThreads) bins[i] = 0;
         __syncthreads();
     }
     int32_t *dst = kSmem ? bins : counts;
-    for_each_row<kVec>(assign, assign, N, kAddThreads, [&](int g, int) {
+    for_each_row<kVec, kMask>(assign, assign, N, kAddThreads, [&](int g, int) {
         if (g >= 0 && g < G) atomicAdd(&dst[g], 1);
-    });
+    }, observed);
     if (kSmem) {
         __syncthreads();
         for (int i = threadIdx.x; i < G; i += kAddThreads)
             if (bins[i]) atomicAdd(&counts[i], bins[i]);
     }
+}
+
+template <bool kSmem, bool kVec>
+__global__ void __launch_bounds__(kAddThreads) count_assignments_kernel(const int32_t *__restrict__ assign, size_t N, int G,
+                                                                        int32_t *__restrict__ counts) {
+    count_assignments<kSmem, kVec, false>(assign, N, G, counts, nullptr);
+}
+
+template <bool kSmem, bool kVec>
+__global__ void __launch_bounds__(kAddThreads) count_observed_kernel(const int32_t *__restrict__ assign, size_t N, int G,
+                                                                     int32_t *__restrict__ counts, const uint32_t *observed) {
+    count_assignments<kSmem, kVec, true>(assign, N, G, counts, observed);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -267,7 +330,8 @@ static unsigned row_tiles(const dist_b200_ctx *ctx, size_t N, int per_sm, int sp
     return static_cast<unsigned>(want < cap ? want : cap);
 }
 
-int launch_add_rows_pooled(dist_b200_ctx *ctx, const AddBatch &b_in, cudaStream_t s) {
+// masks (may be NULL): the batch's observed masks; a batch whose masks are all NULL takes the unmasked kernel
+int launch_add_rows_pooled(dist_b200_ctx *ctx, const AddBatch &b_in, cudaStream_t s, const AddMasks *masks) {
     if (b_in.G == 0 || b_in.n == 0) return DIST_B200_OK;
     const AddBatch &b = b_in;
     // zeroed BEFORE the empty-batch early-out: the merge / pack that follows an empty batch (a rank whose row
@@ -279,7 +343,14 @@ int launch_add_rows_pooled(dist_b200_ctx *ctx, const AddBatch &b_in, cudaStream_
     for (int i = 0; i < b.n; ++i) vec = vec && aligned16(b.d[i].column);
     const bool smem = b.G <= kAddSmemGroups;
     const size_t sb = smem ? static_cast<size_t>(b.G) * 24 : 0;
-    if (smem && vec) add_rows_pooled_kernel<true, true><<<grid, kAddThreads, sb, s>>>(b);
+    bool masked = false;
+    for (int i = 0; masks && i < b.n; ++i) masked = masked || masks->m[i];
+    if (masked) {
+        if (smem && vec) add_rows_pooled_masked_kernel<true, true><<<grid, kAddThreads, sb, s>>>(b, *masks);
+        else if (smem) add_rows_pooled_masked_kernel<true, false><<<grid, kAddThreads, sb, s>>>(b, *masks);
+        else if (vec) add_rows_pooled_masked_kernel<false, true><<<grid, kAddThreads, 0, s>>>(b, *masks);
+        else add_rows_pooled_masked_kernel<false, false><<<grid, kAddThreads, 0, s>>>(b, *masks);
+    } else if (smem && vec) add_rows_pooled_kernel<true, true><<<grid, kAddThreads, sb, s>>>(b);
     else if (smem) add_rows_pooled_kernel<true, false><<<grid, kAddThreads, sb, s>>>(b);
     else if (vec) add_rows_pooled_kernel<false, true><<<grid, kAddThreads, 0, s>>>(b);
     else add_rows_pooled_kernel<false, false><<<grid, kAddThreads, 0, s>>>(b);
@@ -288,9 +359,9 @@ int launch_add_rows_pooled(dist_b200_ctx *ctx, const AddBatch &b_in, cudaStream_
     return DIST_B200_OK;
 }
 
-// dst: the count table to update (nullptr = the feature's own statistics)
+// dst: the count table to update (nullptr = the feature's own statistics); observed: the feature's mask, or NULL
 int launch_add_rows_counts(dist_b200_ctx *ctx, dist_b200_feature *f, const void *column, const int32_t *assign, size_t N,
-                           int sign, cudaStream_t s, int32_t *dst) {
+                           int sign, cudaStream_t s, int32_t *dst, const uint32_t *observed) {
     if (N == 0 || f->G == 0) return DIST_B200_OK;
     CountArgs a{};
     a.model = f->model;
@@ -306,7 +377,15 @@ int launch_add_rows_counts(dist_b200_ctx *ctx, dist_b200_feature *f, const void 
     a.key_rows = f->key_rows_dev;
     const size_t cells = static_cast<size_t>(f->G) * f->dim;
     const bool vec = aligned16(assign) && aligned16(column);
-    if (cells <= kCountSmemBins) {
+    if (observed) {
+        const bool smem = cells <= kCountSmemBins;
+        const unsigned grid = row_tiles(ctx, (N + 3) / 4, smem ? 4 : 8, 1);
+        const size_t sb = smem ? cells * 4 : 0;
+        if (smem && vec) add_rows_counts_masked_kernel<true, true><<<grid, kAddThreads, sb, s>>>(a, observed);
+        else if (smem) add_rows_counts_masked_kernel<true, false><<<grid, kAddThreads, sb, s>>>(a, observed);
+        else if (vec) add_rows_counts_masked_kernel<false, true><<<grid, kAddThreads, 0, s>>>(a, observed);
+        else add_rows_counts_masked_kernel<false, false><<<grid, kAddThreads, 0, s>>>(a, observed);
+    } else if (cells <= kCountSmemBins) {
         const unsigned grid = row_tiles(ctx, (N + 3) / 4, 4, 1);
         if (vec) add_rows_counts_kernel<true, true><<<grid, kAddThreads, cells * 4, s>>>(a);
         else add_rows_counts_kernel<true, false><<<grid, kAddThreads, cells * 4, s>>>(a);
@@ -352,13 +431,18 @@ int launch_merge_counts(dist_b200_ctx *ctx, int32_t *counts, const double *delta
 }
 
 int launch_count_assignments(dist_b200_ctx *ctx, const int32_t *assign, size_t N, int G, int32_t *counts, int accumulate,
-                             cudaStream_t s) {
+                             cudaStream_t s, const uint32_t *observed) {
     if (!accumulate) DISTB200_CUDA(ctx, cudaMemsetAsync(counts, 0, sizeof(int32_t) * G, s));
     if (N == 0) return DIST_B200_OK;
     const unsigned grid = row_tiles(ctx, (N + 3) / 4, 4, 1);
     const bool vec = aligned16(assign), smem = G <= kCountSmemBins;
     const size_t sb = smem ? static_cast<size_t>(G) * 4 : 0;
-    if (smem && vec) count_assignments_kernel<true, true><<<grid, kAddThreads, sb, s>>>(assign, N, G, counts);
+    if (observed) {
+        if (smem && vec) count_observed_kernel<true, true><<<grid, kAddThreads, sb, s>>>(assign, N, G, counts, observed);
+        else if (smem) count_observed_kernel<true, false><<<grid, kAddThreads, sb, s>>>(assign, N, G, counts, observed);
+        else if (vec) count_observed_kernel<false, true><<<grid, kAddThreads, 0, s>>>(assign, N, G, counts, observed);
+        else count_observed_kernel<false, false><<<grid, kAddThreads, 0, s>>>(assign, N, G, counts, observed);
+    } else if (smem && vec) count_assignments_kernel<true, true><<<grid, kAddThreads, sb, s>>>(assign, N, G, counts);
     else if (smem) count_assignments_kernel<true, false><<<grid, kAddThreads, sb, s>>>(assign, N, G, counts);
     else if (vec) count_assignments_kernel<false, true><<<grid, kAddThreads, 0, s>>>(assign, N, G, counts);
     else count_assignments_kernel<false, false><<<grid, kAddThreads, 0, s>>>(assign, N, G, counts);

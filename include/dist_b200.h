@@ -398,6 +398,61 @@ int dist_b200_score_logp_batch_host(dist_b200_ctx *ctx, const dist_b200_feature 
 int dist_b200_logp_from_scores(dist_b200_ctx *ctx, const float *scores_dev, size_t n_rows, int G,
                                float *logp_dev, void *stream);
 
+/* ---- missing cells: per-feature observed masks ------------------------------------------------------------------
+ * A cross-cat table has holes.  As in loom's ProductModel, whose Value carries an `observed` flag per feature, an
+ * unobserved feature simply does not enter the row's score or its group's statistics.  The *_masked entries take the
+ * arguments of their unmasked form plus observed_dev: n_features device pointers, one per feature, each NULL (that
+ * feature is fully observed) or ceil(n_rows / 32) uint32 words; bit n % 32 of word n / 32 is 1 when row n's cell is
+ * observed (bits past n_rows are ignored).  np.packbits(column, bitorder="little") read as little-endian uint32 is this
+ * layout.  observed_dev itself may be NULL (every feature fully observed).
+ *   - Scoring: a missing cell contributes exactly 0: scores[n][g] = prior[g] + sum_f observed_f[n] * score_f(x_f[n]; g).
+ *     Its stored value is never used in arithmetic (it may be NaN, a dd value >= dim, a huge count).  A row with every
+ *     feature missing scores the prior alone: its draw comes from the prior and its logp is logsumexp(prior).
+ *   - add / remove rows, rows_accumulate: a missing cell leaves that feature's statistics alone, exactly as if
+ *     assign_dev[n] were -1 for that feature only.  The row's other features are unaffected.  The exchange layout of
+ *     rows_accumulate is the unmasked one (merge with dist_b200_rows_merge).
+ *   - Imputation (sample_values_batch_masked): a draw is written into every MISSING cell of a row with a valid
+ *     assignment, and nothing else: observed cells and rows with an invalid id keep their values.  The draw is the one
+ *     dist_b200_sample_values_batch writes for the same (seed, row0, row, list position), so the result is
+ *     where(observed, column, unmasked draws) bit for bit.  Here a NULL mask means nothing is imputed for that feature.
+ *   - With every mask NULL the score, sample, logp and rows entries ARE the unmasked entries (bit-identical results).
+ *     Argument checks and error codes are those of the unmasked entries.
+ * Routes and costs.  Lists of row-mapped features (nich / gp / bnb / bb / dd, including a list of one) run the
+ * feature-list kernel with the masks as a separate kernel parameter: one broadcast word per warp and feature, and a
+ * lane whose cell is missing sits that feature out.  dpd and niw features are scored alone (their own kernels) into a
+ * second context [N][G] buffer and added where observed: one extra [N][G] write and read per masked dpd / niw feature
+ * (fully observed ones accumulate directly).  The single-feature, nich_rows2, table, per-value and niw tensor-core
+ * sampling kernels have no masked form; their features take the two routes above.  add / remove rows and
+ * rows_accumulate run masked instantiations of the pooled, count-table and niw histogram / scatter kernels (one mask
+ * word per 32 rows, pooled batches of up to 128 features as unmasked).  Imputation runs the unmasked sampling kernels
+ * over an assignment vector with -1 in the observed rows: one extra N-int pass per masked feature.
+ * Streams: the masked score route (with dpd / niw) and imputation use a context scratch buffer of their own, ordered
+ * only by the stream of the call, as the context's scores buffer is: masked calls of one context on two streams at
+ * once must not overlap.
+ * There are no masked forms of dist_b200_score_push_batch or of the host-buffer entries. */
+int dist_b200_score_batch_masked(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                                 const void *const *columns_dev, size_t n_rows, const float *prior_dev, float *scores_dev,
+                                 int accumulate, const uint32_t *const *observed_dev, void *stream);
+int dist_b200_score_sample_batch_masked(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                                        const void *const *columns_dev, size_t n_rows, const float *prior_dev,
+                                        const float *u_dev, int32_t *assign_dev, float *scores_dev,
+                                        const uint32_t *const *observed_dev, void *stream);
+int dist_b200_score_logp_batch_masked(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                                      const void *const *columns_dev, size_t n_rows, const float *prior_dev, float *logp_dev,
+                                      const uint32_t *const *observed_dev, void *stream);
+int dist_b200_add_rows_batch_masked(dist_b200_ctx *ctx, dist_b200_feature *const *features, int n_features,
+                                    const void *const *columns_dev, const int32_t *assign_dev, size_t n_rows,
+                                    const uint32_t *const *observed_dev, void *stream);
+int dist_b200_remove_rows_batch_masked(dist_b200_ctx *ctx, dist_b200_feature *const *features, int n_features,
+                                       const void *const *columns_dev, const int32_t *assign_dev, size_t n_rows,
+                                       const uint32_t *const *observed_dev, void *stream);
+int dist_b200_rows_accumulate_masked(dist_b200_ctx *ctx, dist_b200_feature *const *features, int n_features,
+                                     const void *const *columns_dev, const int32_t *assign_dev, size_t n_rows, double *xchg_dev,
+                                     const uint32_t *const *observed_dev, void *stream);
+int dist_b200_sample_values_batch_masked(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
+                                         const int32_t *assign_dev, size_t n_rows, uint64_t seed, uint64_t row0,
+                                         void *const *columns_out_dev, const uint32_t *const *observed_dev, void *stream);
+
 /* ---- feature shards over NVLink peer memory (one process per GPU) ----------------------------------
  * scores[n][g] = prior[g] + sum_f s_f[n][g] is a sum over features (SURVEY.md §8e).  With the features of
  * a kind sharded over K ranks, each rank scores its features for every row and stores the partial row
