@@ -521,10 +521,12 @@ score_rows_kernel(const __grid_constant__ FeatList feats, const RowsArgs a, Mask
 #pragma unroll
                     for (int j = 0; j < 32; ++j) tw[lane * 33 + j] = acc[sb * 32 + j];
                     __syncwarp();
-                    if (((G & 3) == 0) && g0 + sb * 32 + 32 <= G && !a.accumulate) {
+                    if (((G & 3) == 0) && g0 + sb * 32 + 32 <= G && !a.accumulate && (!a.n_push || a.block_rows >= 32)) {
                         // 16-byte stores: lane (r, c) = (lane / 8, lane % 8) writes groups [4c, 4c + 4) of rows r, r + 4, ...
                         // -- four conflict-free scalar LDS, one ST.128; a store instruction covers four 128-byte row
-                        // segments (a quarter of the store instructions, 16 B per lane on the NVLink path)
+                        // segments (a quarter of the store instructions, 16 B per lane on the NVLink path).  A push
+                        // takes them only with blocks of >= 32 rows, where the warp's 32 rows span at most two owners;
+                        // smaller blocks take the scalar path below, which walks any number of owners.
                         const int r = lane >> 3, c = lane & 7;
                         const int gq = g0 + sb * 32 + 4 * c;
                         const size_t grow0 = a.row0 + wrow0;
@@ -550,7 +552,7 @@ score_rows_kernel(const __grid_constant__ FeatList feats, const RowsArgs a, Mask
                     if (g >= G) continue;
                     const float *src = tw + lane;
                     if (a.n_push) {
-                        // rows of this warp tile land in at most two owners' slots
+                        // rows of this warp tile land in as many owners' slots as its 32 rows span
                         const size_t grow0 = a.row0 + wrow0;
                         int owner = static_cast<int>(grow0 / a.block_rows);
                         size_t off = grow0 - static_cast<size_t>(owner) * a.block_rows;

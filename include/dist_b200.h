@@ -466,7 +466,9 @@ int dist_b200_peer_close(dist_b200_ctx *ctx, void *dev_ptr);
 int dist_b200_peer_free(dist_b200_ctx *ctx, void *dev_ptr);
 /* Partial scores of rows [row0, row0 + n_rows) for this rank's features, pushed to the owners' slots:
  * slot_ptrs[o] is the (peer-mapped) base of THIS rank's slot in owner o's buffer.  prior_dev is passed
- * by exactly one rank.  Row-mapped models only (nich / gp / bb / dd). */
+ * by exactly one rank.  Row-mapped models only (nich / gp / bnb / bb / dd; dpd and niw return
+ * DIST_B200_ERR_UNSUPPORTED).  Any block_rows >= 1 and any row0 are accepted.  When G % 4 == 0 every slot pointer
+ * must be 16-byte aligned (rows are stored 16 bytes at a time). */
 int dist_b200_score_push_batch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
                                const void *const *columns_dev, size_t n_rows, size_t row0, const float *prior_dev,
                                void *const *slot_ptrs, int n_owners, size_t block_rows, void *stream);
