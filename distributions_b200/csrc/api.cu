@@ -1229,9 +1229,15 @@ int dist_b200_prior_pitman_yor_host(dist_b200_ctx *ctx, float alpha, float d, in
 }
 
 // ---- the hot path ---------------------------------------------------------------------------
-// Describe one row-mapped feature for the score kernel.  In multi-feature lists GammaPoisson goes through
-// its per-(group, value) table (rebuilt lazily, stream-ordered, after any cache update).
+// Make f's GammaPoisson value table current: grown with the feature's capacity, its rebuild queued in `tb` when stale
+// (rebuilt lazily, stream-ordered, after any cache update).  The caller launches what remains queued.
 static int queue_gp_table(dist_b200_ctx *ctx, dist_b200_feature *f, GpTableBatch &tb, cudaStream_t s) {
+    const size_t bytes = sizeof(float) * 2 * kGpTableX * f->capacity;  // [capacity][x] | [x][capacity]
+    if (bytes > f->gp_table_bytes) {
+        if (int rc = grow(ctx, f->gp_table, f->gp_table_bytes, bytes)) return rc;
+        f->gp_table_dirty = true;
+    }
+    if (!f->gp_table_dirty) return DIST_B200_OK;
     if (tb.n == kGpTableBatch) {
         int rc = launch_gp_table_batch(ctx, tb, s);
         if (rc) return rc;
@@ -1245,10 +1251,7 @@ static int queue_gp_table(dist_b200_ctx *ctx, dist_b200_feature *f, GpTableBatch
     return DIST_B200_OK;
 }
 
-// the GammaPoisson value table: [capacity][x] | [x][capacity]
-static size_t gp_table_bytes(const dist_b200_feature *f) { return sizeof(float) * 2 * kGpTableX * f->capacity; }
-
-// stale tables are queued in `tb`; the caller launches the remainder before the score kernel
+// Describe one row-mapped feature for the score kernel.  multi: GammaPoisson goes through its per-(group, value) table.
 static int fill_desc(dist_b200_ctx *ctx, const dist_b200_feature *cf, const void *column, bool multi, FeatDesc &d,
                      GpTableBatch &tb, cudaStream_t s) {
     dist_b200_feature *f = const_cast<dist_b200_feature *>(cf);
@@ -1260,14 +1263,7 @@ static int fill_desc(dist_b200_ctx *ctx, const dist_b200_feature *cf, const void
     d.cap = f->capacity;
     d.pad_ = 0;
     if (multi && f->model == DIST_B200_GP) {
-        if (gp_table_bytes(f) > f->gp_table_bytes) {
-            if (int rc = grow(ctx, f->gp_table, f->gp_table_bytes, gp_table_bytes(f))) return rc;
-            f->gp_table_dirty = true;
-        }
-        if (f->gp_table_dirty) {
-            int rc = queue_gp_table(ctx, f, tb, s);
-            if (rc) return rc;
-        }
+        if (int rc = queue_gp_table(ctx, f, tb, s)) return rc;
         d.params = f->gp_table;
         d.kind = kKindGpTable;
         d.vdim = kGpTableX;
@@ -1282,14 +1278,13 @@ static int refresh_gp_tables(dist_b200_ctx *ctx, const dist_b200_feature *const 
     if (F < 2) return DIST_B200_OK;
     GpTableBatch tb;
     tb.n = 0;
-    FeatDesc scratch_desc;
     bool any = false;
     for (int f = 0; f < F; ++f) {
         if (!features[f] || features[f]->model != DIST_B200_GP) continue;
-        const bool stale = features[f]->gp_table_dirty || features[f]->gp_table_bytes < gp_table_bytes(features[f]);
-        int rc = fill_desc(ctx, features[f], nullptr, true, scratch_desc, tb, s);
+        const int queued = tb.n;
+        int rc = queue_gp_table(ctx, const_cast<dist_b200_feature *>(features[f]), tb, s);
         if (rc) return rc;
-        any = any || stale;
+        any = any || tb.n != queued;
     }
     if (!any) return DIST_B200_OK;
     int rc = launch_gp_table_batch(ctx, tb, s);
@@ -1322,173 +1317,113 @@ static int check_score_args(dist_b200_ctx *ctx, const dist_b200_feature *const *
 // are materialised, every feature accumulates, and the stand-alone sampler finishes.
 static bool solo(const dist_b200_feature *f) { return f->model == DIST_B200_DPD || f->model == DIST_B200_NIW; }
 
-// logp != nullptr (assign = scores = nullptr): logp[n] = log sum_g exp(prior[g] + sum_f score_f) per row
-static int score_dispatch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int F,
-                          const void *const *columns, size_t N, const float *prior, const float *u,
-                          int32_t *assign, float *scores, int accumulate, cudaStream_t s, float *logp = nullptr) {
-    int G = 0;
-    if (int rc = check_score_args(ctx, features, F, columns, prior, u, assign, scores, accumulate, logp, G)) return rc;
-    if (N == 0) return DIST_B200_OK;
-    {
-        int rcw = wait_ready(ctx, features, F, s);
-        if (rcw) return rcw;
-    }
-    int n_solo = 0;
-    for (int f = 0; f < F; ++f) n_solo += solo(features[f]) ? 1 : 0;
-    // ONE table feature (dpd / dd / bb), sampling only: every row with the same value has the same likelihood
-    // vector, so it is evaluated once per distinct value (per-value CDF trees, table_rows.cu).  SURVEY 8(d)
-    // "algorithmic shortcut"; DIST_B200_OPT_VALUE_CDF = 1 keeps the per-cell kernels (what bench.py reports beside it),
-    // 2 = the round-2 tree search instead of the guide-table walk
-    if (F == 1 && assign && !scores && !accumulate && ctx->opt[DIST_B200_OPT_VALUE_CDF] != 1 &&
-        (features[0]->model == DIST_B200_DPD || features[0]->model == DIST_B200_DD || features[0]->model == DIST_B200_BB)) {
-        dist_b200_feature *f = const_cast<dist_b200_feature *>(features[0]);
-        const int R = f->model == DIST_B200_DPD ? f->dim + 1 : (f->model == DIST_B200_DD ? f->dim : 2);
-        int rc = grow(ctx, f->cdf_buf, f->cdf_bytes, sizeof(float) * value_cdf_floats(R, G));
-        if (!rc) rc = launch_value_cdf(ctx, f, f->cdf_buf, columns[0], N, prior, u, assign, s);
-        if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;
-    }
-    // the logp form of the same shortcut: a table feature's log-normaliser is a function of the value alone, so it is one
-    // log-sum-exp per table row and a gather per data row (DIST_B200_OPT_VALUE_CDF = 1 keeps the per-cell kernels here too)
-    if (F == 1 && logp && ctx->opt[DIST_B200_OPT_VALUE_CDF] != 1 &&
-        (features[0]->model == DIST_B200_DPD || features[0]->model == DIST_B200_DD || features[0]->model == DIST_B200_BB)) {
-        dist_b200_feature *f = const_cast<dist_b200_feature *>(features[0]);
-        const int R = f->model == DIST_B200_DPD ? f->dim + 1 : (f->model == DIST_B200_DD ? f->dim : 2);
-        int rc = grow(ctx, f->cdf_buf, f->cdf_bytes, sizeof(float) * R);
-        if (!rc) rc = launch_value_logp(ctx, f, f->cdf_buf, columns[0], N, prior, logp, s);
-        if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;
-    }
-    if (n_solo == 0) {
-        if (F > kMaxFeatures) return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "score: more than 512 features in one call");
-        FeatList fl;
-        fl.n = F;
-        GpTableBatch tb;
-        tb.n = 0;
-        for (int f = 0; f < F; ++f) {
-            int rc = fill_desc(ctx, features[f], columns[f], F > 1, fl.f[f], tb, s);
-            if (rc) return rc;
-        }
-        if (int rc = launch_gp_table_batch(ctx, tb, s)) return rc;
-        return launch_score_rows(ctx, fl, G, N, prior, u, assign, scores, accumulate, s, nullptr, logp);
-    }
-    // one NIW<32> feature, sampling only: quadratic forms, scores and sample_from_scores in one tcgen05 kernel
-    if (F == 1 && features[0]->model == DIST_B200_NIW && features[0]->dim == 32 && features[0]->niw_tc && assign && !scores &&
-        !accumulate && ctx->opt[DIST_B200_OPT_NIW_PATH] == 0)
-        return launch_niw_tc(ctx, G, features[0]->niw_tc, columns[0], N, prior, nullptr, 0, u, assign, s);
-    // one NIW feature with d <= 8, sampling only: the fused FP32 kernel (DIST_B200_OPT_NIW_PATH = 1 keeps the materialising route)
-    if (F == 1 && features[0]->model == DIST_B200_NIW && features[0]->dim <= 8 && assign && !scores && !accumulate &&
-        ctx->opt[DIST_B200_OPT_NIW_PATH] == 0) {
-        const int rc = launch_niw_rows_small(ctx, features[0], columns[0], N, prior, u, assign, s);
-        if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;
-    }
-    // logp over dpd / niw (alone or in a mixed list): the scores are materialised and reduced by logp_scores_kernel
-    if (F == 1 && features[0]->model == DIST_B200_DPD && !logp) {
-        if (assign && !scores && !accumulate && ctx->opt[DIST_B200_OPT_TABLE_KERNEL] != 1) {
-            const int rc = launch_table_rows(ctx, features[0], columns[0], N, prior, u, assign, s);
-            if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;
-        }
-        return launch_gather_rows(ctx, features[0], columns[0], N, prior, u, assign, scores, accumulate, s);
-    }
-    float *buf = scores;
-    if (!buf) {
-        if (int rc = grow(ctx, ctx->scores_scratch, ctx->scores_scratch_bytes, sizeof(float) * N * G)) return rc;
-        buf = static_cast<float *>(ctx->scores_scratch);
-    }
-    FeatList fl;
-    fl.n = 0;
+// The row-mapped part of a feature list (solo features skipped), with each feature's observed mask in `ml` when `ml` is
+// given; stale GammaPoisson value tables are rebuilt on `s`.  multi: see fill_desc.  At most kMaxFeatures row-mapped.
+static int build_list(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int F, const void *const *columns,
+                      const uint32_t *const *observed, bool multi, FeatList &fl, MaskList *ml, cudaStream_t s) {
     GpTableBatch tb;
     tb.n = 0;
+    fl.n = 0;
     for (int f = 0; f < F; ++f) {
         if (solo(features[f])) continue;
-        if (fl.n >= kMaxFeatures) return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "score: more than 512 features in one call");
-        int rc = fill_desc(ctx, features[f], columns[f], true, fl.f[fl.n++], tb, s);
-        if (rc) return rc;
+        if (ml) ml->m[fl.n] = observed[f];
+        if (int rc = fill_desc(ctx, features[f], columns[f], multi, fl.f[fl.n++], tb, s)) return rc;
     }
-    bool started = accumulate != 0;
-    int rc;
-    if ((rc = launch_gp_table_batch(ctx, tb, s))) return rc;
-    if (fl.n) {
-        if ((rc = launch_score_rows(ctx, fl, G, N, prior, nullptr, nullptr, buf, accumulate, s))) return rc;
-        started = true;
-    }
-    for (int f = 0; f < F; ++f) {
-        if (!solo(features[f])) continue;
-        if (features[f]->model == DIST_B200_DPD)
-            rc = launch_gather_rows(ctx, features[f], columns[f], N, started ? nullptr : prior, nullptr, nullptr, buf,
-                                    started ? 1 : 0, s);
-        else
-            rc = launch_niw_scores(ctx, features[f], columns[f], N, started ? nullptr : prior, buf, started ? 1 : 0, s);
-        if (rc) return rc;
-        started = true;
-    }
-    if (assign) return launch_sample_scores(ctx, buf, N, G, u, assign, s);
-    if (logp) return launch_logp_scores(ctx, buf, N, G, logp, s);
-    return DIST_B200_OK;
+    return launch_gp_table_batch(ctx, tb, s);
 }
 
-// ---- missing cells (dist_b200.h: "Missing cells") ----
-static bool any_mask(const uint32_t *const *observed, int F) {
-    for (int f = 0; observed && f < F; ++f)
-        if (observed[f]) return true;
-    return false;
-}
-
-// All-NULL masks take the unmasked dispatch.  Otherwise: every feature row-mapped -> one launch of the masked feature-list
-// kernel; dpd / niw in the list -> the row-mapped features' scores from the masked kernel into [N][G], each masked dpd /
-// niw feature scored alone into a second [N][G] buffer and added where observed (masked_accumulate), fully observed ones
-// accumulated directly as in the unmasked dispatch, then the stand-alone sampler or log-sum-exp.
-static int score_masked(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int F, const void *const *columns,
-                        const uint32_t *const *observed, size_t N, const float *prior, const float *u, int32_t *assign,
-                        float *scores, int accumulate, cudaStream_t s, float *logp = nullptr) {
-    if (!any_mask(observed, F)) return score_dispatch(ctx, features, F, columns, N, prior, u, assign, scores, accumulate, s, logp);
+// Missing cells (dist_b200.h: "Missing cells"): observed[f] is NULL (feature f fully observed) or its mask; observed may
+// be NULL.  A call is masked when any mask is non-NULL.  Then the row-mapped features run the masked feature-list kernel
+// (a list of one too), and each masked dpd / niw feature is scored alone into a second [N][G] buffer and added where
+// observed (masked_accumulate).  The single-feature routes are taken on unmasked calls only.
+// logp != nullptr (assign = scores = nullptr): logp[n] = log sum_g exp(prior[g] + sum_f score_f) per row
+static int score_dispatch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int F, const void *const *columns,
+                          const uint32_t *const *observed, size_t N, const float *prior, const float *u, int32_t *assign,
+                          float *scores, int accumulate, cudaStream_t s, float *logp = nullptr) {
     int G = 0;
     if (int rc = check_score_args(ctx, features, F, columns, prior, u, assign, scores, accumulate, logp, G)) return rc;
     if (N == 0) return DIST_B200_OK;
-    int rc = wait_ready(ctx, features, F, s);
-    if (rc) return rc;
-    int n_solo = 0, n_masked_solo = 0;
+    if (int rc = wait_ready(ctx, features, F, s)) return rc;
+    bool masked = false, masked_solo = false;
+    int n_solo = 0;
     for (int f = 0; f < F; ++f) {
+        const bool m = observed && observed[f];
+        masked = masked || m;
+        masked_solo = masked_solo || (m && solo(features[f]));
         n_solo += solo(features[f]) ? 1 : 0;
-        n_masked_solo += solo(features[f]) && observed[f] ? 1 : 0;
+    }
+    if (!masked && F == 1) {
+        dist_b200_feature *f0 = const_cast<dist_b200_feature *>(features[0]);
+        // ONE table feature (dpd / dd / bb): every row with the same value has the same likelihood vector, so it is evaluated
+        // once per distinct value (table_rows.cu).  SURVEY 8(d) "algorithmic shortcut".  DIST_B200_OPT_VALUE_CDF = 1 keeps
+        // the per-cell kernels (what bench.py reports beside it), 2 = the round-2 tree search instead of the guide-table walk
+        if (ctx->opt[DIST_B200_OPT_VALUE_CDF] != 1 &&
+            (f0->model == DIST_B200_DPD || f0->model == DIST_B200_DD || f0->model == DIST_B200_BB)) {
+            const int R = f0->model == DIST_B200_DPD ? f0->dim + 1 : (f0->model == DIST_B200_DD ? f0->dim : 2);  // table rows
+            // sampling only: per-value CDF trees
+            if (assign && !scores && !accumulate) {
+                int rc = grow(ctx, f0->cdf_buf, f0->cdf_bytes, sizeof(float) * value_cdf_floats(R, G));
+                if (!rc) rc = launch_value_cdf(ctx, f0, f0->cdf_buf, columns[0], N, prior, u, assign, s);
+                if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;
+            }
+            // logp: the log-normaliser is a function of the value alone, one log-sum-exp per table row and a gather per row
+            if (logp) {
+                int rc = grow(ctx, f0->cdf_buf, f0->cdf_bytes, sizeof(float) * R);
+                if (!rc) rc = launch_value_logp(ctx, f0, f0->cdf_buf, columns[0], N, prior, logp, s);
+                if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;
+            }
+        }
+        // one NIW<32> feature, sampling only: quadratic forms, scores and sample_from_scores in one tcgen05 kernel
+        if (f0->model == DIST_B200_NIW && f0->dim == 32 && f0->niw_tc && assign && !scores && !accumulate &&
+            ctx->opt[DIST_B200_OPT_NIW_PATH] == 0)
+            return launch_niw_tc(ctx, G, f0->niw_tc, columns[0], N, prior, nullptr, 0, u, assign, s);
+        // one NIW feature with d <= 8, sampling only: the fused FP32 kernel (DIST_B200_OPT_NIW_PATH = 1 keeps the materialising route)
+        if (f0->model == DIST_B200_NIW && f0->dim <= 8 && assign && !scores && !accumulate && ctx->opt[DIST_B200_OPT_NIW_PATH] == 0) {
+            const int rc = launch_niw_rows_small(ctx, f0, columns[0], N, prior, u, assign, s);
+            if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;
+        }
+        // logp over dpd / niw (alone or in a mixed list): the scores are materialised and reduced by logp_scores_kernel
+        if (f0->model == DIST_B200_DPD && !logp) {
+            if (assign && !scores && !accumulate && ctx->opt[DIST_B200_OPT_TABLE_KERNEL] != 1) {
+                const int rc = launch_table_rows(ctx, f0, columns[0], N, prior, u, assign, s);
+                if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;
+            }
+            return launch_gather_rows(ctx, f0, columns[0], N, prior, u, assign, scores, accumulate, s);
+        }
     }
     if (F - n_solo > kMaxFeatures) return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "score: more than 512 features in one call");
     FeatList fl;
     MaskList ml;
-    fl.n = 0;
-    GpTableBatch tb;
-    tb.n = 0;
-    for (int f = 0; f < F; ++f) {
-        if (solo(features[f])) continue;
-        ml.m[fl.n] = observed[f];
-        if ((rc = fill_desc(ctx, features[f], columns[f], F > 1, fl.f[fl.n++], tb, s))) return rc;
-    }
-    if ((rc = launch_gp_table_batch(ctx, tb, s))) return rc;
-    if (n_solo == 0) return launch_score_rows_masked(ctx, fl, ml, G, N, prior, u, assign, scores, accumulate, logp, s);
+    MaskList *masks = masked ? &ml : nullptr;
+    int rc = build_list(ctx, features, F, columns, observed, F > 1, fl, masks, s);
+    if (rc) return rc;
+    if (n_solo == 0) return launch_score_rows(ctx, fl, G, N, prior, u, assign, scores, accumulate, s, nullptr, logp, masks);
     const size_t cells = N * static_cast<size_t>(G);
     float *buf = scores;
     if (!buf) {
         if ((rc = grow(ctx, ctx->scores_scratch, ctx->scores_scratch_bytes, sizeof(float) * cells))) return rc;
         buf = static_cast<float *>(ctx->scores_scratch);
     }
-    float *tmp = nullptr;
-    if (n_masked_solo) {
+    float *tmp = nullptr;  // a masked dpd / niw feature's scores, before they are added where observed
+    if (masked_solo) {
         if ((rc = grow(ctx, ctx->missing_scratch, ctx->missing_scratch_bytes, sizeof(float) * cells))) return rc;
         tmp = static_cast<float *>(ctx->missing_scratch);
     }
     bool started = accumulate != 0;
     if (fl.n) {
-        if ((rc = launch_score_rows_masked(ctx, fl, ml, G, N, prior, nullptr, nullptr, buf, accumulate, nullptr, s))) return rc;
+        if ((rc = launch_score_rows(ctx, fl, G, N, prior, nullptr, nullptr, buf, accumulate, s, nullptr, nullptr, masks))) return rc;
         started = true;
     }
     for (int f = 0; f < F; ++f) {
         const dist_b200_feature *feat = features[f];
         if (!solo(feat)) continue;
-        const bool m = observed[f] != nullptr;
+        const uint32_t *m = observed ? observed[f] : nullptr;
         float *dst = m ? tmp : buf;
         const float *p = m || started ? nullptr : prior;
         const int acc = !m && started ? 1 : 0;
         if (feat->model == DIST_B200_DPD) rc = launch_gather_rows(ctx, feat, columns[f], N, p, nullptr, nullptr, dst, acc, s);
         else rc = launch_niw_scores(ctx, feat, columns[f], N, p, dst, acc, s);
-        if (!rc && m) rc = launch_masked_accumulate(ctx, buf, tmp, observed[f], N, G, started ? nullptr : prior, started ? 1 : 0, s);
+        if (!rc && m) rc = launch_masked_accumulate(ctx, buf, tmp, m, N, G, started ? nullptr : prior, started ? 1 : 0, s);
         if (rc) return rc;
         started = true;
     }
@@ -1501,8 +1436,8 @@ int dist_b200_score_batch_masked(dist_b200_ctx *ctx, const dist_b200_feature *co
                                  const void *const *columns_dev, size_t n_rows, const float *prior_dev, float *scores_dev,
                                  int accumulate, const uint32_t *const *observed_dev, void *stream) {
     if (!scores_dev) return ctx ? fail(ctx, DIST_B200_ERR_INVALID, "score_batch: scores_dev is null") : DIST_B200_ERR_INVALID;
-    return score_masked(ctx, features, n_features, columns_dev, observed_dev, n_rows, prior_dev, nullptr, nullptr, scores_dev,
-                        accumulate, as_stream(stream));
+    return score_dispatch(ctx, features, n_features, columns_dev, observed_dev, n_rows, prior_dev, nullptr, nullptr, scores_dev,
+                          accumulate, as_stream(stream));
 }
 
 int dist_b200_score_sample_batch_masked(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
@@ -1510,23 +1445,23 @@ int dist_b200_score_sample_batch_masked(dist_b200_ctx *ctx, const dist_b200_feat
                                         const float *u_dev, int32_t *assign_dev, float *scores_dev,
                                         const uint32_t *const *observed_dev, void *stream) {
     if (!assign_dev) return ctx ? fail(ctx, DIST_B200_ERR_INVALID, "score_sample_batch: assign_dev is null") : DIST_B200_ERR_INVALID;
-    return score_masked(ctx, features, n_features, columns_dev, observed_dev, n_rows, prior_dev, u_dev, assign_dev, scores_dev, 0,
-                        as_stream(stream));
+    return score_dispatch(ctx, features, n_features, columns_dev, observed_dev, n_rows, prior_dev, u_dev, assign_dev, scores_dev, 0,
+                          as_stream(stream));
 }
 
 int dist_b200_score_logp_batch_masked(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
                                       const void *const *columns_dev, size_t n_rows, const float *prior_dev, float *logp_dev,
                                       const uint32_t *const *observed_dev, void *stream) {
     if (!logp_dev) return ctx ? fail(ctx, DIST_B200_ERR_INVALID, "score_logp_batch: logp_dev is null") : DIST_B200_ERR_INVALID;
-    return score_masked(ctx, features, n_features, columns_dev, observed_dev, n_rows, prior_dev, nullptr, nullptr, nullptr, 0,
-                        as_stream(stream), logp_dev);
+    return score_dispatch(ctx, features, n_features, columns_dev, observed_dev, n_rows, prior_dev, nullptr, nullptr, nullptr, 0,
+                          as_stream(stream), logp_dev);
 }
 
 int dist_b200_score_batch(dist_b200_ctx *ctx, const dist_b200_feature *const *features, int n_features,
                           const void *const *columns_dev, size_t n_rows, const float *prior_dev, float *scores_dev,
                           int accumulate, void *stream) {
     if (!scores_dev) return ctx ? fail(ctx, DIST_B200_ERR_INVALID, "score_batch: scores_dev is null") : DIST_B200_ERR_INVALID;
-    return score_dispatch(ctx, features, n_features, columns_dev, n_rows, prior_dev, nullptr, nullptr, scores_dev,
+    return score_dispatch(ctx, features, n_features, columns_dev, nullptr, n_rows, prior_dev, nullptr, nullptr, scores_dev,
                           accumulate, as_stream(stream));
 }
 
@@ -1534,7 +1469,7 @@ int dist_b200_score_sample_batch(dist_b200_ctx *ctx, const dist_b200_feature *co
                                  const void *const *columns_dev, size_t n_rows, const float *prior_dev,
                                  const float *u_dev, int32_t *assign_dev, float *scores_dev, void *stream) {
     if (!assign_dev) return ctx ? fail(ctx, DIST_B200_ERR_INVALID, "score_sample_batch: assign_dev is null") : DIST_B200_ERR_INVALID;
-    return score_dispatch(ctx, features, n_features, columns_dev, n_rows, prior_dev, u_dev, assign_dev, scores_dev, 0,
+    return score_dispatch(ctx, features, n_features, columns_dev, nullptr, n_rows, prior_dev, u_dev, assign_dev, scores_dev, 0,
                           as_stream(stream));
 }
 
@@ -1542,7 +1477,7 @@ int dist_b200_score_logp_batch(dist_b200_ctx *ctx, const dist_b200_feature *cons
                                const void *const *columns_dev, size_t n_rows, const float *prior_dev, float *logp_dev,
                                void *stream) {
     if (!logp_dev) return ctx ? fail(ctx, DIST_B200_ERR_INVALID, "score_logp_batch: logp_dev is null") : DIST_B200_ERR_INVALID;
-    return score_dispatch(ctx, features, n_features, columns_dev, n_rows, prior_dev, nullptr, nullptr, nullptr, 0,
+    return score_dispatch(ctx, features, n_features, columns_dev, nullptr, n_rows, prior_dev, nullptr, nullptr, nullptr, 0,
                           as_stream(stream), logp_dev);
 }
 
@@ -1609,18 +1544,14 @@ int dist_b200_score_push_batch(dist_b200_ctx *ctx, const dist_b200_feature *cons
     cudaStream_t s = as_stream(stream);
     int rc = wait_ready(ctx, features, F, s);
     if (rc) return rc;
-    FeatList fl;
-    fl.n = F;
-    GpTableBatch tb;
-    tb.n = 0;
     for (int f = 0; f < F; ++f) {
         if (!features[f] || !columns_dev[f] || features[f]->ctx != ctx || features[f]->G != G)
             return fail(ctx, DIST_B200_ERR_INVALID, "score_push: bad feature list");
-        if (features[f]->model == DIST_B200_DPD || features[f]->model == DIST_B200_NIW)
-            return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "score_push: row-mapped models only");
-        if ((rc = fill_desc(ctx, features[f], columns_dev[f], true, fl.f[f], tb, s))) return rc;
+        if (solo(features[f])) return fail(ctx, DIST_B200_ERR_UNSUPPORTED, "score_push: row-mapped models only");
     }
-    if ((rc = launch_gp_table_batch(ctx, tb, s))) return rc;
+    // multi for a list of one too: a lone GammaPoisson shard is scored through its value table
+    FeatList fl;
+    if ((rc = build_list(ctx, features, F, columns_dev, nullptr, true, fl, nullptr, s))) return rc;
     PushTargets pt{};
     pt.n = n_owners;
     pt.row0 = row0;
@@ -1675,7 +1606,7 @@ static int score_host(dist_b200_ctx *ctx, const dist_b200_feature *const *featur
 
     // per-row output of rows [lo, lo + n) at `out` (device / mapped), u of those rows at `uu`
     auto dispatch = [&](const void *const *cols, size_t n, const float *pr, const float *uu, char *out, float *sc, cudaStream_t str) {
-        return score_dispatch(ctx, features, F, cols, n, pr, uu, logp_host ? nullptr : reinterpret_cast<int32_t *>(out), sc, 0, str,
+        return score_dispatch(ctx, features, F, cols, nullptr, n, pr, uu, logp_host ? nullptr : reinterpret_cast<int32_t *>(out), sc, 0, str,
                               logp_host ? reinterpret_cast<float *>(out) : nullptr);
     };
 
@@ -1833,7 +1764,7 @@ int dist_b200_score_value_host(dist_b200_ctx *ctx, const dist_b200_feature *feat
     if ((rc = wait_ready(ctx, &feature, 1, s))) return rc;
     std::memcpy(pin, value_host, vb);
     const void *col = pin;
-    rc = score_dispatch(ctx, &feature, 1, &col, 1, nullptr, nullptr, nullptr, sc, 0, s);
+    rc = score_dispatch(ctx, &feature, 1, &col, nullptr, 1, nullptr, nullptr, nullptr, sc, 0, s);
     if (rc) return rc;
     DISTB200_CUDA(ctx, cudaStreamSynchronize(s));
     for (int g = 0; g < G; ++g) scores_accum_host[g] += sc[g];  // MixtureSlave::score_value accumulates (mixture.hpp:416-425)

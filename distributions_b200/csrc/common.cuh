@@ -232,15 +232,12 @@ int launch_score_data(dist_b200_ctx *ctx, const dist_b200_feature *f, const uint
 int launch_unpack_caches(dist_b200_ctx *ctx, const dist_b200_feature *f, float *out_dev, cudaStream_t s);
 
 // score_rows.cu: rows mapped to lanes, groups looped (nich / gp / bb / small-dim dd, any F).  logp != nullptr (with
-// assign = scores = nullptr): logp[n] = log sum_g exp(prior[g] + scores of row n)
+// assign = scores = nullptr): logp[n] = log sum_g exp(prior[g] + scores of row n).  masks != nullptr: the list's missing
+// cells (the feature-list kernel with masks, a list of one too; not with push)
 int launch_score_rows(dist_b200_ctx *ctx, const FeatList &feats, int G, size_t N, const float *prior,
                       const float *u, int32_t *assign, float *scores, int accumulate, cudaStream_t s,
-                      const PushTargets *push = nullptr, float *logp = nullptr);
+                      const PushTargets *push = nullptr, float *logp = nullptr, const MaskList *masks = nullptr);
 int launch_gp_table_batch(dist_b200_ctx *ctx, const GpTableBatch &b, cudaStream_t s);
-// score_rows_masked*.cu: the feature-list kernel with missing cells (every feature row-mapped; assign, scores or logp)
-int launch_score_rows_masked(dist_b200_ctx *ctx, const FeatList &feats, const MaskList &masks, int G, size_t N,
-                             const float *prior, const float *u, int32_t *assign, float *scores, int accumulate,
-                             float *logp, cudaStream_t s);
 // missing.cu: out[n] = assign[n] where row n's bit equals `keep` (1: observed cells, 0: missing cells), else -1
 int launch_mask_assign(dist_b200_ctx *ctx, const int32_t *assign, const uint32_t *observed, size_t N, int keep, int32_t *out,
                        cudaStream_t s);

@@ -34,9 +34,15 @@ int launch_gp_table_batch(dist_b200_ctx *ctx, const GpTableBatch &b, cudaStream_
     return DIST_B200_OK;
 }
 
+template <>
+int launch_crosscat_tile<128, false, false>(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s,
+                                            const MaskList *) {
+    return launch_modes<128, -1, 128>(ctx, feats, a, s);
+}
+
 int launch_score_rows(dist_b200_ctx *ctx, const FeatList &feats, int G, size_t N, const float *prior,
                       const float *u, int32_t *assign, float *scores, int accumulate, cudaStream_t s,
-                      const PushTargets *push, float *logp) {
+                      const PushTargets *push, float *logp, const MaskList *masks) {
     if (N == 0 || G == 0) return DIST_B200_OK;
     RowsArgs a{};
     if (push) {
@@ -56,7 +62,7 @@ int launch_score_rows(dist_b200_ctx *ctx, const FeatList &feats, int G, size_t N
     a.t = ctx->tables;
     a.logp = logp;
     if (!assign && !scores && !logp) return fail(ctx, DIST_B200_ERR_INVALID, "score_rows: nothing to produce");
-    if (feats.n == 1) {
+    if (feats.n == 1 && !masks) {  // a masked list of one runs the feature-list kernel
         int rc = DIST_B200_ERR_UNSUPPORTED;
         switch (feats.f[0].kind) {
             case DIST_B200_NICH: rc = launch_single_nich(ctx, feats, a, s); break;
@@ -67,7 +73,7 @@ int launch_score_rows(dist_b200_ctx *ctx, const FeatList &feats, int G, size_t N
         }
         if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;
     }
-    return launch_tiers<-1>(ctx, feats, a, s);
+    return launch_tiers<-1>(ctx, feats, a, s, masks);
 }
 
 }  // namespace distb200

@@ -973,21 +973,31 @@ static int launch_variant(dist_b200_ctx *ctx, const FeatList &feats, RowsArgs a,
     return DIST_B200_OK;
 }
 
-int launch_crosscat_tile32(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s);
-int launch_crosscat_tile64(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s);
-int launch_crosscat_ksub(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s);
+// Feature-list (KIND = -1) launches of one register tile: CHUNK = 32, 64 or 128 groups, kSub = the kSub kernel on
+// 128-group tiles, kMask = with a MaskList.  These instantiations are the heaviest to compile, so every specialisation is
+// defined in one of five translation units: score_rows.cu (128-group tiles), score_rows_cc32.cu (32-group tiles + kSub),
+// score_rows_cc64.cu (64-group tiles), score_rows_masked.cu (masked 128-group tiles + kSub), score_rows_masked_cc.cu
+// (masked 32- and 64-group tiles).
+template <int CHUNK, bool kSub, bool kMask>
+int launch_crosscat_tile(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s, const MaskList *masks);
+// masks: nullptr (the unmasked kernels) or the list's observed masks
+template <int CHUNK, bool kSub = false>
+static int launch_crosscat(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s, const MaskList *masks) {
+    if (masks) return launch_crosscat_tile<CHUNK, kSub, true>(ctx, feats, a, s, masks);
+    return launch_crosscat_tile<CHUNK, kSub, false>(ctx, feats, a, s, nullptr);
+}
 
-template <int CHUNK, int KIND, int THREADS>
-static int launch_modes(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s) {
+template <int CHUNK, int KIND, int THREADS, bool kMask = false>
+static int launch_modes(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s, const MaskList *masks = nullptr) {
     const bool sample = a.assign != nullptr, scores = a.scores != nullptr;
     if (a.logp) {
         // a feature list does not fit a 128-group logp tile in registers: two 64-group tiles instead
-        if constexpr (KIND < 0 && CHUNK == 128) return launch_crosscat_tile64(ctx, feats, a, s);
-        else return launch_variant<CHUNK, KIND, false, false, THREADS>(ctx, feats, a, s);
+        if constexpr (KIND < 0 && CHUNK == 128) return launch_crosscat<64>(ctx, feats, a, s, masks);
+        else return launch_variant<CHUNK, KIND, false, false, THREADS, false, kMask>(ctx, feats, a, s, masks);
     }
-    if (sample && scores) return launch_variant<CHUNK, KIND, true, true, THREADS>(ctx, feats, a, s);
-    if (sample) return launch_variant<CHUNK, KIND, true, false, THREADS>(ctx, feats, a, s);
-    return launch_variant<CHUNK, KIND, false, true, THREADS>(ctx, feats, a, s);
+    if (sample && scores) return launch_variant<CHUNK, KIND, true, true, THREADS, false, kMask>(ctx, feats, a, s, masks);
+    if (sample) return launch_variant<CHUNK, KIND, true, false, THREADS, false, kMask>(ctx, feats, a, s, masks);
+    return launch_variant<CHUNK, KIND, false, true, THREADS, false, kMask>(ctx, feats, a, s, masks);
 }
 
 // kSub launches: heads / tails of every BetaBernoulli feature of the list as two contiguous rows (the float4 caches hold
@@ -1035,28 +1045,27 @@ static int ksub_list(dist_b200_ctx *ctx, const FeatList &feats, int G, FeatList 
 // 64 < G <= 128 of a single feature runs 128-thread blocks, three per SM (12 warps instead of the 8 of one
 // 256-thread block: the row-wide dependent chains of max / total / walk need the extra warps to hide their
 // latency) -- DIST_B200_OPT_SMALL_TILE selects the alternatives for A/B runs.  G > 128: 32-group tiles.
-// the feature-list (KIND = -1) instantiations are the heaviest to compile: they live in three translation units
-// (score_rows.cu: 128-group tiles; score_rows_cc32.cu: 32-group tiles + kSub; score_rows_cc64.cu: 64-group tiles)
+// masks (feature lists only): nullptr, or the observed masks of a list with missing cells, which takes the same tiers
 template <int KIND>
-static int launch_tile32(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s) {
-    if constexpr (KIND < 0) return launch_crosscat_tile32(ctx, feats, a, s);
+static int launch_tile32(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s, const MaskList *masks) {
+    if constexpr (KIND < 0) return launch_crosscat<32>(ctx, feats, a, s, masks);
     else return launch_modes<32, KIND, 256>(ctx, feats, a, s);
 }
 template <int KIND>
-static int launch_tile64(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s) {
-    if constexpr (KIND < 0) return launch_crosscat_tile64(ctx, feats, a, s);
+static int launch_tile64(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s, const MaskList *masks) {
+    if constexpr (KIND < 0) return launch_crosscat<64>(ctx, feats, a, s, masks);
     else return launch_modes<64, KIND, 256>(ctx, feats, a, s);
 }
 
 template <int KIND>
-static int launch_tiers(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s) {
-    if (a.G <= 32) return launch_tile32<KIND>(ctx, feats, a, s);
-    if (a.G <= 64) return launch_tile64<KIND>(ctx, feats, a, s);
+static int launch_tiers(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s, const MaskList *masks = nullptr) {
+    if (a.G <= 32) return launch_tile32<KIND>(ctx, feats, a, s, masks);
+    if (a.G <= 64) return launch_tile64<KIND>(ctx, feats, a, s, masks);
     if (a.G <= 128) {
-        if (KIND < 0) return launch_modes<128, KIND, 128>(ctx, feats, a, s);
+        if (KIND < 0) return launch_crosscat<128>(ctx, feats, a, s, masks);
         const int v = ctx->opt[DIST_B200_OPT_SMALL_TILE];
         if (v == 1) return launch_modes<128, KIND, 256>(ctx, feats, a, s);
-        if (v == 3) return launch_tile32<KIND>(ctx, feats, a, s);
+        if (v == 3) return launch_tile32<KIND>(ctx, feats, a, s, masks);
         if (v != 2 && a.assign && !a.scores) {
             // sampling only: the register tile is G rounded up to 16 groups (G = 100 pads to 112 instead of 128:
             // every padded group is a wasted MUFU.EX2)
@@ -1076,13 +1085,13 @@ static int launch_tiers(dist_b200_ctx *ctx, const FeatList &feats, const RowsArg
         if (ksub_wanted(feats, a.G)) {
             FeatList local;
             if (int rc = ksub_list(ctx, feats, a.G, local, s)) return rc;
-            const int rc = launch_crosscat_ksub(ctx, local, a, s);
+            const int rc = launch_crosscat<128, true>(ctx, local, a, s, masks);
             if (rc != DIST_B200_ERR_UNSUPPORTED) return rc;  // (too many groups for the sub-slot sums in shared memory)
         }
     }
     const int tile = ctx->opt[DIST_B200_OPT_ROW_TILE] ? ctx->opt[DIST_B200_OPT_ROW_TILE] : (a.scores ? 64 : 32);
-    if (tile == 64) return launch_tile64<KIND>(ctx, feats, a, s);
-    return launch_tile32<KIND>(ctx, feats, a, s);
+    if (tile == 64) return launch_tile64<KIND>(ctx, feats, a, s, masks);
+    return launch_tile32<KIND>(ctx, feats, a, s, masks);
 }
 
 // one per model, each in its own translation unit (parallel compilation)

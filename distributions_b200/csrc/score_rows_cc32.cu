@@ -4,11 +4,15 @@
 
 namespace distb200 {
 
-int launch_crosscat_tile32(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s) {
+template <>
+int launch_crosscat_tile<32, false, false>(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s,
+                                           const MaskList *) {
     return launch_modes<32, -1, 256>(ctx, feats, a, s);
 }
 
-int launch_crosscat_ksub(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s) {
+template <>
+int launch_crosscat_tile<128, true, false>(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s,
+                                           const MaskList *) {
     return launch_variant<128, -1, true, false, 128, true>(ctx, feats, a, s);
 }
 

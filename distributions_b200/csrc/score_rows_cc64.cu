@@ -4,7 +4,9 @@
 
 namespace distb200 {
 
-int launch_crosscat_tile64(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s) {
+template <>
+int launch_crosscat_tile<64, false, false>(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s,
+                                           const MaskList *) {
     return launch_modes<64, -1, 256>(ctx, feats, a, s);
 }
 

@@ -3,20 +3,16 @@
 
 namespace distb200 {
 
-template <int CHUNK>
-static int masked_modes(dist_b200_ctx *ctx, const FeatList &feats, const MaskList &masks, const RowsArgs &a, cudaStream_t s) {
-    if (a.logp) return launch_variant<CHUNK, -1, false, false, 256, false, true>(ctx, feats, a, s, &masks);
-    if (a.assign && a.scores) return launch_variant<CHUNK, -1, true, true, 256, false, true>(ctx, feats, a, s, &masks);
-    if (a.assign) return launch_variant<CHUNK, -1, true, false, 256, false, true>(ctx, feats, a, s, &masks);
-    return launch_variant<CHUNK, -1, false, true, 256, false, true>(ctx, feats, a, s, &masks);
+template <>
+int launch_crosscat_tile<32, false, true>(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s,
+                                          const MaskList *masks) {
+    return launch_modes<32, -1, 256, true>(ctx, feats, a, s, masks);
 }
 
-int launch_masked_tile32(dist_b200_ctx *ctx, const FeatList &feats, const MaskList &masks, const RowsArgs &a, cudaStream_t s) {
-    return masked_modes<32>(ctx, feats, masks, a, s);
-}
-
-int launch_masked_tile64(dist_b200_ctx *ctx, const FeatList &feats, const MaskList &masks, const RowsArgs &a, cudaStream_t s) {
-    return masked_modes<64>(ctx, feats, masks, a, s);
+template <>
+int launch_crosscat_tile<64, false, true>(dist_b200_ctx *ctx, const FeatList &feats, const RowsArgs &a, cudaStream_t s,
+                                          const MaskList *masks) {
+    return launch_modes<64, -1, 256, true>(ctx, feats, a, s, masks);
 }
 
 }  // namespace distb200
