@@ -43,6 +43,7 @@ SOURCES = {
     "niw_stats.cu": [],
     "microbench.cu": [],
     "stats.cu": [],
+    "regroup.cu": [],
     "wire.cu": [],
     "sample_values.cu": ["--fmad=false"],
 }

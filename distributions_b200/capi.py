@@ -41,6 +41,7 @@ SIGNATURES = {
     "dist_b200_feature_update_group": (c_i, [c_p, c_i, c_p, c_p]),
     "dist_b200_feature_add_group": (c_i, [c_p, c_p]),
     "dist_b200_feature_remove_group": (c_i, [c_p, c_i, c_p]),
+    "dist_b200_regroup_batch": (c_i, [c_p, c_p, c_i, c_p, c_i, c_i, c_p, c_sz, c_p, c_p, ctypes.POINTER(c_i), c_p]),
     "dist_b200_feature_add_rows": (c_i, [c_p, c_p, c_p, c_sz, c_p]),
     "dist_b200_add_rows_batch": (c_i, [c_p, c_p, c_i, c_p, c_p, c_sz, c_p]),
     "dist_b200_add_rows_batch_host": (c_i, [c_p, c_p, c_i, c_p, c_p, c_sz]),
@@ -375,6 +376,20 @@ class Context:
         self.check(self.L.dist_b200_sample_values_batch_host(self.h, fa, F, _np_ptr(assign), n, int(seed), int(row0), ca),
                    "sample_values_batch_host")
         return out
+
+    def regroup_batch(self, features, counts_dev, G, n_empty, assign_dev=None, n_rows=0, counts_out=None, remap_out=None,
+                      stream=None):
+        """group births and deaths in one batch: drop the groups of size 0 (counts_dev[G] on the device), append n_empty
+        fresh empty groups, relabel assign_dev in place and compact every feature's statistics the same way.  Survivors
+        keep their order.  counts_out (G + n_empty int32) receives the new sizes, remap_out (G int32) old -> new id or -1.
+        Returns the new G.  Reads the new G back to the host once (one drain of `stream`)."""
+        F = len(features)
+        fa = (c_p * max(F, 1))(*[f.h for f in features])
+        g_out = c_i(0)
+        self.check(self.L.dist_b200_regroup_batch(self.h, fa, F, _dev_ptr(counts_dev), int(G), int(n_empty), _dev_ptr(assign_dev),
+                                                  int(n_rows), _dev_ptr(counts_out), _dev_ptr(remap_out), ctypes.byref(g_out), stream),
+                   "regroup_batch")
+        return g_out.value
 
     def count_assignments(self, assign_dev, n_rows, G, counts_dev, accumulate=False, stream=None):
         self.check(self.L.dist_b200_count_assignments(self.h, _dev_ptr(assign_dev), n_rows, G, _dev_ptr(counts_dev),

@@ -306,6 +306,9 @@ void dist_b200_ctx_destroy(dist_b200_ctx *ctx) {
     if (ctx->scratch_dev) cudaFree(ctx->scratch_dev);
     if (ctx->add_acc) cudaFree(ctx->add_acc);
     if (ctx->add_done) cudaEventDestroy(ctx->add_done);
+    if (ctx->regroup_buf) cudaFree(ctx->regroup_buf);
+    if (ctx->regroup_k_host) cudaFreeHost(ctx->regroup_k_host);
+    if (ctx->regroup_done) cudaEventDestroy(ctx->regroup_done);
     if (ctx->scores_scratch) cudaFree(ctx->scores_scratch);
     if (ctx->missing_scratch) cudaFree(ctx->missing_scratch);
     if (ctx->xpack) cudaFree(ctx->xpack);
@@ -546,6 +549,117 @@ int dist_b200_feature_remove_group(dist_b200_feature *f, int groupid, void *stre
     f->gp_table_dirty = true;
     f->log_prod_valid = false;
     return mark_ready(f, rc, s);
+}
+
+static bool pooled_model(int model);
+
+// the per-group device arrays regroup_batch moves with their group: the statistics, and the caches a gather keeps
+// (pooled and dd params, nich aux, a valid gp log_prod, niw records).  dpd's table is rebuilt instead.
+static void regroup_arrays(dist_b200_feature *f, bool log_prod, std::vector<RegroupArray> &out) {
+    for (int a = 0; a < stat_arrays(f); ++a) out.push_back({f->stats[a], f->stats[a], stat_elems(f, a)});
+    uint32_t *params = static_cast<uint32_t *>(f->params);
+    if (pooled_model(f->model) || f->model == DIST_B200_DD) out.push_back({params, params, group_floats(f)});
+    if (f->model == DIST_B200_NICH) out.push_back({reinterpret_cast<uint32_t *>(f->aux), reinterpret_cast<uint32_t *>(f->aux), 1});
+    if (log_prod) out.push_back({reinterpret_cast<uint32_t *>(f->log_prod_dev), reinterpret_cast<uint32_t *>(f->log_prod_dev), 1});
+    if (f->model == DIST_B200_NIW) {
+        uint32_t *recs = reinterpret_cast<uint32_t *>(f->niw_buf);
+        out.push_back({recs, recs, niw_rec_floats(f->dim)});
+    }
+}
+
+// one launch per kRegroupBatch arrays
+static int regroup_launch(dist_b200_ctx *ctx, const std::vector<RegroupArray> &arrays, int rows, const int32_t *inv,
+                          const int32_t *k, cudaStream_t s) {
+    RegroupBatch b;
+    b.rows = rows;
+    b.inv = inv;
+    b.k = k;
+    for (size_t i0 = 0; i0 < arrays.size(); i0 += kRegroupBatch) {
+        b.n = static_cast<int>(std::min<size_t>(kRegroupBatch, arrays.size() - i0));
+        for (int i = 0; i < b.n; ++i) b.a[i] = arrays[i0 + i];
+        if (int rc = launch_regroup_arrays(ctx, b, s)) return rc;
+    }
+    return DIST_B200_OK;
+}
+
+int dist_b200_regroup_batch(dist_b200_ctx *ctx, dist_b200_feature *const *features, int n_features, const int32_t *counts_dev,
+                            int G, int n_empty, int32_t *assign_dev, size_t n_rows, int32_t *counts_out_dev,
+                            int32_t *remap_out_dev, int *G_out, void *stream) {
+    if (!ctx) return DIST_B200_ERR_INVALID;
+    if (!G_out || G < 0 || n_features < 0 || (n_features && !features) || (G && !counts_dev) || (n_rows && !assign_dev))
+        return fail(ctx, DIST_B200_ERR_INVALID, "regroup_batch: null or negative argument");
+    if (n_empty < 1 || n_empty > INT32_MAX - G)
+        return fail(ctx, DIST_B200_ERR_INVALID, "regroup_batch: need n_empty >= 1 (a mixture always keeps an empty group)");
+    for (int i = 0; i < n_features; ++i) {
+        const dist_b200_feature *f = features[i];
+        if (!f || f->ctx != ctx) return fail(ctx, DIST_B200_ERR_INVALID, "regroup_batch: null feature or one of another context");
+        if (!stats_resident(f)) return fail(ctx, DIST_B200_ERR_STATE, "regroup_batch: call update_all first");
+        if (f->G != G) return fail(ctx, DIST_B200_ERR_STATE, "regroup_batch: a feature's G differs from the G given");
+    }
+    cudaStream_t s = as_stream(stream);
+    const int rows = G + n_empty;  // K+ <= G: an upper bound of the new G, so the gather needs no readback
+
+    // the source arrays and the layout of the context buffer: remap | inv | K+ | one gathered copy per array
+    std::vector<RegroupArray> src;
+    std::vector<bool> log_prod(n_features);
+    for (int i = 0; i < n_features; ++i) {
+        log_prod[i] = features[i]->model == DIST_B200_GP && features[i]->log_prod_valid;
+        regroup_arrays(features[i], log_prod[i], src);
+    }
+    size_t bytes = 0;
+    auto region = [&](size_t n) { const size_t off = bytes; bytes += round_up(n, 256); return off; };
+    const size_t remap_off = region(sizeof(int32_t) * G), inv_off = region(sizeof(int32_t) * rows), k_off = region(sizeof(int32_t));
+    std::vector<size_t> arr_off(src.size());
+    for (size_t i = 0; i < src.size(); ++i) arr_off[i] = region(4 * src[i].words * rows);
+    int rc;
+    if (bytes > ctx->regroup_bytes && (rc = grow(ctx, ctx->regroup_buf, ctx->regroup_bytes, bytes + bytes / 4))) return rc;
+    if (!ctx->regroup_k_host) DISTB200_CUDA(ctx, cudaMallocHost(&ctx->regroup_k_host, sizeof(int32_t)));
+    if (!ctx->regroup_done) DISTB200_CUDA(ctx, cudaEventCreateWithFlags(&ctx->regroup_done, cudaEventDisableTiming));
+    char *buf = static_cast<char *>(ctx->regroup_buf);
+    int32_t *remap = remap_out_dev ? remap_out_dev : reinterpret_cast<int32_t *>(buf + remap_off);
+    int32_t *inv = reinterpret_cast<int32_t *>(buf + inv_off), *k_dev = reinterpret_cast<int32_t *>(buf + k_off);
+
+    // phase 1, before K+ is known: the remap, the relabel and every gather into the context buffer.  The buffer is
+    // ordered behind the last regroup's copy-back by the context's regroup_done event.
+    DISTB200_CUDA(ctx, cudaStreamWaitEvent(s, ctx->regroup_done, 0));
+    if ((rc = wait_ready(ctx, features, n_features, s)) ||
+        (rc = launch_regroup_remap(ctx, counts_dev, G, n_empty, remap, inv, counts_out_dev, k_dev, s)) ||
+        (rc = launch_regroup_relabel(ctx, assign_dev, n_rows, remap, G, s)))
+        return rc;
+    std::vector<RegroupArray> gather(src);
+    for (size_t i = 0; i < src.size(); ++i) gather[i].dst = reinterpret_cast<uint32_t *>(buf + arr_off[i]);
+    if ((rc = regroup_launch(ctx, gather, rows, inv, k_dev, s))) return rc;
+    // the one host round trip: the new G sets grid sizes and f->G
+    DISTB200_CUDA(ctx, cudaMemcpyAsync(ctx->regroup_k_host, k_dev, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    DISTB200_CUDA(ctx, cudaStreamSynchronize(s));
+    const int K = *ctx->regroup_k_host, G_new = K + n_empty;
+
+    // phase 2: capacity for G_new (the old contents are in the context buffer, so nothing is kept), then the copy back
+    // of rows [0, max(G, G_new)): survivors, zeroed fresh groups, and zeros over the dropped tail
+    for (int i = 0; i < n_features; ++i) {
+        dist_b200_feature *f = features[i];
+        if ((rc = reserve_stats(f, G_new, false)) || (rc = ensure_params(f, G_new, false)) ||
+            (log_prod[i] && (rc = grow(ctx, f->log_prod_dev, f->log_prod_bytes, sizeof(float) * f->capacity))))
+            return rc;
+    }
+    std::vector<RegroupArray> back;
+    for (int i = 0; i < n_features; ++i) regroup_arrays(features[i], log_prod[i], back);
+    for (size_t i = 0; i < back.size(); ++i) back[i].src = reinterpret_cast<const uint32_t *>(buf + arr_off[i]);
+    if ((rc = regroup_launch(ctx, back, std::max(G, G_new), nullptr, nullptr, s))) return rc;
+
+    // caches of the fresh groups (dpd: the whole table at the new stride; niw: also the tensor-core images, once)
+    for (int i = 0; i < n_features; ++i) {
+        dist_b200_feature *f = features[i];
+        f->G = G_new;
+        rc = f->model == DIST_B200_DPD ? rebuild(f, 0, G_new, s) : rebuild(f, K, n_empty, s);
+        if (rc) return rc;
+        f->gp_table_dirty = true;
+        f->log_prod_valid = log_prod[i];
+        DISTB200_CUDA(ctx, cudaEventRecord(f->ready, s));
+    }
+    DISTB200_CUDA(ctx, cudaEventRecord(ctx->regroup_done, s));
+    *G_out = G_new;
+    return DIST_B200_OK;
 }
 
 // batched Group::add_value over many features of one kind.  Everything is enqueued on `stream`: the

@@ -84,6 +84,21 @@ struct AddMasks {
     const uint32_t *m[kAddBatch];
 };
 
+// dist_b200_regroup_batch: per-group arrays (statistics and caches) of many features moved in one launch, `words`
+// 4-byte words per group, descriptors in kernel-parameter space
+constexpr int kRegroupBatch = 128;
+struct RegroupArray {
+    const uint32_t *src;
+    uint32_t *dst;
+    size_t words;
+};
+struct RegroupBatch {
+    int n, rows;           // arrays in this launch; groups written per array
+    const int32_t *inv;    // gather: new id -> old id (NULL: copy row r to row r)
+    const int32_t *k;      // gather: device K+ (rows from K+ on are zero-filled)
+    RegroupArray a[kRegroupBatch];
+};
+
 }  // namespace distb200
 
 struct dist_b200_ctx {
@@ -110,6 +125,10 @@ struct dist_b200_ctx {
     void *add_acc = nullptr;          // batched add_value: per-feature accumulators (stats.cu)
     size_t add_acc_bytes = 0;
     cudaEvent_t add_done = nullptr;   // recorded after the last merge that read add_acc
+    void *regroup_buf = nullptr;      // regroup_batch: remap | inv | K+ | the gathered per-group arrays
+    size_t regroup_bytes = 0;
+    int32_t *regroup_k_host = nullptr;  // page-locked K+ read back by regroup_batch
+    cudaEvent_t regroup_done = nullptr; // recorded after the last copy-back that read regroup_buf
     int opt[DIST_B200_OPT_COUNT_] = {0};  // dist_b200_ctx_set_option: A/B knobs of bench.py / the profiling scripts
 };
 
@@ -257,6 +276,12 @@ int launch_merge_counts(dist_b200_ctx *ctx, int32_t *counts, const double *delta
 size_t add_rows_acc_bytes(int G);
 int launch_count_assignments(dist_b200_ctx *ctx, const int32_t *assign, size_t N, int G, int32_t *counts, int accumulate,
                              cudaStream_t s, const uint32_t *observed = nullptr);
+// regroup.cu: remap[G] / inv[G + n_empty] / counts_out / K+ from the group sizes (one block), the relabel of the
+// assignments, and the gather / copy of per-group arrays
+int launch_regroup_remap(dist_b200_ctx *ctx, const int32_t *counts, int G, int n_empty, int32_t *remap, int32_t *inv,
+                         int32_t *counts_out, int32_t *k_out, cudaStream_t s);
+int launch_regroup_relabel(dist_b200_ctx *ctx, int32_t *assign, size_t N, const int32_t *remap, int G, cudaStream_t s);
+int launch_regroup_arrays(dist_b200_ctx *ctx, const RegroupBatch &b, cudaStream_t s);
 // gather_rows.cu: one warp per row, groups mapped to lanes (value-major tables: dpd, wide dd) and the
 // stand-alone sampler over materialised scores
 int launch_gather_rows(dist_b200_ctx *ctx, const dist_b200_feature *f, const void *column, size_t N,

@@ -97,6 +97,23 @@ class _Mixture:
         self.groups.pop()
         self.feature.remove_group(groupid)
 
+    # after dist_b200_regroup_batch moved this feature's groups: survivors in order, then n_empty fresh groups
+    def regroup(self, shared, remap, n_empty):
+        """follow a regroup of self.feature (capi.Context.regroup_batch): remap[g] = new id of old group g or -1; the
+        host Groups are reordered the same way, fresh ones appended, and all of them re-read from the device"""
+        remap = np.asarray(remap).ravel()
+        assert remap.size == len(self.groups), "remap must have one entry per group"
+        keep = [self.groups[g] for g in np.flatnonzero(remap >= 0)]
+        assert all(remap[g] == i for i, g in enumerate(np.flatnonzero(remap >= 0))), "remap is not the stable compaction"
+        fresh = []
+        for _ in range(n_empty):
+            grp = self.Group()
+            grp.init(shared)
+            fresh.append(grp)
+        self.groups = keep + fresh
+        assert self.feature.groups == len(self.groups), "the device feature was not regrouped to this G"
+        self._pull_groups(shared)
+
     # mixture.hpp:377-398
     def add_value(self, shared, groupid, value):
         self.groups[groupid].add_value(shared, value)
@@ -535,6 +552,19 @@ class MixtureIdTracker:
             self.packed_to_global_[packed] = last
             self.global_to_packed_[last] = packed
 
+    def regroup(self, remap, n_empty):
+        """follow dist_b200_regroup_batch: remap[p] = new packed id of packed group p, or -1 (dropped: its global id is
+        retired); survivors keep their global ids, and n_empty fresh groups get new global ids at the end"""
+        remap = np.asarray(remap).ravel()
+        assert remap.size == self.packed_size(), "remap must have one entry per packed group"
+        survivors = [self.packed_to_global_[p] for p in np.flatnonzero(remap >= 0)]
+        for p in np.flatnonzero(remap < 0):
+            del self.global_to_packed_[self.packed_to_global_[p]]
+        self.packed_to_global_ = survivors
+        self.global_to_packed_ = {glob: packed for packed, glob in enumerate(survivors)}
+        for _ in range(n_empty):
+            self.add_group()
+
     def packed_to_global(self, packed):
         assert packed < self.packed_size(), "bad packed id: %d" % packed
         return self.packed_to_global_[packed]
@@ -614,6 +644,22 @@ class _ClusteringMixture:
                     self.empty_groupids.add(groupid)
             self.counts.pop()
         return remove_group
+
+    def regroup(self, n_empty=1, counts=None):
+        """the batched form of the bookkeeping above (dist_b200_regroup_batch): groups of size 0 are dropped, the live
+        ones keep their order, and n_empty fresh empty groups follow.  counts (optional) replaces the group sizes first,
+        e.g. the device's count_assignments.  Returns remap[g] = new id of old group g, -1 when dropped."""
+        assert n_empty >= 1, "a mixture keeps at least one empty group"  # mixture.hpp:150
+        if counts is not None:
+            self.counts = [int(c) for c in counts]
+        c = np.asarray(self.counts, dtype=np.int64)
+        live = c > 0
+        remap = np.where(live, np.cumsum(live) - 1, -1).astype(np.int32)
+        K = int(live.sum())
+        self.counts = [int(v) for v in c[live]] + [0] * n_empty
+        self.empty_groupids = set(range(K, K + n_empty))
+        self.sample_size = int(c[live].sum())
+        return remap
 
     def score_value(self, model, scores):
         assert len(scores) == len(self.counts) and scores.dtype == np.float32

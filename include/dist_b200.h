@@ -154,6 +154,48 @@ int dist_b200_feature_update_group(dist_b200_feature *f, int groupid, const void
 int dist_b200_feature_add_group(dist_b200_feature *f, void *stream);
 int dist_b200_feature_remove_group(dist_b200_feature *f, int groupid, void *stream);
 
+/* ---- group births and deaths in one batch: the step that makes a blocked Gibbs pass a DP / Pitman-Yor mixture ------
+ * The batched form of the per-value bookkeeping of MixtureDriver::add_value / remove_value (mixture.hpp:77-122: a value
+ * landing in an empty group appends a fresh one, a group emptied by remove_value is packed_remove'd) and of
+ * packed_add / packed_remove (vector.hpp:39-61), for one clustering and every feature of its kind at once.
+ *   - counts_dev[G]: the group sizes (the clustering's counts, e.g. from dist_b200_count_assignments).  A group is ALIVE
+ *     iff counts_dev[g] > 0.  Feature statistics never decide liveness (with missing cells, a live group may hold no
+ *     observed cell of some feature).
+ *   - Order (canonical and stable): the live groups keep their relative order and become 0 .. K+ - 1; exactly n_empty
+ *     fresh empty groups follow, K+ .. K+ + n_empty - 1; *G_out = K+ + n_empty.  A group of size 0 is dropped even when
+ *     it already was an empty group, and a fresh one replaces it.  This is NOT the order a sequence of swap-with-last
+ *     dist_b200_feature_remove_group calls gives: callers with per-group data of their own follow remap_out_dev.
+ *   - remap_out_dev[G] (nullable): the new id of every old group, -1 for a dropped one.
+ *   - counts_out_dev (nullable, capacity >= G + n_empty): the compacted counts, zeros for the fresh groups: the group
+ *     sizes dist_b200_prior_pitman_yor_dev / dist_b200_prior_low_entropy_dev take at the new G.
+ *   - assign_dev[n_rows] (nullable when n_rows == 0) is relabelled in place: negative ids stay, an id >= 0 becomes its
+ *     group's new id.  An id >= G, or one whose group was dropped, becomes -1; that happens only when counts_dev
+ *     disagrees with the assignments.
+ *   - Every feature of the list (n_features == 0 does the clustering part only): its statistics are compacted the same
+ *     way, each fresh group is Group::init (every statistics word zero) and its G becomes the new G.  Afterwards
+ *     download_stats / download_caches / score / sample / logp / sample_values are bit-identical to those of a feature
+ *     loaded by update_all from the compacted statistics.  gp: a Group::log_prod that was valid moves with its group
+ *     (0 for a fresh group) and stays valid; an invalid one stays invalid.  Hot-cache slots past the new G hold zeros,
+ *     as after dist_b200_feature_remove_group.
+ *   - Checked, with no state changed: every feature has resident statistics (ERR_STATE before its first update_all) and
+ *     G == the feature's G (ERR_STATE); n_empty >= 1, the reference's invariant (mixture.hpp:150-153), and no null
+ *     argument where one is required (ERR_INVALID).
+ *   - Synchronisation: the new G must reach the host (grid sizes and the features' G live there), so the call reads
+ *     K+ back once through page-locked memory, which drains `stream` once.  That is its only synchronisation (plus the
+ *     device-wide one of a buffer that has to grow past its capacity).  Everything else is enqueued on `stream`, and the
+ *     features' ready events are recorded as the other update entries do.
+ * Launches: one remap block, one relabel pass, and per 128 per-group arrays one gather and one copy-back launch
+ * (statistics and gathered caches, out of place through a context buffer), then the caches of the fresh groups: the
+ * model's prep on the n_empty fresh groups only, per feature (dpd: its table rebuilt once at the new stride; niw: the
+ * fresh records and the tensor-core images once; gp: the value table is marked stale).  The count does not depend on
+ * how many groups die or are born.
+ * Row shards (replicated statistics): all-reduce the counts over the ranks, then every rank calls this with the GLOBAL
+ * counts on its replica and its own rows; every replica computes the same remap and stays bit-identical. */
+int dist_b200_regroup_batch(dist_b200_ctx *ctx, dist_b200_feature *const *features, int n_features,
+                            const int32_t *counts_dev, int G, int n_empty,
+                            int32_t *assign_dev, size_t n_rows,
+                            int32_t *counts_out_dev, int32_t *remap_out_dev, int *G_out, void *stream);
+
 /* ---- batched Group::add_value on the device (next row of the path: score -> sample -> UPDATE) -----
  * Folds n_rows values into the groups given by assign_dev[n] (packed ids; negative = skip) with one
  * segmented reduction, merges into the device-resident statistics (the arrays last given to update_all /

@@ -472,6 +472,19 @@ struct MixtureIdTracker {
     }
     size_t packed_size() const { return packed_to_global_.size(); }
     size_t global_size() const { return global_size_; }
+    // NEW: follow dist_b200_regroup_batch.  remap[p] = new packed id of packed group p or -1 (dropped: its global id is
+    // retired); survivors keep their global ids and their order, and n_empty fresh groups get new global ids at the end.
+    void regroup(const std::vector<int32_t> & remap, size_t n_empty) {
+        if (remap.size() != packed_size()) throw std::runtime_error("regroup: remap size != packed size");
+        std::vector<Id> survivors;
+        for (size_t p = 0; p < remap.size(); ++p) {
+            if (remap[p] >= 0) survivors.push_back(packed_to_global_[p]);
+            else global_to_packed_.erase(packed_to_global_[p]);
+        }
+        packed_to_global_ = survivors;
+        for (size_t p = 0; p < survivors.size(); ++p) global_to_packed_[survivors[p]] = static_cast<Id>(p);
+        for (size_t i = 0; i < n_empty; ++i) add_group();
+    }
 
   private:
     std::vector<Id> packed_to_global_;
@@ -501,6 +514,7 @@ class Mixture {
     Group & groups(size_t i) { return groups_[i]; }
     const Group & groups(size_t i) const { return groups_[i]; }
     const dist_b200_feature * feature() const { return f_; }
+    dist_b200_feature * feature() { return f_; }  // for dist_b200_regroup_batch over the features of a kind
 
     // mixture.hpp:354-359: value_scorer_.resize + update_all
     void init(const Shared & shared, rng_t &) {
@@ -577,6 +591,28 @@ class Mixture {
         Model::load_groups(raw.data(), shared, groups_);
     }
 
+    // NEW: follow dist_b200_regroup_batch on feature() (remap[g] = new id of old group g, or -1): the host Groups are
+    // reordered the same way, n_empty fresh Groups (Group::init) appended, and all of them re-read from the device, as
+    // add_values does.
+    void regroup(const Shared & shared, const std::vector<int32_t> & remap, size_t n_empty, rng_t & rng) {
+        if (remap.size() != groups_.size()) throw std::runtime_error("regroup: remap size != group count");
+        std::vector<Group> kept;
+        for (size_t g = 0; g < remap.size(); ++g)
+            if (remap[g] >= 0) kept.push_back(std::move(groups_[g]));
+        for (size_t i = 0; i < n_empty; ++i) {
+            kept.emplace_back();
+            kept.back().init(shared, rng);
+        }
+        groups_ = std::move(kept);
+        if (static_cast<size_t>(dist_b200_feature_groups(f_)) != groups_.size())
+            throw std::runtime_error("regroup: the device feature holds another group count");
+        std::vector<unsigned char> raw(Model::stats_bytes(shared, groups_.size()));
+        size_t got = 0;
+        ctx_->check(dist_b200_feature_download_stats(f_, raw.data(), raw.size(), &got, nullptr), "download_stats");
+        if (got != raw.size()) throw std::runtime_error("regroup: statistics size mismatch");
+        Model::load_groups(raw.data(), shared, groups_);
+    }
+
     // NEW: batched score (+ sample).  values[n] are rows of this feature, prior[G] the clustering
     // prior vector (or null), u[n] uniforms in [0,1); assign[n] receives the sampled packed group ids,
     // scores (optional) the [n][G] log scores.  Host buffers.
@@ -616,6 +652,24 @@ class Mixture {
     dist_b200_feature * f_ = nullptr;
     std::vector<Group> groups_;
 };
+
+// ---------------------------------------------------------------------------------------------
+namespace detail {
+// the batched driver bookkeeping of dist_b200_regroup_batch on host counts: groups of size 0 are dropped, the live
+// ones keep their order and n_empty empty groups follow.  Returns remap[g] = new id of old group g, or -1.
+inline std::vector<int32_t> regroup_counts(std::vector<int32_t> & counts, size_t n_empty) {
+    if (n_empty < 1) throw std::runtime_error("regroup: a mixture keeps at least one empty group");  // mixture.hpp:150
+    std::vector<int32_t> remap(counts.size(), -1), kept;
+    for (size_t g = 0; g < counts.size(); ++g)
+        if (counts[g] > 0) {
+            remap[g] = static_cast<int32_t>(kept.size());
+            kept.push_back(counts[g]);
+        }
+    kept.resize(kept.size() + n_empty, 0);
+    counts = std::move(kept);
+    return remap;
+}
+}  // namespace detail
 
 // ---------------------------------------------------------------------------------------------
 // Clustering<int>::PitmanYor and its Mixture (CachedMixture over MixtureDriver)
@@ -671,6 +725,18 @@ struct PitmanYor {
             }
             return remove_group;
         }
+        // NEW: the batched form of add_value / remove_value's group bookkeeping (dist_b200_regroup_batch on host counts;
+        // counts() may first be overwritten with the device's group sizes).  Returns the remap the features follow.
+        std::vector<int32_t> regroup(const PitmanYor &, size_t n_empty) {
+            std::vector<int32_t> remap = detail::regroup_counts(counts_, n_empty);
+            empty_groupids_.clear();
+            sample_size_ = 0;
+            for (size_t i = 0; i < counts_.size(); ++i) {
+                sample_size_ += counts_[i];
+                if (counts_[i] == 0) empty_groupids_.insert(i);
+            }
+            return remap;
+        }
         // clustering.hpp:195-208: OVERWRITES scores with the prior vector
         void score_value(const PitmanYor & model, Floats scores) const {
             if (scores.size() != counts_.size()) throw std::runtime_error("score_value: size mismatch");
@@ -715,6 +781,8 @@ struct LowEntropy {
             }
             return remove_group;
         }
+        // NEW: as PitmanYor::Mixture::regroup
+        std::vector<int32_t> regroup(const LowEntropy &, size_t n_empty) { return detail::regroup_counts(counts_, n_empty); }
         // mixture.hpp:123-141: OVERWRITES scores with score_add_value of every group
         void score_value(const LowEntropy & model, Floats scores) const {
             if (scores.size() != counts_.size()) throw std::runtime_error("score_value: size mismatch");
