@@ -1062,18 +1062,24 @@ static int launch_tiers(dist_b200_ctx *ctx, const FeatList &feats, const RowsArg
     if (a.G <= 32) return launch_tile32<KIND>(ctx, feats, a, s, masks);
     if (a.G <= 64) return launch_tile64<KIND>(ctx, feats, a, s, masks);
     if (a.G <= 128) {
-        if (KIND < 0) return launch_crosscat<128>(ctx, feats, a, s, masks);
-        const int v = ctx->opt[DIST_B200_OPT_SMALL_TILE];
-        if (v == 1) return launch_modes<128, KIND, 256>(ctx, feats, a, s);
-        if (v == 3) return launch_tile32<KIND>(ctx, feats, a, s, masks);
-        if (v != 2 && a.assign && !a.scores) {
-            // sampling only: the register tile is G rounded up to 16 groups (G = 100 pads to 112 instead of 128:
-            // every padded group is a wasted MUFU.EX2)
-            if (a.G <= 80) return launch_variant<80, KIND, true, false, 128>(ctx, feats, a, s);
-            if (a.G <= 96) return launch_variant<96, KIND, true, false, 128>(ctx, feats, a, s);
-            if (a.G <= 112) return launch_variant<112, KIND, true, false, 128>(ctx, feats, a, s);
+        // (a compile-time branch: the single-feature tiles below are not instantiated for feature lists)
+        if constexpr (KIND < 0) {
+            return launch_crosscat<128>(ctx, feats, a, s, masks);
+        } else {
+            const int v = ctx->opt[DIST_B200_OPT_SMALL_TILE];
+            if (v == 1) return launch_modes<128, KIND, 256>(ctx, feats, a, s);
+            if (v == 3) return launch_tile32<KIND>(ctx, feats, a, s, masks);
+            // (not for dd: its sampling-only launches at G <= 128 take the scaled-table kinds, launch_single_dd, and reach
+            // these tiers only with DIST_B200_OPT_SMALL_TILE set, which then selects the 128-group tile)
+            if constexpr (KIND != DIST_B200_DD) if (v != 2 && a.assign && !a.scores) {
+                // sampling only: the register tile is G rounded up to 16 groups (G = 100 pads to 112 instead of 128:
+                // every padded group is a wasted MUFU.EX2)
+                if (a.G <= 80) return launch_variant<80, KIND, true, false, 128>(ctx, feats, a, s);
+                if (a.G <= 96) return launch_variant<96, KIND, true, false, 128>(ctx, feats, a, s);
+                if (a.G <= 112) return launch_variant<112, KIND, true, false, 128>(ctx, feats, a, s);
+            }
+            return launch_modes<128, KIND, 128>(ctx, feats, a, s);
         }
-        return launch_modes<128, KIND, 128>(ctx, feats, a, s);
     }
     // measured at c2, sampling only: 32-group tiles 0.748 ms, 64-group tiles 0.774 ms; with the [N][G] scores also written
     // (HBM-store bound): 32-group tiles 1.215 ms, 64-group tiles 1.098 ms -- a store instruction then covers 256-byte runs of
