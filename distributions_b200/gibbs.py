@@ -3,17 +3,45 @@
     kind = gibbs.BlockedGibbs(ctx, features, columns, assign, models.PitmanYor(alpha, d), n_empty=1)
     kind.sweep(n_blocks=8, generator=torch.Generator(device="cuda").manual_seed(0))
 
-The rows are split into blocks (boundaries at multiples of 32 rows, so observed-mask words slice cleanly).  Per block:
+sweep() splits the rows into blocks with boundaries at multiples of 32 rows, so observed-mask words slice cleanly;
+block(r0, r1) takes any row range and shifts the mask words of an unaligned one into place.  Per block:
 remove the block's rows from their groups, mark them unassigned, count the group sizes, regroup (drop the emptied
 groups, restore `n_empty` fresh empty groups, relabel the assignments and compact every feature), evaluate the prior
 at the new G, score and sample the block's rows against it, and add them to the groups drawn.  Every block is scored
 against exactly `n_empty` empty groups, so a block can open up to `n_empty` new groups.  The only host round trip per
 block is the new G, read back by regroup_batch; everything else stays on the device, on torch's current stream.
+
+What the chain samples.  The rows of one block are drawn independently of each other, each from its conditional given
+the rows outside the block.  That is a valid Markov kernel, but for blocks of more than one row its stationary
+distribution is not the DP / Pitman-Yor posterior over partitions; blocks of one row (`block(r, r + 1)`) make a
+collapsed Gibbs sampler whose stationary distribution is the posterior (tests/test_gpu_gibbs_exact.py checks both
+against the exact distributions over every partition of tiny tables).  `blocks()` makes one block of every row when
+N <= 32: that block removes every row, regroup leaves only the `n_empty` fresh groups, and each row is drawn uniformly
+among them without looking at the data.
 """
 import numpy as np
 import torch
 
 from . import models
+
+
+def block_mask_words(words, r0, r1):
+    """the observed-mask words of rows [r0, r1) as a call over those rows reads them: bit n % 32 of word n / 32 is row
+    r0 + n.  An aligned r0 is a slice of the kind's words; otherwise each word is the kind's words shifted right by
+    r0 % 32, (w[i] >> s) | (w[i + 1] << (32 - s)), with the bits past r1 cleared (torch ops on the words' device)."""
+    s, w0, n_words = r0 % 32, r0 // 32, -(-(r1 - r0) // 32)
+    if s == 0:
+        return words[w0:(r1 + 31) // 32]
+    w = words[w0:w0 + n_words + 1].to(torch.int64) & 0xFFFFFFFF
+    if w.numel() == n_words:
+        w = torch.cat([w, w.new_zeros(1)])
+    out = ((w[:n_words] >> s) | (w[1:] << (32 - s))) & 0xFFFFFFFF
+    tail = (r1 - r0) % 32
+    if tail:
+        out[-1] &= (1 << tail) - 1
+    if words.dtype == torch.int32:
+        out = torch.where(out >= 1 << 31, out - (1 << 32), out)
+    return out.to(words.dtype)
 
 
 class BlockedGibbs:
@@ -44,7 +72,7 @@ class BlockedGibbs:
         self.prior = torch.zeros(self._cap, dtype=torch.float32, device=self.assign.device)
 
     def blocks(self, n_blocks):
-        """row ranges [r0, r1) of n_blocks blocks whose boundaries are multiples of 32"""
+        """row ranges [r0, r1) of n_blocks blocks whose boundaries are multiples of 32 (one block of every row when N <= 32)"""
         size = -(-self.N // max(1, int(n_blocks)))
         size = -(-size // 32) * 32
         return [(r0, min(self.N, r0 + size)) for r0 in range(0, self.N, size)]
@@ -53,11 +81,12 @@ class BlockedGibbs:
         cols = [c[r0:r1] for c in self.columns]
         obs = None
         if self.observed is not None:
-            obs = [None if m is None else m[r0 // 32:(r1 + 31) // 32] for m in self.observed]
+            obs = [None if m is None else block_mask_words(m, r0, r1) for m in self.observed]
         return cols, obs
 
     def block(self, r0, r1, generator):
-        """one Gibbs block over rows [r0, r1); returns K+ (the live groups the block was scored against)"""
+        """one Gibbs block over rows [r0, r1) (any 0 <= r0 < r1 <= N); returns K+ (the live groups the block was scored
+        against).  The block's rows are drawn independently of each other, given the rows outside the block."""
         # the library calls run on torch's current stream, in order with the torch ops between them
         ctx, s, n = self.ctx, torch.cuda.current_stream(self.assign.device).cuda_stream, r1 - r0
         cols, obs = self._slice(r0, r1)

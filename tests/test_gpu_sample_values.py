@@ -16,6 +16,7 @@ import pytest
 from scipy import special, stats
 
 from distributions_b200 import capi
+from gibbs_exact_ref import bb_predictive, bnb_predictive, dd_predictive, dpd_predictive, gp_predictive, nich_predictive, niw_predictive
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CPP_SRC = os.path.join(ROOT, "tests", "cpp", "test_sample_values.cc")
@@ -46,14 +47,7 @@ def _nich():
     mean = np.array([0.0, -1.0, 0.3], np.float32)
     ctv = np.array([0.0, 3.0, 2.0e6], np.float32)
     w = dict(model="nich", shared=sh, count=count, mean=mean, ctv=ctv)
-    mu, kappa, sigmasq, nu = sh.astype(np.float64)
-    dists = []
-    for n, m, c in zip(count.astype(np.float64), mean.astype(np.float64), ctv.astype(np.float64)):
-        pk, pn = kappa + n, nu + n
-        pm = (kappa * mu + m * n) / pk
-        ps = (nu * sigmasq + c + n * kappa * (mu - m) ** 2 / pk) / pn
-        dists.append(stats.t(df=pn, loc=pm, scale=np.sqrt(ps * (pk + 1) / pk)))
-    return w, dists
+    return w, [nich_predictive(sh, n, m, c) for n, m, c in zip(count.astype(np.float64), mean.astype(np.float64), ctv.astype(np.float64))]
 
 
 def _gp():
@@ -64,8 +58,7 @@ def _gp():
     return w, [_gp_dist(sh[0] + s, sh[1] + c) for c, s in zip(count.astype(np.float64), sm.astype(np.float64))]
 
 
-def _gp_dist(shape, rate):
-    return stats.nbinom(n=float(shape), p=float(rate) / (1.0 + float(rate)))
+_gp_dist = gp_predictive
 
 
 def _bnb():
@@ -77,8 +70,7 @@ def _bnb():
     return w, [_bnb_dist(r, sh[0] + r * c, sh[1] + s) for c, s in zip(count.astype(np.float64), sm.astype(np.float64))]
 
 
-def _bnb_dist(r, a, b):
-    return stats.betanbinom(n=r, a=float(a), b=float(b))
+_bnb_dist = bnb_predictive
 
 
 def _bb():
@@ -86,8 +78,8 @@ def _bb():
     heads = np.array([0, 3, 400_000], np.int32)
     tails = np.array([0, 1, 600_000], np.int32)
     w = dict(model="bb", shared=sh, heads=heads, tails=tails)
-    p = (sh[0] + heads.astype(np.float64)) / (sh[0] + sh[1] + heads.astype(np.float64) + tails.astype(np.float64))
-    return w, [np.array([1 - q, q]) for q in p]
+    a, b = sh.astype(np.float64)
+    return w, [bb_predictive(a, b, h, t) for h, t in zip(heads.astype(np.float64), tails.astype(np.float64))]
 
 
 def _dd(dim):
@@ -97,8 +89,7 @@ def _dd(dim):
     counts[1, rng.integers(0, dim, 10)] += 1
     counts[2] = rng.integers(0, 5000, dim)
     w = dict(model="dd", alphas=alphas, counts=counts)
-    wt = alphas.astype(np.float64)[None, :] + counts
-    return w, list(wt / wt.sum(1, keepdims=True))
+    return w, list(dd_predictive(alphas, counts))
 
 
 def _dpd(beta0):
@@ -113,8 +104,7 @@ def _dpd(beta0):
     counts[1, :4] = [2, 0, 5, 1]
     counts[2] = rng.integers(0, 3000, V)
     w = dict(model="dpd", alpha=alpha, beta0=beta0, keys=keys, betas=betas, counts=counts)
-    wt = np.concatenate([alpha * betas.astype(np.float64)[None, :] + counts, np.full((3, 1), alpha * np.float64(np.float32(beta0)))], 1)
-    return w, list(wt / wt.sum(1, keepdims=True))
+    return w, [dpd_predictive(alpha, betas, np.float32(beta0), c) for c in counts]
 
 
 def _niw(d):
@@ -128,18 +118,8 @@ def _niw(d):
     sum_x = np.stack([np.zeros(d), x.sum(0)]).astype(np.float32)
     sum_xxT = np.stack([np.zeros((d, d)), x.T @ x]).astype(np.float32)
     w = dict(model="niw", mu=mu, kappa=kappa, psi=psi, nu=nu, count=count, sum_x=sum_x, sum_xxT=sum_xxT)
-    dists = []
-    for g in range(2):
-        n = float(count[g])
-        sx, sxx = sum_x[g].astype(np.float64), sum_xxT[g].astype(np.float64)
-        xbar = sx / n if n else np.zeros(d)
-        diff = xbar - mu
-        C = sxx - np.outer(sx, xbar) - np.outer(xbar, sx) + n * np.outer(xbar, xbar)
-        pk, pn = kappa + n, nu + n
-        ppsi = psi.astype(np.float64) + C + kappa * n / (kappa + n) * np.outer(diff, diff)
-        dof = pn - d + 1
-        dists.append(dict(loc=(kappa * mu + n * xbar) / pk, shape=ppsi * (pk + 1) / (pk * dof), df=dof))
-    return w, dists
+    return w, [niw_predictive(mu, kappa, psi, nu, float(count[g]), sum_x[g].astype(np.float64), sum_xxT[g].astype(np.float64))
+               for g in range(2)]
 
 
 MODEL_ID = {"nich": capi.NICH, "gp": capi.GP, "bnb": capi.BNB, "bb": capi.BB, "dd": capi.DD, "dpd": capi.DPD, "niw": capi.NIW}
